@@ -2,11 +2,14 @@
 """bench.py -- headline benchmark of the bev_b200 hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the batched warp over one synthetic batch.  The default workload is
 BASELINE.json configs[1]: 256 synthetic 1080p uint8 frames, one fixed homography (SURVEY.md 8d
 H_canon), bilinear image->BEV warp to 1024x1024.  N > 1 runs one process per GPU (torchrun), each
 with its own 256 frames (weak scaling, no data-path collective); rank 0 prints ONE JSON line.
+The frames come from a seeded generator, so with --dump-outputs two builds run with the same
+arguments can be compared output for output (see dump_output).
 """
 import argparse
 import json
@@ -59,6 +62,33 @@ def measured_peak():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+DUMP_LIMIT = 64 * 10**6  # bytes written by --dump-outputs, all files together
+
+
+def dump_output(out_dir, name, t, limit=DUMP_LIMIT):
+    """Write tensor t (..., C) as out_dir/<name>.npy in float32, so that two builds run with the
+    same arguments can be compared output for output.  If the whole tensor does not fit in `limit`
+    bytes, a fixed sample of its pixels (whole rows of the last axis, positions drawn with seed 0
+    and sorted) is written as (k, C), with their flat pixel indices as <name>_index.npy (float64).
+    Returns the paths written."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    c = t.shape[-1]
+    pixels = t.reshape(-1, c)
+    path = os.path.join(out_dir, name + ".npy")
+    data = limit - 4096  # the rest holds the .npy headers
+    if t.numel() * 4 <= data:
+        np.save(path, t.float().cpu().numpy())
+        return [path]
+    k = data // (4 * c + 8)
+    idx = np.sort(np.random.default_rng(0).choice(pixels.shape[0], k, replace=False, shuffle=False))
+    sample = pixels[torch.from_numpy(idx).to(t.device)].float().cpu().numpy()
+    ipath = os.path.join(out_dir, name + "_index.npy")
+    np.save(path, sample)
+    np.save(ipath, idx.astype(np.float64))
+    return [path, ipath]
 
 
 class ClockSampler:
@@ -213,14 +243,18 @@ def ours(args, wl):
     if rank == 0:
         sampler.start()
         time.sleep(0.05)
-    ev = [torch.cuda.Event(enable_timing=True) for _ in range(args.steps + 1)]
-    barrier()
-    ev[0].record()
-    for i in range(args.steps):
-        step()
-        ev[i + 1].record()
-    barrier()
-    clocks = sampler.stop() if rank == 0 else None
+    try:  # the nvidia-smi sampler must not outlive a failed step
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(args.steps + 1)]
+        barrier()
+        ev[0].record()
+        for i in range(args.steps):
+            step()
+            ev[i + 1].record()
+        barrier()
+    finally:
+        clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_output(args.dump_outputs, "warp_output", out)
     total_ms = ev[0].elapsed_time(ev[-1])
     per_launch_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps)]
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
@@ -610,7 +644,14 @@ def main():
     ap.add_argument("--no-projection", action="store_true", help="skip the rbox projection leg")
     ap.add_argument("--no-other-configs", action="store_true",
                     help="skip the kernel-only numbers of the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's warp output (rank 0) as "
+                         "DIR/warp_output.npy in float32, a seeded sample if it exceeds 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
 
     if args.impl == "reference":
         reference_arm(args, args.workload)
