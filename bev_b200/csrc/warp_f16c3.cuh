@@ -11,13 +11,6 @@
 // for frames that hold Inf / NaN next to the image border).
 #pragma once
 #include "bevk_common.cuh"
-
-#ifndef BEVK_F16_THREADS
-#define BEVK_F16_THREADS 128
-#endif
-#ifndef BEVK_F16_CTAS
-#define BEVK_F16_CTAS 4
-#endif
 #include "warp_u8c3.cuh"  // prmt, st_stream
 
 struct PixF16 {
@@ -30,8 +23,8 @@ struct PxF16C3 {
     static constexpr int kBpp = 6;
     static constexpr int kSegBytes = 192;
     static constexpr int kDtype = BEVK_F16;
-    static constexpr int kLinearThreads = BEVK_F16_THREADS, kNearestThreads = 256;  // CTA size of the staged kernel (warp_fast.cu)
-    static constexpr int kLinearCtas = BEVK_F16_CTAS;   // CTAs per SM of the bilinear kernel (bounds its registers)
+    static constexpr int kLinearThreads = 128, kNearestThreads = 256;  // CTA size of the staged kernel (warp_fast.cu)
+    static constexpr int kLinearCtas = 4;   // CTAs per SM of the bilinear kernel (bounds its registers)
     static constexpr int kWinWords = 8;     // window words the kernel keeps per pixel
     static constexpr bool kPairs = false;
     using Reg = PixF16;

@@ -49,7 +49,6 @@
 
 #include <cuda.h>  // CUtensorMap + enums only; the encoder is fetched through the runtime
 #include <mutex>
-#include <stdlib.h>
 #include <string.h>
 
 namespace {
@@ -83,11 +82,6 @@ constexpr int kMaxBoxes = 3;
 constexpr int kMaxStageFrames = 8;              // frames that share one ring stage / mbarrier phase
 constexpr int kBarBytes = 256;                  // 28 mbarriers: ring depths 2, 4 and 8
 constexpr int kPrefetchAhead = 2;               // depth-2 rings: L2 prefetch runs this many stages ahead
-#ifdef BEVK_EXPERIMENTS
-constexpr bool kExperiments = true;   // build with -DBEVK_EXPERIMENTS: the BEVK_DBG ablation switches exist
-#else
-constexpr bool kExperiments = false;
-#endif
 constexpr int kTailSlack = 64;                  // window words may run a few bytes past a stage
 
 __host__ __device__ constexpr int map_width(int wi)
@@ -145,13 +139,6 @@ struct WarpScratch {
     int *hdr;         // [groups * tiles][kHdrInts]
     uint32_t *rec;    // [groups * tiles][kRecWords][kThreads]
     uint32_t recip_per_chunk, recip_tiles, recip_tiles_y;  // ceil(2^32 / d) for the item decode
-    int no_pairs;     // tuning aid (BEVK_NO_PAIRS): every warp takes the per-pixel path
-    int dbg;          // -DBEVK_EXPERIMENTS builds only (BEVK_DBG): 1 = no stores, 2 = no TMA traffic / waits
-    int slack;        // ring stages NOT in flight ahead of the consumers (0: half the ring)
-    int pf;           // L2 prefetch distance in stages beyond the fills (-1: depth-2 rings only, 2 stages)
-    int pf1;          // the same for depth-2 rings when pf < 0
-    int max_fps;      // frames per ring stage, at most
-    unsigned long long *prof;  // -DBEVK_EXPERIMENTS builds only (BEVK_PROF): cycle counters of thread 0
 };
 
 // ---- PTX wrappers -------------------------------------------------------------------------------
@@ -222,6 +209,7 @@ __device__ __forceinline__ void st_release(int *p, int v)
 }
 // Stops the compiler from re-deriving a loop-invariant value inside the frame loop.
 __device__ __forceinline__ void keep(uint32_t &v) { asm volatile("" : "+r"(v)); }
+__device__ __forceinline__ void keep(int &v) { asm volatile("" : "+r"(v)); }
 
 // What the producing warp needs to fetch the frames' bounding boxes.
 struct BoxPlan {
@@ -260,9 +248,6 @@ struct LoopCtx {
     int n_frames;
     int slog;                      // ring depth 2^slog stages
     int ahead;                     // stages in flight ahead of the one being consumed
-    int pf;                        // L2 prefetch distance in stages beyond that (0: none)
-    int dbg;
-    unsigned long long *prof;      // -DBEVK_EXPERIMENTS builds (BEVK_PROF): cycle counters of thread 0
     const WarpFastMaps *maps;
     const BoxPlan *plan;           // in shared memory
 };
@@ -313,8 +298,8 @@ __device__ __forceinline__ void feed(const LoopCtx &c, int done, uint32_t use, i
     const int turn = ((int)use - warp) & (WARPS - 1);
     const int i_load = done + (c.ahead - 1) * c.fps;  // first frame of the stage `ahead` stages on
     if (turn == 0 && i_load < c.n_frames) produce<true>(c.plan, c.maps, i_load, use + c.ahead, lane);
-    if (c.pf && turn == WARPS / 2 && i_load + c.pf * c.fps < c.n_frames)
-        produce<false>(c.plan, c.maps, i_load + c.pf * c.fps, 0, lane);
+    if (c.slog == 1 && turn == WARPS / 2 && i_load + kPrefetchAhead * c.fps < c.n_frames)
+        produce<false>(c.plan, c.maps, i_load + kPrefetchAhead * c.fps, 0, lane);
 }
 
 // The frame loop of a staged item: ring of 2^slog stages of c.fps frames each, c.ahead of them in
@@ -331,14 +316,11 @@ __device__ __forceinline__ uint32_t stage_loop(const LoopCtx &c, uint32_t use, u
 {
     const uint32_t smask = (1u << c.slog) - 1u;
     const int lane = tid & 31, warp = tid >> 5;
-    const bool live = !(kExperiments && (c.dbg & 2));
     if (warp == 0) {
-        if (live) {
-            for (int s = 0; s < c.ahead && s * c.fps < c.n_frames; ++s)
-                produce<true>(c.plan, c.maps, s * c.fps, use + s, lane);
-            for (int s = c.ahead; s < c.ahead + c.pf && s * c.fps < c.n_frames; ++s)
-                produce<false>(c.plan, c.maps, s * c.fps, 0, lane);
-        }
+        for (int s = 0; s < c.ahead && s * c.fps < c.n_frames; ++s)
+            produce<true>(c.plan, c.maps, s * c.fps, use + s, lane);
+        for (int s = c.ahead; c.slog == 1 && s < c.ahead + kPrefetchAhead && s * c.fps < c.n_frames; ++s)
+            produce<false>(c.plan, c.maps, s * c.fps, 0, lane);
         if (tid == 0) started();
     }
     int done = 0;
@@ -346,21 +328,15 @@ __device__ __forceinline__ uint32_t stage_loop(const LoopCtx &c, uint32_t use, u
     while (done < c.n_frames) {
         const uint32_t slot = use & smask;
         const uint32_t fb = c.full0 + 8 * slot;
-        long long tw0 = 0;
-        if (kExperiments && c.prof && tid == 0) tw0 = clock64();
-        if (live) mbar_wait(fb, (use >> c.slog) & 1u);
-        if (kExperiments && c.prof && tid == 0)
-            atomicAdd(c.prof + (done == 0 ? 1 : 2), (unsigned long long)(clock64() - tw0));
+        mbar_wait(fb, (use >> c.slog) & 1u);
         uint32_t sa = c.ring + slot * c.stride;  // first frame of the stage
         int nf = min(c.fps, c.n_frames - done);
         done += nf;
 #pragma unroll 1
         for (; nf > 0; --nf, sa += c.frame_bytes, d += d_step) body(sa, d);
-        if (live) {
-            __syncwarp();
-            if (lane == 0) mbar_arrive(fb + (8u << c.slog));
-            feed<WARPS>(c, done, use, lane, warp);
-        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(fb + (8u << c.slog));
+        feed<WARPS>(c, done, use, lane, warp);
         ++use;
     }
     return use;
@@ -532,7 +508,6 @@ warp_fast_kernel(const __grid_constant__ BevkWarpParams p,
         o.stride = p.g[gi].stride;
         o.chunk = chunk;
         // one item ahead of its use: by then the first chunk's CTA has nearly always published
-        // one item ahead of its use: by then the first chunk's CTA has nearly always published
         o.ready = (sc.ready != nullptr && chunk > 0)
                       ? ld_acquire(sc.ready + (gi * n_tiles + o.tile_x * tiles_y + o.tile_y))
                       : 1;
@@ -566,8 +541,6 @@ warp_fast_kernel(const __grid_constant__ BevkWarpParams p,
         const int y0 = tile_y * tile_h(SEGS, kWarps) + warp_px_y<SEGS, kPairMap>(warp);
         const int tile_id = gi * n_tiles + tile_x * tiles_y + tile_y;
         par ^= 1;
-        long long t_item = 0;
-        if (kExperiments && sc.prof && tid == 0) t_item = clock64();
 
         // ---- 1. set-up: window position and tap weights of the thread's four pixels, the tile's
         //         source bounding box -- computed by the tile's first chunk, re-read by the others
@@ -684,11 +657,9 @@ warp_fast_kernel(const __grid_constant__ BevkWarpParams p,
         // staged for nothing (and fetched from HBM for nothing) -- gather those tiles directly
         if (!LINEAR && frame_bytes > 3u * 1024u * (uint32_t)kBpp) staged = false;
         // frames per stage: as many as still leave a ring of 4 stages
-        const int fps = (4 * 8 * frame_bytes <= (uint32_t)ring_bytes && sc.max_fps >= 8)
-                            ? 8
-                            : ((4 * 4 * frame_bytes <= (uint32_t)ring_bytes && sc.max_fps >= 4)
-                                   ? 4
-                                   : (8 * frame_bytes <= (uint32_t)ring_bytes && sc.max_fps >= 2 ? 2 : 1));
+        const int fps = 4 * kMaxStageFrames * frame_bytes <= (uint32_t)ring_bytes ? kMaxStageFrames
+                        : 4 * 4 * frame_bytes <= (uint32_t)ring_bytes ? 4
+                        : 8 * frame_bytes <= (uint32_t)ring_bytes ? 2 : 1;
         const int stage_stride = fps * (int)frame_bytes;
         const int slog = (8 * stage_stride <= ring_bytes) ? 3 : (4 * stage_stride <= ring_bytes ? 2 : 1);
         const uint32_t full0 = bar0 + 16 * (1 << slog) - 32;  // the set's empty[] follow its full[]
@@ -748,7 +719,6 @@ warp_fast_kernel(const __grid_constant__ BevkWarpParams p,
             const int row = px_row<SEGS, kPairMap>(k), seg = px_seg<SEGS, kPairMap>(k);
             return (row & 1 ? dd1 : dd) + (row >> 1) * 2 * (size_t)row_bytes + PX::kSegBytes * seg;
         };
-        if (kExperiments && (sc.dbg & 1)) seg_ok[0] = seg_ok[1] = seg_ok[2] = seg_ok[3] = false;
         uint32_t d_step = (uint32_t)g_stride * (uint32_t)dst_frame_bytes;  // < 2^32 (host check)
         keep(d_step);
         uint8_t *d = dst + (long long)(g_first + f0 * g_stride) * dst_frame_bytes +
@@ -771,25 +741,23 @@ warp_fast_kernel(const __grid_constant__ BevkWarpParams p,
             c.fps = fps;
             c.n_frames = n_frames;
             c.slog = slog;
-            // stages in flight ahead of the one being consumed.  Two-slot rings refill the slot that was
-            // just released (the producing warp waits for the other warps' release), so that the copy of
-            // stage n + 2 runs under stage n + 1 -- with one stage ahead the copy only started when the
-            // frame before it was done (cfg 5 0.424 -> 0.393 ms, cfg 2 0.391 -> 0.382 ms).
-            c.ahead = slog == 1 ? 2 : (sc.slack > 0 ? max(1, (1 << slog) - sc.slack) : (sc.slack < 0 ? (1 << slog) : (1 << (slog - 1))));
-            c.pf = sc.pf >= 0 ? sc.pf : (slog == 1 ? sc.pf1 : 0);
-            c.dbg = sc.dbg;
-            c.prof = sc.prof;
+            // stages in flight ahead of the one being consumed: all but one.  With a whole warp issuing
+            // a stage in one pass the producer's detour is short, and every kernel does best this way
+            // (against half the ring: float16 cfg 5 0.792 -> 0.749 ms, uint8 x 4 0.441 -> 0.430 ms,
+            // nearest 0.316 -> 0.310 ms); the whole ring in flight is worse again for the 4-warp kernels.
+            // Two-slot rings refill the slot that was just released (the producing warp waits for the
+            // other warps' release), so that the copy of stage n + 2 runs under stage n + 1 -- with one
+            // stage ahead the copy only started when the frame before it was done (cfg 5 0.424 -> 0.393
+            // ms, cfg 2 0.391 -> 0.382 ms).  Only those rings prefetch into L2, kPrefetchAhead stages
+            // further on (feed).
+            c.ahead = slog == 1 ? 2 : (1 << slog) - 1;
             c.maps = &maps;
             c.plan = &s_plan;
             keep(c.ring);
             keep(c.full0);
+            keep(c.slog);  // else the stage loop re-derives the ring depth from ring_bytes in every stage
             // every thread tracks the counter in a register; thread 0 publishes it for the next item
             uint32_t use = s_use[slog - 1];
-            long long t_loop = 0;
-            if (kExperiments && sc.prof && tid == 0) {
-                t_loop = clock64();
-                atomicAdd(sc.prof + 0, (unsigned long long)(t_loop - t_item));  // set-up
-            }
 
             // Pair path (uint8 x 3 bilinear): can every vertical pair of this warp share its
             // window loads?  Needs windows at most one column apart and the same row step --
@@ -819,7 +787,6 @@ warp_fast_kernel(const __grid_constant__ BevkWarpParams p,
                         ok2 = ok2 && by1 - by0 >= 2;
                     }
                 }
-                if (sc.no_pairs) ok0 = ok1 = ok2 = false;
                 var = __all_sync(0xffffffffu, ok0) ? 0
                       : (__all_sync(0xffffffffu, ok1) ? 1 : (__all_sync(0xffffffffu, ok2) ? 2 : 3));
             }
@@ -926,15 +893,8 @@ warp_fast_kernel(const __grid_constant__ BevkWarpParams p,
                     for (int k = 0; k < 4; ++k) PX::store(seg_ptr(dd, dd + row_bytes, k), P[k], seg_ok[k], st, lane);
                 }, next_item_decode);
             }
-            long long t_end = 0;
-            if (kExperiments && sc.prof && tid == 0) t_end = clock64();
             __syncthreads();  // every warp has read s_use and left the ring
             if (tid == 0) s_use[slog - 1] = use;
-            if (kExperiments && sc.prof && tid == 0) {
-                atomicAdd(sc.prof + 3, (unsigned long long)(t_end - t_loop));         // frame loops incl. waits
-                atomicAdd(sc.prof + 4, (unsigned long long)(clock64() - t_end));      // end-of-item barrier (warp skew)
-                atomicAdd(sc.prof + 5, 1ULL);
-            }
             continue;
         } else if (p.hard) {
             // split launch: leave the tile to the direct-gather kernel that follows on the stream
@@ -978,15 +938,6 @@ warp_fast_kernel(const __grid_constant__ BevkWarpParams p,
         }
         __syncthreads();  // the next item's descriptor (s_item) is complete and visible
     }
-}
-
-// Tuning switches (BEVK_* environment variables) exist only in -DBEVK_EXPERIMENTS builds; the
-// product build reads no environment on the launch path.
-inline const char *tune_env(const char *name) { return kExperiments ? getenv(name) : nullptr; }
-inline int tune_int(const char *name, int dflt)
-{
-    const char *v = tune_env(name);
-    return v ? atoi(v) : dflt;
 }
 
 // ---- host side: tensor-map menu ---------------------------------------------------------------
@@ -1068,11 +1019,9 @@ struct KernelConfig {
     int ctas_per_sm = 0;
     int ring_bytes = 0;
 };
-// CTAs per SM the register allocation is bounded for: bilinear needs 80 registers per thread (a
-// 64-register build spills in the frame loop and is slower), nearest fits 64 without spilling and
-// gains 5 % from the fourth CTA.
-// CTAs per SM the register allocation of a kernel is bounded for (PX::kLinearCtas for the bilinear
-// kernels; nearest kernels fit 64 registers: 4 CTAs of 8 warps).
+// CTAs per SM the register allocation of a kernel is bounded for: PX::kLinearCtas for the bilinear
+// kernels (a 64-register build spills in the frame loop and is slower); nearest kernels fit 64
+// registers without spilling (4 CTAs of 8 warps) and gain 5 % from the fourth CTA.
 template <typename PX, bool LINEAR> constexpr int min_ctas()
 {
     return LINEAR ? PX::kLinearCtas : 4 * (256 / cta_threads<PX, LINEAR>());
@@ -1286,9 +1235,7 @@ int pick_tile_shape(const BevkWarpParams &p, int linear, int bpp, int warps, int
     int best = 0;
     double best_frac = 2.0;
     static const int shapes[3] = {4, 2, 1};
-    const char *env = tune_env("BEVK_FAST_SEGS");  // tuning aid: force a tile shape
     for (int si = 0; si < 3; ++si) {
-        if (env && atoi(env) != shapes[si]) continue;
         const double f = unstaged_fraction(p, linear, bpp, shapes[si], warps, ring_bytes);
         if (f < best_frac - 1e-9) {
             best_frac = f;
@@ -1400,17 +1347,7 @@ int bevk_launch_warp_fast(const BevkWarpParams &p_in, int channels, int dtype, i
     ChunkPlan plan;
     memset(&plan, 0, sizeof(plan));
     const long long tile_groups = n_tiles * p.n_groups;
-    if (const char *env = tune_env("BEVK_CHUNKS")) {  // tuning aid: chunk lengths in 1/256ths, e.g. "96,64,48,32,16"
-        int k = 0, acc = 0;
-        for (const char *q = env; *q && k < kMaxChunks;) {
-            acc += atoi(q);
-            plan.cum[++k] = (uint32_t)(acc * 256);
-            while (*q && *q != ',') ++q;
-            if (*q == ',') ++q;
-        }
-        plan.cum[k] = 65536;
-        plan.n_chunks = k;
-    } else if (max_count >= 128 && tile_groups * 5 >= 2LL * ctas) {
+    if (max_count >= 128 && tile_groups * 5 >= 2LL * ctas) {
         static const uint32_t cum[8] = {0, 20480, 36864, 49152, 57344, 61952, 64512, 65536};
         plan.n_chunks = 7;
         memcpy(plan.cum, cum, sizeof(cum));
@@ -1430,15 +1367,13 @@ int bevk_launch_warp_fast(const BevkWarpParams &p_in, int channels, int dtype, i
     // Per-launch scratch, allocated and freed in stream order (launches on other streams or from
     // other threads get their own): [item counter | split flags | set-up ready flags] zeroed, then
     // the tiles' set-up headers and records.
-    split = split && !tune_env("BEVK_NO_SPLIT");
     // Sharing a tile's set-up between its frame chunks pays where the set-up is expensive relative to
     // the per-frame work and the issue slots are the scarce resource: uint8 x 3 bilinear (cfg 2: 0.444 ->
     // 0.428 ms) and uint8 x 1 bilinear (0.277 -> 0.256 ms).  The other kernels have issue slots to spare
     // and gain nothing (float16, uint8 x 4, float32) or lose a little to the extra round trips
     // (nearest 0.326 -> 0.331 ms), so they recompute.
     const bool share_setup = (fmt == 0 || fmt == 2) && linear && plan.n_chunks > 1 &&
-                             tile_groups * kRecWords * threads * 4 <= (512LL << 20) &&
-                             !tune_env("BEVK_NO_SETUP_CACHE");
+                             tile_groups * kRecWords * threads * 4 <= (512LL << 20);
     const size_t off_hard = 256;
     const size_t off_ready = off_hard + (((size_t)(split ? tile_groups : 0) + 255) & ~(size_t)255);
     const size_t off_hdr = off_ready + (((size_t)(share_setup ? tile_groups * 4 : 0) + 255) & ~(size_t)255);
@@ -1456,17 +1391,6 @@ int bevk_launch_warp_fast(const BevkWarpParams &p_in, int channels, int dtype, i
     sc.recip_per_chunk = recip(tile_groups);
     sc.recip_tiles = recip(n_tiles);
     sc.recip_tiles_y = recip(tiles_y);
-    sc.no_pairs = tune_env("BEVK_NO_PAIRS") ? 1 : 0;
-    sc.dbg = tune_int("BEVK_DBG", 0);
-    // stages of the ring NOT in flight ahead of the consumers: one (0 = half the ring, < 0 = none).
-    // With a whole warp issuing a stage in one pass the producer's detour is short, and every kernel
-    // does best with all but one stage in flight (float16 cfg 5 0.792 -> 0.749 ms, uint8 x 4 0.441 ->
-    // 0.430 ms, nearest 0.316 -> 0.310 ms); none as slack is worse again for the 4-warp kernels.
-    sc.slack = tune_int("BEVK_SLACK", 1);
-    sc.pf = tune_int("BEVK_PF", -1);
-    sc.pf1 = tune_int("BEVK_PF1", kPrefetchAhead);
-    sc.max_fps = tune_int("BEVK_MAXFPS", kMaxStageFrames);
-    sc.prof = tune_env("BEVK_PROF") ? (unsigned long long *)(scratch + 64) : nullptr;  // (zeroed with the item counter)
     if (split) {
         // one byte per (group, tile): the staged kernel marks the tiles it leaves to the second launch
         p.hard = scratch + off_hard;
@@ -1490,13 +1414,6 @@ int bevk_launch_warp_fast(const BevkWarpParams &p_in, int channels, int dtype, i
             rc2 = bevk_plan_generic_chunks(p, channels);
             if (!rc2) rc2 = bevk_launch_warp_generic(p, channels, dtype, linear, stream);
         }
-    }
-    if (kExperiments && sc.prof) {  // BEVK_PROF: where thread 0 of every CTA spent its cycles
-        unsigned long long h[8];
-        cudaStreamSynchronize(stream);
-        cudaMemcpy(h, sc.prof, sizeof(h), cudaMemcpyDeviceToHost);
-        fprintf(stderr, "BEVK_PROF thread-0 cycles: set-up %llu first-wait %llu later-waits %llu loops %llu end-barrier %llu items %llu (grid %d)\n",
-                h[0], h[1], h[2], h[3], h[4], h[5], grid);
     }
     const cudaError_t ef = cudaFreeAsync(scratch, stream);  // stream-ordered: after the kernels above
     if (e != cudaSuccess) {

@@ -5,10 +5,6 @@
 #pragma once
 #include "bevk_common.cuh"
 
-#ifndef BEVK_U8C3_LINEAR_THREADS
-#define BEVK_U8C3_LINEAR_THREADS 128
-#endif
-
 __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
 {
     return __byte_perm(a, b, sel);
@@ -91,7 +87,7 @@ struct PxU8C3 {
     static constexpr int kBpp = 3;         // bytes per pixel
     static constexpr int kSegBytes = 96;   // bytes of a 32-pixel row segment
     static constexpr int kDtype = BEVK_U8;
-    static constexpr int kLinearThreads = BEVK_U8C3_LINEAR_THREADS, kNearestThreads = 256;  // CTA size of the staged kernel (warp_fast.cu)
+    static constexpr int kLinearThreads = 128, kNearestThreads = 256;  // CTA size of the staged kernel (warp_fast.cu)
     static constexpr int kLinearCtas = 6;   // CTAs per SM of the bilinear kernel (bounds its registers)
     static constexpr int kWinWords = 8;     // window words the kernel keeps per pixel
     static constexpr bool kPairs = true;   // the staged kernel's shared-window pair path exists for this format

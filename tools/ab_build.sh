@@ -1,6 +1,7 @@
 #!/bin/bash
-# Development aid: build a variant of the library (extra -D switches for warp_fast.cu) into
-# tools/_ab/<name>.so for same-box A/B runs (tools/kbench.py --lib).   tools/ab_build.sh name -DX=1 ...
+# Development aid: build the working tree's warp_fast.cu, linked with the other objects of the last
+# make, as the named library variant tools/_ab/<name>.so for same-box A/B runs (tools/ab_run.sh,
+# tools/kbench.py --lib).   tools/ab_build.sh name [nvcc flags]
 set -e
 cd "$(dirname "$0")/../bev_b200/csrc"
 name=$1; shift
