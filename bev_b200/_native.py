@@ -41,6 +41,9 @@ SIGNATURES = {
     "bevk_warp_host_rows": (_c_int, [_c_int, _c_int, _c_int, _c_int, _dp, _c_int, _c_int, _ip]),
     "bevk_warp_set_path": (_c_int, [_c_int]),
     "bevk_warp_touched_pixels": (_c_i64, [_c_int, _c_int, _c_int, _c_int, _dp, _c_int, _ip]),
+    "bevk_nv12_to_bgr": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _vp]),
+    "bevk_warp_perspective_nv12": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int,
+                                            _dp, _c_int, _i32p, _c_int, _c_int, _dp, _vp]),
     "bevk_resize": (_c_int, [_vp, _vp] + [_c_int] * 8 + [_vp]),
     "bevk_composite_u8c3": (_c_int, [_vp, _vp, _vp, _vp, _c_i64, _c_int, _vp]),
     "bevk_composite_bev_u8c3": (_c_int, [_vp, _vp, _vp, _vp] + [_c_int] * 8 + [_dp, _dp, _c_int, _vp]),
@@ -270,6 +273,79 @@ def warp_perspective_host(src, M, dsize, dst=None, flags=1, borderMode=0, border
         int(borderMode), _dptr(b))
     _check(rc, "bevk_warp_perspective_host")
     return dst if dst is not None else undo(out4)
+
+
+def _nv12_frames(src):
+    """(frames view (N, H*3/2, W), N, H, W, pitch, frame stride) of an NV12 tensor (H*3/2, W) or
+    (N, H*3/2, W).  Pitch and frame stride come from the tensor's strides, so a decoder surface
+    with padded rows is used as it is."""
+    import torch
+    if not isinstance(src, torch.Tensor):
+        raise TypeError("src must be a torch.Tensor, got %s" % type(src).__name__)
+    if not src.is_cuda:
+        raise ValueError("src is on %s: bev_b200 runs on CUDA (sm_100a) only, there is no CPU fallback"
+                         % (src.device,))
+    if src.dtype != torch.uint8:
+        raise ValueError("NV12 frames are uint8, got %s" % (src.dtype,))
+    if src.dim() not in (2, 3):
+        raise ValueError("NV12 frames must be (H*3/2, W) or (N, H*3/2, W); got shape %s" % (tuple(src.shape),))
+    s3 = src[None] if src.dim() == 2 else src
+    n, rows, w = s3.shape
+    if rows == 0 or rows % 3 or w % 2:
+        raise ValueError("NV12 frames need H*3/2 rows for an even H and an even width W; got %d rows x %d"
+                         % (rows, w))
+    if s3.stride(2) != 1:
+        raise ValueError("NV12 rows must be contiguous (inner stride 1), got stride %d" % s3.stride(2))
+    pitch = s3.stride(1)
+    if pitch < w:
+        raise ValueError("NV12 row pitch %d is smaller than the width %d" % (pitch, w))
+    fstride = s3.stride(0) if n > 1 else pitch * rows
+    return s3, n, rows // 3 * 2, w, pitch, fstride
+
+
+def nv12_to_bgr(src, dst=None):
+    """cv2.cvtColor(f, COLOR_YUV2BGR_NV12) on CUDA uint8 NV12 frames (H*3/2, W) or (N, H*3/2, W)
+    -> (H, W, 3) or (N, H, W, 3) BGR."""
+    import torch
+    s3, n, h, w, pitch, fstride = _nv12_frames(src)
+    want = (n, h, w, 3) if src.dim() == 3 else (h, w, 3)
+    if dst is None:
+        dst = torch.empty(want, dtype=torch.uint8, device=src.device)
+    else:
+        _require_cuda(dst, "dst")
+        if tuple(dst.shape) != want or dst.dtype != torch.uint8 or not dst.is_contiguous() \
+                or dst.device != src.device:
+            raise ValueError("dst must be a contiguous uint8 tensor of shape %s on %s" % (want, src.device))
+    with torch.cuda.device(src.device):
+        rc = lib().bevk_nv12_to_bgr(_vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride,
+                                    _stream_ptr(src))
+    _check(rc, "bevk_nv12_to_bgr")
+    return dst
+
+
+def warp_perspective_nv12(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue=0, mat_index=None):
+    """warp_perspective of nv12_to_bgr(src) in one pass: (H*3/2, W) -> (h, w, 3), (N, H*3/2, W) ->
+    (N, h, w, 3) BGR uint8.  M / mat_index as for warp_perspective."""
+    import torch
+    s3, n, h, w, pitch, fstride = _nv12_frames(src)
+    dw, dh = int(dsize[0]), int(dsize[1])
+    Ms, idx = _prep_mats(M, n, mat_index)
+    want = (n, dh, dw, 3) if src.dim() == 3 else (dh, dw, 3)
+    if dst is None:
+        dst = torch.empty(want, dtype=torch.uint8, device=src.device)
+    else:
+        _require_cuda(dst, "dst")
+        if tuple(dst.shape) != want or dst.dtype != torch.uint8 or not dst.is_contiguous() \
+                or dst.device != src.device:
+            raise ValueError("dst must be a contiguous uint8 tensor of shape %s on %s" % (want, src.device))
+    b = _border(borderValue)
+    with torch.cuda.device(src.device):
+        rc = lib().bevk_warp_perspective_nv12(
+            _vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride, dh, dw, _dptr(Ms), Ms.shape[0],
+            idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags), int(borderMode), _dptr(b),
+            _stream_ptr(src))
+    _check(rc, "bevk_warp_perspective_nv12")
+    return dst
 
 
 def warp_touched_pixels(ssize, dsize, M, flags=1):

@@ -138,6 +138,14 @@ struct BevkWarpParams {
     BevkWarpGroup g[BEVK_MAX_GROUPS];
 };
 
+// The warp of NV12 frames (nv12.cu): w.src is frame 0's first luma byte, w.src_h / w.src_w the luma
+// size; w.src_frame_elems is unused, the two strides below replace it.
+struct BevkNv12Params {
+    BevkWarpParams w;
+    int pitch;               // bytes from one luma or chroma row to the next
+    long long frame_stride;  // bytes from one frame to the next
+};
+
 // kernels-side entry points implemented in the .cu files
 int bevk_launch_warp_generic(const BevkWarpParams &p, int channels, int dtype, int linear,
                              cudaStream_t stream);
@@ -147,3 +155,7 @@ int bevk_plan_generic_chunks(BevkWarpParams &p, int channels);
 // `force`, is too small a batch to amortise its per-tile set-up), <0 on error
 int bevk_launch_warp_fast(const BevkWarpParams &p, int channels, int dtype, int linear, int force,
                           cudaStream_t stream);
+// NV12 -> BGR warp over the chunks bevk_plan_generic_chunks planned for P.w
+int bevk_launch_warp_nv12(const BevkNv12Params &P, int linear, cudaStream_t stream);
+int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int w, int pitch,
+                            long long frame_stride, cudaStream_t stream);

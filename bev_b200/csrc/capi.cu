@@ -384,6 +384,83 @@ int bevk_warp_perspective_path(const void *src, void *dst, int n_frames, int src
     return run_warp_device(src, dst, a, groups, path, (cudaStream_t)stream);
 }
 
+}  // extern "C"
+
+namespace {
+// The NV12 frame rules of both NV12 entry points: even sizes, rows at least a luma row apart.
+int check_nv12_layout(const char *what, int n_frames, int h, int w, int pitch, int64_t frame_stride)
+{
+    if (n_frames < 0) BEVK_FAIL(BEVK_E_ARG, "%s: n_frames must be >= 0", what);
+    if (h <= 0 || w <= 0 || (h % 2) != 0 || (w % 2) != 0)
+        BEVK_FAIL(BEVK_E_ARG, "%s: NV12 frames need an even, positive width and height (got %dx%d)", what, w, h);
+    if (pitch < w) BEVK_FAIL(BEVK_E_ARG, "%s: pitch %d is smaller than the width %d", what, pitch, w);
+    if (frame_stride < 0) BEVK_FAIL(BEVK_E_ARG, "%s: negative frame stride", what);
+    return BEVK_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int bevk_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int w, int pitch,
+                     int64_t frame_stride, void *stream)
+{
+    int rc = check_nv12_layout("nv12_to_bgr", n_frames, h, w, pitch, frame_stride);
+    if (rc) return rc;
+    if (n_frames > 0 && (!src || !dst)) BEVK_FAIL(BEVK_E_ARG, "nv12_to_bgr: null src / dst");
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    return bevk_launch_nv12_to_bgr(src, dst, n_frames, h, w, pitch, frame_stride, (cudaStream_t)stream);
+}
+
+int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w,
+                               int pitch, int64_t frame_stride, int dst_h, int dst_w,
+                               const double *M, int n_mats, const int32_t *mat_index, int flags,
+                               int border_mode, const double *border_value, void *stream)
+{
+    int rc = check_nv12_layout("warp_nv12", n_frames, src_h, src_w, pitch, frame_stride);
+    if (rc) return rc;
+    // the kernel addresses a frame with 32-bit byte offsets
+    if ((int64_t)pitch * (src_h / 2 * 3) > 0xffffffffLL)
+        BEVK_FAIL(BEVK_E_ARG, "warp_nv12: a frame of pitch %d and %d rows spans 4 GB or more", pitch, src_h / 2 * 3);
+    WarpArgs a;
+    rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index,
+                         flags, border_mode, border_value, a);
+    if (rc) return rc;
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    std::vector<double> maps;
+    effective_maps(M, n_mats, flags, maps);
+    std::vector<BevkWarpGroup> groups;
+    build_groups(n_frames, n_mats, mat_index, maps, groups);
+
+    BevkNv12Params P;
+    memset(&P, 0, sizeof(P));
+    BevkWarpParams &p = P.w;
+    p.src = src;
+    p.dst = dst;
+    p.src_h = src_h;
+    p.src_w = src_w;
+    p.dst_h = dst_h;
+    p.dst_w = dst_w;
+    p.dst_frame_elems = (long long)dst_h * dst_w * 3;
+    p.bw0 = bevk_block_width(dst_w, dst_h);
+    for (int c = 0; c < 4; ++c) p.border[c] = a.border[c];
+    P.pitch = pitch;
+    P.frame_stride = frame_stride;
+    for (size_t g0 = 0; g0 < groups.size(); g0 += BEVK_MAX_GROUPS) {
+        const int ng = (int)std::min<size_t>(BEVK_MAX_GROUPS, groups.size() - g0);
+        p.n_groups = ng;
+        for (int i = 0; i < ng; ++i) p.g[i] = groups[g0 + i];
+        rc = bevk_plan_generic_chunks(p, 3);
+        if (rc) return rc;
+        rc = bevk_launch_warp_nv12(P, a.linear, (cudaStream_t)stream);
+        if (rc) return rc;
+    }
+    return BEVK_OK;
+}
+
 int bevk_warp_host_rows(int src_h, int src_w, int dst_h, int dst_w, const double *M, int n_mats,
                         int flags, int rows[2])
 {

@@ -7,6 +7,9 @@
 //   torch.ops.bev_cuda.rbox_corners_project(Tensor xywhr, Tensor? H, int mode) -> Tensor
 //   torch.ops.bev_cuda.corners_to_rbox(Tensor xy8, Tensor? H, int mode) -> Tensor
 //   torch.ops.bev_cuda.rbox_similarity(Tensor rbox, Tensor H, int src_mode) -> Tensor
+//   torch.ops.bev_cuda.nv12_to_bgr(Tensor src) -> Tensor
+//   torch.ops.bev_cuda.warp_perspective_nv12(Tensor src, Tensor M, int w, int h, int flags, int border_mode,
+//                                            float border_val, Tensor? mat_index) -> Tensor
 //
 // Every implementation only checks tensors, allocates the result with torch's caching allocator,
 // takes the current CUDA stream and calls the extern "C" entry point of include/bev_b200.h with raw
@@ -16,7 +19,8 @@
 //
 // Reference interfaces replaced: cv2.warpPerspective at vis_homo.py:85-91, rbox.pts_world_bev
 // (bev/rbox.py:136-151), rbox_torch.xywhr2xyxy (bev/rbox_torch.py:52-99) + the projection of
-// rbox_vis.py:38-55, rbox.xy82xywhr (bev/rbox.py:50-63), rbox_torch.rbox_world_bev (:123-168).
+// rbox_vis.py:38-55, rbox.xy82xywhr (bev/rbox.py:50-63), rbox_torch.rbox_world_bev (:123-168); the NV12
+// operators serve the frame loop of vis_homo.py:85-91 with frames from a GPU video decoder.
 #include <ATen/ATen.h>
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
@@ -86,6 +90,66 @@ at::Tensor warp_perspective(const at::Tensor &src, const at::Tensor &M, int64_t 
     return out;
 }
 
+// NV12 frames (H*3/2, W) or (N, H*3/2, W): row pitch and frame stride from the tensor's strides
+struct Nv12View {
+    at::Tensor s3;
+    int64_t n, h, w, pitch, frame_stride;
+};
+
+Nv12View nv12_view(const at::Tensor &src)
+{
+    TORCH_CHECK(src.is_cuda(), "src must be a CUDA tensor");
+    TORCH_CHECK(src.scalar_type() == at::kByte, "NV12 frames are uint8, got ", src.scalar_type());
+    TORCH_CHECK(src.dim() == 2 || src.dim() == 3, "NV12 frames must be (H*3/2, W) or (N, H*3/2, W)");
+    Nv12View v;
+    v.s3 = src.dim() == 2 ? src.unsqueeze(0) : src;
+    v.n = v.s3.size(0);
+    const int64_t rows = v.s3.size(1);
+    v.w = v.s3.size(2);
+    TORCH_CHECK(rows > 0 && rows % 3 == 0 && v.w % 2 == 0,
+                "NV12 frames need H*3/2 rows for an even H and an even width; got ", rows, " x ", v.w);
+    TORCH_CHECK(v.s3.stride(2) == 1, "NV12 rows must be contiguous (inner stride 1)");
+    v.h = rows / 3 * 2;
+    v.pitch = v.s3.stride(1);
+    v.frame_stride = v.n > 1 ? v.s3.stride(0) : v.pitch * rows;
+    return v;
+}
+
+at::Tensor nv12_to_bgr(const at::Tensor &src)
+{
+    Nv12View v = nv12_view(src);
+    at::Tensor out = at::empty({v.n, v.h, v.w, 3}, v.s3.options());
+    c10::cuda::CUDAGuard guard(src.device());
+    check_rc(bevk_nv12_to_bgr(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w, (int)v.pitch,
+                              v.frame_stride, current_stream(src)),
+             "bevk_nv12_to_bgr");
+    return src.dim() == 2 ? out.squeeze(0) : out;
+}
+
+at::Tensor warp_perspective_nv12(const at::Tensor &src, const at::Tensor &M, int64_t w, int64_t h, int64_t flags,
+                                 int64_t border_mode, double border_val,
+                                 const c10::optional<at::Tensor> &mat_index)
+{
+    Nv12View v = nv12_view(src);
+    at::Tensor Ms = host_f64(M, "M").reshape({-1, 3, 3});
+    at::Tensor idx;
+    const int32_t *idx_ptr = nullptr;
+    if (mat_index.has_value()) {
+        idx = mat_index->to(at::kCPU, at::kInt).contiguous();
+        TORCH_CHECK(idx.numel() == v.n, "mat_index has ", idx.numel(), " entries for ", v.n, " frames");
+        idx_ptr = idx.data_ptr<int32_t>();
+    }
+    at::Tensor out = at::empty({v.n, h, w, 3}, v.s3.options());
+    const double border[4] = {border_val, border_val, border_val, border_val};
+    c10::cuda::CUDAGuard guard(src.device());
+    check_rc(bevk_warp_perspective_nv12(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w,
+                                        (int)v.pitch, v.frame_stride, (int)h, (int)w, Ms.data_ptr<double>(),
+                                        (int)Ms.size(0), idx_ptr, (int)flags, (int)border_mode, border,
+                                        current_stream(src)),
+             "bevk_warp_perspective_nv12");
+    return src.dim() == 2 ? out.squeeze(0) : out;
+}
+
 // rows (N, in_cols) -> (N, out_cols) through fn(in, out, n, ..., stream)
 template <typename FN> at::Tensor rows(const at::Tensor &x, int64_t in_cols, int64_t out_cols, FN fn, const char *what)
 {
@@ -143,6 +207,9 @@ TORCH_LIBRARY(bev_cuda, m)
     m.def("rbox_corners_project(Tensor xywhr, Tensor? H, int mode) -> Tensor");
     m.def("corners_to_rbox(Tensor xy8, Tensor? H, int mode) -> Tensor");
     m.def("rbox_similarity(Tensor rbox, Tensor H, int src_mode) -> Tensor");
+    m.def("nv12_to_bgr(Tensor src) -> Tensor");
+    m.def("warp_perspective_nv12(Tensor src, Tensor M, int w, int h, int flags=1, int border_mode=0, "
+          "float border_val=0., Tensor? mat_index=None) -> Tensor");
 }
 
 TORCH_LIBRARY_IMPL(bev_cuda, CUDA, m)
@@ -152,4 +219,6 @@ TORCH_LIBRARY_IMPL(bev_cuda, CUDA, m)
     m.impl("rbox_corners_project", &rbox_corners_project);
     m.impl("corners_to_rbox", &corners_to_rbox);
     m.impl("rbox_similarity", &rbox_similarity);
+    m.impl("nv12_to_bgr", &nv12_to_bgr);
+    m.impl("warp_perspective_nv12", &warp_perspective_nv12);
 }

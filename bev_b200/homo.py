@@ -17,6 +17,7 @@ INTER_NEAREST = 0
 INTER_LINEAR = 1
 WARP_INVERSE_MAP = 16
 BORDER_CONSTANT = 0
+COLOR_YUV2BGR_NV12 = 91
 
 
 # ----------------------------------------------------------------------------- host geometry
@@ -231,6 +232,31 @@ def warp_img_to_bev(frames, calib, bspec, flags=INTER_LINEAR):
     """Image -> BEV warp of a frame batch with the calibration objects (vis_homo.py:61-63,89)."""
     H = compose_H_bev_img(calib, bspec)
     return warp_perspective(frames, H, (int(bspec.u_size), int(bspec.v_size)), flags=flags)
+
+
+def nv12_to_bgr(src, dst=None):
+    """Drop-in for ``cv2.cvtColor(f, cv2.COLOR_YUV2BGR_NV12)`` on CUDA tensors, batched: NV12 frames
+    as a GPU video decoder gives them, (H*3/2, W) or (N, H*3/2, W) uint8 with H and W even, to
+    (H, W, 3) / (N, H, W, 3) BGR, byte-identical to cv2 4.13.  Rows may be padded (a row stride,
+    the decoder's pitch, larger than W) and frames may lie apart; the strides are read from the
+    tensor."""
+    return _native.nv12_to_bgr(src, dst)
+
+
+def warp_perspective_nv12(src, M, dsize, dst=None, flags=INTER_LINEAR, borderMode=BORDER_CONSTANT,
+                          borderValue=0, mat_index=None):
+    """``warp_perspective(nv12_to_bgr(src), M, dsize, ...)`` in one pass, without the BGR copy of
+    the frames: byte-identical to ``cv2.warpPerspective(cv2.cvtColor(f, COLOR_YUV2BGR_NV12), M,
+    dsize, flags=flags, borderValue=borderValue)``.  src as for :func:`nv12_to_bgr`; M, mat_index,
+    flags and borderValue (B, G, R) as for :func:`warp_perspective`.  Returns (h, w, 3) or
+    (N, h, w, 3) BGR uint8; the kernel is launched asynchronously on the current CUDA stream."""
+    return _native.warp_perspective_nv12(src, M, dsize, dst, flags, borderMode, borderValue, mat_index)
+
+
+def warp_nv12_img_to_bev(frames, calib, bspec, flags=INTER_LINEAR):
+    """:func:`warp_img_to_bev` for NV12 frames from a GPU video decoder (vis_homo.py:61-63,89)."""
+    H = compose_H_bev_img(calib, bspec)
+    return warp_perspective_nv12(frames, H, (int(bspec.u_size), int(bspec.v_size)), flags=flags)
 
 
 def warp_bev_to_img(bev_frames, calib, bspec, flags=INTER_LINEAR):

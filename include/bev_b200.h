@@ -105,6 +105,36 @@ int bevk_warp_perspective_path(const void *src, void *dst, int n_frames, int src
 int bevk_warp_set_path(int path);
 
 /*
+ * NV12 frames, as a GPU video decoder hands them out, to BGR: cv2.cvtColor(f, COLOR_YUV2BGR_NV12)
+ * (cv2 4.13: BT.601 limited range, chroma shared by each 2x2 luma block) on a batch, byte-identical.
+ * Serves the decode half of "decode -> warp without a host round trip" (SURVEY.md 8f rank 4) for
+ * the frame loop of vis_homo.py:85-91, whose frames are BGR.
+ *   src  device buffer; frame n starts at src + n * frame_stride bytes and holds h luma rows then
+ *        h / 2 rows of interleaved U, V bytes, each row `pitch` bytes after the previous one
+ *        (pitch >= w; a contiguous (n, h * 3 / 2, w) buffer has pitch = w, frame_stride = w * h * 3 / 2)
+ *   dst  [n_frames][h][w][3] contiguous uint8 BGR
+ *   h, w even and positive.
+ */
+int bevk_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int w, int pitch,
+                     int64_t frame_stride, void *stream);
+
+/*
+ * Perspective warp of NV12 frames straight to BGR: dst[i] is byte-identical to
+ *     cv2.warpPerspective(cv2.cvtColor(src[i], COLOR_YUV2BGR_NV12), M[k], (dst_w, dst_h), flags,
+ *                         BORDER_CONSTANT, border_value)
+ * in one pass, without the BGR copy of the frames.  Replaces the warp of vis_homo.py:85-91 for
+ * frames decoded on the GPU (SURVEY.md 8f rank 4).  src layout, pitch and frame_stride as for
+ * bevk_nv12_to_bgr with src_h x src_w luma pixels (both even); dst [n_frames][dst_h][dst_w][3]
+ * uint8.  M, n_mats, mat_index, flags, border_mode and border_value mean what they mean for
+ * bevk_warp_perspective (border_value: B, G, R).  A frame must span less than 4 GB
+ * (pitch * src_h * 3 / 2 < 2^32).
+ */
+int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w,
+                               int pitch, int64_t frame_stride, int dst_h, int dst_w,
+                               const double *M, int n_mats, const int32_t *mat_index, int flags,
+                               int border_mode, const double *border_value, void *stream);
+
+/*
  * Roofline accounting helper (SURVEY.md 8d): number of distinct in-bounds source pixels that the
  * coordinate map of one matrix references (4 taps bilinear / 1 tap nearest), computed on the
  * device with the same coordinate code as the warp.  row_range (HOST int[2], may be NULL)

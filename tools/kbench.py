@@ -287,8 +287,121 @@ def cfg1_cold_warm(steps=50):
     print("cfg1 one 1080p frame -> 1024^2: warm %.1f us, cold (L2 flushed) %.1f us per call" % (res["warm"], res["cold"]))
 
 
+def card():
+    """Name and power limit of GPU 0 (read-only nvidia-smi query): part of every number printed."""
+    import subprocess
+    try:
+        r = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=60)
+        return r.stdout.strip() or r.stderr.strip()
+    except (OSError, subprocess.TimeoutExpired) as e:
+        return "unknown (%s)" % e
+
+
+def _alternate(routes, rounds, steps):
+    """ms per call of each route, timed with CUDA events in rounds that alternate the routes."""
+    times = {name: [] for name in routes}
+    for name, fn in routes.items():  # warm-up: module loads, allocations, the staged kernel's set-up
+        for _ in range(2):
+            fn()
+    torch.cuda.synchronize()
+    for _ in range(rounds):
+        for name, fn in routes.items():
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(steps):
+                fn()
+            e1.record()
+            torch.cuda.synchronize()
+            times[name].append(e0.elapsed_time(e1) / steps)
+    return times
+
+
+def _report(label, times, algo_bytes, peak):
+    for name, t in times.items():
+        t = np.array(t)
+        med = float(np.median(t))
+        print("%s | %s: median %.4f ms (min %.4f, max %.4f, spread %.1f %%), %.0f GB/s algorithmic = %.3f of %.1f GB/s"
+              % (label, name, med, t.min(), t.max(), 100.0 * (t.max() - t.min()) / med,
+                 algo_bytes / (med * 1e-3) / 1e9, algo_bytes / (med * 1e-3) / 1e9 / peak, peak), flush=True)
+    names = list(times)
+    if len(names) == 2:
+        a, b = np.array(times[names[0]]), np.array(times[names[1]])
+        print("%s | %s / %s per round: %s" % (label, names[0], names[1],
+                                             " ".join("%.3f" % v for v in a / b)), flush=True)
+
+
+def nv12_bench(rounds=5):
+    """NV12 frames (GPU decoder output) to BGR BEVs: the fused warp against converting to BGR and
+    then warping, alternating the two routes in one process; the conversion alone.  Algorithmic
+    bytes: touched luma + 2 x touched chroma samples (oracle coordinate map, host) + 3 x dst pixels.
+    Every frame set is larger than the 126 MB L2."""
+    import json
+    from oracle import nv12_oracle
+    print("card: %s" % card(), flush=True)
+    peak, src = bench.measured_peak()
+    print("peak: %.1f GB/s (%s)" % (peak, src), flush=True)
+    dev = torch.device("cuda", 0)
+    g = torch.Generator(device=dev).manual_seed(1234)
+
+    # cfg 2: 256 x 1080p -> 1024^2, the canonical map
+    n, dsize, H = 256, (1024, 1024), bench.h_canon(1)
+    frames = torch.randint(0, 256, (n, 1620, 1920), dtype=torch.uint8, device=dev, generator=g)
+    bgr = torch.empty((n, 1080, 1920, 3), dtype=torch.uint8, device=dev)
+    out_a = torch.empty((n, 1024, 1024, 3), dtype=torch.uint8, device=dev)
+    out_b = torch.empty_like(out_a)
+    for flags, fname in ((1, "bilinear"), (0, "nearest")):
+        luma, chroma = nv12_oracle.touched_samples((1920, 1080), dsize, H, flags)
+        algo = n * (luma + 2 * chroma + 3 * dsize[0] * dsize[1])
+
+        def fused():
+            homo.warp_perspective_nv12(frames, H, dsize, dst=out_a, flags=flags)
+
+        def two_pass():
+            homo.nv12_to_bgr(frames, dst=bgr)
+            homo.warp_perspective(bgr, H, dsize, dst=out_b, flags=flags, path="fast")
+        times = _alternate({"fused": fused, "nv12_to_bgr + staged warp": two_pass}, rounds, 10)
+        assert torch.equal(out_a, out_b), "routes differ"
+        print("cfg2 %s: touched luma %d, chroma %d per frame, %.2f MB algorithmic per frame"
+              % (fname, luma, chroma, algo / n / 1e6))
+        _report("cfg2 x%d 1080p NV12 -> 1024^2 %s" % (n, fname), times, algo, peak)
+
+    # the conversion alone: reads 1.5 B and writes 3 B per pixel
+    conv_bytes = n * 1080 * 1920 * 9 // 2
+    times = _alternate({"nv12_to_bgr": lambda: homo.nv12_to_bgr(frames, dst=bgr)}, rounds, 10)
+    _report("conversion x%d 1080p" % n, times, conv_bytes, peak)
+    del frames, bgr, out_a, out_b
+    torch.cuda.empty_cache()
+
+    # cfg 4: 8 cameras x 1000 frames, one homography and BEV size per camera
+    cams = json.load(open(os.path.join(ROOT, "tests", "golden", "cfg4_cams.json")))
+    n = 1000
+    frames = torch.randint(0, 256, (n, 1620, 1920), dtype=torch.uint8, device=dev, generator=g)
+    bgr = torch.empty((n, 1080, 1920, 3), dtype=torch.uint8, device=dev)
+    jobs, algo = [], 0
+    for c in cams:
+        Hc = np.array(c["H_bev_img"])
+        ds = (int(c["bspec"]["u_size"]), int(c["bspec"]["v_size"]))
+        luma, chroma = nv12_oracle.touched_samples((1920, 1080), ds, Hc, 1)
+        algo += n * (luma + 2 * chroma + 3 * ds[0] * ds[1])
+        jobs.append((Hc, ds, torch.empty((n, ds[1], ds[0], 3), dtype=torch.uint8, device=dev)))
+
+    def fused4():
+        for Hc, ds, o in jobs:
+            homo.warp_perspective_nv12(frames, Hc, ds, dst=o)
+
+    def two_pass4():
+        for Hc, ds, o in jobs:
+            homo.nv12_to_bgr(frames, dst=bgr)
+            homo.warp_perspective(bgr, Hc, ds, dst=o)
+    times = _alternate({"fused": fused4, "nv12_to_bgr + warp per camera": two_pass4}, rounds, 2)
+    _report("cfg4 8 cameras x%d 1080p NV12" % n, times, algo, peak)
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "cfg4":
+    if len(sys.argv) > 1 and sys.argv[1] == "nv12":
+        nv12_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "cfg4":
         if len(sys.argv) > 3:
             _native.set_warp_path(sys.argv[3])
         cfg4(int(sys.argv[2]) if len(sys.argv) > 2 else 1000)
