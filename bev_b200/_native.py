@@ -45,6 +45,7 @@ SIGNATURES = {
     "bevk_warp_perspective_nv12": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int,
                                             _dp, _c_int, _i32p, _c_int, _c_int, _dp, _vp]),
     "bevk_resize": (_c_int, [_vp, _vp] + [_c_int] * 8 + [_vp]),
+    "bevk_resize_nv12": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int, _vp]),
     "bevk_composite_u8c3": (_c_int, [_vp, _vp, _vp, _vp, _c_i64, _c_int, _vp]),
     "bevk_composite_bev_u8c3": (_c_int, [_vp, _vp, _vp, _vp] + [_c_int] * 8 + [_dp, _dp, _c_int, _vp]),
     "bevk_pts_project": (_c_int, [_vp, _vp, _c_i64, _c_int, _c_int, _dp, _vp]),
@@ -440,6 +441,27 @@ def resize(src, dsize, interpolation=1, dst=None):
         return dst.reshape(h, w)
     if src.dim() == 3:
         return dst.reshape(h, w, c)
+    return dst
+
+
+def resize_nv12(src, dsize, dst=None):
+    """resize(nv12_to_bgr(src), dsize) in one pass: CUDA uint8 NV12 frames (H*3/2, W) or
+    (N, H*3/2, W) -> (h, w, 3) or (N, h, w, 3) BGR; dsize = (width, height)."""
+    import torch
+    s3, n, h, w, pitch, fstride = _nv12_frames(src)
+    dw, dh = int(dsize[0]), int(dsize[1])
+    want = (n, dh, dw, 3) if src.dim() == 3 else (dh, dw, 3)
+    if dst is None:
+        dst = torch.empty(want, dtype=torch.uint8, device=src.device)
+    else:
+        _require_cuda(dst, "dst")
+        if tuple(dst.shape) != want or dst.dtype != torch.uint8 or not dst.is_contiguous() \
+                or dst.device != src.device:
+            raise ValueError("dst must be a contiguous uint8 tensor of shape %s on %s" % (want, src.device))
+    with torch.cuda.device(src.device):
+        rc = lib().bevk_resize_nv12(_vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride, dh, dw,
+                                    _stream_ptr(src))
+    _check(rc, "bevk_resize_nv12")
     return dst
 
 

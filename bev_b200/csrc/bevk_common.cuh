@@ -159,3 +159,6 @@ int bevk_launch_warp_fast(const BevkWarpParams &p, int channels, int dtype, int 
 int bevk_launch_warp_nv12(const BevkNv12Params &P, int linear, cudaStream_t stream);
 int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int w, int pitch,
                             long long frame_stride, cudaStream_t stream);
+// cv2.resize(NV12 -> BGR) of n_frames > 0 frames; arguments already checked by bevk_resize_nv12
+int bevk_launch_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                            long long frame_stride, int dst_h, int dst_w, cudaStream_t stream);

@@ -387,7 +387,7 @@ int bevk_warp_perspective_path(const void *src, void *dst, int n_frames, int src
 }  // extern "C"
 
 namespace {
-// The NV12 frame rules of both NV12 entry points: even sizes, rows at least a luma row apart.
+// The NV12 frame rules of the NV12 entry points: even sizes, rows at least a luma row apart.
 int check_nv12_layout(const char *what, int n_frames, int h, int w, int pitch, int64_t frame_stride)
 {
     if (n_frames < 0) BEVK_FAIL(BEVK_E_ARG, "%s: n_frames must be >= 0", what);
@@ -459,6 +459,26 @@ int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src
         if (rc) return rc;
     }
     return BEVK_OK;
+}
+
+int bevk_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                     int64_t frame_stride, int dst_h, int dst_w, void *stream)
+{
+    int rc = check_nv12_layout("resize_nv12", n_frames, src_h, src_w, pitch, frame_stride);
+    if (rc) return rc;
+    if (dst_h <= 0 || dst_w <= 0)
+        BEVK_FAIL(BEVK_E_ARG, "resize_nv12: dst sizes must be positive (got %dx%d)", dst_w, dst_h);
+    if (src_h > 32767 || src_w > 32767 || dst_h > 32767 || dst_w > 32767)
+        BEVK_FAIL(BEVK_E_ARG, "resize_nv12: sizes above 32767 are not supported");
+    // the kernel addresses a frame with 32-bit byte offsets
+    if ((int64_t)pitch * (src_h / 2 * 3) > 0xffffffffLL)
+        BEVK_FAIL(BEVK_E_ARG, "resize_nv12: a frame of pitch %d and %d rows spans 4 GB or more", pitch, src_h / 2 * 3);
+    if (n_frames > 0 && (!src || !dst)) BEVK_FAIL(BEVK_E_ARG, "resize_nv12: null src / dst");
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    return bevk_launch_resize_nv12(src, dst, n_frames, src_h, src_w, pitch, frame_stride, dst_h, dst_w,
+                                   (cudaStream_t)stream);
 }
 
 int bevk_warp_host_rows(int src_h, int src_w, int dst_h, int dst_w, const double *M, int n_mats,

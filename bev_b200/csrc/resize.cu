@@ -19,6 +19,7 @@
 // dp2a for the horizontal pass, 32 pixels packed into one 96-byte store per warp) and a byte-wise
 // one for every other channel count / width.
 #include "bevk_common.cuh"
+#include "resize_coef.cuh"
 #include "warp_u8c3.cuh"
 
 namespace {
@@ -32,8 +33,6 @@ __device__ __forceinline__ uint32_t ldg_dense(const uint32_t *p)
     return v;
 }
 
-constexpr int kCoefScale = 2048;  // INTER_RESIZE_COEF_SCALE
-
 struct ResizeParams {
     const uint8_t *src;
     uint8_t *dst;
@@ -42,32 +41,6 @@ struct ResizeParams {
     double scale_x, scale_y;
     int n_frames, frames_per_chunk;
 };
-
-// (index, w0, w1) of dst position d along one axis; `clamp` = the column rule
-__device__ __forceinline__ void axis_coef(int d, double scale, int ssize, bool clamp, int &s, int &w0, int &w1)
-{
-    float f = __double2float_rn(__dsub_rn(__dmul_rn(__dadd_rn((double)d, 0.5), scale), 0.5));
-    int si = __float2int_rd(f);  // cvFloor
-    f = __fsub_rn(f, (float)si);
-    if (clamp) {
-        if (si < 0) {
-            f = 0.f;
-            si = 0;
-        }
-        if (si >= ssize - 1) {
-            f = 0.f;
-            si = ssize - 1;
-        }
-    }
-    w0 = __float2int_rn(__fmul_rn(__fsub_rn(1.f, f), (float)kCoefScale));
-    w1 = __float2int_rn(__fmul_rn(f, (float)kCoefScale));
-    s = si;
-}
-
-__device__ __forceinline__ uint32_t vpass(int b0, int b1, int s0, int s1)
-{
-    return (uint32_t)((((b0 * (s0 >> 4)) >> 16) + ((b1 * (s1 >> 4)) >> 16) + 2) >> 2);
-}
 
 // ---- any channel count: one thread per dst pixel, byte loads -----------------------------------
 template <int C>
@@ -184,12 +157,7 @@ extern "C" int bevk_resize(const void *src, void *dst, int n_frames, int src_h, 
     p.scale_x = 1.0 / ((double)dst_w / (double)src_w);
     p.scale_y = 1.0 / ((double)dst_h / (double)src_h);
     p.n_frames = n_frames;
-    const long long tiles = (long long)((dst_w + 31) / 32) * ((dst_h + 7) / 8);
-    const long long want_blocks = (long long)bevk_sm_count() * 8 * 2;
-    int fpc = n_frames < 64 ? n_frames : 64;
-    while (fpc > 1 && tiles * ((n_frames + fpc - 1) / fpc) < want_blocks) fpc = (fpc + 1) / 2;
-    // ~12 waves of blocks while a chunk keeps 8 frames: few long blocks leave a costly last wave
-    while (fpc >= 16 && tiles * ((n_frames + fpc - 1) / fpc) < 6 * want_blocks) fpc = (fpc + 1) / 2;
+    const int fpc = bevk_resize_frames_per_chunk(n_frames, dst_h, dst_w);
     p.frames_per_chunk = fpc;
     const int z = (n_frames + fpc - 1) / fpc;
     if (z > 65535) BEVK_FAIL(BEVK_E_ARG, "resize: too many frame chunks (%d) for one launch", z);

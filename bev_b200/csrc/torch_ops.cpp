@@ -10,6 +10,7 @@
 //   torch.ops.bev_cuda.nv12_to_bgr(Tensor src) -> Tensor
 //   torch.ops.bev_cuda.warp_perspective_nv12(Tensor src, Tensor M, int w, int h, int flags, int border_mode,
 //                                            float border_val, Tensor? mat_index) -> Tensor
+//   torch.ops.bev_cuda.resize_nv12(Tensor src, int w, int h) -> Tensor
 //
 // Every implementation only checks tensors, allocates the result with torch's caching allocator,
 // takes the current CUDA stream and calls the extern "C" entry point of include/bev_b200.h with raw
@@ -20,7 +21,8 @@
 // Reference interfaces replaced: cv2.warpPerspective at vis_homo.py:85-91, rbox.pts_world_bev
 // (bev/rbox.py:136-151), rbox_torch.xywhr2xyxy (bev/rbox_torch.py:52-99) + the projection of
 // rbox_vis.py:38-55, rbox.xy82xywhr (bev/rbox.py:50-63), rbox_torch.rbox_world_bev (:123-168); the NV12
-// operators serve the frame loop of vis_homo.py:85-91 with frames from a GPU video decoder.
+// operators serve the frame loop of vis_homo.py:85-91 with frames from a GPU video decoder
+// (resize_nv12: its small-frame copy, vis_homo.py:90).
 #include <ATen/ATen.h>
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
@@ -150,6 +152,17 @@ at::Tensor warp_perspective_nv12(const at::Tensor &src, const at::Tensor &M, int
     return src.dim() == 2 ? out.squeeze(0) : out;
 }
 
+at::Tensor resize_nv12(const at::Tensor &src, int64_t w, int64_t h)
+{
+    Nv12View v = nv12_view(src);
+    at::Tensor out = at::empty({v.n, h, w, 3}, v.s3.options());
+    c10::cuda::CUDAGuard guard(src.device());
+    check_rc(bevk_resize_nv12(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w, (int)v.pitch,
+                              v.frame_stride, (int)h, (int)w, current_stream(src)),
+             "bevk_resize_nv12");
+    return src.dim() == 2 ? out.squeeze(0) : out;
+}
+
 // rows (N, in_cols) -> (N, out_cols) through fn(in, out, n, ..., stream)
 template <typename FN> at::Tensor rows(const at::Tensor &x, int64_t in_cols, int64_t out_cols, FN fn, const char *what)
 {
@@ -210,6 +223,7 @@ TORCH_LIBRARY(bev_cuda, m)
     m.def("nv12_to_bgr(Tensor src) -> Tensor");
     m.def("warp_perspective_nv12(Tensor src, Tensor M, int w, int h, int flags=1, int border_mode=0, "
           "float border_val=0., Tensor? mat_index=None) -> Tensor");
+    m.def("resize_nv12(Tensor src, int w, int h) -> Tensor");
 }
 
 TORCH_LIBRARY_IMPL(bev_cuda, CUDA, m)
@@ -221,4 +235,5 @@ TORCH_LIBRARY_IMPL(bev_cuda, CUDA, m)
     m.impl("rbox_similarity", &rbox_similarity);
     m.impl("nv12_to_bgr", &nv12_to_bgr);
     m.impl("warp_perspective_nv12", &warp_perspective_nv12);
+    m.impl("resize_nv12", &resize_nv12);
 }

@@ -280,3 +280,22 @@ def warp_small_img_to_bev(frames, calib, bspec, new_u, new_v, flags=INTER_LINEAR
     H_small = np.linalg.inv(bspec.gen_H_world_bev()).dot(calib_small.gen_H_world_img())
     small = resize(frames, (int(new_u), int(new_v)))
     return small, warp_perspective(small, H_small, (int(bspec.u_size), int(bspec.v_size)), flags=flags)
+
+
+def resize_nv12(src, dsize, dst=None):
+    """``resize(nv12_to_bgr(src), dsize)`` in one pass, without the BGR copy of the frames:
+    byte-identical to ``cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12), dsize)`` (default
+    INTER_LINEAR).  src as for :func:`nv12_to_bgr`; dsize = (width, height), 1..32767 each.
+    Returns (h, w, 3) or (N, h, w, 3) BGR uint8; the kernel is launched asynchronously on the
+    current CUDA stream."""
+    return _native.resize_nv12(src, dsize, dst)
+
+
+def warp_small_nv12_img_to_bev(frames, calib, bspec, new_u, new_v, flags=INTER_LINEAR):
+    """:func:`warp_small_img_to_bev` for NV12 frames from a GPU video decoder (vis_homo.py:73-78,
+    90-91): the small BGR frames come from :func:`resize_nv12`, without a full-size BGR copy.
+    Returns (small_frames, bev_small)."""
+    calib_small = calib.scale(align_corners=False, new_u=new_u, new_v=new_v)
+    H_small = np.linalg.inv(bspec.gen_H_world_bev()).dot(calib_small.gen_H_world_img())
+    small = resize_nv12(frames, (int(new_u), int(new_v)))
+    return small, warp_perspective(small, H_small, (int(bspec.u_size), int(bspec.v_size)), flags=flags)

@@ -154,6 +154,18 @@ int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, 
                 int dst_w, int channels, int dtype, int interpolation, void *stream);
 
 /*
+ * Batched cv2.resize of NV12 frames straight to small BGR frames: dst[i] is byte-identical to
+ *     cv2.resize(cv2.cvtColor(src[i], COLOR_YUV2BGR_NV12), (dst_w, dst_h))
+ * with the default INTER_LINEAR, in one pass, without the BGR copy of the frames.  Replaces the
+ * small-frame copy at vis_homo.py:90 for frames decoded on the GPU (SURVEY.md 8f rank 4).  src
+ * layout, pitch and frame_stride as for bevk_nv12_to_bgr with src_h x src_w luma pixels (both
+ * even); dst [n_frames][dst_h][dst_w][3] contiguous uint8 BGR.  All sizes 1..32767; a frame must
+ * span less than 4 GB (pitch * src_h * 3 / 2 < 2^32).
+ */
+int bevk_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                     int64_t frame_stride, int dst_h, int dst_w, void *stream);
+
+/*
  * Alpha compositing of uint8 BGR frames, the blend behind the three warps of
  * bev/tool/compo.py:38,46,47 -- replaces composite_reg_img (bev/tool/compo.py:5-24):
  *     out = uint8(min(round_half_even(fg * (mask / 255) + bg * (1 - mask / 255)), 255))

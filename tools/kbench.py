@@ -398,9 +398,47 @@ def nv12_bench(rounds=5):
     _report("cfg4 8 cameras x%d 1080p NV12" % n, times, algo, peak)
 
 
+def resize_nv12_bench(rounds=5):
+    """The small frame of the reference's frame loop (vis_homo.py:90) from NV12 frames: the fused
+    resize against converting to BGR and then resizing, alternating the two routes in one process.
+    Algorithmic bytes: touched luma + 2 x touched chroma samples (taps with a non-zero weight) +
+    3 x dst pixels.  Every frame set is larger than the 126 MB L2."""
+    from oracle import resize_nv12_oracle
+    print("card: %s" % card(), flush=True)
+    peak, src = bench.measured_peak()
+    print("peak: %.1f GB/s (%s)" % (peak, src), flush=True)
+    dev = torch.device("cuda", 0)
+    g = torch.Generator(device=dev).manual_seed(1234)
+    for n, (h, w), dsize in ((256, (1080, 1920), (852, 480)), (256, (1080, 1920), (960, 540)),
+                             (64, (2160, 3840), (1920, 1080))):
+        frames = torch.randint(0, 256, (n, h * 3 // 2, w), dtype=torch.uint8, device=dev, generator=g)
+        bgr = torch.empty((n, h, w, 3), dtype=torch.uint8, device=dev)
+        out_a = torch.empty((n, dsize[1], dsize[0], 3), dtype=torch.uint8, device=dev)
+        out_b = torch.empty_like(out_a)
+        luma, chroma = resize_nv12_oracle.resize_touched_samples((w, h), dsize)
+        algo = n * (luma + 2 * chroma + 3 * dsize[0] * dsize[1])
+
+        def fused():
+            homo.resize_nv12(frames, dsize, dst=out_a)
+
+        def two_pass():
+            homo.nv12_to_bgr(frames, dst=bgr)
+            homo.resize(bgr, dsize, dst=out_b)
+        times = _alternate({"fused": fused, "nv12_to_bgr + resize": two_pass}, rounds, 10)
+        assert torch.equal(out_a, out_b), "routes differ"
+        label = "x%d %dx%d NV12 -> %dx%d" % (n, w, h, dsize[0], dsize[1])
+        print("%s: touched luma %d, chroma %d per frame, %.2f MB algorithmic per frame"
+              % (label, luma, chroma, algo / n / 1e6))
+        _report(label, times, algo, peak)
+        del frames, bgr, out_a, out_b
+        torch.cuda.empty_cache()
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "nv12":
         nv12_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "resize_nv12":
+        resize_nv12_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "cfg4":
         if len(sys.argv) > 3:
             _native.set_warp_path(sys.argv[3])
