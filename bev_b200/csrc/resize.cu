@@ -10,6 +10,8 @@
 //   rint(fx * 2048) in float.  Row dy: the same without that clamp, the two row indices clipped
 //   into the image instead.  S = p[sx] * a0 + p[sx + 1] * a1 per row, then
 //   (((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >> 16) + 2) >> 2.
+//   2-channel frames downscaled by exactly 2 in both axes take the round-half-even mean of each
+//   2x2 block instead (cv2's INTER_AREA special case).
 // The coefficients are recomputed per thread from (dx, dy) with unfused IEEE float / double
 // operations (the library is built with -fmad=false) -- no tables to upload, nothing to keep alive
 // across the asynchronous launch -- and amortised over the frames of the thread's chunk.
@@ -57,6 +59,25 @@ __global__ void __launch_bounds__(256) resize_bytes_kernel(const __grid_constant
     const long long o10 = ((long long)r1 * p.src_w + sx) * C, o11 = ((long long)r1 * p.src_w + sx1) * C;
     const long long od = ((long long)y * p.dst_w + x) * C;
     const int f0 = blockIdx.z * p.frames_per_chunk, f1 = min(f0 + p.frames_per_chunk, p.n_frames);
+    if constexpr (C == 2) {
+        // cv2 sends an exact 2x downscale to INTER_AREA, which for 2 channels rounds the mean of
+        // the 2x2 block half to even (for 1, 3, 4 channels it equals the bilinear result).  The
+        // window above is then exactly that block.
+        if (p.src_w == 2 * p.dst_w && p.src_h == 2 * p.dst_h) {
+            for (int f = f0; f < f1; ++f) {
+                const uint8_t *s = p.src + f * p.src_frame;
+                uint8_t *d = p.dst + f * p.dst_frame + od;
+#pragma unroll
+                for (int c = 0; c < C; ++c) {
+                    const int sum = (int)__ldg(s + o00 + c) + (int)__ldg(s + o01 + c) +
+                                    (int)__ldg(s + o10 + c) + (int)__ldg(s + o11 + c);
+                    const int q = sum >> 2;
+                    d[c] = (uint8_t)(q + ((sum & 3) + (q & 1) > 2));
+                }
+            }
+            return;
+        }
+    }
     for (int f = f0; f < f1; ++f) {
         const uint8_t *s = p.src + f * p.src_frame;
         uint8_t *d = p.dst + f * p.dst_frame + od;

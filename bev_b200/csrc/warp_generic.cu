@@ -107,6 +107,22 @@ __global__ void __launch_bounds__(256) warp_linear_kernel(const __grid_constant_
         const float omx = __fsub_rn(1.0f, tx), omy = __fsub_rn(1.0f, ty);
         const float w00 = __fmul_rn(omy, omx), w01 = __fmul_rn(omy, tx);
         const float w10 = __fmul_rn(ty, omx), w11 = __fmul_rn(ty, tx);
+        if (!(in00 || in01 || in10 || in11)) {
+            // no tap inside: cv2 stores the border value itself, not the weighted sum of four
+            // copies of it (which can miss it by an ulp)
+            for (int f = f0; f < f1; ++f) {
+                const long long fr = (long long)(g.first + f * g.stride);
+                T *d = dst + fr * p.dst_frame_elems + od;
+#pragma unroll
+                for (int c = 0; c < C; ++c) {
+                    if constexpr (sizeof(T) == 2)
+                        d[c] = __float2half_rn(p.border[c]);
+                    else
+                        d[c] = p.border[c];
+                }
+            }
+            return;
+        }
         for (int f = f0; f < f1; ++f) {
             const long long fr = (long long)(g.first + f * g.stride);
             const T *s = src + fr * p.src_frame_elems;

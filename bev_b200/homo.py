@@ -221,7 +221,8 @@ def warp_perspective(src, M, dsize, dst=None, flags=INTER_LINEAR, borderMode=BOR
     launched asynchronously on the current CUDA stream.
 
     uint8/float32 results are bit-identical to cv2 4.13 (nearest and bilinear); float16 equals
-    float16(cv2(float32(src))).  Only BORDER_CONSTANT is implemented (all reference call sites
+    float16(cv2(float32(src))).  Exception: float nearest warps of 1 or 4 channels follow cv2's own
+    remap, not the IPP path cv2 takes for most of those shapes (DESIGN.md section 4).  Only BORDER_CONSTANT is implemented (all reference call sites
     use the default).  ``path`` ("auto" / "generic" / "fast") pins the kernel family for this call
     (tests and benchmarks); None leaves the choice to the library.
     """

@@ -15,6 +15,8 @@ opencv-python-headless 4.13.0.92); its published algorithm for 8-bit bilinear re
   row indices sy, sy + 1 are clipped into the image instead.
 * horizontal pass in int: S = p[sx] * a0 + p[sx + 1] * a1; vertical pass
   ((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >> 16) + 2) >> 2.
+* one exception: 2-channel frames downscaled by exactly 2 in both axes take the round-half-even
+  mean of each 2x2 block (``half_mean_2x2``).
 
 Pinned bit-for-bit against cv2 4.13.0.92 in the build container by oracle/gen_golden.py (all
 shapes of tests/golden/resize_kat.json: the generator asserts equality before it stores cv2's
@@ -52,8 +54,11 @@ def resize(img, dsize):
     squeeze = img.ndim == 2
     if squeeze:
         img = img[:, :, None]
-    h, w = img.shape[:2]
+    h, w, c = img.shape
     dw, dh = int(dsize[0]), int(dsize[1])
+    if c == 2 and w == 2 * dw and h == 2 * dh:
+        out = half_mean_2x2(img)
+        return out[:, :, 0] if squeeze else out
     sx, a0, a1 = axis_coefficients(w, dw, True)
     sy, b0, b1 = axis_coefficients(h, dh, False)
     px = img.astype(np.int32)
@@ -64,6 +69,16 @@ def resize(img, dsize):
     out = (((b0[:, None, None] * (s0 >> 4)) >> 16) + ((b1[:, None, None] * (s1 >> 4)) >> 16) + 2) >> 2
     out = out.astype(np.uint8)
     return out[:, :, 0] if squeeze else out
+
+
+def half_mean_2x2(img):
+    """cv2 sends an exact 2x downscale in both axes to INTER_AREA; for 2-channel uint8 frames that
+    gives the mean of each 2x2 block rounded half to even.  (For 1, 3 and 4 channels it gives
+    (a + b + c + d + 2) >> 2, which the bilinear formula above already equals.)"""
+    p = img.astype(np.int32)
+    s = p[0::2, 0::2] + p[0::2, 1::2] + p[1::2, 0::2] + p[1::2, 1::2]
+    q, r = s >> 2, s & 3
+    return (q + ((r > 2) | ((r == 2) & ((q & 1) == 1)))).astype(np.uint8)
 
 
 def touched_pixels(ssize, dsize):

@@ -165,6 +165,11 @@ int bevo_warp_perspective(const void *src_, int src_h, int src_w, int ch, int dt
                     const int v = (w00 * p00 + w01 * p01 + w10 * p10 + w11 * p11 + 16384) >> 15;
                     d[c] = (uint8_t)(v < 0 ? 0 : (v > 255 ? 255 : v));
                 }
+            } else if (!(in00 || in01 || in10 || in11)) {
+                /* no tap inside: cv2 stores the border value itself, not the weighted sum of four
+                 * copies of it (which can miss it by an ulp) */
+                float *d = (float *)dst_ + ((size_t)y * dst_w + x) * ch;
+                for (int c = 0; c < ch; ++c) d[c] = (float)border[c];
             } else {
                 const float tx = (float)ax * (1.0f / 32.0f), ty = (float)ay * (1.0f / 32.0f);
                 const float w00 = (1.0f - ty) * (1.0f - tx), w01 = (1.0f - ty) * tx;

@@ -52,3 +52,12 @@ def test_scaled_calibration_reproduces_the_small_homography():
     small = calib.scale(align_corners=False, new_u=ch["new_uv"][0], new_v=ch["new_uv"][1])
     H = np.linalg.inv(bspec.gen_H_world_bev()).dot(small.gen_H_world_img())
     assert np.allclose(H, np.array(ch["H_bev_img_small"]), rtol=1e-9, atol=1e-9)
+
+
+def test_two_channel_exact_half_matches_cv2_hashes():
+    """cv2 sends an exact 2x downscale to INTER_AREA; for 2 channels that rounds the 2x2 mean half
+    to even, which the bilinear formula does not (tests/golden/resize_c2_half_hash.json)."""
+    for case in util.load_json("resize_c2_half_hash.json")["cases"]:
+        h, w, c = case["shape"]
+        out = ro.resize(util.seeded_frame(case["seed"], h, w, c, "uint8"), case["dsize"])
+        assert util.sha256(out) == case["sha256"], case

@@ -101,3 +101,13 @@ def test_argument_errors():
     with pytest.raises(RuntimeError):
         homo.resize(t.cpu(), (4, 4))
     assert homo.resize(torch.zeros(0, 8, 8, 3, dtype=torch.uint8, device=DEV), (4, 4)).shape == (0, 4, 4, 3)
+
+
+def test_two_channel_exact_half_matches_cv2_hashes():
+    """2-channel frames downscaled by exactly 2 take cv2's round-half-even 2x2 mean, batched."""
+    for case in util.load_json("resize_c2_half_hash.json")["cases"]:
+        h, w, c = case["shape"]
+        src = util.seeded_frame(case["seed"], h, w, c, "uint8")
+        out = homo.resize(cu(np.stack([src] * 3)), case["dsize"]).cpu().numpy()
+        for i in range(3):
+            assert util.sha256(out[i]) == case["sha256"], (case, i)
