@@ -46,6 +46,8 @@ SIGNATURES = {
                                             _dp, _c_int, _i32p, _c_int, _c_int, _dp, _vp]),
     "bevk_resize": (_c_int, [_vp, _vp] + [_c_int] * 8 + [_vp]),
     "bevk_resize_nv12": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int, _vp]),
+    "bevk_resize_nv12_interp": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int, _c_int,
+                                         _vp]),
     "bevk_composite_u8c3": (_c_int, [_vp, _vp, _vp, _vp, _c_i64, _c_int, _vp]),
     "bevk_composite_bev_u8c3": (_c_int, [_vp, _vp, _vp, _vp] + [_c_int] * 8 + [_dp, _dp, _c_int, _vp]),
     "bevk_pts_project": (_c_int, [_vp, _vp, _c_i64, _c_int, _c_int, _dp, _vp]),
@@ -409,8 +411,9 @@ def rows_op(name, x, in_cols, out_shape_tail, *extra, H=None, has_H=False):
 
 
 def resize(src, dsize, interpolation=1, dst=None):
-    """cv2.resize(src, dsize) (INTER_LINEAR) on uint8 CUDA frames (H,W), (H,W,C) or (N,H,W,C);
-    dsize = (width, height).  Replaces the per-frame call at vis_homo.py:90."""
+    """cv2.resize(src, dsize, interpolation=interpolation) (INTER_LINEAR = 1 or INTER_AREA = 3) on
+    uint8 CUDA frames (H,W), (H,W,C) or (N,H,W,C); dsize = (width, height).  Replaces the
+    per-frame call at vis_homo.py:90."""
     import torch
     _require_cuda(src, "src")
     if src.dtype != torch.uint8:
@@ -444,9 +447,10 @@ def resize(src, dsize, interpolation=1, dst=None):
     return dst
 
 
-def resize_nv12(src, dsize, dst=None):
-    """resize(nv12_to_bgr(src), dsize) in one pass: CUDA uint8 NV12 frames (H*3/2, W) or
-    (N, H*3/2, W) -> (h, w, 3) or (N, h, w, 3) BGR; dsize = (width, height)."""
+def resize_nv12(src, dsize, dst=None, interpolation=1):
+    """resize(nv12_to_bgr(src), dsize, interpolation) in one pass: CUDA uint8 NV12 frames
+    (H*3/2, W) or (N, H*3/2, W) -> (h, w, 3) or (N, h, w, 3) BGR; dsize = (width, height);
+    interpolation INTER_LINEAR = 1 or INTER_AREA = 3."""
     import torch
     s3, n, h, w, pitch, fstride = _nv12_frames(src)
     dw, dh = int(dsize[0]), int(dsize[1])
@@ -459,9 +463,9 @@ def resize_nv12(src, dsize, dst=None):
                 or dst.device != src.device:
             raise ValueError("dst must be a contiguous uint8 tensor of shape %s on %s" % (want, src.device))
     with torch.cuda.device(src.device):
-        rc = lib().bevk_resize_nv12(_vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride, dh, dw,
-                                    _stream_ptr(src))
-    _check(rc, "bevk_resize_nv12")
+        rc = lib().bevk_resize_nv12_interp(_vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride, dh,
+                                           dw, int(interpolation), _stream_ptr(src))
+    _check(rc, "bevk_resize_nv12_interp")
     return dst
 
 

@@ -464,6 +464,16 @@ int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src
 int bevk_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
                      int64_t frame_stride, int dst_h, int dst_w, void *stream)
 {
+    return bevk_resize_nv12_interp(src, dst, n_frames, src_h, src_w, pitch, frame_stride, dst_h, dst_w,
+                                   BEVK_INTER_LINEAR, stream);
+}
+
+int bevk_resize_nv12_interp(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                            int64_t frame_stride, int dst_h, int dst_w, int interpolation, void *stream)
+{
+    if (interpolation != BEVK_INTER_LINEAR && interpolation != BEVK_INTER_AREA)
+        BEVK_FAIL(BEVK_E_ARG, "resize_nv12: only INTER_LINEAR (cv2.resize's default) and INTER_AREA are "
+                  "implemented, got %d", interpolation);
     int rc = check_nv12_layout("resize_nv12", n_frames, src_h, src_w, pitch, frame_stride);
     if (rc) return rc;
     if (dst_h <= 0 || dst_w <= 0)
@@ -477,6 +487,9 @@ int bevk_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int sr
     rc = bevk_require_device();
     if (rc) return rc;
     if (n_frames == 0) return BEVK_OK;
+    if (interpolation == BEVK_INTER_AREA)
+        return bevk_launch_resize_area(src, dst, n_frames, src_h, src_w, 3, 1, pitch, frame_stride, dst_h, dst_w,
+                                       (cudaStream_t)stream);
     return bevk_launch_resize_nv12(src, dst, n_frames, src_h, src_w, pitch, frame_stride, dst_h, dst_w,
                                    (cudaStream_t)stream);
 }

@@ -157,13 +157,16 @@ extern "C" int bevk_resize(const void *src, void *dst, int n_frames, int src_h, 
         BEVK_FAIL(BEVK_E_ARG, "resize: sizes above 32767 are not supported");
     if (channels < 1 || channels > 4) BEVK_FAIL(BEVK_E_ARG, "resize: channels must be 1..4, got %d", channels);
     if (dtype != BEVK_U8) BEVK_FAIL(BEVK_E_ARG, "resize: only uint8 frames are implemented (dtype code %d)", dtype);
-    if (interpolation != BEVK_INTER_LINEAR)
-        BEVK_FAIL(BEVK_E_ARG, "resize: only INTER_LINEAR (cv2.resize's default) is implemented, got %d",
-                  interpolation);
+    if (interpolation != BEVK_INTER_LINEAR && interpolation != BEVK_INTER_AREA)
+        BEVK_FAIL(BEVK_E_ARG, "resize: only INTER_LINEAR (cv2.resize's default) and INTER_AREA are implemented, "
+                  "got %d", interpolation);
     int rc = bevk_require_device();
     if (rc) return rc;
     if (n_frames == 0) return BEVK_OK;
     if (!src || !dst) BEVK_FAIL(BEVK_E_ARG, "resize: null src / dst");
+    if (interpolation == BEVK_INTER_AREA)
+        return bevk_launch_resize_area(src, dst, n_frames, src_h, src_w, channels, 0, (long long)src_w * channels,
+                                       (long long)src_h * src_w * channels, dst_h, dst_w, (cudaStream_t)stream);
 
     ResizeParams p;
     p.src = (const uint8_t *)src;

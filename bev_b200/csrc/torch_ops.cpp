@@ -10,7 +10,7 @@
 //   torch.ops.bev_cuda.nv12_to_bgr(Tensor src) -> Tensor
 //   torch.ops.bev_cuda.warp_perspective_nv12(Tensor src, Tensor M, int w, int h, int flags, int border_mode,
 //                                            float border_val, Tensor? mat_index) -> Tensor
-//   torch.ops.bev_cuda.resize_nv12(Tensor src, int w, int h) -> Tensor
+//   torch.ops.bev_cuda.resize_nv12(Tensor src, int w, int h, int interpolation=1) -> Tensor
 //
 // Every implementation only checks tensors, allocates the result with torch's caching allocator,
 // takes the current CUDA stream and calls the extern "C" entry point of include/bev_b200.h with raw
@@ -152,14 +152,14 @@ at::Tensor warp_perspective_nv12(const at::Tensor &src, const at::Tensor &M, int
     return src.dim() == 2 ? out.squeeze(0) : out;
 }
 
-at::Tensor resize_nv12(const at::Tensor &src, int64_t w, int64_t h)
+at::Tensor resize_nv12(const at::Tensor &src, int64_t w, int64_t h, int64_t interpolation)
 {
     Nv12View v = nv12_view(src);
     at::Tensor out = at::empty({v.n, h, w, 3}, v.s3.options());
     c10::cuda::CUDAGuard guard(src.device());
-    check_rc(bevk_resize_nv12(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w, (int)v.pitch,
-                              v.frame_stride, (int)h, (int)w, current_stream(src)),
-             "bevk_resize_nv12");
+    check_rc(bevk_resize_nv12_interp(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w, (int)v.pitch,
+                                     v.frame_stride, (int)h, (int)w, (int)interpolation, current_stream(src)),
+             "bevk_resize_nv12_interp");
     return src.dim() == 2 ? out.squeeze(0) : out;
 }
 
@@ -223,7 +223,7 @@ TORCH_LIBRARY(bev_cuda, m)
     m.def("nv12_to_bgr(Tensor src) -> Tensor");
     m.def("warp_perspective_nv12(Tensor src, Tensor M, int w, int h, int flags=1, int border_mode=0, "
           "float border_val=0., Tensor? mat_index=None) -> Tensor");
-    m.def("resize_nv12(Tensor src, int w, int h) -> Tensor");
+    m.def("resize_nv12(Tensor src, int w, int h, int interpolation=1) -> Tensor");
 }
 
 TORCH_LIBRARY_IMPL(bev_cuda, CUDA, m)

@@ -15,6 +15,7 @@ from . import _native
 # flag values follow cv2 so existing call sites keep working unchanged
 INTER_NEAREST = 0
 INTER_LINEAR = 1
+INTER_AREA = 3
 WARP_INVERSE_MAP = 16
 BORDER_CONSTANT = 0
 COLOR_YUV2BGR_NV12 = 91
@@ -267,36 +268,40 @@ def warp_bev_to_img(bev_frames, calib, bspec, flags=INTER_LINEAR):
 
 
 def resize(src, dsize, dst=None, interpolation=INTER_LINEAR):
-    """Drop-in for ``cv2.resize(src, dsize)`` (default INTER_LINEAR, uint8) on CUDA tensors, batched:
+    """Drop-in for ``cv2.resize(src, dsize, interpolation=...)`` (uint8) on CUDA tensors, batched:
     the small-frame copy of the reference's frame loop (vis_homo.py:90).  src (H, W), (H, W, C)
-    or (N, H, W, C); dsize = (width, height).  Bit-identical to cv2 4.13."""
+    or (N, H, W, C); dsize = (width, height); interpolation INTER_LINEAR (cv2's default) or
+    INTER_AREA (what OpenCV recommends for downscaling: no aliasing of fine texture).
+    Bit-identical to cv2 4.13."""
     return _native.resize(src, dsize, interpolation, dst)
 
 
-def warp_small_img_to_bev(frames, calib, bspec, new_u, new_v, flags=INTER_LINEAR):
-    """The small-frame path of vis_homo.py:73-78,90-91 on a frame batch: resize to (new_u, new_v),
-    rescale the calibration with ``Calib.scale(align_corners=False)`` and warp the small frames
-    to the same BEV.  Returns (small_frames, bev_small)."""
+def warp_small_img_to_bev(frames, calib, bspec, new_u, new_v, flags=INTER_LINEAR, interpolation=INTER_LINEAR):
+    """The small-frame path of vis_homo.py:73-78,90-91 on a frame batch: resize to (new_u, new_v)
+    with ``interpolation``, rescale the calibration with ``Calib.scale(align_corners=False)`` and
+    warp the small frames to the same BEV with ``flags``.  Returns (small_frames, bev_small)."""
     calib_small = calib.scale(align_corners=False, new_u=new_u, new_v=new_v)
     H_small = np.linalg.inv(bspec.gen_H_world_bev()).dot(calib_small.gen_H_world_img())
-    small = resize(frames, (int(new_u), int(new_v)))
+    small = resize(frames, (int(new_u), int(new_v)), interpolation=interpolation)
     return small, warp_perspective(small, H_small, (int(bspec.u_size), int(bspec.v_size)), flags=flags)
 
 
-def resize_nv12(src, dsize, dst=None):
-    """``resize(nv12_to_bgr(src), dsize)`` in one pass, without the BGR copy of the frames:
-    byte-identical to ``cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12), dsize)`` (default
-    INTER_LINEAR).  src as for :func:`nv12_to_bgr`; dsize = (width, height), 1..32767 each.
-    Returns (h, w, 3) or (N, h, w, 3) BGR uint8; the kernel is launched asynchronously on the
-    current CUDA stream."""
-    return _native.resize_nv12(src, dsize, dst)
+def resize_nv12(src, dsize, dst=None, interpolation=INTER_LINEAR):
+    """``resize(nv12_to_bgr(src), dsize, interpolation=interpolation)`` in one pass, without the
+    BGR copy of the frames: byte-identical to
+    ``cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12), dsize, interpolation=interpolation)`` with
+    INTER_LINEAR (the default) or INTER_AREA.  src as for :func:`nv12_to_bgr`; dsize = (width,
+    height), 1..32767 each.  Returns (h, w, 3) or (N, h, w, 3) BGR uint8; the kernel is launched
+    asynchronously on the current CUDA stream."""
+    return _native.resize_nv12(src, dsize, dst, interpolation)
 
 
-def warp_small_nv12_img_to_bev(frames, calib, bspec, new_u, new_v, flags=INTER_LINEAR):
+def warp_small_nv12_img_to_bev(frames, calib, bspec, new_u, new_v, flags=INTER_LINEAR,
+                               interpolation=INTER_LINEAR):
     """:func:`warp_small_img_to_bev` for NV12 frames from a GPU video decoder (vis_homo.py:73-78,
-    90-91): the small BGR frames come from :func:`resize_nv12`, without a full-size BGR copy.
-    Returns (small_frames, bev_small)."""
+    90-91): the small BGR frames come from :func:`resize_nv12` with ``interpolation``, without a
+    full-size BGR copy.  Returns (small_frames, bev_small)."""
     calib_small = calib.scale(align_corners=False, new_u=new_u, new_v=new_v)
     H_small = np.linalg.inv(bspec.gen_H_world_bev()).dot(calib_small.gen_H_world_img())
-    small = resize_nv12(frames, (int(new_u), int(new_v)))
+    small = resize_nv12(frames, (int(new_u), int(new_v)), interpolation=interpolation)
     return small, warp_perspective(small, H_small, (int(bspec.u_size), int(bspec.v_size)), flags=flags)

@@ -26,6 +26,8 @@ extern "C" {
 /* flags: same numeric values as cv2.INTER_NEAREST / INTER_LINEAR / WARP_INVERSE_MAP */
 #define BEVK_INTER_NEAREST 0
 #define BEVK_INTER_LINEAR 1
+/* resize only: cv2.INTER_AREA */
+#define BEVK_INTER_AREA 3
 #define BEVK_WARP_INVERSE_MAP 16
 /* border_mode: cv2.BORDER_CONSTANT (the only mode any reference call site uses) */
 #define BEVK_BORDER_CONSTANT 0
@@ -144,11 +146,12 @@ int64_t bevk_warp_touched_pixels(int src_h, int src_w, int dst_h, int dst_w, con
                                  int flags, int *row_range);
 
 /*
- * Batched cv2.resize(img, (dst_w, dst_h)) with the default INTER_LINEAR on uint8 frames: replaces
- * the per-frame call at vis_homo.py:90 (the small-frame path; its result feeds the warp at
+ * Batched cv2.resize(img, (dst_w, dst_h), interpolation=...) on uint8 frames: replaces the
+ * per-frame call at vis_homo.py:90 (the small-frame path; its result feeds the warp at
  * vis_homo.py:91 through the homography of Calib.scale(align_corners=False), bev/calib.py:142-198).
  * src [n_frames][src_h][src_w][channels], dst [n_frames][dst_h][dst_w][channels], device buffers,
- * channels 1..4, dtype BEVK_U8, interpolation BEVK_INTER_LINEAR.  Bit-identical to OpenCV 4.13.
+ * channels 1..4, dtype BEVK_U8, interpolation BEVK_INTER_LINEAR (cv2's default) or BEVK_INTER_AREA
+ * (what OpenCV recommends for downscaling).  Bit-identical to OpenCV 4.13.
  */
 int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
                 int dst_w, int channels, int dtype, int interpolation, void *stream);
@@ -164,6 +167,14 @@ int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, 
  */
 int bevk_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
                      int64_t frame_stride, int dst_h, int dst_w, void *stream);
+
+/*
+ * bevk_resize_nv12 with a choice of interpolation: BEVK_INTER_LINEAR, or BEVK_INTER_AREA for
+ *     cv2.resize(cv2.cvtColor(src[i], COLOR_YUV2BGR_NV12), (dst_w, dst_h), interpolation=INTER_AREA).
+ * bevk_resize_nv12 is this function with BEVK_INTER_LINEAR.  Same layouts and limits.
+ */
+int bevk_resize_nv12_interp(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                            int64_t frame_stride, int dst_h, int dst_w, int interpolation, void *stream);
 
 /*
  * Alpha compositing of uint8 BGR frames, the blend behind the three warps of

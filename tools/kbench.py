@@ -434,11 +434,90 @@ def resize_nv12_bench(rounds=5):
         torch.cuda.empty_cache()
 
 
+AREA_WORKLOADS = ((256, (1080, 1920), (852, 480)), (256, (1080, 1920), (960, 540)),
+                  (64, (2160, 3840), (1920, 1080)))
+
+
+def resize_area_bench(rounds=5):
+    """INTER_AREA resize of BGR frames against the INTER_LINEAR kernel on the same shapes,
+    alternating the two in one process.  Algorithmic bytes: 3 x (touched source pixels + dst
+    pixels); a downscale touches the whole frame.  Every frame set is larger than the 126 MB L2.
+    Frame 0 of the area route is checked against the oracle."""
+    from oracle import resize_area_oracle
+    print("card: %s" % card(), flush=True)
+    peak, src = bench.measured_peak()
+    print("peak: %.1f GB/s (%s)" % (peak, src), flush=True)
+    dev = torch.device("cuda", 0)
+    g = torch.Generator(device=dev).manual_seed(1234)
+    for n, (h, w), dsize in AREA_WORKLOADS:
+        frames = torch.randint(0, 256, (n, h, w, 3), dtype=torch.uint8, device=dev, generator=g)
+        out_a = torch.empty((n, dsize[1], dsize[0], 3), dtype=torch.uint8, device=dev)
+        out_b = torch.empty_like(out_a)
+        algo = n * 3 * (resize_area_oracle.touched_pixels((w, h), dsize) + dsize[0] * dsize[1])
+
+        def area():
+            homo.resize(frames, dsize, dst=out_a, interpolation=homo.INTER_AREA)
+
+        def linear():
+            homo.resize(frames, dsize, dst=out_b)
+        times = _alternate({"area": area, "linear": linear}, rounds, 10)
+        ref = resize_area_oracle.resize(frames[0].cpu().numpy(), dsize)
+        assert np.array_equal(out_a[0].cpu().numpy(), ref), "area route differs from the oracle"
+        label = "x%d %dx%d BGR -> %dx%d (%s)" % (n, w, h, dsize[0], dsize[1], resize_area_oracle.branch((w, h), dsize))
+        print("%s: %.2f MB algorithmic per frame" % (label, algo / n / 1e6))
+        _report(label, times, algo, peak)
+        del frames, out_a, out_b
+        torch.cuda.empty_cache()
+
+
+def resize_nv12_area_bench(rounds=5):
+    """INTER_AREA resize of NV12 frames: the fused kernel against the fused INTER_LINEAR kernel
+    and against nv12_to_bgr + INTER_AREA resize, alternating the three in one process.
+    Algorithmic bytes: touched luma + 2 x touched chroma samples + 3 x dst pixels.  Every frame set
+    is larger than the 126 MB L2."""
+    from oracle import resize_area_oracle
+    print("card: %s" % card(), flush=True)
+    peak, src = bench.measured_peak()
+    print("peak: %.1f GB/s (%s)" % (peak, src), flush=True)
+    dev = torch.device("cuda", 0)
+    g = torch.Generator(device=dev).manual_seed(1234)
+    for n, (h, w), dsize in AREA_WORKLOADS:
+        frames = torch.randint(0, 256, (n, h * 3 // 2, w), dtype=torch.uint8, device=dev, generator=g)
+        bgr = torch.empty((n, h, w, 3), dtype=torch.uint8, device=dev)
+        out_a = torch.empty((n, dsize[1], dsize[0], 3), dtype=torch.uint8, device=dev)
+        out_b, out_c = torch.empty_like(out_a), torch.empty_like(out_a)
+        luma, chroma = resize_area_oracle.touched_samples_nv12((w, h), dsize)
+        algo = n * (luma + 2 * chroma + 3 * dsize[0] * dsize[1])
+
+        def fused_area():
+            homo.resize_nv12(frames, dsize, dst=out_a, interpolation=homo.INTER_AREA)
+
+        def fused_linear():
+            homo.resize_nv12(frames, dsize, dst=out_b)
+
+        def two_pass_area():
+            homo.nv12_to_bgr(frames, dst=bgr)
+            homo.resize(bgr, dsize, dst=out_c, interpolation=homo.INTER_AREA)
+        times = _alternate({"fused area": fused_area, "fused linear": fused_linear,
+                            "nv12_to_bgr + area resize": two_pass_area}, rounds, 10)
+        assert torch.equal(out_a, out_c), "area routes differ"
+        label = "x%d %dx%d NV12 -> %dx%d (%s)" % (n, w, h, dsize[0], dsize[1], resize_area_oracle.branch((w, h), dsize))
+        print("%s: touched luma %d, chroma %d per frame, %.2f MB algorithmic per frame"
+              % (label, luma, chroma, algo / n / 1e6))
+        _report(label, times, algo, peak)
+        del frames, bgr, out_a, out_b, out_c
+        torch.cuda.empty_cache()
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "nv12":
         nv12_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_nv12":
         resize_nv12_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "resize_area":
+        resize_area_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "resize_nv12_area":
+        resize_nv12_area_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "cfg4":
         if len(sys.argv) > 3:
             _native.set_warp_path(sys.argv[3])
