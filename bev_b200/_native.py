@@ -157,13 +157,17 @@ def _aligned(t, align=4):
     return t
 
 
-def _check_out(out, like, what):
-    """`out` must be a contiguous tensor of `like`'s shape, dtype and device."""
+def _out(out, shape, dtype, device, what="dst"):
+    """A new tensor of this shape, dtype and device, or `out` after checking that it is a contiguous one."""
+    import torch
+    shape = tuple(shape)
+    if out is None:
+        return torch.empty(shape, dtype=dtype, device=device)
     _require_cuda(out, what)
-    if tuple(out.shape) != tuple(like.shape) or out.dtype != like.dtype or out.device != like.device \
-            or not out.is_contiguous():
-        raise ValueError("%s must be a contiguous %s tensor of shape %s on %s"
-                         % (what, like.dtype, tuple(like.shape), like.device))
+    if tuple(out.shape) != shape or out.dtype != dtype or out.device != device or not out.is_contiguous():
+        raise ValueError("%s must be a contiguous %s tensor of shape %s on %s, got %s %s on %s"
+                         % (what, dtype, shape, device, out.dtype, tuple(out.shape), out.device))
+    return out
 
 
 def _warp_dtype(t):
@@ -198,12 +202,12 @@ def _border(borderValue):
 
 
 def _frames_view(src):
-    """(N, H, W, C) view of a (H,W) / (H,W,C) / (N,H,W,C) tensor + how to undo it."""
-    if src.dim() == 2:
+    """(N, H, W, C) view of a (H,W) / (H,W,C) / (N,H,W,C) tensor or array + how to undo it."""
+    if src.ndim == 2:
         return src[None, :, :, None], lambda o: o[0, :, :, 0]
-    if src.dim() == 3:
+    if src.ndim == 3:
         return src[None], lambda o: o[0]
-    if src.dim() == 4:
+    if src.ndim == 4:
         return src, lambda o: o
     raise ValueError("src must be (H,W), (H,W,C) or (N,H,W,C); got shape %s" % (tuple(src.shape),))
 
@@ -223,16 +227,11 @@ def warp_perspective(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue
     n, h, w, c = s4.shape
     dw, dh = int(dsize[0]), int(dsize[1])
     Ms, idx = _prep_mats(M, n, mat_index)
-    if dst is not None:
+    d4 = None
+    if dst is not None:  # any rank whose (N, H, W, C) view has the output's shape
         _require_cuda(dst, "dst")
         d4, _ = _frames_view(dst)
-        if tuple(d4.shape) != (n, dh, dw, c) or dst.dtype != src.dtype or not dst.is_contiguous() \
-                or dst.device != src.device:
-            raise ValueError("dst must be a contiguous %s tensor of shape %s on %s"
-                             % (src.dtype, (n, dh, dw, c), src.device))
-        out4 = d4
-    else:
-        out4 = torch.empty((n, dh, dw, c), dtype=src.dtype, device=src.device)
+    out4 = _out(d4, (n, dh, dw, c), src.dtype, src.device)
     b = _border(borderValue)
     with torch.cuda.device(src.device):
         rc = lib().bevk_warp_perspective_path(
@@ -250,14 +249,7 @@ def warp_perspective_host(src, M, dsize, dst=None, flags=1, borderMode=0, border
     code = {np.dtype("uint8"): U8, np.dtype("float16"): F16, np.dtype("float32"): F32}.get(s.dtype)
     if code is None:
         raise TypeError("warp_perspective_host supports uint8/float16/float32, got %s" % s.dtype)
-    if s.ndim == 2:
-        s4, undo = s[None, :, :, None], (lambda o: o[0, :, :, 0])
-    elif s.ndim == 3:
-        s4, undo = s[None], (lambda o: o[0])
-    elif s.ndim == 4:
-        s4, undo = s, (lambda o: o)
-    else:
-        raise ValueError("src must be (H,W), (H,W,C) or (N,H,W,C)")
+    s4, undo = _frames_view(s)
     s4 = np.ascontiguousarray(s4)
     n, h, w, c = s4.shape
     dw, dh = int(dsize[0]), int(dsize[1])
@@ -311,14 +303,7 @@ def nv12_to_bgr(src, dst=None):
     -> (H, W, 3) or (N, H, W, 3) BGR."""
     import torch
     s3, n, h, w, pitch, fstride = _nv12_frames(src)
-    want = (n, h, w, 3) if src.dim() == 3 else (h, w, 3)
-    if dst is None:
-        dst = torch.empty(want, dtype=torch.uint8, device=src.device)
-    else:
-        _require_cuda(dst, "dst")
-        if tuple(dst.shape) != want or dst.dtype != torch.uint8 or not dst.is_contiguous() \
-                or dst.device != src.device:
-            raise ValueError("dst must be a contiguous uint8 tensor of shape %s on %s" % (want, src.device))
+    dst = _out(dst, (n, h, w, 3) if src.dim() == 3 else (h, w, 3), torch.uint8, src.device)
     with torch.cuda.device(src.device):
         rc = lib().bevk_nv12_to_bgr(_vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride,
                                     _stream_ptr(src))
@@ -333,14 +318,7 @@ def warp_perspective_nv12(src, M, dsize, dst=None, flags=1, borderMode=0, border
     s3, n, h, w, pitch, fstride = _nv12_frames(src)
     dw, dh = int(dsize[0]), int(dsize[1])
     Ms, idx = _prep_mats(M, n, mat_index)
-    want = (n, dh, dw, 3) if src.dim() == 3 else (dh, dw, 3)
-    if dst is None:
-        dst = torch.empty(want, dtype=torch.uint8, device=src.device)
-    else:
-        _require_cuda(dst, "dst")
-        if tuple(dst.shape) != want or dst.dtype != torch.uint8 or not dst.is_contiguous() \
-                or dst.device != src.device:
-            raise ValueError("dst must be a contiguous uint8 tensor of shape %s on %s" % (want, src.device))
+    dst = _out(dst, (n, dh, dw, 3) if src.dim() == 3 else (dh, dw, 3), torch.uint8, src.device)
     b = _border(borderValue)
     with torch.cuda.device(src.device):
         rc = lib().bevk_warp_perspective_nv12(
@@ -418,32 +396,15 @@ def resize(src, dsize, interpolation=1, dst=None):
     _require_cuda(src, "src")
     if src.dtype != torch.uint8:
         raise TypeError("resize: only uint8 frames are implemented, got %s" % (src.dtype,))
-    if src.dim() not in (2, 3, 4):
-        raise ValueError("resize: src must be (H,W), (H,W,C) or (N,H,W,C); got %s" % (tuple(src.shape),))
-    w, h = int(dsize[0]), int(dsize[1])
-    s4 = src.contiguous()
-    if src.dim() == 2:
-        s4 = s4[None, :, :, None]
-    elif src.dim() == 3:
-        s4 = s4[None]
+    s4, _ = _frames_view(src)
+    s4 = s4.contiguous()
     n, sh, sw, c = s4.shape
-    want = {2: (h, w), 3: (h, w, c), 4: (n, h, w, c)}[src.dim()]
-    if dst is None:
-        dst = torch.empty((n, h, w, c), dtype=torch.uint8, device=src.device)
-    else:
-        _require_cuda(dst, "dst")
-        if tuple(dst.shape) != want or dst.dtype != torch.uint8 or not dst.is_contiguous() \
-                or dst.device != src.device:
-            raise ValueError("resize: dst must be a contiguous uint8 tensor of shape %s on %s, got %s %s on %s"
-                             % (want, src.device, dst.dtype, tuple(dst.shape), dst.device))
+    w, h = int(dsize[0]), int(dsize[1])
+    dst = _out(dst, {2: (h, w), 3: (h, w, c), 4: (n, h, w, c)}[src.dim()], torch.uint8, src.device)
     with torch.cuda.device(src.device):
         rc = lib().bevk_resize(_vp(s4.data_ptr()), _vp(dst.data_ptr()), n, sh, sw, h, w, c, 0,
                                int(interpolation), _stream_ptr(src))
     _check(rc, "bevk_resize")
-    if src.dim() == 2:
-        return dst.reshape(h, w)
-    if src.dim() == 3:
-        return dst.reshape(h, w, c)
     return dst
 
 
@@ -454,14 +415,7 @@ def resize_nv12(src, dsize, dst=None, interpolation=1):
     import torch
     s3, n, h, w, pitch, fstride = _nv12_frames(src)
     dw, dh = int(dsize[0]), int(dsize[1])
-    want = (n, dh, dw, 3) if src.dim() == 3 else (dh, dw, 3)
-    if dst is None:
-        dst = torch.empty(want, dtype=torch.uint8, device=src.device)
-    else:
-        _require_cuda(dst, "dst")
-        if tuple(dst.shape) != want or dst.dtype != torch.uint8 or not dst.is_contiguous() \
-                or dst.device != src.device:
-            raise ValueError("dst must be a contiguous uint8 tensor of shape %s on %s" % (want, src.device))
+    dst = _out(dst, (n, dh, dw, 3) if src.dim() == 3 else (dh, dw, 3), torch.uint8, src.device)
     with torch.cuda.device(src.device):
         rc = lib().bevk_resize_nv12_interp(_vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride, dh,
                                            dw, int(interpolation), _stream_ptr(src))
@@ -486,12 +440,9 @@ def composite_u8c3(bg, fg, fg_mask, bw_mode=False, out=None):
     # the kernel reads 4-byte words: views at an odd byte offset (the mask half of a concatenated
     # warp output, user slices) are realigned by a copy
     bg, fg, fg_mask = _aligned(bg), _aligned(fg), _aligned(fg_mask)
-    if out is None:
-        out = torch.empty_like(bg)
-    else:
-        _check_out(out, bg, "out")
-        if out.data_ptr() % 4:
-            raise ValueError("out must be 4-byte aligned")
+    out = _out(out, bg.shape, torch.uint8, bg.device, "out")
+    if out.data_ptr() % 4:
+        raise ValueError("out must be 4-byte aligned")
     n_pixels = bg.numel() // 3
     with torch.cuda.device(bg.device):
         rc = lib().bevk_composite_u8c3(_vp(bg.data_ptr()), _vp(fg.data_ptr()), _vp(fg_mask.data_ptr()),
@@ -532,14 +483,9 @@ def composite_bev_u8c3(bg, fg, fg_mask, H_bg, H_fg, dsize, out=None):
                          % (bg.device, fg.device, fg_mask.device))
     bg, fg, fg_mask = _aligned(bg, 16), _aligned(fg, 16), _aligned(fg_mask, 16)
     w, h = int(dsize[0]), int(dsize[1])
-    if out is None:
-        out = torch.empty((n, h, w, 3), dtype=torch.uint8, device=fg.device)
-    else:
-        _require_cuda(out, "out")
-        if tuple(out.shape) != (n, h, w, 3) or out.dtype != torch.uint8 or not out.is_contiguous() \
-                or out.device != fg.device or out.data_ptr() % 4:
-            raise ValueError("out must be a contiguous, 4-byte aligned uint8 tensor of shape %s on %s"
-                             % ((n, h, w, 3), fg.device))
+    out = _out(out, (n, h, w, 3), torch.uint8, fg.device, "out")
+    if out.data_ptr() % 4:
+        raise ValueError("out must be 4-byte aligned")
     with torch.cuda.device(fg.device):
         rc = lib().bevk_composite_bev_u8c3(
             _vp(bg.data_ptr()), _vp(fg.data_ptr()), _vp(fg_mask.data_ptr()), _vp(out.data_ptr()),

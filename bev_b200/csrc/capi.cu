@@ -149,17 +149,25 @@ struct WarpArgs {
     float border[4];
 };
 
+// The frame sizes every warp and resize takes: 1..32767.
+int check_sizes(const char *what, int src_h, int src_w, int dst_h, int dst_w)
+{
+    if (src_h <= 0 || src_w <= 0 || dst_h <= 0 || dst_w <= 0)
+        BEVK_FAIL(BEVK_E_ARG, "%s: image sizes must be positive (src %dx%d, dst %dx%d)", what, src_w, src_h,
+                  dst_w, dst_h);
+    if (src_h > 32767 || src_w > 32767 || dst_h > 32767 || dst_w > 32767)
+        BEVK_FAIL(BEVK_E_ARG, "%s: sizes above 32767 are not supported (cv2 SHRT_MAX limit)", what);
+    return BEVK_OK;
+}
+
 int check_warp_args(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
                     int dst_w, int channels, int dtype, const double *M, int n_mats,
                     const int32_t *mat_index, int flags, int border_mode,
                     const double *border_value, WarpArgs &a)
 {
     if (n_frames < 0) BEVK_FAIL(BEVK_E_ARG, "warp: n_frames must be >= 0");
-    if (src_h <= 0 || src_w <= 0 || dst_h <= 0 || dst_w <= 0)
-        BEVK_FAIL(BEVK_E_ARG, "warp: image sizes must be positive (src %dx%d, dst %dx%d)", src_w,
-                  src_h, dst_w, dst_h);
-    if (src_h > 32767 || src_w > 32767 || dst_h > 32767 || dst_w > 32767)
-        BEVK_FAIL(BEVK_E_ARG, "warp: sizes above 32767 are not supported (cv2 SHRT_MAX limit)");
+    int rc = check_sizes("warp", src_h, src_w, dst_h, dst_w);
+    if (rc) return rc;
     if (channels < 1 || channels > 4) BEVK_FAIL(BEVK_E_ARG, "warp: channels must be 1..4, got %d", channels);
     if (dtype != BEVK_U8 && dtype != BEVK_F16 && dtype != BEVK_F32)
         BEVK_FAIL(BEVK_E_ARG, "warp: dtype must be uint8, float16 or float32 (code %d)", dtype);
@@ -241,10 +249,12 @@ void build_groups(int n_frames, int n_mats, const int32_t *mat_index, const std:
     }
 }
 
-int run_warp_device(const void *src, void *dst, const WarpArgs &a,
-                    const std::vector<BevkWarpGroup> &groups, int path, cudaStream_t stream)
+// Fill p from a and walk the groups in launches of up to BEVK_MAX_GROUPS: launch() plans and
+// launches the groups p holds.
+template <typename Launch>
+int launch_warp_groups(BevkWarpParams &p, const void *src, void *dst, const WarpArgs &a,
+                       const std::vector<BevkWarpGroup> &groups, Launch launch)
 {
-    BevkWarpParams p;
     memset(&p, 0, sizeof(p));
     p.src = src;
     p.dst = dst;
@@ -261,21 +271,28 @@ int run_warp_device(const void *src, void *dst, const WarpArgs &a,
         const int ng = (int)std::min<size_t>(BEVK_MAX_GROUPS, groups.size() - g0);
         p.n_groups = ng;
         for (int i = 0; i < ng; ++i) p.g[i] = groups[g0 + i];
-        int launched = 0;
-        if (path != 1) {
-            launched = bevk_launch_warp_fast(p, a.channels, a.dtype, a.linear, path == 2, stream);
-            if (launched < 0) return launched;
-            if (!launched && path == 2)
-                BEVK_FAIL(BEVK_E_ARG, "warp: shape does not qualify for the staged fast path");
-        }
-        if (!launched) {
-            int rc = bevk_plan_generic_chunks(p, a.channels);
-            if (rc) return rc;
-            rc = bevk_launch_warp_generic(p, a.channels, a.dtype, a.linear, stream);
-            if (rc) return rc;
-        }
+        const int rc = launch();
+        if (rc) return rc;
     }
     return BEVK_OK;
+}
+
+// The BGR warp: the staged kernel where it qualifies (path 0 or 2), else the direct-gather kernels.
+int run_warp_device(const void *src, void *dst, const WarpArgs &a,
+                    const std::vector<BevkWarpGroup> &groups, int path, cudaStream_t stream)
+{
+    BevkWarpParams p;
+    return launch_warp_groups(p, src, dst, a, groups, [&]() -> int {
+        if (path != 1) {
+            const int launched = bevk_launch_warp_fast(p, a.channels, a.dtype, a.linear, path == 2, stream);
+            if (launched < 0) return launched;
+            if (launched) return BEVK_OK;
+            if (path == 2) BEVK_FAIL(BEVK_E_ARG, "warp: shape does not qualify for the staged fast path");
+        }
+        const int rc = bevk_plan_generic_chunks(p, a.channels);
+        if (rc) return rc;
+        return bevk_launch_warp_generic(p, a.channels, a.dtype, a.linear, stream);
+    });
 }
 
 // Source rows referenced by one dst->src map.  A projective map restricted to a line is monotone
@@ -397,6 +414,41 @@ int check_nv12_layout(const char *what, int n_frames, int h, int w, int pitch, i
     if (frame_stride < 0) BEVK_FAIL(BEVK_E_ARG, "%s: negative frame stride", what);
     return BEVK_OK;
 }
+
+// check_nv12_layout for the fused kernels, which address a frame with 32-bit byte offsets
+int check_nv12_layout32(const char *what, int n_frames, int h, int w, int pitch, int64_t frame_stride)
+{
+    int rc = check_nv12_layout(what, n_frames, h, w, pitch, frame_stride);
+    if (rc) return rc;
+    if ((int64_t)pitch * (h / 2 * 3) > 0xffffffffLL)
+        BEVK_FAIL(BEVK_E_ARG, "%s: a frame of pitch %d and %d rows spans 4 GB or more", what, pitch, h / 2 * 3);
+    return BEVK_OK;
+}
+
+// The resize entry points after their frame-format checks: n_frames >= 0 frames of `channels`
+// uint8 channels, or NV12 frames (nv12, channels 3) converted to BGR; rows `pitch` and frames
+// `frame_stride` bytes apart.
+int resize_frames(const char *what, const void *src, void *dst, int n_frames, int src_h, int src_w, int channels,
+                  int nv12, long long pitch, long long frame_stride, int dst_h, int dst_w, int interpolation,
+                  void *stream)
+{
+    if (interpolation != BEVK_INTER_LINEAR && interpolation != BEVK_INTER_AREA)
+        BEVK_FAIL(BEVK_E_ARG, "%s: only INTER_LINEAR (cv2.resize's default) and INTER_AREA are implemented, got %d",
+                  what, interpolation);
+    int rc = check_sizes(what, src_h, src_w, dst_h, dst_w);
+    if (rc) return rc;
+    if (n_frames > 0 && (!src || !dst)) BEVK_FAIL(BEVK_E_ARG, "%s: null src / dst", what);
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (interpolation == BEVK_INTER_AREA)
+        return bevk_launch_resize_area(src, dst, n_frames, src_h, src_w, channels, nv12, pitch, frame_stride, dst_h,
+                                       dst_w, st);
+    if (nv12)
+        return bevk_launch_resize_nv12(src, dst, n_frames, src_h, src_w, (int)pitch, frame_stride, dst_h, dst_w, st);
+    return bevk_launch_resize(src, dst, n_frames, src_h, src_w, channels, dst_h, dst_w, st);
+}
 }  // namespace
 
 extern "C" {
@@ -418,11 +470,8 @@ int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src
                                const double *M, int n_mats, const int32_t *mat_index, int flags,
                                int border_mode, const double *border_value, void *stream)
 {
-    int rc = check_nv12_layout("warp_nv12", n_frames, src_h, src_w, pitch, frame_stride);
+    int rc = check_nv12_layout32("warp_nv12", n_frames, src_h, src_w, pitch, frame_stride);
     if (rc) return rc;
-    // the kernel addresses a frame with 32-bit byte offsets
-    if ((int64_t)pitch * (src_h / 2 * 3) > 0xffffffffLL)
-        BEVK_FAIL(BEVK_E_ARG, "warp_nv12: a frame of pitch %d and %d rows spans 4 GB or more", pitch, src_h / 2 * 3);
     WarpArgs a;
     rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index,
                          flags, border_mode, border_value, a);
@@ -437,28 +486,23 @@ int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src
 
     BevkNv12Params P;
     memset(&P, 0, sizeof(P));
-    BevkWarpParams &p = P.w;
-    p.src = src;
-    p.dst = dst;
-    p.src_h = src_h;
-    p.src_w = src_w;
-    p.dst_h = dst_h;
-    p.dst_w = dst_w;
-    p.dst_frame_elems = (long long)dst_h * dst_w * 3;
-    p.bw0 = bevk_block_width(dst_w, dst_h);
-    for (int c = 0; c < 4; ++c) p.border[c] = a.border[c];
     P.pitch = pitch;
     P.frame_stride = frame_stride;
-    for (size_t g0 = 0; g0 < groups.size(); g0 += BEVK_MAX_GROUPS) {
-        const int ng = (int)std::min<size_t>(BEVK_MAX_GROUPS, groups.size() - g0);
-        p.n_groups = ng;
-        for (int i = 0; i < ng; ++i) p.g[i] = groups[g0 + i];
-        rc = bevk_plan_generic_chunks(p, 3);
+    return launch_warp_groups(P.w, src, dst, a, groups, [&]() {
+        const int rc = bevk_plan_generic_chunks(P.w, 3);
         if (rc) return rc;
-        rc = bevk_launch_warp_nv12(P, a.linear, (cudaStream_t)stream);
-        if (rc) return rc;
-    }
-    return BEVK_OK;
+        return bevk_launch_warp_nv12(P, a.linear, (cudaStream_t)stream);
+    });
+}
+
+int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h, int dst_w, int channels,
+                int dtype, int interpolation, void *stream)
+{
+    if (n_frames < 0) BEVK_FAIL(BEVK_E_ARG, "resize: n_frames must be >= 0");
+    if (channels < 1 || channels > 4) BEVK_FAIL(BEVK_E_ARG, "resize: channels must be 1..4, got %d", channels);
+    if (dtype != BEVK_U8) BEVK_FAIL(BEVK_E_ARG, "resize: only uint8 frames are implemented (dtype code %d)", dtype);
+    return resize_frames("resize", src, dst, n_frames, src_h, src_w, channels, 0, (long long)src_w * channels,
+                         (long long)src_h * src_w * channels, dst_h, dst_w, interpolation, stream);
 }
 
 int bevk_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
@@ -471,27 +515,10 @@ int bevk_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int sr
 int bevk_resize_nv12_interp(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
                             int64_t frame_stride, int dst_h, int dst_w, int interpolation, void *stream)
 {
-    if (interpolation != BEVK_INTER_LINEAR && interpolation != BEVK_INTER_AREA)
-        BEVK_FAIL(BEVK_E_ARG, "resize_nv12: only INTER_LINEAR (cv2.resize's default) and INTER_AREA are "
-                  "implemented, got %d", interpolation);
-    int rc = check_nv12_layout("resize_nv12", n_frames, src_h, src_w, pitch, frame_stride);
+    const int rc = check_nv12_layout32("resize_nv12", n_frames, src_h, src_w, pitch, frame_stride);
     if (rc) return rc;
-    if (dst_h <= 0 || dst_w <= 0)
-        BEVK_FAIL(BEVK_E_ARG, "resize_nv12: dst sizes must be positive (got %dx%d)", dst_w, dst_h);
-    if (src_h > 32767 || src_w > 32767 || dst_h > 32767 || dst_w > 32767)
-        BEVK_FAIL(BEVK_E_ARG, "resize_nv12: sizes above 32767 are not supported");
-    // the kernel addresses a frame with 32-bit byte offsets
-    if ((int64_t)pitch * (src_h / 2 * 3) > 0xffffffffLL)
-        BEVK_FAIL(BEVK_E_ARG, "resize_nv12: a frame of pitch %d and %d rows spans 4 GB or more", pitch, src_h / 2 * 3);
-    if (n_frames > 0 && (!src || !dst)) BEVK_FAIL(BEVK_E_ARG, "resize_nv12: null src / dst");
-    rc = bevk_require_device();
-    if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
-    if (interpolation == BEVK_INTER_AREA)
-        return bevk_launch_resize_area(src, dst, n_frames, src_h, src_w, 3, 1, pitch, frame_stride, dst_h, dst_w,
-                                       (cudaStream_t)stream);
-    return bevk_launch_resize_nv12(src, dst, n_frames, src_h, src_w, pitch, frame_stride, dst_h, dst_w,
-                                   (cudaStream_t)stream);
+    return resize_frames("resize_nv12", src, dst, n_frames, src_h, src_w, 3, 1, pitch, frame_stride, dst_h, dst_w,
+                         interpolation, stream);
 }
 
 int bevk_warp_host_rows(int src_h, int src_w, int dst_h, int dst_w, const double *M, int n_mats,

@@ -35,15 +35,6 @@ __device__ __forceinline__ uint32_t border_bgr(const float *b)
     return px;
 }
 
-__device__ __forceinline__ const BevkWarpGroup &find_group(const BevkWarpParams &p, int z)
-{
-    int gi = 0;
-#pragma unroll 1
-    for (int i = 1; i < p.n_groups; ++i)
-        if (z >= p.g[i].chunk0) gi = i;
-    return p.g[gi];
-}
-
 // ---- fused warp -------------------------------------------------------------------------------
 // One lane per dst pixel, as warp_u8c3_direct_kernel (warp_generic.cu): the coordinate is computed
 // once per frame chunk with bevk_map_pixel, then every frame of the chunk gathers the window's two
@@ -59,7 +50,8 @@ __global__ void __launch_bounds__(256) warp_nv12_kernel(const __grid_constant__ 
     const int lane = threadIdx.x, x0 = blockIdx.x * 32;
     const int x = x0 + lane, y = blockIdx.y * 8 + threadIdx.y;
     if (y >= p.dst_h) return;  // a warp is one dst row segment: uniform exit, shuffles stay legal
-    const BevkWarpGroup &g = find_group(p, blockIdx.z);
+    int gi;
+    const BevkWarpGroup &g = find_group(p, blockIdx.z, gi);
     const int c_local = blockIdx.z - g.chunk0;
     const int f0 = c_local * p.frames_per_chunk;
     const int f1 = min(f0 + p.frames_per_chunk, g.count);
@@ -472,6 +464,9 @@ int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int
 int bevk_launch_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
                             long long frame_stride, int dst_h, int dst_w, cudaStream_t stream)
 {
+    BevkResizePlan plan;
+    int rc = bevk_plan_resize(n_frames, src_h, src_w, dst_h, dst_w, plan);
+    if (rc) return rc;
     ResizeNv12Params p;
     p.src = (const uint8_t *)src;
     p.dst = (uint8_t *)dst;
@@ -482,17 +477,13 @@ int bevk_launch_resize_nv12(const void *src, void *dst, int n_frames, int src_h,
     p.pitch = (uint32_t)pitch;
     p.frame_stride = frame_stride;
     p.dst_frame = (long long)dst_h * dst_w * 3;
-    // cv2: inv_scale = (double)dsize / ssize; scale = 1. / inv_scale
-    p.scale_x = 1.0 / ((double)dst_w / (double)src_w);
-    p.scale_y = 1.0 / ((double)dst_h / (double)src_h);
+    p.scale_x = plan.scale_x;
+    p.scale_y = plan.scale_y;
     p.n_frames = n_frames;
-    p.frames_per_chunk = bevk_resize_frames_per_chunk(n_frames, dst_h, dst_w);
-    const int z = (n_frames + p.frames_per_chunk - 1) / p.frames_per_chunk;
-    if (z > 65535) BEVK_FAIL(BEVK_E_ARG, "resize_nv12: too many frame chunks (%d) for one launch", z);
-    const dim3 grid((dst_w + 31) / 32, (dst_h + 7) / 8, z);
+    p.frames_per_chunk = plan.frames_per_chunk;
     const bool words = ((uintptr_t)src % 4) == 0 && (pitch % 4) == 0 && (frame_stride % 4) == 0;
     const bool packed = (dst_w % 4) == 0 && ((uintptr_t)dst % 4) == 0;
-    words ? launch_resize<true>(p, packed, grid, stream) : launch_resize<false>(p, packed, grid, stream);
+    words ? launch_resize<true>(p, packed, plan.grid, stream) : launch_resize<false>(p, packed, plan.grid, stream);
     BEVK_CUDA(cudaGetLastError());
     return BEVK_OK;
 }

@@ -146,28 +146,12 @@ template <int C> void launch_bytes(const ResizeParams &p, dim3 grid, cudaStream_
 
 }  // namespace
 
-extern "C" int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
-                           int dst_w, int channels, int dtype, int interpolation, void *stream)
+int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels, int dst_h,
+                       int dst_w, cudaStream_t stream)
 {
-    if (n_frames < 0) BEVK_FAIL(BEVK_E_ARG, "resize: n_frames must be >= 0");
-    if (src_h <= 0 || src_w <= 0 || dst_h <= 0 || dst_w <= 0)
-        BEVK_FAIL(BEVK_E_ARG, "resize: image sizes must be positive (src %dx%d, dst %dx%d)", src_w, src_h,
-                  dst_w, dst_h);
-    if (src_h > 32767 || src_w > 32767 || dst_h > 32767 || dst_w > 32767)
-        BEVK_FAIL(BEVK_E_ARG, "resize: sizes above 32767 are not supported");
-    if (channels < 1 || channels > 4) BEVK_FAIL(BEVK_E_ARG, "resize: channels must be 1..4, got %d", channels);
-    if (dtype != BEVK_U8) BEVK_FAIL(BEVK_E_ARG, "resize: only uint8 frames are implemented (dtype code %d)", dtype);
-    if (interpolation != BEVK_INTER_LINEAR && interpolation != BEVK_INTER_AREA)
-        BEVK_FAIL(BEVK_E_ARG, "resize: only INTER_LINEAR (cv2.resize's default) and INTER_AREA are implemented, "
-                  "got %d", interpolation);
-    int rc = bevk_require_device();
+    BevkResizePlan plan;
+    int rc = bevk_plan_resize(n_frames, src_h, src_w, dst_h, dst_w, plan);
     if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
-    if (!src || !dst) BEVK_FAIL(BEVK_E_ARG, "resize: null src / dst");
-    if (interpolation == BEVK_INTER_AREA)
-        return bevk_launch_resize_area(src, dst, n_frames, src_h, src_w, channels, 0, (long long)src_w * channels,
-                                       (long long)src_h * src_w * channels, dst_h, dst_w, (cudaStream_t)stream);
-
     ResizeParams p;
     p.src = (const uint8_t *)src;
     p.dst = (uint8_t *)dst;
@@ -177,26 +161,20 @@ extern "C" int bevk_resize(const void *src, void *dst, int n_frames, int src_h, 
     p.dst_w = dst_w;
     p.src_frame = (long long)src_h * src_w * channels;
     p.dst_frame = (long long)dst_h * dst_w * channels;
-    // cv2: inv_scale = (double)dsize / ssize; scale = 1. / inv_scale
-    p.scale_x = 1.0 / ((double)dst_w / (double)src_w);
-    p.scale_y = 1.0 / ((double)dst_h / (double)src_h);
+    p.scale_x = plan.scale_x;
+    p.scale_y = plan.scale_y;
     p.n_frames = n_frames;
-    const int fpc = bevk_resize_frames_per_chunk(n_frames, dst_h, dst_w);
-    p.frames_per_chunk = fpc;
-    const int z = (n_frames + fpc - 1) / fpc;
-    if (z > 65535) BEVK_FAIL(BEVK_E_ARG, "resize: too many frame chunks (%d) for one launch", z);
-    const dim3 grid((dst_w + 31) / 32, (dst_h + 7) / 8, z);
-    cudaStream_t st = (cudaStream_t)stream;
+    p.frames_per_chunk = plan.frames_per_chunk;
     const bool words = channels == 3 && src_w >= 2 && (src_w % 4) == 0 && (dst_w % 4) == 0 &&
                        ((uintptr_t)src % 4) == 0 && ((uintptr_t)dst % 4) == 0;
     if (words) {
-        resize_u8c3_kernel<<<grid, dim3(32, 8, 1), 0, st>>>(p);
+        resize_u8c3_kernel<<<plan.grid, dim3(32, 8, 1), 0, stream>>>(p);
     } else {
         switch (channels) {
-        case 1: launch_bytes<1>(p, grid, st); break;
-        case 2: launch_bytes<2>(p, grid, st); break;
-        case 3: launch_bytes<3>(p, grid, st); break;
-        default: launch_bytes<4>(p, grid, st); break;
+        case 1: launch_bytes<1>(p, plan.grid, stream); break;
+        case 2: launch_bytes<2>(p, plan.grid, stream); break;
+        case 3: launch_bytes<3>(p, plan.grid, stream); break;
+        default: launch_bytes<4>(p, plan.grid, stream); break;
         }
     }
     BEVK_CUDA(cudaGetLastError());

@@ -218,6 +218,9 @@ int bevk_launch_resize_area(const void *src, void *dst, int n_frames, int src_h,
                             int nv12, long long pitch, long long frame_stride, int dst_h, int dst_w,
                             cudaStream_t stream)
 {
+    BevkResizePlan plan;
+    int rc = bevk_plan_resize(n_frames, src_h, src_w, dst_h, dst_w, plan);
+    if (rc) return rc;
     AreaParams p;
     p.src = (const uint8_t *)src;
     p.dst = (uint8_t *)dst;
@@ -228,28 +231,25 @@ int bevk_launch_resize_area(const void *src, void *dst, int n_frames, int src_h,
     p.pitch = pitch;
     p.src_frame = frame_stride;
     p.dst_frame = (long long)dst_h * dst_w * channels;
-    p.inv_x = (double)dst_w / (double)src_w;
-    p.inv_y = (double)dst_h / (double)src_h;
-    p.scale_x = 1.0 / p.inv_x;
-    p.scale_y = 1.0 / p.inv_y;
+    p.inv_x = plan.inv_x;
+    p.inv_y = plan.inv_y;
+    p.scale_x = plan.scale_x;
+    p.scale_y = plan.scale_y;
     int mode = kLinear;
     p.kx = p.ky = 1;
     if (p.scale_x >= 1 && p.scale_y >= 1)
         mode = integer_scale(p.scale_x, p.kx) && integer_scale(p.scale_y, p.ky) ? kFast : kArea;
     p.inv_area = 1.f / (float)(p.kx * p.ky);
     p.n_frames = n_frames;
-    p.frames_per_chunk = bevk_resize_frames_per_chunk(n_frames, dst_h, dst_w);
-    const int z = (n_frames + p.frames_per_chunk - 1) / p.frames_per_chunk;
-    if (z > 65535) BEVK_FAIL(BEVK_E_ARG, "resize: too many frame chunks (%d) for one launch", z);
-    const dim3 grid((dst_w + 31) / 32, (dst_h + 7) / 8, z);
+    p.frames_per_chunk = plan.frames_per_chunk;
     if (nv12) {
-        launch<3, true>(p, mode, grid, stream);
+        launch<3, true>(p, mode, plan.grid, stream);
     } else {
         switch (channels) {
-        case 1: launch<1, false>(p, mode, grid, stream); break;
-        case 2: launch<2, false>(p, mode, grid, stream); break;
-        case 3: launch<3, false>(p, mode, grid, stream); break;
-        default: launch<4, false>(p, mode, grid, stream); break;
+        case 1: launch<1, false>(p, mode, plan.grid, stream); break;
+        case 2: launch<2, false>(p, mode, plan.grid, stream); break;
+        case 3: launch<3, false>(p, mode, plan.grid, stream); break;
+        default: launch<4, false>(p, mode, plan.grid, stream); break;
         }
     }
     BEVK_CUDA(cudaGetLastError());

@@ -62,6 +62,23 @@ at::Tensor host_f64(const at::Tensor &m, const char *what)
     return m.to(at::kDouble).contiguous();
 }
 
+// The matrices of a warp of n frames on the host: (K, 3, 3) float64 and the optional per-frame index
+struct WarpMats {
+    at::Tensor M, idx;
+    const int32_t *idx_ptr() const { return idx.defined() ? idx.data_ptr<int32_t>() : nullptr; }
+};
+
+WarpMats warp_mats(const at::Tensor &M, const c10::optional<at::Tensor> &mat_index, int64_t n)
+{
+    WarpMats m;
+    m.M = host_f64(M, "M").reshape({-1, 3, 3});
+    if (mat_index.has_value()) {
+        m.idx = mat_index->to(at::kCPU, at::kInt).contiguous();
+        TORCH_CHECK(m.idx.numel() == n, "mat_index has ", m.idx.numel(), " entries for ", n, " frames");
+    }
+    return m;
+}
+
 at::Tensor warp_perspective(const at::Tensor &src, const at::Tensor &M, int64_t w, int64_t h, int64_t flags,
                             int64_t border_mode, double border_val, const c10::optional<at::Tensor> &mat_index)
 {
@@ -72,19 +89,12 @@ at::Tensor warp_perspective(const at::Tensor &src, const at::Tensor &M, int64_t 
     if (src.dim() == 2) s4 = s4.unsqueeze(0).unsqueeze(-1);
     else if (src.dim() == 3) s4 = s4.unsqueeze(0);
     const int64_t n = s4.size(0), sh = s4.size(1), sw = s4.size(2), c = s4.size(3);
-    at::Tensor Ms = host_f64(M, "M").reshape({-1, 3, 3});
-    at::Tensor idx;
-    const int32_t *idx_ptr = nullptr;
-    if (mat_index.has_value()) {
-        idx = mat_index->to(at::kCPU, at::kInt).contiguous();
-        TORCH_CHECK(idx.numel() == n, "mat_index has ", idx.numel(), " entries for ", n, " frames");
-        idx_ptr = idx.data_ptr<int32_t>();
-    }
+    const WarpMats m = warp_mats(M, mat_index, n);
     at::Tensor out = at::empty({n, h, w, c}, s4.options());
     const double border[4] = {border_val, border_val, border_val, border_val};
     c10::cuda::CUDAGuard guard(src.device());
     check_rc(bevk_warp_perspective(s4.data_ptr(), out.data_ptr(), (int)n, (int)sh, (int)sw, (int)h, (int)w, (int)c,
-                                   dtype, Ms.data_ptr<double>(), (int)Ms.size(0), idx_ptr, (int)flags,
+                                   dtype, m.M.data_ptr<double>(), (int)m.M.size(0), m.idx_ptr(), (int)flags,
                                    (int)border_mode, border, current_stream(src)),
              "bevk_warp_perspective");
     if (src.dim() == 2) return out.squeeze(-1).squeeze(0);
@@ -133,20 +143,13 @@ at::Tensor warp_perspective_nv12(const at::Tensor &src, const at::Tensor &M, int
                                  const c10::optional<at::Tensor> &mat_index)
 {
     Nv12View v = nv12_view(src);
-    at::Tensor Ms = host_f64(M, "M").reshape({-1, 3, 3});
-    at::Tensor idx;
-    const int32_t *idx_ptr = nullptr;
-    if (mat_index.has_value()) {
-        idx = mat_index->to(at::kCPU, at::kInt).contiguous();
-        TORCH_CHECK(idx.numel() == v.n, "mat_index has ", idx.numel(), " entries for ", v.n, " frames");
-        idx_ptr = idx.data_ptr<int32_t>();
-    }
+    const WarpMats m = warp_mats(M, mat_index, v.n);
     at::Tensor out = at::empty({v.n, h, w, 3}, v.s3.options());
     const double border[4] = {border_val, border_val, border_val, border_val};
     c10::cuda::CUDAGuard guard(src.device());
     check_rc(bevk_warp_perspective_nv12(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w,
-                                        (int)v.pitch, v.frame_stride, (int)h, (int)w, Ms.data_ptr<double>(),
-                                        (int)Ms.size(0), idx_ptr, (int)flags, (int)border_mode, border,
+                                        (int)v.pitch, v.frame_stride, (int)h, (int)w, m.M.data_ptr<double>(),
+                                        (int)m.M.size(0), m.idx_ptr(), (int)flags, (int)border_mode, border,
                                         current_stream(src)),
              "bevk_warp_perspective_nv12");
     return src.dim() == 2 ? out.squeeze(0) : out;

@@ -22,15 +22,6 @@ template <> struct Px<float> {
     static __device__ __forceinline__ float ld(const float *p) { return __ldg(p); }
 };
 
-__device__ __forceinline__ const BevkWarpGroup &find_group(const BevkWarpParams &p, int z, int &gi)
-{
-    gi = 0;
-#pragma unroll 1
-    for (int i = 1; i < p.n_groups; ++i)
-        if (z >= p.g[i].chunk0) gi = i;
-    return p.g[gi];
-}
-
 // Second half of a split launch (BevkWarpParams::hard): is this 32x8 block's staged tile unmarked,
 // i.e. already written by the staged kernel?  Block-uniform.
 __device__ __forceinline__ bool skip_block(const BevkWarpParams &p, int gi)

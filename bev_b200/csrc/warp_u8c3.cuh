@@ -27,6 +27,16 @@ __device__ __forceinline__ uint32_t ldg_sparse(const uint32_t *p)
     return v;
 }
 
+// The (matrix, frame-run) group gi that grid z-block z of a direct-gather warp works on.
+__device__ __forceinline__ const BevkWarpGroup &find_group(const BevkWarpParams &p, int z, int &gi)
+{
+    gi = 0;
+#pragma unroll 1
+    for (int i = 1; i < p.n_groups; ++i)
+        if (z >= p.g[i].chunk0) gi = i;
+    return p.g[gi];
+}
+
 // 2-tap window along one axis: first index (clamped into the image) and the weight each of the
 // two window positions receives.  Taps outside [0, n) contribute nothing (border value 0).
 __device__ __forceinline__ void window(int s, int frac, int n, int &first, int &w0, int &w1)
