@@ -159,15 +159,9 @@ int bevk_launch_warp_fast(const BevkWarpParams &p, int channels, int dtype, int 
 int bevk_launch_warp_nv12(const BevkNv12Params &P, int linear, cudaStream_t stream);
 int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int w, int pitch,
                             long long frame_stride, cudaStream_t stream);
-// cv2.resize (INTER_LINEAR) of n_frames > 0 uint8 frames with `channels` channels; arguments
-// already checked by bevk_resize
-int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels, int dst_h,
-                       int dst_w, cudaStream_t stream);
-// cv2.resize(NV12 -> BGR) of n_frames > 0 frames; arguments already checked by bevk_resize_nv12
-int bevk_launch_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
-                            long long frame_stride, int dst_h, int dst_w, cudaStream_t stream);
-// cv2.resize(..., INTER_AREA) of n_frames > 0 frames, uint8 with `channels` channels or (nv12) NV12
-// to BGR; rows `pitch` and frames `frame_stride` bytes apart; arguments already checked
-int bevk_launch_resize_area(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels,
-                            int nv12, long long pitch, long long frame_stride, int dst_h, int dst_w,
-                            cudaStream_t stream);
+// cv2.resize of n_frames > 0 frames with `interpolation` (BEVK_INTER_LINEAR or BEVK_INTER_AREA):
+// uint8 frames with `channels` channels, or (nv12, channels 3) NV12 frames converted to BGR; rows
+// `pitch` and frames `frame_stride` bytes apart; arguments already checked by the entry points
+int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels, int nv12,
+                       long long pitch, long long frame_stride, int dst_h, int dst_w, int interpolation,
+                       cudaStream_t stream);

@@ -441,13 +441,8 @@ int resize_frames(const char *what, const void *src, void *dst, int n_frames, in
     rc = bevk_require_device();
     if (rc) return rc;
     if (n_frames == 0) return BEVK_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (interpolation == BEVK_INTER_AREA)
-        return bevk_launch_resize_area(src, dst, n_frames, src_h, src_w, channels, nv12, pitch, frame_stride, dst_h,
-                                       dst_w, st);
-    if (nv12)
-        return bevk_launch_resize_nv12(src, dst, n_frames, src_h, src_w, (int)pitch, frame_stride, dst_h, dst_w, st);
-    return bevk_launch_resize(src, dst, n_frames, src_h, src_w, channels, dst_h, dst_w, st);
+    return bevk_launch_resize(src, dst, n_frames, src_h, src_w, channels, nv12, pitch, frame_stride, dst_h, dst_w,
+                              interpolation, (cudaStream_t)stream);
 }
 }  // namespace
 

@@ -6,22 +6,16 @@
 // replicated over each 2x2 luma block; the warp equals cv2.warpPerspective of the converted frame
 // (reference frame loop vis_homo.py:85-91), i.e. every bilinear tap is converted on its own and
 // the four are then interpolated with the uint8 x 3 arithmetic of warp_u8c3.cuh.  A tap outside
-// the frame takes the BGR border colour; it is never converted from YUV.
-//
-// The resize equals cv2.resize of the converted frame with INTER_LINEAR (the small frame of
-// vis_homo.py:90): the four taps of a dst pixel are converted on their own and then interpolated
-// with the arithmetic of resize.cu.
+// the frame takes the BGR border colour; it is never converted from YUV.  The resize of NV12
+// frames is in resize.cu.
 //
 // Layout of frame n: luma rows 0..H-1 then chroma rows 0..H/2-1 (interleaved U, V bytes), each
 // row `pitch` bytes after the previous one, the frame at src + n * frame_stride bytes.
 #include "bevk_common.cuh"
-#include "resize_coef.cuh"
 #include "warp_u8c3.cuh"
 #include "yuv_bgr.cuh"
 
 namespace {
-
-__device__ __forceinline__ uint32_t byte_of(uint32_t w, int i) { return (w >> (8 * i)) & 0xffu; }
 
 __device__ __forceinline__ uint32_t border_bgr(const float *b)
 {
@@ -203,144 +197,6 @@ void launch_warp(const BevkNv12Params &P, bool packed, cudaStream_t stream)
         warp_nv12_kernel<LINEAR, WORDS, false, kBatch><<<grid, block, 0, stream>>>(P);
 }
 
-// ---- resize -----------------------------------------------------------------------------------
-struct ResizeNv12Params {
-    const uint8_t *src;
-    uint8_t *dst;
-    int src_h, src_w, dst_h, dst_w;  // luma size of a source frame; dst size
-    uint32_t pitch;                  // bytes from one luma or chroma row to the next
-    long long frame_stride, dst_frame;  // bytes from one source / dst frame to the next
-    double scale_x, scale_y;
-    int n_frames, frames_per_chunk;
-};
-
-// One lane per dst pixel, as resize_u8c3_kernel (resize.cu): the coefficients are computed once
-// per frame chunk with axis_coef, and the 2-pixel window starts inside the frame (cs = min(sx,
-// src_w - 2), weights swapped when it moved).  Every frame gathers two luma rows r0, r1 (2 bytes
-// at cs each; one row twice at the top and bottom edges) and the chroma rows r0 / 2, r1 / 2 under
-// them (4 bytes each: the U,V pairs of columns cs and cs + 1, one pair twice when cs is even),
-// converts the 4 taps on their own, then runs cv2's horizontal pass per channel as one dp2a on
-// the weight pair and its vertical pass.  WORDS and PACKED as in warp_nv12_kernel.
-// The gather is that kernel's with the second luma row at r1 instead of the next row.  It is kept
-// separate: moving it into a helper both kernels call changed the register allocation and SASS
-// of warp_nv12_kernel's bilinear variants.
-template <bool WORDS, bool PACKED, int kBatch>
-__global__ void __launch_bounds__(256) resize_nv12_kernel(const __grid_constant__ ResizeNv12Params p)
-{
-    const int lane = threadIdx.x, x0 = blockIdx.x * 32;
-    const int x = x0 + lane, y = blockIdx.y * 8 + threadIdx.y;
-    if (y >= p.dst_h) return;  // a warp is one dst row segment: uniform exit, shuffles stay legal
-    int sx, a0, a1, sy, b0, b1;
-    axis_coef(min(x, p.dst_w - 1), p.scale_x, p.src_w, true, sx, a0, a1);
-    axis_coef(y, p.scale_y, p.src_h, false, sy, b0, b1);
-    const int cs = min(sx, p.src_w - 2);
-    const int wa = cs == sx ? a0 : a1, wb = cs == sx ? a1 : a0;  // sx == src_w - 1 has a1 == 0
-    const uint32_t w16 = (uint32_t)wa | ((uint32_t)wb << 16);
-    const int r0 = min(max(sy, 0), p.src_h - 1), r1 = min(max(sy + 1, 0), p.src_h - 1);
-    const uint32_t pitch = p.pitch;
-    // byte offsets inside a frame: luma row r0 at column cs, and from it to row r1 (0 or pitch);
-    // chroma rows r0 / 2 and r1 / 2 at the U of column cs
-    const uint32_t lo = (uint32_t)r0 * pitch + (uint32_t)cs;
-    const uint32_t l1 = (uint32_t)(r1 - r0) * pitch;
-    const uint32_t cx = 2u * (uint32_t)(cs >> 1);
-    const uint32_t co = ((uint32_t)p.src_h + (uint32_t)(r0 >> 1)) * pitch + cx;
-    const uint32_t co_b = ((uint32_t)p.src_h + (uint32_t)(r1 >> 1)) * pitch + cx;
-    // the right column uses the next chroma column when cs is odd (else duplicate the one pair)
-    const uint32_t csel = (cs & 1) ? 0x3210u : 0x1010u;
-    // WORDS: the second word of a row is needed when the 2 luma / 4 chroma bytes straddle it
-    const bool l_two = (lo & 3u) == 3u;
-    const bool c_two = (co & 3u) == 2u && (cs & 1);
-
-    const int j = lane >> 2, r4 = lane & 3;
-    const uint32_t sel_pack = r4 == 0 ? 0x4210u : (r4 == 1 ? 0x5421u : 0x6542u);
-    const bool st_ok = PACKED ? (r4 < 3 && 4 * j < min(32, p.dst_w - x0)) : x < p.dst_w;
-    uint8_t *dst = p.dst + ((long long)y * p.dst_w + x0) * 3 + (PACKED ? (3 * j + r4) * 4 : 3 * lane);
-
-    constexpr int kWords = WORDS ? 8 : 4;
-    auto LD = [](const uint8_t *a) { return ldg_sparse(reinterpret_cast<const uint32_t *>(a)); };
-    auto B = [](const uint8_t *a) { return (uint32_t)__ldg(a); };
-    auto load = [&](int f, uint32_t(&w)[kWords]) {
-        const uint8_t *s = p.src + (long long)f * p.frame_stride;
-        if (WORDS) {
-            const uint8_t *la = s + (lo & ~3u), *ca = s + (co & ~3u), *cb = s + (co_b & ~3u);
-            w[0] = LD(la);
-            w[1] = l_two ? LD(la + 4) : 0u;
-            w[2] = LD(la + l1);
-            w[3] = l_two ? LD(la + l1 + 4) : 0u;
-            w[4] = LD(ca);
-            w[5] = c_two ? LD(ca + 4) : 0u;
-            w[6] = LD(cb);
-            w[7] = c_two ? LD(cb + 4) : 0u;
-        } else {
-            const uint8_t *la = s + lo, *ca = s + co, *cb = s + co_b;
-            const uint32_t cn = (cs & 1) ? 2u : 0u;  // offset of the right column's U,V pair
-            w[0] = B(la) | (B(la + 1) << 8);
-            w[1] = B(la + l1) | (B(la + l1 + 1) << 8);
-            w[2] = B(ca) | (B(ca + 1) << 8) | (B(ca + cn) << 16) | (B(ca + cn + 1) << 24);
-            w[3] = B(cb) | (B(cb + 1) << 8) | (B(cb + cn) << 16) | (B(cb + cn + 1) << 24);
-        }
-    };
-    auto finish = [&](int f, const uint32_t(&w)[kWords]) {
-        uint32_t L0, L1, C0, C1;  // [Y Y' . .] of window rows 0 / 1, [U V U' V'] under them
-        if (WORDS) {
-            L0 = __funnelshift_r(w[0], w[1], 8 * (lo & 3u));
-            L1 = __funnelshift_r(w[2], w[3], 8 * (lo & 3u));
-            C0 = prmt(__funnelshift_r(w[4], w[5], 8 * (co & 3u)), 0u, csel);
-            C1 = prmt(__funnelshift_r(w[6], w[7], 8 * (co_b & 3u)), 0u, csel);
-        } else {
-            L0 = w[0];
-            L1 = w[1];
-            C0 = w[2];
-            C1 = w[3];
-        }
-        const uint32_t p00 = yuv_to_bgr(byte_of(L0, 0), byte_of(C0, 0), byte_of(C0, 1));
-        const uint32_t p01 = yuv_to_bgr(byte_of(L0, 1), byte_of(C0, 2), byte_of(C0, 3));
-        const uint32_t p10 = yuv_to_bgr(byte_of(L1, 0), byte_of(C1, 0), byte_of(C1, 1));
-        const uint32_t p11 = yuv_to_bgr(byte_of(L1, 1), byte_of(C1, 2), byte_of(C1, 3));
-        // per window row [B B' G G'] and [R R' . .]: channel c of the horizontal pass is
-        // p[cs][c] * wa + p[cs + 1][c] * wb, one dp2a on the low or high byte pair
-        const uint32_t xa = prmt(p00, p01, 0x5140u), ya = prmt(p00, p01, 0x0062u);
-        const uint32_t xb = prmt(p10, p11, 0x5140u), yb = prmt(p10, p11, 0x0062u);
-        const int s00 = __dp2a_lo(w16, xa, 0u), s01 = __dp2a_hi(w16, xa, 0u), s02 = __dp2a_lo(w16, ya, 0u);
-        const int s10 = __dp2a_lo(w16, xb, 0u), s11 = __dp2a_hi(w16, xb, 0u), s12 = __dp2a_lo(w16, yb, 0u);
-        const uint32_t P0 = vpass(b0, b1, s00, s10) | (vpass(b0, b1, s01, s11) << 8) | (vpass(b0, b1, s02, s12) << 16);
-        uint8_t *d = dst + (long long)f * p.dst_frame;
-        if (PACKED) {
-            const uint32_t word = prmt(P0, __shfl_down_sync(0xffffffffu, P0, 1), sel_pack);
-            if (st_ok) st_stream_free(reinterpret_cast<uint32_t *>(d), word);
-        } else if (st_ok) {
-            d[0] = (uint8_t)P0;
-            d[1] = (uint8_t)(P0 >> 8);
-            d[2] = (uint8_t)(P0 >> 16);
-        }
-    };
-    // the windows of kBatch frames are requested before the first one is converted
-    const int f0 = blockIdx.z * p.frames_per_chunk, f1 = min(f0 + p.frames_per_chunk, p.n_frames);
-    int f = f0;
-    for (; f + kBatch <= f1; f += kBatch) {
-        uint32_t w[kBatch][kWords];
-#pragma unroll
-        for (int u = 0; u < kBatch; ++u) load(f + u, w[u]);
-#pragma unroll
-        for (int u = 0; u < kBatch; ++u) finish(f + u, w[u]);
-    }
-    for (; f < f1; ++f) {
-        uint32_t w[kWords];
-        load(f, w);
-        finish(f, w);
-    }
-}
-
-template <bool WORDS>
-void launch_resize(const ResizeNv12Params &p, bool packed, dim3 grid, cudaStream_t stream)
-{
-    constexpr int kBatch = 2;
-    if (packed)
-        resize_nv12_kernel<WORDS, true, kBatch><<<grid, dim3(32, 8, 1), 0, stream>>>(p);
-    else
-        resize_nv12_kernel<WORDS, false, kBatch><<<grid, dim3(32, 8, 1), 0, stream>>>(p);
-}
-
 // ---- conversion -------------------------------------------------------------------------------
 // A thread owns a 2x2 luma block and its one U,V pair, for kRowPairs block rows 4 apart (all
 // loads issued before the first conversion); a warp covers 64 columns, i.e. 64 luma bytes per
@@ -457,33 +313,6 @@ int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int
               n_frames < 65535 ? n_frames : 65535);
     nv12_to_bgr_kernel<<<grid, block, 0, stream>>>((const uint8_t *)src, (uint8_t *)dst, n_frames, h, w, pitch,
                                                    frame_stride);
-    BEVK_CUDA(cudaGetLastError());
-    return BEVK_OK;
-}
-
-int bevk_launch_resize_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
-                            long long frame_stride, int dst_h, int dst_w, cudaStream_t stream)
-{
-    BevkResizePlan plan;
-    int rc = bevk_plan_resize(n_frames, src_h, src_w, dst_h, dst_w, plan);
-    if (rc) return rc;
-    ResizeNv12Params p;
-    p.src = (const uint8_t *)src;
-    p.dst = (uint8_t *)dst;
-    p.src_h = src_h;
-    p.src_w = src_w;
-    p.dst_h = dst_h;
-    p.dst_w = dst_w;
-    p.pitch = (uint32_t)pitch;
-    p.frame_stride = frame_stride;
-    p.dst_frame = (long long)dst_h * dst_w * 3;
-    p.scale_x = plan.scale_x;
-    p.scale_y = plan.scale_y;
-    p.n_frames = n_frames;
-    p.frames_per_chunk = plan.frames_per_chunk;
-    const bool words = ((uintptr_t)src % 4) == 0 && (pitch % 4) == 0 && (frame_stride % 4) == 0;
-    const bool packed = (dst_w % 4) == 0 && ((uintptr_t)dst % 4) == 0;
-    words ? launch_resize<true>(p, packed, plan.grid, stream) : launch_resize<false>(p, packed, plan.grid, stream);
     BEVK_CUDA(cudaGetLastError());
     return BEVK_OK;
 }

@@ -1,10 +1,12 @@
 // yuv_bgr.cuh -- one NV12 sample to BGR, cv2.cvtColor(COLOR_YUV2BGR_NV12)'s arithmetic (BT.601
-// limited range, 20-bit fixed point), shared by the NV12 kernels (nv12.cu) and the NV12 area
-// resize (resize_area.cu).
+// limited range, 20-bit fixed point), shared by the NV12 conversion and warp (nv12.cu) and the NV12
+// resizes (resize.cu).
 #pragma once
 #include "bevk_common.cuh"
 
 namespace {
+
+__device__ __forceinline__ uint32_t byte_of(uint32_t w, int i) { return (w >> (8 * i)) & 0xffu; }
 
 __device__ __forceinline__ int clamp8(int v) { return min(max(v, 0), 255); }
 

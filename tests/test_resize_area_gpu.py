@@ -1,5 +1,5 @@
 """GPU: cv2.resize(..., interpolation=cv2.INTER_AREA) through homo.resize and homo.resize_nv12
-(csrc/resize_area.cu) against the oracle (oracle/resize_area_oracle.py, pinned to cv2 4.13), live
+(csrc/resize.cu) against the oracle (oracle/resize_area_oracle.py, pinned to cv2 4.13), live
 cv2 where it is installed, and the committed cv2 hashes of tests/golden/resize_area_hash.json.
 Every comparison is bit for bit."""
 import numpy as np
@@ -80,15 +80,19 @@ def test_cv2_hashes(case):
         assert util.sha256(bev.cpu().numpy()) == case["sha256_bev"]
 
 
-# one shape per branch: (src h, w), dsize
-BRANCH_SHAPES = {"fast": ((96, 130), (65, 32)), "area": ((96, 130), (57, 41)), "linear": ((40, 62), (97, 30))}
+# one shape per branch: (src h, w), dsize.  The upscaling branch runs the bilinear kernels: with
+# src_w % 4 == 2 the byte gathers; with src_w and dst_w multiples of 4 ("words") the BGR word-gather
+# kernel and the NV12 word-gather one with packed stores; and with dst_w % 4 == 2 the NV12
+# word-gather one with unpacked stores.
+BRANCH_SHAPES = {"fast": ((96, 130), (65, 32)), "area": ((96, 130), (57, 41)), "linear": ((40, 62), (97, 30)),
+                 "linear_words": ((40, 64), (96, 30)), "linear_words_unpacked": ((40, 64), (98, 52))}
 
 
 @pytest.mark.parametrize("branch", sorted(BRANCH_SHAPES))
 @pytest.mark.parametrize("channels", [1, 2, 3, 4, "nv12"])
 def test_every_kernel_variant(branch, channels):
     (h, w), dsize = BRANCH_SHAPES[branch]
-    assert ra.branch((w, h), dsize) == branch
+    assert ra.branch((w, h), dsize) == branch.split("_")[0]
     rng = np.random.default_rng([7, h, w, dsize[0]])
     if channels == "nv12":
         frames = rng.integers(0, 256, (3, h * 3 // 2, w), dtype=np.uint8)

@@ -1,4 +1,4 @@
-"""GPU: the NV12 resize (csrc/nv12.cu, resize_nv12_kernel) against the composed oracle
+"""GPU: the NV12 resize (csrc/resize.cu, resize_nv12_kernel) against the composed oracle
 (oracle/resize_nv12_oracle.py, pinned to cv2 4.13), the committed cv2 hashes of
 tests/golden/nv12_resize_hash.json and the two-pass route nv12_to_bgr + resize.  Every comparison
 is bit for bit."""

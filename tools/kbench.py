@@ -435,14 +435,14 @@ def resize_nv12_bench(rounds=5):
 
 
 AREA_WORKLOADS = ((256, (1080, 1920), (852, 480)), (256, (1080, 1920), (960, 540)),
-                  (64, (2160, 3840), (1920, 1080)))
+                  (64, (2160, 3840), (1920, 1080)), (256, (480, 852), (1920, 1080)))
 
 
 def resize_area_bench(rounds=5):
     """INTER_AREA resize of BGR frames against the INTER_LINEAR kernel on the same shapes,
-    alternating the two in one process.  Algorithmic bytes: 3 x (touched source pixels + dst
-    pixels); a downscale touches the whole frame.  Every frame set is larger than the 126 MB L2.
-    Frame 0 of the area route is checked against the oracle."""
+    alternating the two in one process; the last shape upscales.  Algorithmic bytes: 3 x (touched
+    source pixels + dst pixels); a downscale touches the whole frame.  Every frame set is larger
+    than the 126 MB L2.  Frame 0 of the area route is checked against the oracle."""
     from oracle import resize_area_oracle
     print("card: %s" % card(), flush=True)
     peak, src = bench.measured_peak()
