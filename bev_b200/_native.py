@@ -44,6 +44,12 @@ SIGNATURES = {
     "bevk_nv12_to_bgr": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _vp]),
     "bevk_warp_perspective_nv12": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int,
                                             _dp, _c_int, _i32p, _c_int, _c_int, _dp, _vp]),
+    "bevk_bgr_to_yuv420": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_int, _c_i64, _vp]),
+    "bevk_warp_perspective_yuv420": (_c_int, [_vp, _vp] + [_c_int] * 6 + [_c_int, _c_i64, _dp, _c_int, _i32p, _c_int,
+                                                                          _c_int, _dp, _vp]),
+    "bevk_warp_perspective_nv12_yuv420": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int,
+                                                   _c_int, _c_int, _c_i64, _dp, _c_int, _i32p, _c_int, _c_int, _dp,
+                                                   _vp]),
     "bevk_resize": (_c_int, [_vp, _vp] + [_c_int] * 8 + [_vp]),
     "bevk_resize_nv12": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int, _vp]),
     "bevk_resize_nv12_interp": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int, _c_int,
@@ -326,6 +332,100 @@ def warp_perspective_nv12(src, M, dsize, dst=None, flags=1, borderMode=0, border
             idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags), int(borderMode), _dptr(b),
             _stream_ptr(src))
     _check(rc, "bevk_warp_perspective_nv12")
+    return dst
+
+
+YUV_LAYOUTS = {"i420": 0, "nv12": 1}
+
+
+def _yuv_layout(layout):
+    code = YUV_LAYOUTS.get(layout)
+    if code is None:
+        raise ValueError("layout must be 'i420' or 'nv12', got %r" % (layout,))
+    return code
+
+
+def _yuv_dst(dst, n, h, w, batched, device):
+    """(frames view (N, H*3/2, W), pitch, frame stride) of a new or given YUV 4:2:0 dst of n frames of
+    h x w: (H*3/2, W) or (N, H*3/2, W) uint8.  Pitch and frame stride come from the tensor's strides,
+    so an encoder surface with padded rows is written as it is."""
+    import torch
+    if h % 2 or w % 2:
+        raise ValueError("YUV 4:2:0 frames need an even width and height, got %dx%d" % (w, h))
+    shape = (n, h * 3 // 2, w) if batched else (h * 3 // 2, w)
+    if dst is None:
+        dst = torch.empty(shape, dtype=torch.uint8, device=device)
+    _require_cuda(dst, "dst")
+    if tuple(dst.shape) != shape or dst.dtype != torch.uint8 or dst.device != device:
+        raise ValueError("dst must be a uint8 tensor of shape %s on %s, got %s %s on %s"
+                         % (shape, device, dst.dtype, tuple(dst.shape), dst.device))
+    d3 = dst if batched else dst[None]
+    if d3.stride(2) != 1 or d3.stride(1) < w:
+        raise ValueError("dst rows must be contiguous and at least %d bytes apart, got strides %s"
+                         % (w, tuple(d3.stride())))
+    pitch = d3.stride(1)
+    return dst, d3, pitch, d3.stride(0) if n > 1 else pitch * (h * 3 // 2)
+
+
+def bgr_to_yuv420(src, layout="i420", dst=None):
+    """cv2.cvtColor(f, COLOR_BGR2YUV_I420) (layout "i420") or its NV12 relayout ("nv12") on CUDA
+    uint8 BGR frames (H, W, 3) or (N, H, W, 3) -> (H*3/2, W) or (N, H*3/2, W)."""
+    import torch
+    _require_cuda(src, "src")
+    if src.dtype != torch.uint8 or src.dim() not in (3, 4) or src.shape[-1] != 3:
+        raise ValueError("src must be uint8 (H, W, 3) or (N, H, W, 3), got %s %s" % (src.dtype, tuple(src.shape)))
+    code = _yuv_layout(layout)
+    s4 = (src[None] if src.dim() == 3 else src).contiguous()
+    n, h, w, _ = s4.shape
+    dst, d3, pitch, fstride = _yuv_dst(dst, n, h, w, src.dim() == 4, src.device)
+    with torch.cuda.device(src.device):
+        rc = lib().bevk_bgr_to_yuv420(_vp(s4.data_ptr()), _vp(d3.data_ptr()), n, h, w, code, pitch, fstride,
+                                      _stream_ptr(src))
+    _check(rc, "bevk_bgr_to_yuv420")
+    return dst
+
+
+def warp_perspective_yuv420(src, M, dsize, layout="i420", dst=None, flags=1, borderMode=0, borderValue=0,
+                            mat_index=None):
+    """bgr_to_yuv420(warp_perspective(src, M, dsize, ...), layout) in one pass: CUDA uint8 BGR
+    frames (H, W, 3) or (N, H, W, 3) -> (h*3/2, w) or (N, h*3/2, w)."""
+    import torch
+    _require_cuda(src, "src")
+    if src.dtype != torch.uint8 or src.dim() not in (3, 4) or src.shape[-1] != 3:
+        raise ValueError("src must be uint8 (H, W, 3) or (N, H, W, 3), got %s %s" % (src.dtype, tuple(src.shape)))
+    code = _yuv_layout(layout)
+    s4 = (src[None] if src.dim() == 3 else src).contiguous()
+    n, h, w, _ = s4.shape
+    dw, dh = int(dsize[0]), int(dsize[1])
+    Ms, idx = _prep_mats(M, n, mat_index)
+    dst, d3, pitch, fstride = _yuv_dst(dst, n, dh, dw, src.dim() == 4, src.device)
+    b = _border(borderValue)
+    with torch.cuda.device(src.device):
+        rc = lib().bevk_warp_perspective_yuv420(
+            _vp(s4.data_ptr()), _vp(d3.data_ptr()), n, h, w, dh, dw, code, pitch, fstride, _dptr(Ms), Ms.shape[0],
+            idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags), int(borderMode), _dptr(b),
+            _stream_ptr(src))
+    _check(rc, "bevk_warp_perspective_yuv420")
+    return dst
+
+
+def warp_perspective_nv12_yuv420(src, M, dsize, layout="i420", dst=None, flags=1, borderMode=0, borderValue=0,
+                                 mat_index=None):
+    """bgr_to_yuv420(warp_perspective_nv12(src, M, dsize, ...), layout) in one pass: CUDA uint8 NV12
+    frames (H*3/2, W) or (N, H*3/2, W), any pitch and frame stride -> (h*3/2, w) or (N, h*3/2, w)."""
+    import torch
+    s3, n, h, w, pitch, fstride = _nv12_frames(src)
+    code = _yuv_layout(layout)
+    dw, dh = int(dsize[0]), int(dsize[1])
+    Ms, idx = _prep_mats(M, n, mat_index)
+    dst, d3, dpitch, dfstride = _yuv_dst(dst, n, dh, dw, src.dim() == 3, src.device)
+    b = _border(borderValue)
+    with torch.cuda.device(src.device):
+        rc = lib().bevk_warp_perspective_nv12_yuv420(
+            _vp(s3.data_ptr()), _vp(d3.data_ptr()), n, h, w, pitch, fstride, dh, dw, code, dpitch, dfstride,
+            _dptr(Ms), Ms.shape[0], idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags),
+            int(borderMode), _dptr(b), _stream_ptr(src))
+    _check(rc, "bevk_warp_perspective_nv12_yuv420")
     return dst
 
 

@@ -146,6 +146,16 @@ struct BevkNv12Params {
     long long frame_stride;  // bytes from one frame to the next
 };
 
+// The warps to YUV 4:2:0 (yuv420.cu): w.dst is frame 0's first luma byte, w.src_frame_elems and
+// w.dst_frame_elems are unused; BGR sources have pitch = 3 * src_w and frame_stride = pitch * src_h.
+struct BevkYuvParams {
+    BevkWarpParams w;
+    int pitch;                   // source bytes from one (luma or chroma) row to the next
+    long long frame_stride;      // source bytes from one frame to the next
+    int dst_pitch;               // dst bytes from one luma or chroma row to the next
+    long long dst_frame_stride;  // dst bytes from one frame to the next
+};
+
 // kernels-side entry points implemented in the .cu files
 int bevk_launch_warp_generic(const BevkWarpParams &p, int channels, int dtype, int linear,
                              cudaStream_t stream);
@@ -165,3 +175,9 @@ int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int
 int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels, int nv12,
                        long long pitch, long long frame_stride, int dst_h, int dst_w, int interpolation,
                        cudaStream_t stream);
+// BGR (nv12_src 0) or NV12 frames warped to YUV 4:2:0 (nv12_out: NV12, else I420) over the chunks
+// planned for P.w on the grid of 2x2 dst blocks
+int bevk_launch_warp_yuv420(const BevkYuvParams &P, int nv12_src, int nv12_out, int linear, cudaStream_t stream);
+// n_frames > 0 contiguous BGR frames of h x w (both even) to YUV 4:2:0 (nv12_out: NV12, else I420)
+int bevk_launch_bgr_to_yuv420(const void *src, void *dst, int n_frames, int h, int w, int nv12_out, int dst_pitch,
+                              long long dst_frame_stride, cudaStream_t stream);

@@ -444,6 +444,55 @@ int resize_frames(const char *what, const void *src, void *dst, int n_frames, in
     return bevk_launch_resize(src, dst, n_frames, src_h, src_w, channels, nv12, pitch, frame_stride, dst_h, dst_w,
                               interpolation, (cudaStream_t)stream);
 }
+// The YUV 4:2:0 destinations (I420 or NV12 frames of h x w): even sizes, rows at least w bytes
+// apart, in-frame offsets below 4 GB.
+int check_yuv420_dst(const char *what, int n_frames, int h, int w, int layout, int pitch, int64_t frame_stride)
+{
+    if (layout != BEVK_YUV_I420 && layout != BEVK_YUV_NV12)
+        BEVK_FAIL(BEVK_E_ARG, "%s: layout must be BEVK_YUV_I420 (0) or BEVK_YUV_NV12 (1), got %d", what, layout);
+    if (h <= 0 || w <= 0 || (h % 2) != 0 || (w % 2) != 0)
+        BEVK_FAIL(BEVK_E_ARG, "%s: YUV 4:2:0 frames need an even, positive width and height (got %dx%d)", what, w, h);
+    return check_nv12_layout32(what, n_frames, h, w, pitch, frame_stride);
+}
+
+// The fused warps to YUV 4:2:0 after their source-layout checks: BGR (nv12 0, contiguous frames)
+// or NV12 frames, rows `pitch` and frames `frame_stride` bytes apart.
+int warp_yuv420(const char *what, const void *src, void *dst, int n_frames, int src_h, int src_w, int nv12,
+                long long pitch, long long frame_stride, int dst_h, int dst_w, int layout, int dst_pitch,
+                int64_t dst_frame_stride, const double *M, int n_mats, const int32_t *mat_index, int flags,
+                int border_mode, const double *border_value, void *stream)
+{
+    int rc = check_yuv420_dst(what, n_frames, dst_h, dst_w, layout, dst_pitch, dst_frame_stride);
+    if (rc) return rc;
+    WarpArgs a;
+    rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index, flags,
+                         border_mode, border_value, a);
+    if (rc) return rc;
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    std::vector<double> maps;
+    effective_maps(M, n_mats, flags, maps);
+    std::vector<BevkWarpGroup> groups;
+    build_groups(n_frames, n_mats, mat_index, maps, groups);
+
+    BevkYuvParams P;
+    memset(&P, 0, sizeof(P));
+    P.pitch = (int)pitch;
+    P.frame_stride = frame_stride;
+    P.dst_pitch = dst_pitch;
+    P.dst_frame_stride = dst_frame_stride;
+    return launch_warp_groups(P.w, src, dst, a, groups, [&]() {
+        // a thread owns a 2x2 dst block: plan the frame chunks over the grid of blocks
+        P.w.dst_w /= 2;
+        P.w.dst_h /= 2;
+        const int rc = bevk_plan_generic_chunks(P.w, 3);
+        P.w.dst_w *= 2;
+        P.w.dst_h *= 2;
+        if (rc) return rc;
+        return bevk_launch_warp_yuv420(P, nv12, layout == BEVK_YUV_NV12, a.linear, (cudaStream_t)stream);
+    });
+}
 }  // namespace
 
 extern "C" {
@@ -488,6 +537,43 @@ int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src
         if (rc) return rc;
         return bevk_launch_warp_nv12(P, a.linear, (cudaStream_t)stream);
     });
+}
+
+int bevk_bgr_to_yuv420(const void *src, void *dst, int n_frames, int h, int w, int layout, int dst_pitch,
+                       int64_t dst_frame_stride, void *stream)
+{
+    int rc = check_yuv420_dst("bgr_to_yuv420", n_frames, h, w, layout, dst_pitch, dst_frame_stride);
+    if (rc) return rc;
+    if (w > 32767 || h > 32767) BEVK_FAIL(BEVK_E_ARG, "bgr_to_yuv420: sizes above 32767 are not supported");
+    if (n_frames > 0 && (!src || !dst)) BEVK_FAIL(BEVK_E_ARG, "bgr_to_yuv420: null src / dst");
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    return bevk_launch_bgr_to_yuv420(src, dst, n_frames, h, w, layout == BEVK_YUV_NV12, dst_pitch, dst_frame_stride,
+                                     (cudaStream_t)stream);
+}
+
+int bevk_warp_perspective_yuv420(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
+                                 int dst_w, int layout, int dst_pitch, int64_t dst_frame_stride, const double *M,
+                                 int n_mats, const int32_t *mat_index, int flags, int border_mode,
+                                 const double *border_value, void *stream)
+{
+    return warp_yuv420("warp_yuv420", src, dst, n_frames, src_h, src_w, 0, 3LL * src_w, 3LL * src_w * src_h, dst_h,
+                       dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index, flags, border_mode,
+                       border_value, stream);
+}
+
+int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                                      int64_t frame_stride, int dst_h, int dst_w, int layout, int dst_pitch,
+                                      int64_t dst_frame_stride, const double *M, int n_mats,
+                                      const int32_t *mat_index, int flags, int border_mode,
+                                      const double *border_value, void *stream)
+{
+    const int rc = check_nv12_layout32("warp_nv12_yuv420", n_frames, src_h, src_w, pitch, frame_stride);
+    if (rc) return rc;
+    return warp_yuv420("warp_nv12_yuv420", src, dst, n_frames, src_h, src_w, 1, pitch, frame_stride, dst_h, dst_w,
+                       layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index, flags, border_mode, border_value,
+                       stream);
 }
 
 int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h, int dst_w, int channels,

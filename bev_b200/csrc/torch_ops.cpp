@@ -11,6 +11,10 @@
 //   torch.ops.bev_cuda.warp_perspective_nv12(Tensor src, Tensor M, int w, int h, int flags, int border_mode,
 //                                            float border_val, Tensor? mat_index) -> Tensor
 //   torch.ops.bev_cuda.resize_nv12(Tensor src, int w, int h, int interpolation=1) -> Tensor
+//   torch.ops.bev_cuda.bgr_to_yuv420(Tensor src, int layout=0) -> Tensor
+//   torch.ops.bev_cuda.warp_perspective_yuv420(Tensor src, Tensor M, int w, int h, int layout=0, int flags=1,
+//                                              int border_mode=0, float border_val=0., Tensor? mat_index=None)
+//                                              -> Tensor
 //
 // Every implementation only checks tensors, allocates the result with torch's caching allocator,
 // takes the current CUDA stream and calls the extern "C" entry point of include/bev_b200.h with raw
@@ -22,7 +26,8 @@
 // (bev/rbox.py:136-151), rbox_torch.xywhr2xyxy (bev/rbox_torch.py:52-99) + the projection of
 // rbox_vis.py:38-55, rbox.xy82xywhr (bev/rbox.py:50-63), rbox_torch.rbox_world_bev (:123-168); the NV12
 // operators serve the frame loop of vis_homo.py:85-91 with frames from a GPU video decoder
-// (resize_nv12: its small-frame copy, vis_homo.py:90).
+// (resize_nv12: its small-frame copy, vis_homo.py:90); the YUV 4:2:0 operators serve its
+// VideoWriter.write (vis_homo.py:110-111) with frames for a video encoder.
 #include <ATen/ATen.h>
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
@@ -166,6 +171,52 @@ at::Tensor resize_nv12(const at::Tensor &src, int64_t w, int64_t h, int64_t inte
     return src.dim() == 2 ? out.squeeze(0) : out;
 }
 
+// BGR frames (H, W, 3) or (N, H, W, 3) uint8, contiguous
+at::Tensor bgr_frames(const at::Tensor &src)
+{
+    TORCH_CHECK(src.is_cuda(), "src must be a CUDA tensor");
+    TORCH_CHECK(src.scalar_type() == at::kByte, "BGR frames are uint8, got ", src.scalar_type());
+    TORCH_CHECK((src.dim() == 3 || src.dim() == 4) && src.size(-1) == 3, "src must be (H, W, 3) or (N, H, W, 3)");
+    return (src.dim() == 3 ? src.unsqueeze(0) : src).contiguous();
+}
+
+// (N, h*3/2, w) contiguous YUV 4:2:0 frames, squeezed back for an unbatched src
+at::Tensor yuv420_out(const at::Tensor &s4, int64_t h, int64_t w)
+{
+    TORCH_CHECK(h % 2 == 0 && w % 2 == 0, "YUV 4:2:0 frames need an even width and height, got ", w, "x", h);
+    return at::empty({s4.size(0), h / 2 * 3, w}, s4.options());
+}
+
+at::Tensor bgr_to_yuv420(const at::Tensor &src, int64_t layout)
+{
+    const at::Tensor s4 = bgr_frames(src);
+    const int64_t n = s4.size(0), h = s4.size(1), w = s4.size(2);
+    at::Tensor out = yuv420_out(s4, h, w);
+    c10::cuda::CUDAGuard guard(src.device());
+    check_rc(bevk_bgr_to_yuv420(s4.data_ptr(), out.data_ptr(), (int)n, (int)h, (int)w, (int)layout, (int)w,
+                                w * (h / 2 * 3), current_stream(src)),
+             "bevk_bgr_to_yuv420");
+    return src.dim() == 3 ? out.squeeze(0) : out;
+}
+
+at::Tensor warp_perspective_yuv420(const at::Tensor &src, const at::Tensor &M, int64_t w, int64_t h, int64_t layout,
+                                   int64_t flags, int64_t border_mode, double border_val,
+                                   const c10::optional<at::Tensor> &mat_index)
+{
+    const at::Tensor s4 = bgr_frames(src);
+    const int64_t n = s4.size(0);
+    const WarpMats m = warp_mats(M, mat_index, n);
+    at::Tensor out = yuv420_out(s4, h, w);
+    const double border[4] = {border_val, border_val, border_val, border_val};
+    c10::cuda::CUDAGuard guard(src.device());
+    check_rc(bevk_warp_perspective_yuv420(s4.data_ptr(), out.data_ptr(), (int)n, (int)s4.size(1), (int)s4.size(2),
+                                          (int)h, (int)w, (int)layout, (int)w, w * (h / 2 * 3),
+                                          m.M.data_ptr<double>(), (int)m.M.size(0), m.idx_ptr(), (int)flags,
+                                          (int)border_mode, border, current_stream(src)),
+             "bevk_warp_perspective_yuv420");
+    return src.dim() == 3 ? out.squeeze(0) : out;
+}
+
 // rows (N, in_cols) -> (N, out_cols) through fn(in, out, n, ..., stream)
 template <typename FN> at::Tensor rows(const at::Tensor &x, int64_t in_cols, int64_t out_cols, FN fn, const char *what)
 {
@@ -227,6 +278,9 @@ TORCH_LIBRARY(bev_cuda, m)
     m.def("warp_perspective_nv12(Tensor src, Tensor M, int w, int h, int flags=1, int border_mode=0, "
           "float border_val=0., Tensor? mat_index=None) -> Tensor");
     m.def("resize_nv12(Tensor src, int w, int h, int interpolation=1) -> Tensor");
+    m.def("bgr_to_yuv420(Tensor src, int layout=0) -> Tensor");
+    m.def("warp_perspective_yuv420(Tensor src, Tensor M, int w, int h, int layout=0, int flags=1, "
+          "int border_mode=0, float border_val=0., Tensor? mat_index=None) -> Tensor");
 }
 
 TORCH_LIBRARY_IMPL(bev_cuda, CUDA, m)
@@ -239,4 +293,6 @@ TORCH_LIBRARY_IMPL(bev_cuda, CUDA, m)
     m.impl("nv12_to_bgr", &nv12_to_bgr);
     m.impl("warp_perspective_nv12", &warp_perspective_nv12);
     m.impl("resize_nv12", &resize_nv12);
+    m.impl("bgr_to_yuv420", &bgr_to_yuv420);
+    m.impl("warp_perspective_yuv420", &warp_perspective_yuv420);
 }

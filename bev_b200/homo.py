@@ -19,6 +19,7 @@ INTER_AREA = 3
 WARP_INVERSE_MAP = 16
 BORDER_CONSTANT = 0
 COLOR_YUV2BGR_NV12 = 91
+COLOR_BGR2YUV_I420 = 128
 
 
 # ----------------------------------------------------------------------------- host geometry
@@ -259,6 +260,52 @@ def warp_nv12_img_to_bev(frames, calib, bspec, flags=INTER_LINEAR):
     """:func:`warp_img_to_bev` for NV12 frames from a GPU video decoder (vis_homo.py:61-63,89)."""
     H = compose_H_bev_img(calib, bspec)
     return warp_perspective_nv12(frames, H, (int(bspec.u_size), int(bspec.v_size)), flags=flags)
+
+
+def bgr_to_yuv420(src, layout="i420", dst=None):
+    """Drop-in for ``cv2.cvtColor(f, cv2.COLOR_BGR2YUV_I420)`` on CUDA tensors, batched: the colour
+    conversion a video writer does to every BEV (vis_homo.py:110-111), on the GPU, so that 1.5
+    instead of 3 bytes per pixel leave it.  src (H, W, 3) or (N, H, W, 3) uint8 BGR with H and W
+    even; returns (H*3/2, W) or (N, H*3/2, W) uint8, byte-identical to cv2 4.13 for layout "i420"
+    (libx264 / PyAV ``yuv420p``), or the same Y rows followed by H/2 rows of interleaved U, V for
+    layout "nv12" (what GPU encoders take).  ``dst`` may have padded rows (a row stride, the
+    encoder's pitch, larger than W) and frames that lie apart: it is written in place, the padding
+    is left as it is."""
+    return _native.bgr_to_yuv420(src, layout, dst)
+
+
+def warp_perspective_yuv420(src, M, dsize, layout="i420", dst=None, flags=INTER_LINEAR,
+                            borderMode=BORDER_CONSTANT, borderValue=0, mat_index=None):
+    """``bgr_to_yuv420(warp_perspective(src, M, dsize, ...), layout)`` in one pass, without the BGR
+    BEV: byte-identical to ``cv2.cvtColor(cv2.warpPerspective(f, M, dsize, flags=flags,
+    borderValue=borderValue), COLOR_BGR2YUV_I420)`` (or its NV12 relayout).  src (H, W, 3) or
+    (N, H, W, 3) uint8 BGR; M, mat_index, flags and borderValue (B, G, R) as for
+    :func:`warp_perspective`; dsize = (w, h), both even; dst as for :func:`bgr_to_yuv420`.  Returns
+    (h*3/2, w) or (N, h*3/2, w) uint8; the kernel is launched asynchronously on the current CUDA
+    stream."""
+    return _native.warp_perspective_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index)
+
+
+def warp_perspective_nv12_yuv420(src, M, dsize, layout="i420", dst=None, flags=INTER_LINEAR,
+                                 borderMode=BORDER_CONSTANT, borderValue=0, mat_index=None):
+    """:func:`warp_perspective_yuv420` of NV12 frames from a GPU video decoder (src as for
+    :func:`nv12_to_bgr`): decoder frames to encoder frames in one pass, byte-identical to
+    ``cv2.cvtColor(cv2.warpPerspective(cv2.cvtColor(f, COLOR_YUV2BGR_NV12), M, dsize, ...),
+    COLOR_BGR2YUV_I420)`` (or its NV12 relayout)."""
+    return _native.warp_perspective_nv12_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue,
+                                                mat_index)
+
+
+def warp_img_to_bev_yuv420(frames, calib, bspec, layout="i420", flags=INTER_LINEAR):
+    """:func:`warp_img_to_bev` with YUV 4:2:0 BEVs for a video encoder (vis_homo.py:61-63,89,110-111)."""
+    H = compose_H_bev_img(calib, bspec)
+    return warp_perspective_yuv420(frames, H, (int(bspec.u_size), int(bspec.v_size)), layout, flags=flags)
+
+
+def warp_nv12_img_to_bev_yuv420(frames, calib, bspec, layout="i420", flags=INTER_LINEAR):
+    """:func:`warp_nv12_img_to_bev` with YUV 4:2:0 BEVs for a video encoder (vis_homo.py:61-63,89,110-111)."""
+    H = compose_H_bev_img(calib, bspec)
+    return warp_perspective_nv12_yuv420(frames, H, (int(bspec.u_size), int(bspec.v_size)), layout, flags=flags)
 
 
 def warp_bev_to_img(bev_frames, calib, bspec, flags=INTER_LINEAR):

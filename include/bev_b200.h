@@ -32,6 +32,10 @@ extern "C" {
 /* border_mode: cv2.BORDER_CONSTANT (the only mode any reference call site uses) */
 #define BEVK_BORDER_CONSTANT 0
 
+/* YUV 4:2:0 frame layouts (bevk_bgr_to_yuv420 and the warps to YUV) */
+#define BEVK_YUV_I420 0 /* cv2.COLOR_BGR2YUV_I420's: Y plane, U plane, V plane (libx264 / PyAV yuv420p) */
+#define BEVK_YUV_NV12 1 /* Y plane, then rows of interleaved U, V (what GPU video encoders take) */
+
 /* element types */
 #define BEVK_U8 0
 #define BEVK_F16 1
@@ -135,6 +139,53 @@ int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src
                                int pitch, int64_t frame_stride, int dst_h, int dst_w,
                                const double *M, int n_mats, const int32_t *mat_index, int flags,
                                int border_mode, const double *border_value, void *stream);
+
+/*
+ * BGR frames to YUV 4:2:0 for a video encoder: dst[i] is byte-identical to
+ *     cv2.cvtColor(src[i], cv2.COLOR_BGR2YUV_I420)
+ * (cv2 4.13: BT.601 limited range; U and V of each 2x2 block from its top-left pixel), or its NV12
+ * relayout.  Replaces the colour conversion the VideoWriter.write of vis_homo.py:110-111 does on
+ * the CPU for every BEV, so that 1.5 instead of 3 bytes per pixel leave the GPU.
+ *   src  [n_frames][h][w][3] contiguous uint8 BGR, h and w even (1..32767)
+ *   dst  device buffer; frame n starts at dst + n * dst_frame_stride bytes and holds h luma rows
+ *        then h / 2 chroma rows, each row dst_pitch bytes after the previous one (dst_pitch >= w);
+ *        bytes of a row past w are not written.  layout BEVK_YUV_NV12: chroma row r is the U, V
+ *        pairs of block row r.  BEVK_YUV_I420: the U plane then the V plane, each (h/2) x (w/2),
+ *        packed row-major into the chroma rows as cv2 packs them (U row r at chroma row r / 2,
+ *        column (r % 2) * w / 2); with dst_pitch = w and dst_frame_stride = w * h * 3 / 2 that is
+ *        cv2's (h * 3 / 2, w) array.  A frame must span less than 4 GB.
+ */
+int bevk_bgr_to_yuv420(const void *src, void *dst, int n_frames, int h, int w, int layout, int dst_pitch,
+                       int64_t dst_frame_stride, void *stream);
+
+/*
+ * Perspective warp of BGR frames straight to YUV 4:2:0 BEVs: dst[i] is byte-identical to
+ *     cv2.cvtColor(cv2.warpPerspective(src[i], M[k], (dst_w, dst_h), flags, BORDER_CONSTANT,
+ *                                      border_value), COLOR_BGR2YUV_I420)
+ * (or its NV12 relayout) in one pass, without the BGR BEV.  Replaces the warp of vis_homo.py:89
+ * together with the conversion of its VideoWriter.write (vis_homo.py:110-111).  src
+ * [n_frames][src_h][src_w][3] contiguous uint8 BGR; dst, layout, dst_pitch and dst_frame_stride as
+ * for bevk_bgr_to_yuv420 with dst_h x dst_w pixels (both even); M, n_mats, mat_index, flags,
+ * border_mode and border_value (B, G, R) as for bevk_warp_perspective.
+ */
+int bevk_warp_perspective_yuv420(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
+                                 int dst_w, int layout, int dst_pitch, int64_t dst_frame_stride, const double *M,
+                                 int n_mats, const int32_t *mat_index, int flags, int border_mode,
+                                 const double *border_value, void *stream);
+
+/*
+ * bevk_warp_perspective_yuv420 of NV12 frames: dst[i] is byte-identical to
+ *     cv2.cvtColor(cv2.warpPerspective(cv2.cvtColor(src[i], COLOR_YUV2BGR_NV12), M[k], (dst_w, dst_h),
+ *                                      flags, BORDER_CONSTANT, border_value), COLOR_BGR2YUV_I420)
+ * (or its NV12 relayout): decoder frames to encoder frames in one pass (vis_homo.py:85-111 with a
+ * GPU decoder and encoder).  src, pitch and frame_stride as for bevk_warp_perspective_nv12; dst as
+ * for bevk_warp_perspective_yuv420.
+ */
+int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                                      int64_t frame_stride, int dst_h, int dst_w, int layout, int dst_pitch,
+                                      int64_t dst_frame_stride, const double *M, int n_mats,
+                                      const int32_t *mat_index, int flags, int border_mode,
+                                      const double *border_value, void *stream);
 
 /*
  * Roofline accounting helper (SURVEY.md 8d): number of distinct in-bounds source pixels that the

@@ -398,6 +398,89 @@ def nv12_bench(rounds=5):
     _report("cfg4 8 cameras x%d 1080p NV12" % n, times, algo, peak)
 
 
+def yuv420_bench(rounds=5):
+    """YUV 4:2:0 BEVs for a video encoder (vis_homo.py:110-111): the fused warps to I420 against the
+    BGR warp followed by bgr_to_yuv420, for BGR and NV12 frames, alternating the routes in one
+    process; and the conversion alone.  Algorithmic bytes of a warp: the touched source bytes (3 per
+    touched BGR pixel; touched luma + 2 x touched chroma samples for NV12) + 1.5 per dst pixel; of
+    the conversion: 3 + 1.5 bytes per pixel.  Every frame set is larger than the 126 MB L2."""
+    import json
+    from oracle import nv12_oracle
+    print("card: %s" % card(), flush=True)
+    peak, src = bench.measured_peak()
+    print("peak: %.1f GB/s (%s)" % (peak, src), flush=True)
+    dev = torch.device("cuda", 0)
+    g = torch.Generator(device=dev).manual_seed(1234)
+
+    def src_bytes(ds, Hm, flags, nv12):
+        if nv12:
+            luma, chroma = nv12_oracle.touched_samples((1920, 1080), ds, Hm, flags)
+            return luma + 2 * chroma
+        return 3 * _native.warp_touched_pixels((1920, 1080), ds, Hm, flags)[0]
+
+    # cfg 2: 256 x 1080p -> 1024^2, the canonical map
+    n, dsize, H = 256, (1024, 1024), bench.h_canon(1)
+    bgr = torch.randint(0, 256, (n, 1080, 1920, 3), dtype=torch.uint8, device=dev, generator=g)
+    nv12 = torch.randint(0, 256, (n, 1620, 1920), dtype=torch.uint8, device=dev, generator=g)
+    bev = torch.empty((n, 1024, 1024, 3), dtype=torch.uint8, device=dev)
+    out_a = torch.empty((n, 1536, 1024), dtype=torch.uint8, device=dev)
+    out_b = torch.empty_like(out_a)
+    for flags, fname in ((1, "bilinear"), (0, "nearest")):
+        for nv, frames in ((False, bgr), (True, nv12)):
+            algo = n * (src_bytes(dsize, H, flags, nv) + 3 * dsize[0] * dsize[1] // 2)
+            if nv:
+                routes = {"fused": lambda: homo.warp_perspective_nv12_yuv420(frames, H, dsize, dst=out_a, flags=flags),
+                          "warp_perspective_nv12 + bgr_to_yuv420": lambda: (
+                              homo.warp_perspective_nv12(frames, H, dsize, dst=bev, flags=flags),
+                              homo.bgr_to_yuv420(bev, dst=out_b))}
+            else:
+                routes = {"fused": lambda: homo.warp_perspective_yuv420(frames, H, dsize, dst=out_a, flags=flags),
+                          "staged warp + bgr_to_yuv420": lambda: (
+                              homo.warp_perspective(frames, H, dsize, dst=bev, flags=flags, path="fast"),
+                              homo.bgr_to_yuv420(bev, dst=out_b))}
+            times = _alternate(routes, rounds, 10)
+            assert torch.equal(out_a, out_b), "routes differ"
+            _report("cfg2 x%d 1080p %s -> 1024^2 I420 %s" % (n, "NV12" if nv else "BGR", fname), times, algo, peak)
+    del bgr, nv12, out_a, out_b
+    torch.cuda.empty_cache()
+
+    # the conversion alone, on 256 1024^2 BEVs
+    yuv = torch.empty((n, 1536, 1024), dtype=torch.uint8, device=dev)
+    bev.random_(0, 256, generator=g)
+    for layout in ("i420", "nv12"):
+        times = _alternate({"bgr_to_yuv420 " + layout: lambda: homo.bgr_to_yuv420(bev, layout, dst=yuv)}, rounds, 10)
+        _report("conversion x%d 1024^2" % n, times, n * 1024 * 1024 * 9 // 2, peak)
+    del bev, yuv
+    torch.cuda.empty_cache()
+
+    # cfg 4: 8 cameras x 1000 frames, one homography and BEV size per camera
+    cams = json.load(open(os.path.join(ROOT, "tests", "golden", "cfg4_cams.json")))
+    n = 1000
+    for nv in (False, True):
+        frames = torch.randint(0, 256, (n, 1620, 1920) if nv else (n, 1080, 1920, 3), dtype=torch.uint8, device=dev,
+                               generator=g)
+        jobs, algo = [], 0
+        for c in cams:
+            Hc = np.array(c["H_bev_img"])
+            ds = (int(c["bspec"]["u_size"]), int(c["bspec"]["v_size"]))
+            algo += n * (src_bytes(ds, Hc, 1, nv) + 3 * ds[0] * ds[1] // 2)
+            jobs.append((Hc, ds, torch.empty((n, ds[1], ds[0], 3), dtype=torch.uint8, device=dev),
+                         torch.empty((n, ds[1] * 3 // 2, ds[0]), dtype=torch.uint8, device=dev)))
+
+        def fused4():
+            for Hc, ds, _, o in jobs:
+                (homo.warp_perspective_nv12_yuv420 if nv else homo.warp_perspective_yuv420)(frames, Hc, ds, dst=o)
+
+        def two_pass4():
+            for Hc, ds, b, o in jobs:
+                (homo.warp_perspective_nv12 if nv else homo.warp_perspective)(frames, Hc, ds, dst=b)
+                homo.bgr_to_yuv420(b, dst=o)
+        times = _alternate({"fused": fused4, "warp + bgr_to_yuv420 per camera": two_pass4}, rounds, 2)
+        _report("cfg4 8 cameras x%d 1080p %s -> I420" % (n, "NV12" if nv else "BGR"), times, algo, peak)
+        del frames, jobs
+        torch.cuda.empty_cache()
+
+
 def resize_nv12_bench(rounds=5):
     """The small frame of the reference's frame loop (vis_homo.py:90) from NV12 frames: the fused
     resize against converting to BGR and then resizing, alternating the two routes in one process.
@@ -512,6 +595,8 @@ def resize_nv12_area_bench(rounds=5):
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "nv12":
         nv12_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "yuv420":
+        yuv420_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_nv12":
         resize_nv12_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_area":
