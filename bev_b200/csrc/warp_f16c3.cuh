@@ -8,7 +8,8 @@
 // A pixel is 6 bytes; a 2-tap window row is 12 bytes starting on any even byte, i.e. up to 4 aligned
 // words; 32 pixels are 192 bytes = 48 words.  Out-of-image taps carry weight 0 and a clamped
 // address (value * 0 = 0 for every finite neighbour; the direct-gather kernel is the exact path
-// for frames that hold Inf / NaN next to the image border).
+// for frames that hold Inf / NaN next to the image border).  A pixel with no tap inside the image
+// is written as +0, the border value cv2 writes: its sum of zero-weighted negative taps is -0.
 #pragma once
 #include "bevk_common.cuh"
 #include "warp_u8c3.cuh"  // prmt, st_stream
@@ -16,6 +17,7 @@
 struct PixF16 {
     uint32_t addr;  // byte offset (4-aligned) of the first window word, row 0
     uint32_t sh;    // 0 or 16: the window starts on the low / high half of that word
+    uint32_t keep;  // all ones if any tap is inside the image, else 0 (ANDed onto the bilinear result)
     float w00, w01, w10, w11;  // bilinear weights of the window positions; nearest: w00 = 1 or 0
 };
 
@@ -42,6 +44,7 @@ struct PxF16C3 {
         Reg q;
         q.addr = A & ~3u;
         q.sh = 8 * (A & 3);  // A is even: 0 or 16
+        q.keep = act ? 0xffffffffu : 0u;
         if (LINEAR) {
             // wc / wr are 32 - frac, frac or 0: dividing by 32 is exact, so c0 = 1 - tx, c1 = tx ...
             const float c0 = __fmul_rn((float)wc0, 1.0f / 32.0f), c1 = __fmul_rn((float)wc1, 1.0f / 32.0f);
@@ -108,8 +111,8 @@ struct PxF16C3 {
             const float c1 = blend(q, hi(a0), lo(a2), hi(b0), lo(b2));
             const float c2 = blend(q, lo(a1), hi(a2), lo(b1), hi(b2));
             const __half2 h01 = __floats2half2_rn(c0, c1);
-            o.x = *reinterpret_cast<const uint32_t *>(&h01);
-            o.y = (uint32_t)__half_as_ushort(__float2half_rn(c2));
+            o.x = *reinterpret_cast<const uint32_t *>(&h01) & q.keep;
+            o.y = (uint32_t)__half_as_ushort(__float2half_rn(c2)) & q.keep;
         } else {
             const uint32_t a0 = __funnelshift_r(w[0], w[1], q.sh);
             const uint32_t a1 = __funnelshift_r(w[1], 0u, q.sh) & 0xffffu;

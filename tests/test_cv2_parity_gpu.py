@@ -10,6 +10,7 @@ import pytest
 import torch
 
 from bev_b200 import _native, homo, torch_ops
+from oracle import yuv420_oracle as yo
 from tests import cv2_cases as cc
 from tests import util
 
@@ -130,6 +131,28 @@ def test_warp_perspective_nv12_vs_cv2():
             ref = cv2_warp(bgr[i], case["H"], case, border)
             assert util.bits_equal(out[i], ref), "nv12 warp != cv2 at %d px, frame %d: %s" % (
                 int(np.sum(out[i] != ref)), i, cc.describe(case))
+
+
+def test_warp_perspective_yuv420_vs_cv2():
+    """The fused warps to YUV 4:2:0 from BGR and NV12 sources: 3 channels, dst sizes rounded up to
+    even (so rows shorter than 16 give odd block widths, whose 2x2 dst blocks straddle two cv2 block
+    columns), against cv2's warp followed by cv2's BGR -> I420 conversion (and its NV12 relayout)."""
+    for case in cc.warp_cases(WARP_SEED, N_WARP // 2, dtypes=("uint8",)):
+        n = batch_size(case)
+        dw, dh = (v + v % 2 for v in case["dsize"])
+        case = dict(case, channels=3, dsize=(dw, dh), bw0=cc.block_width(dw, dh))
+        border = (list(case["border"]) + [0.0, 0.0])[:3]
+        nv12, nv12_bgr = nv12_batch(case, n)
+        bgr = cc.warp_src(case, n)
+        for what, src, fn, refs in (("bgr", cu(bgr), homo.warp_perspective_yuv420, bgr),
+                                    ("nv12", cu(nv12), homo.warp_perspective_nv12_yuv420, nv12_bgr)):
+            i420 = [cv2.cvtColor(cv2_warp(f, case["H"], case, border), cv2.COLOR_BGR2YUV_I420) for f in refs]
+            for layout in ("i420", "nv12"):
+                out = fn(src, case["H"], (dw, dh), layout, flags=case["flags"], borderValue=border).cpu().numpy()
+                for i in range(n):
+                    ref = i420[i] if layout == "i420" else yo.i420_to_nv12(i420[i])
+                    assert util.bits_equal(out[i], ref), "%s source, %s output != cv2 at %d bytes, frame %d: %s" % (
+                        what, layout, int(np.sum(out[i] != ref)), i, cc.describe(case))
 
 
 def test_resize_vs_cv2():

@@ -168,6 +168,9 @@ MAPS = [  # (H, dsize) on a 96 x 128 source
     (np.array([[3.0, 0.2, -7.0], [0.1, 2.7, -5.0], [0, 0, 1.0]]), (382, 290)),
     (np.array([[1.0, 0.2, -3.0], [0.1, 1.1, -2.0], [0.0, 0.03, -0.5]]), (130, 96)),  # horizon crossing
     (np.array([[1.0, 0, 2.0], [0, 1.0, 1.0], [0, 0, 1.0]]), (2, 2)),
+    # rows shorter than 16: odd block widths 85 and 73, so some 2x2 dst blocks straddle two cv2 block columns
+    (np.array([[0.7, 0.05, 3.5], [0.02, 0.9, 2.5], [0.0, 0.001, 1.0]]), (170, 12)),
+    (np.array([[0.75, 0.0, 0.5], [0.0, 0.5, 0.5], [0.0, 0.0, 1.0]]), (146, 14)),
 ]
 
 
