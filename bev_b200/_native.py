@@ -38,6 +38,8 @@ SIGNATURES = {
     "bevk_warp_perspective_host": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_int,
                                             _c_int, _c_int, _dp, _c_int, _i32p, _c_int, _c_int,
                                             _dp]),
+    "bevk_warp_perspective_video_host": (_c_int, [_vp, _c_int, _vp, _c_int] + [_c_int] * 5 + [_dp, _c_int, _i32p,
+                                                                                       _c_int, _c_int, _dp]),
     "bevk_warp_host_rows": (_c_int, [_c_int, _c_int, _c_int, _c_int, _dp, _c_int, _c_int, _ip]),
     "bevk_warp_set_path": (_c_int, [_c_int]),
     "bevk_warp_touched_pixels": (_c_i64, [_c_int, _c_int, _c_int, _c_int, _dp, _c_int, _ip]),
@@ -427,6 +429,70 @@ def warp_perspective_nv12_yuv420(src, M, dsize, layout="i420", dst=None, flags=1
             int(borderMode), _dptr(b), _stream_ptr(src))
     _check(rc, "bevk_warp_perspective_nv12_yuv420")
     return dst
+
+
+VIDEO_FORMATS = {"i420": 0, "nv12": 1, "bgr": 2}
+
+
+def _video_frames(a, fmt, what):
+    """(frames view, n, h, w, batched) of a host BGR (H, W, 3) / (N, H, W, 3) or YUV 4:2:0
+    (H*3/2, W) / (N, H*3/2, W) uint8 buffer (numpy array or CPU tensor)."""
+    if hasattr(a, "detach"):
+        if a.is_cuda:
+            raise ValueError("%s is on %s: warp_perspective_video_host takes host buffers" % (what, a.device))
+        a = a.detach().numpy()
+    a = np.asarray(a)
+    if a.dtype != np.uint8:
+        raise ValueError("%s frames are uint8, got %s" % (what, a.dtype))
+    if not a.flags["C_CONTIGUOUS"]:
+        raise ValueError("%s must be C-contiguous" % what)
+    if fmt == "bgr":
+        if a.ndim not in (3, 4) or a.shape[-1] != 3:
+            raise ValueError("%s BGR frames must be (H, W, 3) or (N, H, W, 3), got shape %s" % (what, a.shape))
+        f = a[None] if a.ndim == 3 else a
+        return f, f.shape[0], f.shape[1], f.shape[2], a.ndim == 4
+    if a.ndim not in (2, 3):
+        raise ValueError("%s %s frames must be (H*3/2, W) or (N, H*3/2, W), got shape %s"
+                         % (what, fmt.upper(), a.shape))
+    f = a[None] if a.ndim == 2 else a
+    rows, w = f.shape[1], f.shape[2]
+    if rows == 0 or rows % 3 or w % 2 or w == 0:
+        raise ValueError("%s %s frames need H*3/2 rows for an even H and an even width W, got %d rows x %d"
+                         % (what, fmt.upper(), rows, w))
+    return f, f.shape[0], rows // 3 * 2, w, a.ndim == 3
+
+
+def warp_perspective_video_host(src, M, dsize, src_format="bgr", dst_format="i420", dst=None, flags=1,
+                                borderMode=0, borderValue=0, mat_index=None):
+    """Host-buffer warp between video frame formats ("bgr", "i420", "nv12"): src / dst are numpy
+    arrays or CPU tensors (pinned for full speed), BGR (H, W, 3) / (N, H, W, 3) or YUV 4:2:0
+    (H*3/2, W) / (N, H*3/2, W) uint8."""
+    for name, fmt in (("src_format", src_format), ("dst_format", dst_format)):
+        if fmt not in VIDEO_FORMATS:
+            raise ValueError("%s must be 'bgr', 'i420' or 'nv12', got %r" % (name, fmt))
+    s, n, h, w, batched = _video_frames(src, src_format, "src")
+    dw, dh = int(dsize[0]), int(dsize[1])
+    if dst_format != "bgr" and (dw % 2 or dh % 2):
+        raise ValueError("YUV 4:2:0 frames need an even width and height, got dsize %dx%d" % (dw, dh))
+    Ms, idx = _prep_mats(M, n, mat_index)
+    frame = (dh, dw, 3) if dst_format == "bgr" else (dh * 3 // 2, dw)
+    shape = (n,) + frame if batched else frame
+    if dst is None:
+        out = np.empty(shape, np.uint8)
+    else:
+        if getattr(dst, "is_cuda", False):
+            raise ValueError("dst is on %s: warp_perspective_video_host takes host buffers" % (dst.device,))
+        out = _to_numpy(dst) if not isinstance(dst, np.ndarray) else dst
+        if out.shape != shape or out.dtype != np.uint8 or not out.flags["C_CONTIGUOUS"]:
+            raise ValueError("dst must be a C-contiguous uint8 array of shape %s, got %s %s"
+                             % (shape, out.dtype, out.shape))
+    b = _border(borderValue)
+    rc = lib().bevk_warp_perspective_video_host(
+        _vp(s.ctypes.data), VIDEO_FORMATS[src_format], _vp(out.ctypes.data), VIDEO_FORMATS[dst_format], n, h, w,
+        dh, dw, _dptr(Ms), Ms.shape[0], idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags),
+        int(borderMode), _dptr(b))
+    _check(rc, "bevk_warp_perspective_video_host")
+    return dst if dst is not None else out
 
 
 def warp_touched_pixels(ssize, dsize, M, flags=1):

@@ -138,8 +138,8 @@ struct BevkWarpParams {
     BevkWarpGroup g[BEVK_MAX_GROUPS];
 };
 
-// The warp of NV12 frames (nv12.cu): w.src is frame 0's first luma byte, w.src_h / w.src_w the luma
-// size; w.src_frame_elems is unused, the two strides below replace it.
+// The warp of NV12 or I420 frames to BGR (nv12.cu): w.src is frame 0's first luma byte, w.src_h /
+// w.src_w the luma size; w.src_frame_elems is unused, the two strides below replace it.
 struct BevkNv12Params {
     BevkWarpParams w;
     int pitch;               // bytes from one luma or chroma row to the next
@@ -165,8 +165,9 @@ int bevk_plan_generic_chunks(BevkWarpParams &p, int channels);
 // `force`, is too small a batch to amortise its per-tile set-up), <0 on error
 int bevk_launch_warp_fast(const BevkWarpParams &p, int channels, int dtype, int linear, int force,
                           cudaStream_t stream);
-// NV12 -> BGR warp over the chunks bevk_plan_generic_chunks planned for P.w
-int bevk_launch_warp_nv12(const BevkNv12Params &P, int linear, cudaStream_t stream);
+// NV12 or I420 (src_format BEVK_YUV_NV12 / BEVK_YUV_I420) -> BGR warp over the chunks
+// bevk_plan_generic_chunks planned for P.w
+int bevk_launch_warp_nv12(const BevkNv12Params &P, int src_format, int linear, cudaStream_t stream);
 int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int w, int pitch,
                             long long frame_stride, cudaStream_t stream);
 // cv2.resize of n_frames > 0 frames with `interpolation` (BEVK_INTER_LINEAR or BEVK_INTER_AREA):
@@ -175,9 +176,9 @@ int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int
 int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels, int nv12,
                        long long pitch, long long frame_stride, int dst_h, int dst_w, int interpolation,
                        cudaStream_t stream);
-// BGR (nv12_src 0) or NV12 frames warped to YUV 4:2:0 (nv12_out: NV12, else I420) over the chunks
-// planned for P.w on the grid of 2x2 dst blocks
-int bevk_launch_warp_yuv420(const BevkYuvParams &P, int nv12_src, int nv12_out, int linear, cudaStream_t stream);
+// BGR, NV12 or I420 frames (src_format BEVK_BGR / BEVK_YUV_NV12 / BEVK_YUV_I420) warped to YUV
+// 4:2:0 (nv12_out: NV12, else I420) over the chunks planned for P.w on the grid of 2x2 dst blocks
+int bevk_launch_warp_yuv420(const BevkYuvParams &P, int src_format, int nv12_out, int linear, cudaStream_t stream);
 // n_frames > 0 contiguous BGR frames of h x w (both even) to YUV 4:2:0 (nv12_out: NV12, else I420)
 int bevk_launch_bgr_to_yuv420(const void *src, void *dst, int n_frames, int h, int w, int nv12_out, int dst_pitch,
                               long long dst_frame_stride, cudaStream_t stream);

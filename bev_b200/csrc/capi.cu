@@ -367,6 +367,110 @@ struct HostWorkspace {
 };
 HostWorkspace g_ws[kMaxDevices];
 
+// A byte range of every source frame that the host pipeline uploads.
+struct HostBand {
+    size_t offset, bytes;
+};
+
+// The pipelined host-buffer warp of the n_frames > 0 frames of a: frames of src_frame_bytes, of which
+// only `bands` are uploaded, to frames of dst_frame_bytes.  Chunks of frames go through the device
+// workspace, kHostSlots at a time, so that the copies and kernels of neighbouring chunks overlap.
+// run(d_src, d_dst, args, groups, stream) enqueues the kernels of one chunk; maps are the dst->src
+// maps of all n_mats matrices.
+template <typename Run>
+int host_pipeline(const void *src, void *dst, const WarpArgs &a, const std::vector<double> &maps, int n_mats,
+                  const int32_t *mat_index, size_t src_frame_bytes, size_t dst_frame_bytes,
+                  const std::vector<HostBand> &bands, Run run)
+{
+    const int n_frames = a.n_frames;
+    int chunk = (int)std::max<size_t>(1, (size_t)(64u << 20) / std::max(src_frame_bytes, dst_frame_bytes));
+    chunk = std::min(chunk, std::max(1, (n_frames + 3) / 4));
+    chunk = std::min(chunk, n_frames);
+
+    int dev = 0;
+    BEVK_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= kMaxDevices) BEVK_FAIL(BEVK_E_ARG, "warp: device ordinal %d is not supported", dev);
+    HostWorkspace &ws = g_ws[dev];
+    std::lock_guard<std::mutex> lock(ws.mu);  // concurrent host calls on one device take turns
+    if (!ws.ready) {
+        for (int i = 0; i < kHostSlots; ++i)
+            BEVK_CUDA(cudaStreamCreateWithFlags(&ws.stream[i], cudaStreamNonBlocking));
+        ws.ready = true;
+    }
+    if (ws.src_cap < src_frame_bytes * chunk) {
+        for (int i = 0; i < kHostSlots; ++i) {
+            // the previous call synchronised every slot stream before it returned: nothing is in flight
+            if (ws.d_src[i]) cudaFree(ws.d_src[i]);
+            ws.d_src[i] = nullptr;
+        }
+        ws.src_cap = 0;
+        for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA(cudaMalloc(&ws.d_src[i], src_frame_bytes * chunk));
+        ws.src_cap = src_frame_bytes * chunk;
+    }
+    if (ws.dst_cap < dst_frame_bytes * chunk) {
+        for (int i = 0; i < kHostSlots; ++i) {
+            if (ws.d_dst[i]) cudaFree(ws.d_dst[i]);
+            ws.d_dst[i] = nullptr;
+        }
+        ws.dst_cap = 0;
+        for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA(cudaMalloc(&ws.d_dst[i], dst_frame_bytes * chunk));
+        ws.dst_cap = dst_frame_bytes * chunk;
+    }
+
+    // From the first enqueue on, every exit -- also an error exit -- first waits for the slot
+    // streams: copies in flight still read / write the caller's host buffers.
+    auto drain = [&ws]() {
+        for (int i = 0; i < kHostSlots; ++i) cudaStreamSynchronize(ws.stream[i]);
+    };
+#define BEVK_CUDA_DRAIN(expr)                                                                       \
+    do {                                                                                            \
+        cudaError_t _e = (expr);                                                                    \
+        if (_e != cudaSuccess) {                                                                    \
+            drain();                                                                                \
+            bevk_set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__); \
+            return BEVK_E_CUDA;                                                                     \
+        }                                                                                           \
+    } while (0)
+
+    int slot = 0;
+    for (int f0 = 0; f0 < n_frames; f0 += chunk, slot = (slot + 1) % kHostSlots) {
+        const int nf = std::min(chunk, n_frames - f0);
+        cudaStream_t st = ws.stream[slot];
+        // frames are "rows" of a 2-D copy: pitch = whole frame, width = the band
+        for (const HostBand &b : bands)
+            BEVK_CUDA_DRAIN(cudaMemcpy2DAsync((char *)ws.d_src[slot] + b.offset, src_frame_bytes,
+                                              (const char *)src + (size_t)f0 * src_frame_bytes + b.offset,
+                                              src_frame_bytes, b.bytes, nf, cudaMemcpyHostToDevice, st));
+        std::vector<BevkWarpGroup> groups;
+        std::vector<int32_t> idx;
+        const int32_t *idx_ptr = nullptr;
+        std::vector<double> chunk_maps;
+        const std::vector<double> *use_maps = &maps;
+        int use_n_mats = n_mats;
+        if (mat_index) {
+            idx.assign(mat_index + f0, mat_index + f0 + nf);
+            idx_ptr = idx.data();
+        } else if (n_mats != 1) {  // one matrix per frame: this chunk's slice
+            chunk_maps.assign(maps.begin() + (size_t)f0 * 9, maps.begin() + (size_t)(f0 + nf) * 9);
+            use_maps = &chunk_maps;
+            use_n_mats = nf;
+        }
+        build_groups(nf, use_n_mats, idx_ptr, *use_maps, groups);
+        WarpArgs ac = a;
+        ac.n_frames = nf;
+        const int rc = run(ws.d_src[slot], ws.d_dst[slot], ac, groups, st);
+        if (rc) {
+            drain();
+            return rc;
+        }
+        BEVK_CUDA_DRAIN(cudaMemcpyAsync((char *)dst + (size_t)f0 * dst_frame_bytes, ws.d_dst[slot],
+                                        dst_frame_bytes * nf, cudaMemcpyDeviceToHost, st));
+    }
+    for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA_DRAIN(cudaStreamSynchronize(ws.stream[i]));
+    return BEVK_OK;
+#undef BEVK_CUDA_DRAIN
+}
+
 }  // namespace
 
 extern "C" {
@@ -455,9 +559,48 @@ int check_yuv420_dst(const char *what, int n_frames, int h, int w, int layout, i
     return check_nv12_layout32(what, n_frames, h, w, pitch, frame_stride);
 }
 
-// The fused warps to YUV 4:2:0 after their source-layout checks: BGR (nv12 0, contiguous frames)
-// or NV12 frames, rows `pitch` and frames `frame_stride` bytes apart.
-int warp_yuv420(const char *what, const void *src, void *dst, int n_frames, int src_h, int src_w, int nv12,
+// The fused warps to YUV 4:2:0 of these groups on device buffers: BGR (src_format BEVK_BGR,
+// contiguous frames), NV12 or I420 frames, rows `pitch` and frames `frame_stride` bytes apart.
+int run_warp_yuv420(const void *src, void *dst, const WarpArgs &a, const std::vector<BevkWarpGroup> &groups,
+                    int src_format, long long pitch, long long frame_stride, int layout, int dst_pitch,
+                    int64_t dst_frame_stride, cudaStream_t stream)
+{
+    BevkYuvParams P;
+    memset(&P, 0, sizeof(P));
+    P.pitch = (int)pitch;
+    P.frame_stride = frame_stride;
+    P.dst_pitch = dst_pitch;
+    P.dst_frame_stride = dst_frame_stride;
+    return launch_warp_groups(P.w, src, dst, a, groups, [&]() {
+        // a thread owns a 2x2 dst block: plan the frame chunks over the grid of blocks
+        P.w.dst_w /= 2;
+        P.w.dst_h /= 2;
+        const int rc = bevk_plan_generic_chunks(P.w, 3);
+        P.w.dst_w *= 2;
+        P.w.dst_h *= 2;
+        if (rc) return rc;
+        return bevk_launch_warp_yuv420(P, src_format, layout == BEVK_YUV_NV12, a.linear, stream);
+    });
+}
+
+// The NV12 or I420 (src_format) to BGR warp of these groups on device buffers.
+int run_warp_yuv_bgr(const void *src, void *dst, const WarpArgs &a, const std::vector<BevkWarpGroup> &groups,
+                     int src_format, int pitch, int64_t frame_stride, cudaStream_t stream)
+{
+    BevkNv12Params P;
+    memset(&P, 0, sizeof(P));
+    P.pitch = pitch;
+    P.frame_stride = frame_stride;
+    return launch_warp_groups(P.w, src, dst, a, groups, [&]() {
+        const int rc = bevk_plan_generic_chunks(P.w, 3);
+        if (rc) return rc;
+        return bevk_launch_warp_nv12(P, src_format, a.linear, stream);
+    });
+}
+
+// The fused warps to YUV 4:2:0 after their source-layout checks: BGR (src_format BEVK_BGR,
+// contiguous frames) or NV12 frames, rows `pitch` and frames `frame_stride` bytes apart.
+int warp_yuv420(const char *what, const void *src, void *dst, int n_frames, int src_h, int src_w, int src_format,
                 long long pitch, long long frame_stride, int dst_h, int dst_w, int layout, int dst_pitch,
                 int64_t dst_frame_stride, const double *M, int n_mats, const int32_t *mat_index, int flags,
                 int border_mode, const double *border_value, void *stream)
@@ -475,23 +618,8 @@ int warp_yuv420(const char *what, const void *src, void *dst, int n_frames, int 
     effective_maps(M, n_mats, flags, maps);
     std::vector<BevkWarpGroup> groups;
     build_groups(n_frames, n_mats, mat_index, maps, groups);
-
-    BevkYuvParams P;
-    memset(&P, 0, sizeof(P));
-    P.pitch = (int)pitch;
-    P.frame_stride = frame_stride;
-    P.dst_pitch = dst_pitch;
-    P.dst_frame_stride = dst_frame_stride;
-    return launch_warp_groups(P.w, src, dst, a, groups, [&]() {
-        // a thread owns a 2x2 dst block: plan the frame chunks over the grid of blocks
-        P.w.dst_w /= 2;
-        P.w.dst_h /= 2;
-        const int rc = bevk_plan_generic_chunks(P.w, 3);
-        P.w.dst_w *= 2;
-        P.w.dst_h *= 2;
-        if (rc) return rc;
-        return bevk_launch_warp_yuv420(P, nv12, layout == BEVK_YUV_NV12, a.linear, (cudaStream_t)stream);
-    });
+    return run_warp_yuv420(src, dst, a, groups, src_format, pitch, frame_stride, layout, dst_pitch, dst_frame_stride,
+                           (cudaStream_t)stream);
 }
 }  // namespace
 
@@ -527,16 +655,7 @@ int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src
     effective_maps(M, n_mats, flags, maps);
     std::vector<BevkWarpGroup> groups;
     build_groups(n_frames, n_mats, mat_index, maps, groups);
-
-    BevkNv12Params P;
-    memset(&P, 0, sizeof(P));
-    P.pitch = pitch;
-    P.frame_stride = frame_stride;
-    return launch_warp_groups(P.w, src, dst, a, groups, [&]() {
-        const int rc = bevk_plan_generic_chunks(P.w, 3);
-        if (rc) return rc;
-        return bevk_launch_warp_nv12(P, a.linear, (cudaStream_t)stream);
-    });
+    return run_warp_yuv_bgr(src, dst, a, groups, BEVK_YUV_NV12, pitch, frame_stride, (cudaStream_t)stream);
 }
 
 int bevk_bgr_to_yuv420(const void *src, void *dst, int n_frames, int h, int w, int layout, int dst_pitch,
@@ -558,9 +677,9 @@ int bevk_warp_perspective_yuv420(const void *src, void *dst, int n_frames, int s
                                  int n_mats, const int32_t *mat_index, int flags, int border_mode,
                                  const double *border_value, void *stream)
 {
-    return warp_yuv420("warp_yuv420", src, dst, n_frames, src_h, src_w, 0, 3LL * src_w, 3LL * src_w * src_h, dst_h,
-                       dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index, flags, border_mode,
-                       border_value, stream);
+    return warp_yuv420("warp_yuv420", src, dst, n_frames, src_h, src_w, BEVK_BGR, 3LL * src_w,
+                       3LL * src_w * src_h, dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index,
+                       flags, border_mode, border_value, stream);
 }
 
 int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
@@ -571,9 +690,9 @@ int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, 
 {
     const int rc = check_nv12_layout32("warp_nv12_yuv420", n_frames, src_h, src_w, pitch, frame_stride);
     if (rc) return rc;
-    return warp_yuv420("warp_nv12_yuv420", src, dst, n_frames, src_h, src_w, 1, pitch, frame_stride, dst_h, dst_w,
-                       layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index, flags, border_mode, border_value,
-                       stream);
+    return warp_yuv420("warp_nv12_yuv420", src, dst, n_frames, src_h, src_w, BEVK_YUV_NV12, pitch, frame_stride,
+                       dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index, flags, border_mode,
+                       border_value, stream);
 }
 
 int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h, int dst_w, int channels,
@@ -638,96 +757,76 @@ int bevk_warp_perspective_host(const void *src, void *dst, int n_frames, int src
     int r0, r1;
     referenced_rows_union(maps, n_mats, a, r0, r1);
     const size_t row_bytes = (size_t)a.src_w * a.channels * a.elem_size;
-    const size_t src_frame_bytes = row_bytes * a.src_h;
     const size_t dst_frame_bytes = (size_t)a.dst_w * a.dst_h * a.channels * a.elem_size;
-    const size_t up_bytes = row_bytes * (size_t)(r1 - r0 + 1);
+    return host_pipeline(src, dst, a, maps, n_mats, mat_index, row_bytes * a.src_h, dst_frame_bytes,
+                         {{r0 * row_bytes, row_bytes * (size_t)(r1 - r0 + 1)}},
+                         [](const void *s, void *d, const WarpArgs &ac, const std::vector<BevkWarpGroup> &groups,
+                            cudaStream_t st) { return run_warp_device(s, d, ac, groups, g_warp_path, st); });
+}
 
-    // chunk so that copies and kernels of neighbouring chunks overlap (kHostSlots streams and buffers)
-    int chunk = (int)std::max<size_t>(1, (size_t)(64u << 20) / std::max(src_frame_bytes, dst_frame_bytes));
-    chunk = std::min(chunk, std::max(1, (n_frames + 3) / 4));
-    chunk = std::min(chunk, n_frames);
+int bevk_warp_perspective_video_host(const void *src, int src_format, void *dst, int dst_format, int n_frames,
+                                     int src_h, int src_w, int dst_h, int dst_w, const double *M, int n_mats,
+                                     const int32_t *mat_index, int flags, int border_mode,
+                                     const double *border_value)
+{
+    const char *what = "warp_video_host";
+    auto known = [](int f) { return f == BEVK_BGR || f == BEVK_YUV_I420 || f == BEVK_YUV_NV12; };
+    if (!known(src_format) || !known(dst_format))
+        BEVK_FAIL(BEVK_E_ARG, "%s: formats must be BEVK_YUV_I420 (0), BEVK_YUV_NV12 (1) or BEVK_BGR (2), got src %d, "
+                  "dst %d", what, src_format, dst_format);
+    const bool yuv_src = src_format != BEVK_BGR, yuv_dst = dst_format != BEVK_BGR;
+    int rc;
+    if (yuv_src) {
+        rc = check_nv12_layout32(what, n_frames, src_h, src_w, src_w, (int64_t)src_w * src_h / 2 * 3);
+        if (rc) return rc;
+    }
+    if (yuv_dst) {
+        rc = check_yuv420_dst(what, n_frames, dst_h, dst_w, dst_format, dst_w, (int64_t)dst_w * dst_h / 2 * 3);
+        if (rc) return rc;
+    }
+    WarpArgs a;
+    rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index, flags,
+                         border_mode, border_value, a);
+    if (rc) return rc;
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    std::vector<double> maps;
+    effective_maps(M, n_mats, flags, maps);
 
-    int dev = 0;
-    BEVK_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= kMaxDevices) BEVK_FAIL(BEVK_E_ARG, "warp: device ordinal %d is not supported", dev);
-    HostWorkspace &ws = g_ws[dev];
-    std::lock_guard<std::mutex> lock(ws.mu);  // concurrent host calls on one device take turns
-    if (!ws.ready) {
-        for (int i = 0; i < kHostSlots; ++i)
-            BEVK_CUDA(cudaStreamCreateWithFlags(&ws.stream[i], cudaStreamNonBlocking));
-        ws.ready = true;
-    }
-    if (ws.src_cap < src_frame_bytes * chunk) {
-        for (int i = 0; i < kHostSlots; ++i) {
-            // the previous call synchronised every slot stream before it returned: nothing is in flight
-            if (ws.d_src[i]) cudaFree(ws.d_src[i]);
-            ws.d_src[i] = nullptr;
+    // the referenced luma (BGR) row band [r0, r1] and, for YUV, the chroma rows under it
+    int r0, r1;
+    referenced_rows_union(maps, n_mats, a, r0, r1);
+    const size_t h = (size_t)src_h, w = (size_t)src_w, rows = (size_t)(r1 - r0 + 1);
+    size_t src_frame_bytes;
+    std::vector<HostBand> bands;
+    if (!yuv_src) {
+        src_frame_bytes = 3 * w * h;
+        bands.push_back({3 * w * r0, 3 * w * rows});
+    } else {
+        src_frame_bytes = w * h / 2 * 3;
+        bands.push_back({w * r0, w * rows});
+        const size_t c0 = (size_t)(r0 / 2), nc = (size_t)(r1 / 2) - c0 + 1;
+        if (src_format == BEVK_YUV_NV12) {
+            bands.push_back({w * (h + c0), w * nc});
+        } else {  // the U plane, then the V plane: (h / 2) x (w / 2) each, contiguous
+            const size_t cw = w / 2;
+            bands.push_back({w * h + cw * c0, cw * nc});
+            bands.push_back({w * h + cw * (h / 2 + c0), cw * nc});
         }
-        ws.src_cap = 0;
-        for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA(cudaMalloc(&ws.d_src[i], src_frame_bytes * chunk));
-        ws.src_cap = src_frame_bytes * chunk;
     }
-    if (ws.dst_cap < dst_frame_bytes * chunk) {
-        for (int i = 0; i < kHostSlots; ++i) {
-            if (ws.d_dst[i]) cudaFree(ws.d_dst[i]);
-            ws.d_dst[i] = nullptr;
-        }
-        ws.dst_cap = 0;
-        for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA(cudaMalloc(&ws.d_dst[i], dst_frame_bytes * chunk));
-        ws.dst_cap = dst_frame_bytes * chunk;
-    }
-
-    // From the first enqueue on, every exit -- also an error exit -- first waits for the slot
-    // streams: copies in flight still read / write the caller's host buffers.
-    auto drain = [&ws]() {
-        for (int i = 0; i < kHostSlots; ++i) cudaStreamSynchronize(ws.stream[i]);
-    };
-#define BEVK_CUDA_DRAIN(expr)                                                                       \
-    do {                                                                                            \
-        cudaError_t _e = (expr);                                                                    \
-        if (_e != cudaSuccess) {                                                                    \
-            drain();                                                                                \
-            bevk_set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__); \
-            return BEVK_E_CUDA;                                                                     \
-        }                                                                                           \
-    } while (0)
-
-    int slot = 0;
-    for (int f0 = 0; f0 < n_frames; f0 += chunk, slot = (slot + 1) % kHostSlots) {
-        const int nf = std::min(chunk, n_frames - f0);
-        cudaStream_t st = ws.stream[slot];
-        // frames are "rows" of a 2-D copy: pitch = whole frame, width = the referenced row band
-        BEVK_CUDA_DRAIN(cudaMemcpy2DAsync((char *)ws.d_src[slot] + r0 * row_bytes, src_frame_bytes,
-                                    (const char *)src + (size_t)f0 * src_frame_bytes + r0 * row_bytes,
-                                    src_frame_bytes, up_bytes, nf, cudaMemcpyHostToDevice, st));
-        std::vector<BevkWarpGroup> groups;
-        std::vector<int32_t> idx;
-        const int32_t *idx_ptr = nullptr;
-        std::vector<double> chunk_maps;
-        const std::vector<double> *use_maps = &maps;
-        int use_n_mats = n_mats;
-        if (mat_index) {
-            idx.assign(mat_index + f0, mat_index + f0 + nf);
-            idx_ptr = idx.data();
-        } else if (n_mats != 1) {  // one matrix per frame: this chunk's slice
-            chunk_maps.assign(maps.begin() + (size_t)f0 * 9, maps.begin() + (size_t)(f0 + nf) * 9);
-            use_maps = &chunk_maps;
-            use_n_mats = nf;
-        }
-        build_groups(nf, use_n_mats, idx_ptr, *use_maps, groups);
-        WarpArgs ac = a;
-        ac.n_frames = nf;
-        rc = run_warp_device(ws.d_src[slot], ws.d_dst[slot], ac, groups, g_warp_path, st);
-        if (rc) {
-            drain();
-            return rc;
-        }
-        BEVK_CUDA_DRAIN(cudaMemcpyAsync((char *)dst + (size_t)f0 * dst_frame_bytes, ws.d_dst[slot],
-                                  dst_frame_bytes * nf, cudaMemcpyDeviceToHost, st));
-    }
-    for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA_DRAIN(cudaStreamSynchronize(ws.stream[i]));
-    return BEVK_OK;
-#undef BEVK_CUDA_DRAIN
+    const size_t dst_frame_bytes = (size_t)dst_w * dst_h * (yuv_dst ? 1 : 2) * 3 / 2;
+    const long long pitch = yuv_src ? src_w : 3LL * src_w;
+    return host_pipeline(src, dst, a, maps, n_mats, mat_index, src_frame_bytes, dst_frame_bytes, bands,
+                         [&](const void *s, void *d, const WarpArgs &ac, const std::vector<BevkWarpGroup> &groups,
+                             cudaStream_t st) -> int {
+                             if (yuv_dst)
+                                 return run_warp_yuv420(s, d, ac, groups, src_format, pitch, src_frame_bytes,
+                                                        dst_format, dst_w, dst_frame_bytes, st);
+                             if (yuv_src)
+                                 return run_warp_yuv_bgr(s, d, ac, groups, src_format, src_w, src_frame_bytes, st);
+                             return run_warp_device(s, d, ac, groups, g_warp_path, st);
+                         });
 }
 
 }  // extern "C"

@@ -1,6 +1,7 @@
 // nv12.cu -- NV12 video frames (what a GPU video decoder hands out) to BGR: the conversion
-// cv2.cvtColor(f, COLOR_YUV2BGR_NV12) on frame batches, and the perspective warp of NV12 frames
-// fused with it, so that decoded frames reach the BEV without a BGR copy of every frame.
+// cv2.cvtColor(f, COLOR_YUV2BGR_NV12) on frame batches, and the perspective warp of NV12 or I420
+// frames (what CPU decoders hand out) fused with it, so that decoded frames reach the BEV without a
+// BGR copy of every frame.
 //
 // Semantics: cv2 4.13.  The conversion is BT.601 limited range in 20-bit fixed point with chroma
 // replicated over each 2x2 luma block; the warp equals cv2.warpPerspective of the converted frame
@@ -9,25 +10,13 @@
 // the frame takes the BGR border colour; it is never converted from YUV.  The resize of NV12
 // frames is in resize.cu.
 //
-// Layout of frame n: luma rows 0..H-1 then chroma rows 0..H/2-1 (interleaved U, V bytes), each
-// row `pitch` bytes after the previous one, the frame at src + n * frame_stride bytes.
+// Layout of frame n: luma rows 0..H-1 then chroma rows 0..H/2-1 (NV12: interleaved U, V bytes;
+// I420: the U plane then the V plane, see yuv_src.cuh), each row `pitch` bytes after the previous
+// one, the frame at src + n * frame_stride bytes.
 #include "bevk_common.cuh"
-#include "warp_u8c3.cuh"
-#include "yuv_bgr.cuh"
+#include "yuv_src.cuh"
 
 namespace {
-
-__device__ __forceinline__ uint32_t border_bgr(const float *b)
-{
-    uint32_t px = 0;
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        // cv2: saturate_cast<uchar>(borderValue[c])
-        const int v = __float2int_rn(b[c]);
-        px |= (uint32_t)(v < 0 ? 0 : (v > 255 ? 255 : v)) << (8 * c);
-    }
-    return px;
-}
 
 // ---- fused warp -------------------------------------------------------------------------------
 // One lane per dst pixel, as warp_u8c3_direct_kernel (warp_generic.cu): the coordinate is computed
@@ -197,6 +186,86 @@ void launch_warp(const BevkNv12Params &P, bool packed, cudaStream_t stream)
         warp_nv12_kernel<LINEAR, WORDS, false, kBatch><<<grid, block, 0, stream>>>(P);
 }
 
+// warp_nv12_kernel over a source format S of yuv_src.cuh (S::make, S::load, S::math): the warp of
+// I420 frames.  NV12 frames keep warp_nv12_kernel, which holds the NV12 addressing of Nv12Src with
+// the window's border constants and straddle flags computed once per pixel; through Nv12Src the
+// bilinear instances took 48 instead of 40 registers and ran 3-7 % slower (DESIGN.md 3.11).
+template <class S, bool PACKED, int kBatch>
+__global__ void __launch_bounds__(256) warp_yuv_src_kernel(const __grid_constant__ BevkNv12Params P)
+{
+    const BevkWarpParams &p = P.w;
+    const int lane = threadIdx.x, x0 = blockIdx.x * 32;
+    const int x = x0 + lane, y = blockIdx.y * 8 + threadIdx.y;
+    if (y >= p.dst_h) return;  // a warp is one dst row segment: uniform exit, shuffles stay legal
+    int gi;
+    const BevkWarpGroup &g = find_group(p, blockIdx.z, gi);
+    const int c_local = blockIdx.z - g.chunk0;
+    const int f0 = c_local * p.frames_per_chunk;
+    const int f1 = min(f0 + p.frames_per_chunk, g.count);
+
+    const uint32_t bpx = border_bgr(p.border);
+    const typename S::Tap t = S::make(P, g.M, min(x, p.dst_w - 1), y, bpx);
+
+    const int j = lane >> 2, r4 = lane & 3;
+    const uint32_t sel_pack = r4 == 0 ? 0x4210u : (r4 == 1 ? 0x5421u : 0x6542u);
+    const bool st_ok = PACKED ? (r4 < 3 && 4 * j < min(32, p.dst_w - x0)) : x < p.dst_w;
+    uint8_t *dst = (uint8_t *)p.dst + ((long long)y * p.dst_w + x0) * 3 + (PACKED ? (3 * j + r4) * 4 : 3 * lane);
+    const uint8_t *src = (const uint8_t *)p.src;
+
+    auto load = [&](int f, uint32_t(&w)[S::kWords]) {
+        S::load(P, src + (long long)(g.first + f * g.stride) * P.frame_stride, t, w);
+    };
+    auto finish = [&](int f, const uint32_t(&w)[S::kWords]) {
+        const uint32_t P0 = S::math(t, w, bpx);
+        uint8_t *d = dst + (long long)(g.first + f * g.stride) * p.dst_frame_elems;
+        if (PACKED) {
+            const uint32_t word = prmt(P0, __shfl_down_sync(0xffffffffu, P0, 1), sel_pack);
+            if (st_ok) st_stream_free(reinterpret_cast<uint32_t *>(d), word);
+        } else if (st_ok) {
+            d[0] = (uint8_t)P0;
+            d[1] = (uint8_t)(P0 >> 8);
+            d[2] = (uint8_t)(P0 >> 16);
+        }
+    };
+    // the windows of kBatch frames are requested before the first one is converted
+    int f = f0;
+    for (; f + kBatch <= f1; f += kBatch) {
+        uint32_t w[kBatch][S::kWords];
+#pragma unroll
+        for (int u = 0; u < kBatch; ++u) load(f + u, w[u]);
+#pragma unroll
+        for (int u = 0; u < kBatch; ++u) finish(f + u, w[u]);
+    }
+    for (; f < f1; ++f) {
+        uint32_t w[S::kWords];
+        load(f, w);
+        finish(f, w);
+    }
+}
+
+template <class S, int kBatch>
+void launch_yuv_warp(const BevkNv12Params &P, bool packed, cudaStream_t stream)
+{
+    dim3 block(32, 8, 1);
+    dim3 grid((P.w.dst_w + 31) / 32, (P.w.dst_h + 7) / 8, P.w.total_chunks);
+    if (packed)
+        warp_yuv_src_kernel<S, true, kBatch><<<grid, block, 0, stream>>>(P);
+    else
+        warp_yuv_src_kernel<S, false, kBatch><<<grid, block, 0, stream>>>(P);
+}
+
+// the four kernels of a YUV source format: bilinear / nearest, word / byte gathers
+template <template <bool, bool> class S>
+void launch_yuv_src(const BevkNv12Params &P, bool words, bool packed, int linear, cudaStream_t stream)
+{
+    if (linear)
+        words ? launch_yuv_warp<S<true, true>, 2>(P, packed, stream)
+              : launch_yuv_warp<S<true, false>, 2>(P, packed, stream);
+    else
+        words ? launch_yuv_warp<S<false, true>, 4>(P, packed, stream)
+              : launch_yuv_warp<S<false, false>, 4>(P, packed, stream);
+}
+
 // ---- conversion -------------------------------------------------------------------------------
 // A thread owns a 2x2 luma block and its one U,V pair, for kRowPairs block rows 4 apart (all
 // loads issued before the first conversion); a warp covers 64 columns, i.e. 64 luma bytes per
@@ -292,11 +361,13 @@ nv12_to_bgr_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, i
 
 }  // namespace
 
-int bevk_launch_warp_nv12(const BevkNv12Params &P, int linear, cudaStream_t stream)
+int bevk_launch_warp_nv12(const BevkNv12Params &P, int src_format, int linear, cudaStream_t stream)
 {
     const bool words = ((uintptr_t)P.w.src % 4) == 0 && (P.pitch % 4) == 0 && (P.frame_stride % 4) == 0;
     const bool packed = (P.w.dst_w % 4) == 0 && ((uintptr_t)P.w.dst % 4) == 0;
-    if (linear)
+    if (src_format == BEVK_YUV_I420)
+        launch_yuv_src<I420Src>(P, words, packed, linear, stream);
+    else if (linear)
         words ? launch_warp<true, true>(P, packed, stream) : launch_warp<true, false>(P, packed, stream);
     else
         words ? launch_warp<false, true>(P, packed, stream) : launch_warp<false, false>(P, packed, stream);

@@ -7,15 +7,14 @@
 // Semantics: cv2 4.13.  BT.601 limited range in 20-bit fixed point; Y per pixel, U and V of a 2x2
 // block from its top-left pixel alone.  The warps compute each BEV pixel's BGR bit-exactly as
 // warp_generic.cu / nv12.cu do (cv2.warpPerspective, border colour included) and convert it in
-// registers.
+// registers.  Sources: BGR, NV12 or I420 frames.
 //
 // dst layout of frame n (both layouts): h luma rows, then h / 2 rows of chroma, each row `pitch`
 // bytes after the previous one, the frame at dst + n * frame_stride bytes.  NV12 chroma row r holds
 // the U, V pairs of block row r.  I420 chroma follows cv2's packing with a row step: U of block row
 // r at row h + r / 2, column (r % 2) * w / 2; V of block row r as U of block row r + h / 2.
 #include "bevk_common.cuh"
-#include "warp_u8c3.cuh"
-#include "yuv_bgr.cuh"
+#include "yuv_src.cuh"
 
 namespace {
 
@@ -134,56 +133,8 @@ bgr_to_yuv420_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst,
 // the chunk, its BGR value with the arithmetic of the BGR-output kernel for its source format; the
 // four values are converted in registers and only Y and the top-left pixel's U, V are stored.
 // A source format S provides the frame-invariant state of one pixel (S::Tap, S::make), the window
-// loads of one frame (S::load, S::kWords words) and the BGR value (S::math).
-
-__device__ __forceinline__ uint32_t border_bgr(const float *b)
-{
-    uint32_t px = 0;
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        // cv2: saturate_cast<uchar>(borderValue[c])
-        const int v = __float2int_rn(b[c]);
-        px |= (uint32_t)(v < 0 ? 0 : (v > 255 ? 255 : v)) << (8 * c);
-    }
-    return px;
-}
-
-// The clamped 2x2 window of warp_u8c3_direct_kernel / warp_nv12_kernel: first column / row and the
-// integer weights (0..32; nearest: 1 for the tap when it is inside) of its two columns / rows.
-template <bool LINEAR>
-__device__ __forceinline__ bool clamped_window(const BevkWarpParams &p, const double *M, int x, int y, int &cs,
-                                               int &rs, int &wc0, int &wc1, int &wr0, int &wr1)
-{
-    int X, Y;
-    bevk_map_pixel(M, x, y, p.bw0, LINEAR ? 32.0 : 1.0, X, Y);
-    if (LINEAR) {
-        window(bevk_sat16(X >> 5), X & 31, p.src_w, cs, wc0, wc1);
-        window(bevk_sat16(Y >> 5), Y & 31, p.src_h, rs, wr0, wr1);
-    } else {
-        const int sx = bevk_sat16(X), sy = bevk_sat16(Y);
-        const bool in = sx >= 0 && sx < p.src_w && sy >= 0 && sy < p.src_h;
-        cs = min(max(sx, 0), p.src_w - 1);
-        rs = min(max(sy, 0), p.src_h - 1);
-        wc0 = wr0 = in ? 1 : 0;
-        wc1 = wr1 = 0;
-    }
-    const bool act = (wc0 | wc1) != 0 && (wr0 | wr1) != 0;
-    if (!act) cs = rs = 0;  // the loads of an all-border pixel hit one cached line
-    return act;
-}
-
-// dp2a bilinear of warp_u8c3.cuh's lerp_xy with the border folded into the rounding constant:
-// wout = the weight of the taps outside the frame (x 64, cv2's scale doubled).
-__device__ __forceinline__ uint32_t lerp_border(uint32_t w0, uint32_t w1, uint32_t wout, uint32_t bpx, uint32_t xa,
-                                                uint32_t ya, uint32_t xb, uint32_t yb)
-{
-    const uint32_t t0 = __dp2a_lo(w1, xb, __dp2a_lo(w0, xa, 32768u + byte_of(bpx, 0) * wout));
-    const uint32_t t1 = __dp2a_hi(w1, xb, __dp2a_hi(w0, xa, 32768u + byte_of(bpx, 1) * wout));
-    const uint32_t t2 = __dp2a_lo(w1, yb, __dp2a_lo(w0, ya, 32768u + byte_of(bpx, 2) * wout));
-    return prmt(prmt(t0, t1, 0x4462u), t2, 0x7610u);
-}
-
-constexpr uint32_t kInside = 0xffffffffu;  // nearest: "the tap is inside", else the border colour
+// loads of one frame (S::load, S::kWords words) and the BGR value (S::math); the YUV sources
+// Nv12Src and I420Src are in yuv_src.cuh.
 
 // BGR frames, src, row and frame 4-byte aligned: warp_u8c3_direct_kernel's aligned word gathers
 template <bool LINEAR> struct BgrWords {
@@ -303,94 +254,6 @@ template <bool LINEAR> struct BgrBytes {
     }
 };
 
-// NV12 frames: warp_nv12_kernel's gathers (WORDS: src, pitch and frame stride 4-byte aligned) and
-// per-tap conversion
-template <bool LINEAR, bool WORDS> struct Nv12Src {
-    static constexpr int kWords = LINEAR ? (WORDS ? 8 : 4) : 2;
-    struct Tap {
-        uint32_t lo;    // luma row rs at column cs
-        uint32_t co;    // chroma row rs / 2 at the U of column cs
-        uint32_t co_b;  // the chroma row under window row 1
-        uint32_t odd;   // cs is odd: the right column uses the next U,V pair
-        uint32_t w0, w1, k;
-    };
-    static __device__ __forceinline__ Tap make(const BevkYuvParams &P, const double *M, int x, int y, uint32_t bpx)
-    {
-        int cs, rs, wc0, wc1, wr0, wr1;
-        const bool act = clamped_window<LINEAR>(P.w, M, x, y, cs, rs, wc0, wc1, wr0, wr1);
-        const uint32_t pitch = (uint32_t)P.pitch;
-        Tap t;
-        t.lo = (uint32_t)rs * pitch + (uint32_t)cs;
-        t.co = ((uint32_t)P.w.src_h + (uint32_t)(rs >> 1)) * pitch + 2u * (uint32_t)(cs >> 1);
-        t.co_b = t.co + ((rs & 1) ? pitch : 0u);
-        t.odd = cs & 1;
-        t.w0 = tap_weight(wc0, wr0) | (tap_weight(wc1, wr0) << 16);
-        t.w1 = tap_weight(wc0, wr1) | (tap_weight(wc1, wr1) << 16);
-        t.k = LINEAR ? 64u * (uint32_t)(1024 - (wc0 + wc1) * (wr0 + wr1)) : (act ? kInside : bpx);
-        return t;
-    }
-    static __device__ __forceinline__ void load(const BevkYuvParams &P, const uint8_t *s, const Tap &t,
-                                                uint32_t (&w)[kWords])
-    {
-        const uint32_t pitch = (uint32_t)P.pitch;
-        auto LD = [](const uint8_t *a) { return ldg_sparse(reinterpret_cast<const uint32_t *>(a)); };
-        auto B = [](const uint8_t *a) { return (uint32_t)__ldg(a); };
-        if (LINEAR && WORDS) {
-            // the second word of a row only when the 2 luma / 4 chroma bytes straddle it
-            const bool l_two = (t.lo & 3u) == 3u, c_two = (t.co & 3u) == 2u && t.odd;
-            const uint8_t *la = s + (t.lo & ~3u), *ca = s + (t.co & ~3u), *cb = s + (t.co_b & ~3u);
-            w[0] = LD(la);
-            w[1] = l_two ? LD(la + 4) : 0u;
-            w[2] = LD(la + pitch);
-            w[3] = l_two ? LD(la + pitch + 4) : 0u;
-            w[4] = LD(ca);
-            w[5] = c_two ? LD(ca + 4) : 0u;
-            w[6] = LD(cb);
-            w[7] = c_two ? LD(cb + 4) : 0u;
-        } else if (LINEAR) {
-            const uint8_t *la = s + t.lo, *ca = s + t.co, *cb = s + t.co_b;
-            const uint32_t cn = t.odd ? 2u : 0u;  // offset of the right column's U,V pair
-            w[0] = B(la) | (B(la + 1) << 8);
-            w[1] = B(la + pitch) | (B(la + pitch + 1) << 8);
-            w[2] = B(ca) | (B(ca + 1) << 8) | (B(ca + cn) << 16) | (B(ca + cn + 1) << 24);
-            w[3] = B(cb) | (B(cb + 1) << 8) | (B(cb + cn) << 16) | (B(cb + cn + 1) << 24);
-        } else if (WORDS) {
-            w[0] = LD(s + (t.lo & ~3u));
-            w[1] = LD(s + (t.co & ~3u));
-        } else {
-            w[0] = B(s + t.lo);
-            w[1] = B(s + t.co) | (B(s + t.co + 1) << 8);
-        }
-    }
-    static __device__ __forceinline__ uint32_t math(const Tap &t, const uint32_t (&w)[kWords], uint32_t bpx)
-    {
-        if (!LINEAR) {
-            const uint32_t Yw = WORDS ? byte_of(w[0], t.lo & 3u) : w[0];
-            const uint32_t Cw = WORDS ? (w[1] >> (8 * (t.co & 2u))) : w[1];
-            return t.k == kInside ? yuv_to_bgr(Yw, byte_of(Cw, 0), byte_of(Cw, 1)) : t.k;
-        }
-        uint32_t L0, L1, C0, C1;  // [Y Y' . .] of window rows 0 / 1, [U V U' V'] under them
-        if (WORDS) {
-            const uint32_t csel = t.odd ? 0x3210u : 0x1010u;
-            L0 = __funnelshift_r(w[0], w[1], 8 * (t.lo & 3u));
-            L1 = __funnelshift_r(w[2], w[3], 8 * (t.lo & 3u));
-            C0 = prmt(__funnelshift_r(w[4], w[5], 8 * (t.co & 3u)), 0u, csel);
-            C1 = prmt(__funnelshift_r(w[6], w[7], 8 * (t.co_b & 3u)), 0u, csel);
-        } else {
-            L0 = w[0];
-            L1 = w[1];
-            C0 = w[2];
-            C1 = w[3];
-        }
-        const uint32_t p00 = yuv_to_bgr(byte_of(L0, 0), byte_of(C0, 0), byte_of(C0, 1));
-        const uint32_t p01 = yuv_to_bgr(byte_of(L0, 1), byte_of(C0, 2), byte_of(C0, 3));
-        const uint32_t p10 = yuv_to_bgr(byte_of(L1, 0), byte_of(C1, 0), byte_of(C1, 1));
-        const uint32_t p11 = yuv_to_bgr(byte_of(L1, 1), byte_of(C1, 2), byte_of(C1, 3));
-        return lerp_border(t.w0, t.w1, t.k, bpx, prmt(p00, p01, 0x5140u), prmt(p00, p01, 0x0062u),
-                           prmt(p10, p11, 0x5140u), prmt(p10, p11, 0x0062u));
-    }
-};
-
 template <class S, bool NV12_OUT, int kBatch>
 __global__ void __launch_bounds__(256) warp_yuv420_kernel(const __grid_constant__ BevkYuvParams P)
 {
@@ -449,19 +312,26 @@ void launch_warp(const BevkYuvParams &P, bool nv12_out, cudaStream_t stream)
         warp_yuv420_kernel<S, false, kBatch><<<grid, block, 0, stream>>>(P);
 }
 
+// the four kernels of a YUV source format: bilinear / nearest, word / byte gathers
+template <template <bool, bool> class S>
+void launch_yuv_src(const BevkYuvParams &P, bool aligned, bool out, int linear, cudaStream_t stream)
+{
+    if (linear)
+        aligned ? launch_warp<S<true, true>, 1>(P, out, stream) : launch_warp<S<true, false>, 1>(P, out, stream);
+    else
+        aligned ? launch_warp<S<false, true>, 2>(P, out, stream) : launch_warp<S<false, false>, 2>(P, out, stream);
+}
+
 }  // namespace
 
-int bevk_launch_warp_yuv420(const BevkYuvParams &P, int nv12_src, int nv12_out, int linear, cudaStream_t stream)
+int bevk_launch_warp_yuv420(const BevkYuvParams &P, int src_format, int nv12_out, int linear, cudaStream_t stream)
 {
     const bool out = nv12_out != 0;
     const bool aligned = ((uintptr_t)P.w.src % 4) == 0 && (P.pitch % 4) == 0 && (P.frame_stride % 4) == 0;
-    if (nv12_src) {
-        if (linear)
-            aligned ? launch_warp<Nv12Src<true, true>, 1>(P, out, stream)
-                    : launch_warp<Nv12Src<true, false>, 1>(P, out, stream);
-        else
-            aligned ? launch_warp<Nv12Src<false, true>, 2>(P, out, stream)
-                    : launch_warp<Nv12Src<false, false>, 2>(P, out, stream);
+    if (src_format == BEVK_YUV_NV12) {
+        launch_yuv_src<Nv12Src>(P, aligned, out, linear, stream);
+    } else if (src_format == BEVK_YUV_I420) {
+        launch_yuv_src<I420Src>(P, aligned, out, linear, stream);
     } else {
         // word gathers: rows of a multiple of 4 bytes (both window rows share one word alignment)
         // and a 2x2 window inside the frame

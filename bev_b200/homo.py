@@ -308,6 +308,33 @@ def warp_nv12_img_to_bev_yuv420(frames, calib, bspec, layout="i420", flags=INTER
     return warp_perspective_nv12_yuv420(frames, H, (int(bspec.u_size), int(bspec.v_size)), layout, flags=flags)
 
 
+def warp_perspective_video_host(src, M, dsize, src_format="bgr", dst_format="i420", dst=None, flags=INTER_LINEAR,
+                                borderMode=BORDER_CONSTANT, borderValue=0, mat_index=None):
+    """The frame loop of vis_homo.py:85-111 for a CPU decoder and / or encoder: host frames in,
+    host BEVs out, each format "bgr", "i420" (planar yuv420p, what PyAV's ``to_ndarray(format=
+    "yuv420p")`` and ffmpeg ``-pix_fmt yuv420p`` pipes give and take) or "nv12".  Byte-identical to
+    cv2's chain for the pair: ``cv2.cvtColor(f, COLOR_YUV2BGR_I420 / _NV12)`` for a YUV source,
+    then ``cv2.warpPerspective(..., M, dsize, flags=flags, borderValue=borderValue)``, then
+    ``cv2.cvtColor(..., COLOR_BGR2YUV_I420)`` (or its NV12 relayout) for a YUV destination.
+
+    src / dst: numpy arrays or CPU tensors, uint8, contiguous; BGR (H, W, 3) / (N, H, W, 3), YUV
+    (H*3/2, W) / (N, H*3/2, W) with H and W even.  Pinned memory gives full speed; pageable works.
+    M, mat_index, flags and borderValue (B, G, R) as for :func:`warp_perspective`; dsize = (w, h),
+    both even for a YUV destination.  Only the source rows the homographies reference (and the
+    chroma rows under them) are uploaded, so a YUV frame moves half the bytes of a BGR one; copies
+    and kernels overlap.  Synchronous: returns when the BEVs are in the host buffer."""
+    return _native.warp_perspective_video_host(src, M, dsize, src_format, dst_format, dst, flags, borderMode,
+                                               borderValue, mat_index)
+
+
+def warp_img_to_bev_video_host(frames, calib, bspec, src_format="i420", dst_format="i420", flags=INTER_LINEAR):
+    """:func:`warp_img_to_bev` on host video frames for a CPU codec (vis_homo.py:61-63,85-111):
+    see :func:`warp_perspective_video_host`."""
+    H = compose_H_bev_img(calib, bspec)
+    return warp_perspective_video_host(frames, H, (int(bspec.u_size), int(bspec.v_size)), src_format, dst_format,
+                                       flags=flags)
+
+
 def warp_bev_to_img(bev_frames, calib, bspec, flags=INTER_LINEAR):
     """Inverse BEV -> image warp (north_star extension; same kernel, H inverted on the host)."""
     H = np.linalg.inv(compose_H_bev_img(calib, bspec))

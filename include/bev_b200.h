@@ -35,6 +35,8 @@ extern "C" {
 /* YUV 4:2:0 frame layouts (bevk_bgr_to_yuv420 and the warps to YUV) */
 #define BEVK_YUV_I420 0 /* cv2.COLOR_BGR2YUV_I420's: Y plane, U plane, V plane (libx264 / PyAV yuv420p) */
 #define BEVK_YUV_NV12 1 /* Y plane, then rows of interleaved U, V (what GPU video encoders take) */
+/* the third frame format of bevk_warp_perspective_video_host */
+#define BEVK_BGR 2 /* packed uint8 (h, w, 3), cv2's BGR image */
 
 /* element types */
 #define BEVK_U8 0
@@ -186,6 +188,27 @@ int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, 
                                       int64_t dst_frame_stride, const double *M, int n_mats,
                                       const int32_t *mat_index, int flags, int border_mode,
                                       const double *border_value, void *stream);
+
+/*
+ * The host-buffer warp of video frames for CPU codecs: the frame loop of vis_homo.py:85-111 with a
+ * CPU decoder and / or encoder (PyAV, an ffmpeg rawvideo pipe), whose native frames are planar
+ * yuv420p.  dst[i] is byte-identical to cv2's chain for the format pair:
+ *     cv2.cvtColor(src[i], COLOR_YUV2BGR_I420 / _NV12)     (YUV sources only)
+ *     cv2.warpPerspective(..., M[k], (dst_w, dst_h), flags, BORDER_CONSTANT, border_value)
+ *     cv2.cvtColor(..., COLOR_BGR2YUV_I420) or its NV12 relayout   (YUV destinations only)
+ *   src_format, dst_format  BEVK_BGR, BEVK_YUV_I420 or BEVK_YUV_NV12 (any of the nine pairs)
+ *   src, dst  HOST buffers (pinned for full speed, pageable works too), contiguous uint8 frames:
+ *             BGR [n_frames][h][w][3]; YUV [n_frames][h * 3 / 2][w] as cv2 lays it out (h, w even)
+ *   M, n_mats, mat_index, flags, border_mode and border_value (B, G, R) as for
+ *   bevk_warp_perspective.
+ * Like bevk_warp_perspective_host, only the source rows the homographies reference are uploaded
+ * (bevk_warp_host_rows), and for YUV sources the chroma rows under them, so a YUV frame moves 1.5
+ * instead of 3 bytes per pixel each way; copies and kernels overlap chunk by chunk.
+ */
+int bevk_warp_perspective_video_host(const void *src, int src_format, void *dst, int dst_format, int n_frames,
+                                     int src_h, int src_w, int dst_h, int dst_w, const double *M, int n_mats,
+                                     const int32_t *mat_index, int flags, int border_mode,
+                                     const double *border_value);
 
 /*
  * Roofline accounting helper (SURVEY.md 8d): number of distinct in-bounds source pixels that the

@@ -16,6 +16,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import bench  # noqa: E402
 from bev_b200 import _native, homo  # noqa: E402
+from oracle import yuv420_oracle  # noqa: E402
 
 
 def main():
@@ -592,11 +593,111 @@ def resize_nv12_area_bench(rounds=5):
         torch.cuda.empty_cache()
 
 
+def video_host_bench(rounds=5, n=256):
+    """Host video frames to host BEVs through bevk_warp_perspective_video_host (vis_homo.py:85-111
+    with a CPU codec): cfg 2, n pinned 1080p frames -> 1024^2 bilinear with the canonical map, for
+    every pair of frame formats that a CPU decoder / encoder / cv2 user takes.  Per route: the host
+    clock around the synchronous call (warm-up first, routes alternated in rounds), the bytes the
+    call moves up (the referenced row band, and the chroma rows under it) and down, the link ceiling
+    for those bytes (plain pinned copies up and down at the same time, as bench.py does for e2e),
+    and the route's share of it.  The kernel time per route is the sum of the device durations of
+    the kernels one call runs (torch.profiler: the I420-source kernels have no device entry point
+    to bracket with events).  Every route's output equals the device route on the same frames."""
+    import time
+    from torch.profiler import ProfilerActivity, profile
+    print("card: %s" % card(), flush=True)
+    dev = torch.device("cuda", 0)
+    H, ssize, dsize = bench.h_canon(1), (1920, 1080), (1024, 1024)
+    w, h, dw, dh = ssize[0], ssize[1], dsize[0], dsize[1]
+    r0, r1 = _native.warp_host_rows(ssize, dsize, H, 1)
+    rows, crows = r1 - r0 + 1, r1 // 2 - r0 // 2 + 1
+    up = {"bgr": 3 * w * rows, "i420": w * rows + w * crows, "nv12": w * rows + w * crows}
+    down = {"bgr": 3 * dw * dh, "i420": dw * dh * 3 // 2, "nv12": dw * dh * 3 // 2}
+    routes = [("bgr", "bgr"), ("bgr", "i420"), ("i420", "bgr"), ("i420", "i420"), ("nv12", "nv12")]
+    print("cfg2 x%d 1080p -> 1024^2 bilinear, uploaded rows [%d, %d]" % (n, r0, r1), flush=True)
+
+    g = torch.Generator().manual_seed(1234)
+    bgr = torch.randint(0, 256, (n, h, w, 3), dtype=torch.uint8, generator=g).pin_memory()
+    i420 = torch.randint(0, 256, (n, h * 3 // 2, w), dtype=torch.uint8, generator=g).pin_memory()
+    nv12 = torch.from_numpy(np.stack([yuv420_oracle.i420_to_nv12(f) for f in i420.numpy()])).pin_memory()
+    src = {"bgr": bgr, "i420": i420, "nv12": nv12}
+    out = {r: torch.empty((n, dh, dw, 3) if r[1] == "bgr" else (n, dh * 3 // 2, dw), dtype=torch.uint8).pin_memory()
+           for r in routes}
+
+    def call(r):
+        homo.warp_perspective_video_host(src[r[0]], H, dsize, r[0], r[1], dst=out[r])
+
+    for r in routes:  # warm-up: workspace allocations, module loads
+        call(r)
+    times = {r: [] for r in routes}
+    for _ in range(rounds):
+        for r in routes:
+            t0 = time.perf_counter()
+            call(r)
+            times[r].append((time.perf_counter() - t0) * 1e3)
+
+    # the device route on the same frames (I420 frames as their NV12 relayout)
+    for r in routes:
+        s = src["nv12" if r[0] == "i420" else r[0]].to(dev)
+        if r[0] == "bgr":
+            ref = (homo.warp_perspective(s, H, dsize) if r[1] == "bgr"
+                   else homo.warp_perspective_yuv420(s, H, dsize, r[1]))
+        else:
+            ref = (homo.warp_perspective_nv12(s, H, dsize) if r[1] == "bgr"
+                   else homo.warp_perspective_nv12_yuv420(s, H, dsize, r[1]))
+        assert torch.equal(ref.cpu(), out[r]), "%s -> %s differs from the device route" % r
+        del s, ref
+    torch.cuda.empty_cache()
+
+    # the link ceiling for each route's byte counts: plain pinned copies, both directions at once
+    flat = bgr.view(-1)
+    d_up = torch.empty(max(up.values()) * n, dtype=torch.uint8, device=dev)
+    d_dn = torch.empty(max(down.values()) * n, dtype=torch.uint8, device=dev)
+    h_dn = out[("bgr", "bgr")].view(-1)
+    s_up, s_dn = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
+
+    def ceiling(nu, nd):
+        best = None
+        for _ in range(3):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            with torch.cuda.stream(s_up):
+                d_up[:nu].copy_(flat[:nu], non_blocking=True)
+            with torch.cuda.stream(s_dn):
+                h_dn[:nd].copy_(d_dn[:nd], non_blocking=True)
+            s_up.synchronize()
+            s_dn.synchronize()
+            dt = (time.perf_counter() - t0) * 1e3
+            best = dt if best is None else min(best, dt)
+        return best
+
+    def kernel_ms(r):
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            call(r)
+        us = 0.0
+        for e in prof.key_averages():
+            if "warp" in e.key:
+                us += getattr(e, "self_device_time_total", None) or getattr(e, "self_cuda_time_total", 0.0)
+        return us / 1e3
+
+    for r in routes:
+        nu, nd = up[r[0]] * n, down[r[1]] * n
+        ceil = ceiling(nu, nd)
+        t = np.array(times[r])
+        med = float(np.median(t))
+        print("%s -> %s: median %.2f ms (min %.2f, max %.2f, spread %.1f %%), %.2f Gpix/s | H2D %.1f MB, D2H %.1f MB "
+              "per step, ceiling %.2f ms (%.1f GB/s both ways) -> %.1f %% of it | kernels %.2f ms"
+              % (r[0], r[1], med, t.min(), t.max(), 100.0 * (t.max() - t.min()) / med, n * dw * dh / med / 1e6,
+                 nu / 1e6, nd / 1e6, ceil, (nu + nd) / ceil / 1e6, 100.0 * ceil / med, kernel_ms(r)), flush=True)
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "nv12":
         nv12_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "yuv420":
         yuv420_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "video_host":
+        video_host_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_nv12":
         resize_nv12_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_area":
