@@ -40,6 +40,8 @@ SIGNATURES = {
                                             _dp]),
     "bevk_warp_perspective_video_host": (_c_int, [_vp, _c_int, _vp, _c_int] + [_c_int] * 5 + [_dp, _c_int, _i32p,
                                                                                        _c_int, _c_int, _dp]),
+    "bevk_warp_perspective_video_host_small": (_c_int, [_vp, _c_int, _vp, _c_int, _vp, _vp] + [_c_int] * 7
+                                               + [_dp, _dp, _c_int, _i32p, _c_int, _c_int, _c_int, _dp]),
     "bevk_warp_host_rows": (_c_int, [_c_int, _c_int, _c_int, _c_int, _dp, _c_int, _c_int, _ip]),
     "bevk_warp_set_path": (_c_int, [_c_int]),
     "bevk_warp_touched_pixels": (_c_i64, [_c_int, _c_int, _c_int, _c_int, _dp, _c_int, _ip]),
@@ -434,12 +436,12 @@ def warp_perspective_nv12_yuv420(src, M, dsize, layout="i420", dst=None, flags=1
 VIDEO_FORMATS = {"i420": 0, "nv12": 1, "bgr": 2}
 
 
-def _video_frames(a, fmt, what):
+def _video_frames(a, fmt, what, caller="warp_perspective_video_host"):
     """(frames view, n, h, w, batched) of a host BGR (H, W, 3) / (N, H, W, 3) or YUV 4:2:0
     (H*3/2, W) / (N, H*3/2, W) uint8 buffer (numpy array or CPU tensor)."""
     if hasattr(a, "detach"):
         if a.is_cuda:
-            raise ValueError("%s is on %s: warp_perspective_video_host takes host buffers" % (what, a.device))
+            raise ValueError("%s is on %s: %s takes host buffers" % (what, a.device, caller))
         a = a.detach().numpy()
     a = np.asarray(a)
     if a.dtype != np.uint8:
@@ -462,6 +464,19 @@ def _video_frames(a, fmt, what):
     return f, f.shape[0], rows // 3 * 2, w, a.ndim == 3
 
 
+def _host_out(dst, shape, what, caller="warp_perspective_video_host"):
+    """A new uint8 host array of this shape, or dst after checking that it is one."""
+    if dst is None:
+        return np.empty(shape, np.uint8)
+    if getattr(dst, "is_cuda", False):
+        raise ValueError("%s is on %s: %s takes host buffers" % (what, dst.device, caller))
+    out = _to_numpy(dst) if not isinstance(dst, np.ndarray) else dst
+    if out.shape != shape or out.dtype != np.uint8 or not out.flags["C_CONTIGUOUS"]:
+        raise ValueError("%s must be a C-contiguous uint8 array of shape %s, got %s %s"
+                         % (what, shape, out.dtype, out.shape))
+    return out
+
+
 def warp_perspective_video_host(src, M, dsize, src_format="bgr", dst_format="i420", dst=None, flags=1,
                                 borderMode=0, borderValue=0, mat_index=None):
     """Host-buffer warp between video frame formats ("bgr", "i420", "nv12"): src / dst are numpy
@@ -476,16 +491,7 @@ def warp_perspective_video_host(src, M, dsize, src_format="bgr", dst_format="i42
         raise ValueError("YUV 4:2:0 frames need an even width and height, got dsize %dx%d" % (dw, dh))
     Ms, idx = _prep_mats(M, n, mat_index)
     frame = (dh, dw, 3) if dst_format == "bgr" else (dh * 3 // 2, dw)
-    shape = (n,) + frame if batched else frame
-    if dst is None:
-        out = np.empty(shape, np.uint8)
-    else:
-        if getattr(dst, "is_cuda", False):
-            raise ValueError("dst is on %s: warp_perspective_video_host takes host buffers" % (dst.device,))
-        out = _to_numpy(dst) if not isinstance(dst, np.ndarray) else dst
-        if out.shape != shape or out.dtype != np.uint8 or not out.flags["C_CONTIGUOUS"]:
-            raise ValueError("dst must be a C-contiguous uint8 array of shape %s, got %s %s"
-                             % (shape, out.dtype, out.shape))
+    out = _host_out(dst, (n,) + frame if batched else frame, "dst")
     b = _border(borderValue)
     rc = lib().bevk_warp_perspective_video_host(
         _vp(s.ctypes.data), VIDEO_FORMATS[src_format], _vp(out.ctypes.data), VIDEO_FORMATS[dst_format], n, h, w,
@@ -493,6 +499,45 @@ def warp_perspective_video_host(src, M, dsize, src_format="bgr", dst_format="i42
         int(borderMode), _dptr(b))
     _check(rc, "bevk_warp_perspective_video_host")
     return dst if dst is not None else out
+
+
+def warp_perspective_video_host_small(src, M, M_small, dsize, small_size, src_format="bgr", dst_format="i420",
+                                      flags=1, interpolation=1, borderMode=0, borderValue=0, mat_index=None,
+                                      dst=None, small=None, dst_small=None):
+    """warp_perspective_video_host plus the small frames (BGR, small_size = (w, h)) and their BEVs
+    through M_small, from one upload of each frame.  Returns (dst, small, dst_small)."""
+    for name, fmt in (("src_format", src_format), ("dst_format", dst_format)):
+        if fmt not in VIDEO_FORMATS:
+            raise ValueError("%s must be 'bgr', 'i420' or 'nv12', got %r" % (name, fmt))
+    caller = "warp_perspective_video_host_small"
+    s, n, h, w, batched = _video_frames(src, src_format, "src", caller)
+    dw, dh = int(dsize[0]), int(dsize[1])
+    sw, sh = int(small_size[0]), int(small_size[1])
+    if dst_format != "bgr" and (dw % 2 or dh % 2):
+        raise ValueError("YUV 4:2:0 frames need an even width and height, got dsize %dx%d" % (dw, dh))
+    if interpolation not in (1, 3):
+        raise ValueError("interpolation must be INTER_LINEAR (1) or INTER_AREA (3), got %r" % (interpolation,))
+    Ms, idx = _prep_mats(M, n, mat_index)
+    Mss = np.ascontiguousarray(_to_numpy(M_small), dtype=np.float64)
+    if Mss.ndim == 2:
+        Mss = Mss[None]
+    if Mss.shape != Ms.shape:
+        raise ValueError("M_small must hold one 3x3 matrix per matrix of M, shape %s, got %s"
+                         % (Ms.shape, Mss.shape))
+    lead = (n,) if batched else ()
+    frame = (dh, dw, 3) if dst_format == "bgr" else (dh * 3 // 2, dw)
+    out = _host_out(dst, lead + frame, "dst", caller)
+    out_small = _host_out(small, lead + (sh, sw, 3), "small", caller)
+    out_bev_small = _host_out(dst_small, lead + frame, "dst_small", caller)
+    b = _border(borderValue)
+    rc = lib().bevk_warp_perspective_video_host_small(
+        _vp(s.ctypes.data), VIDEO_FORMATS[src_format], _vp(out.ctypes.data), VIDEO_FORMATS[dst_format],
+        _vp(out_small.ctypes.data), _vp(out_bev_small.ctypes.data), n, h, w, dh, dw, sh, sw, _dptr(Ms), _dptr(Mss),
+        Ms.shape[0], idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags), int(interpolation),
+        int(borderMode), _dptr(b))
+    _check(rc, "bevk_warp_perspective_video_host_small")
+    return (dst if dst is not None else out, small if small is not None else out_small,
+            dst_small if dst_small is not None else out_bev_small)
 
 
 def warp_touched_pixels(ssize, dsize, M, flags=1):

@@ -171,9 +171,10 @@ int bevk_launch_warp_nv12(const BevkNv12Params &P, int src_format, int linear, c
 int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int w, int pitch,
                             long long frame_stride, cudaStream_t stream);
 // cv2.resize of n_frames > 0 frames with `interpolation` (BEVK_INTER_LINEAR or BEVK_INTER_AREA):
-// uint8 frames with `channels` channels, or (nv12, channels 3) NV12 frames converted to BGR; rows
-// `pitch` and frames `frame_stride` bytes apart; arguments already checked by the entry points
-int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels, int nv12,
+// src_format BEVK_BGR, uint8 frames with `channels` channels, or BEVK_YUV_NV12 / BEVK_YUV_I420
+// (channels 3) YUV 4:2:0 frames converted to BGR; rows `pitch` and frames `frame_stride` bytes
+// apart; arguments already checked by the entry points
+int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels, int src_format,
                        long long pitch, long long frame_stride, int dst_h, int dst_w, int interpolation,
                        cudaStream_t stream);
 // BGR, NV12 or I420 frames (src_format BEVK_BGR / BEVK_YUV_NV12 / BEVK_YUV_I420) warped to YUV

@@ -353,9 +353,10 @@ void referenced_rows_union(const std::vector<double> &maps, int n_mats, const Wa
     }
 }
 
-// grow-only device workspace of the host-buffer entry point, one per device: kHostSlots chunks in
-// flight, each with its own stream and device buffers.  A workspace is only ever touched under its
-// own mutex and is never freed because another device is being used.
+// grow-only device workspace of the host-buffer entry points, one per device: kHostSlots chunks in
+// flight, each with its own stream and device buffers (d_dst holds every output of a chunk).  A
+// workspace is only ever touched under its own mutex and is never freed because another device is
+// being used.
 constexpr int kHostSlots = 3;
 struct HostWorkspace {
     std::mutex mu;
@@ -372,20 +373,54 @@ struct HostBand {
     size_t offset, bytes;
 };
 
+// One output of the host pipeline: host frames of frame_bytes each.
+struct HostOut {
+    void *host;
+    size_t frame_bytes;
+};
+
+// The (matrix, frame-run) groups of frames [f0, f0 + nf) of a host call: the chunk's slice of
+// mat_index, or of the per-frame matrices.
+void chunk_groups(const std::vector<double> &maps, int n_mats, const int32_t *mat_index, int f0, int nf,
+                  std::vector<BevkWarpGroup> &groups)
+{
+    groups.clear();
+    if (mat_index) {
+        const std::vector<int32_t> idx(mat_index + f0, mat_index + f0 + nf);
+        build_groups(nf, n_mats, idx.data(), maps, groups);
+    } else if (n_mats != 1) {  // one matrix per frame: this chunk's slice
+        const std::vector<double> chunk_maps(maps.begin() + (size_t)f0 * 9, maps.begin() + (size_t)(f0 + nf) * 9);
+        build_groups(nf, nf, nullptr, chunk_maps, groups);
+    } else {
+        build_groups(nf, 1, nullptr, maps, groups);
+    }
+}
+
 // The pipelined host-buffer warp of the n_frames > 0 frames of a: frames of src_frame_bytes, of which
-// only `bands` are uploaded, to frames of dst_frame_bytes.  Chunks of frames go through the device
+// only `bands` are uploaded, to one or more outputs.  Chunks of frames go through the device
 // workspace, kHostSlots at a time, so that the copies and kernels of neighbouring chunks overlap.
-// run(d_src, d_dst, args, groups, stream) enqueues the kernels of one chunk; maps are the dst->src
-// maps of all n_mats matrices.
+// run(d_src, d_out, args, f0, groups, stream) enqueues the kernels of the chunk that starts at frame
+// f0, where d_out[k] is the device buffer of outs[k] (256-byte aligned, its frames contiguous);
+// every output is then downloaded to its host buffer.  groups come from maps, the dst->src maps of
+// all n_mats matrices.
 template <typename Run>
-int host_pipeline(const void *src, void *dst, const WarpArgs &a, const std::vector<double> &maps, int n_mats,
-                  const int32_t *mat_index, size_t src_frame_bytes, size_t dst_frame_bytes,
-                  const std::vector<HostBand> &bands, Run run)
+int host_pipeline(const void *src, const WarpArgs &a, const std::vector<double> &maps, int n_mats,
+                  const int32_t *mat_index, size_t src_frame_bytes, const std::vector<HostBand> &bands,
+                  const std::vector<HostOut> &outs, Run run)
 {
     const int n_frames = a.n_frames;
-    int chunk = (int)std::max<size_t>(1, (size_t)(64u << 20) / std::max(src_frame_bytes, dst_frame_bytes));
+    size_t largest = src_frame_bytes;
+    for (const HostOut &o : outs) largest = std::max(largest, o.frame_bytes);
+    int chunk = (int)std::max<size_t>(1, (size_t)(64u << 20) / largest);
     chunk = std::min(chunk, std::max(1, (n_frames + 3) / 4));
     chunk = std::min(chunk, n_frames);
+    // the outputs' regions of a slot's d_dst
+    std::vector<size_t> out_off;
+    size_t dst_bytes = 0;
+    for (const HostOut &o : outs) {
+        out_off.push_back(dst_bytes);
+        dst_bytes += (o.frame_bytes * chunk + 255) / 256 * 256;
+    }
 
     int dev = 0;
     BEVK_CUDA(cudaGetDevice(&dev));
@@ -407,14 +442,14 @@ int host_pipeline(const void *src, void *dst, const WarpArgs &a, const std::vect
         for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA(cudaMalloc(&ws.d_src[i], src_frame_bytes * chunk));
         ws.src_cap = src_frame_bytes * chunk;
     }
-    if (ws.dst_cap < dst_frame_bytes * chunk) {
+    if (ws.dst_cap < dst_bytes) {
         for (int i = 0; i < kHostSlots; ++i) {
             if (ws.d_dst[i]) cudaFree(ws.d_dst[i]);
             ws.d_dst[i] = nullptr;
         }
         ws.dst_cap = 0;
-        for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA(cudaMalloc(&ws.d_dst[i], dst_frame_bytes * chunk));
-        ws.dst_cap = dst_frame_bytes * chunk;
+        for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA(cudaMalloc(&ws.d_dst[i], dst_bytes));
+        ws.dst_cap = dst_bytes;
     }
 
     // From the first enqueue on, every exit -- also an error exit -- first waits for the slot
@@ -442,29 +477,19 @@ int host_pipeline(const void *src, void *dst, const WarpArgs &a, const std::vect
                                               (const char *)src + (size_t)f0 * src_frame_bytes + b.offset,
                                               src_frame_bytes, b.bytes, nf, cudaMemcpyHostToDevice, st));
         std::vector<BevkWarpGroup> groups;
-        std::vector<int32_t> idx;
-        const int32_t *idx_ptr = nullptr;
-        std::vector<double> chunk_maps;
-        const std::vector<double> *use_maps = &maps;
-        int use_n_mats = n_mats;
-        if (mat_index) {
-            idx.assign(mat_index + f0, mat_index + f0 + nf);
-            idx_ptr = idx.data();
-        } else if (n_mats != 1) {  // one matrix per frame: this chunk's slice
-            chunk_maps.assign(maps.begin() + (size_t)f0 * 9, maps.begin() + (size_t)(f0 + nf) * 9);
-            use_maps = &chunk_maps;
-            use_n_mats = nf;
-        }
-        build_groups(nf, use_n_mats, idx_ptr, *use_maps, groups);
+        chunk_groups(maps, n_mats, mat_index, f0, nf, groups);
         WarpArgs ac = a;
         ac.n_frames = nf;
-        const int rc = run(ws.d_src[slot], ws.d_dst[slot], ac, groups, st);
+        std::vector<void *> d_out;
+        for (size_t k = 0; k < outs.size(); ++k) d_out.push_back((char *)ws.d_dst[slot] + out_off[k]);
+        const int rc = run(ws.d_src[slot], d_out.data(), ac, f0, groups, st);
         if (rc) {
             drain();
             return rc;
         }
-        BEVK_CUDA_DRAIN(cudaMemcpyAsync((char *)dst + (size_t)f0 * dst_frame_bytes, ws.d_dst[slot],
-                                        dst_frame_bytes * nf, cudaMemcpyDeviceToHost, st));
+        for (size_t k = 0; k < outs.size(); ++k)
+            BEVK_CUDA_DRAIN(cudaMemcpyAsync((char *)outs[k].host + (size_t)f0 * outs[k].frame_bytes, d_out[k],
+                                            outs[k].frame_bytes * nf, cudaMemcpyDeviceToHost, st));
     }
     for (int i = 0; i < kHostSlots; ++i) BEVK_CUDA_DRAIN(cudaStreamSynchronize(ws.stream[i]));
     return BEVK_OK;
@@ -529,23 +554,29 @@ int check_nv12_layout32(const char *what, int n_frames, int h, int w, int pitch,
     return BEVK_OK;
 }
 
-// The resize entry points after their frame-format checks: n_frames >= 0 frames of `channels`
-// uint8 channels, or NV12 frames (nv12, channels 3) converted to BGR; rows `pitch` and frames
-// `frame_stride` bytes apart.
-int resize_frames(const char *what, const void *src, void *dst, int n_frames, int src_h, int src_w, int channels,
-                  int nv12, long long pitch, long long frame_stride, int dst_h, int dst_w, int interpolation,
-                  void *stream)
+// The interpolation and sizes of a resize, checked before any device is looked for.
+int check_resize_args(const char *what, int src_h, int src_w, int dst_h, int dst_w, int interpolation)
 {
     if (interpolation != BEVK_INTER_LINEAR && interpolation != BEVK_INTER_AREA)
         BEVK_FAIL(BEVK_E_ARG, "%s: only INTER_LINEAR (cv2.resize's default) and INTER_AREA are implemented, got %d",
                   what, interpolation);
-    int rc = check_sizes(what, src_h, src_w, dst_h, dst_w);
+    return check_sizes(what, src_h, src_w, dst_h, dst_w);
+}
+
+// The resize entry points after their frame-format checks: n_frames >= 0 frames of `channels`
+// uint8 channels (src_format BEVK_BGR), or NV12 frames (BEVK_YUV_NV12, channels 3) converted to
+// BGR; rows `pitch` and frames `frame_stride` bytes apart.
+int resize_frames(const char *what, const void *src, void *dst, int n_frames, int src_h, int src_w, int channels,
+                  int src_format, long long pitch, long long frame_stride, int dst_h, int dst_w, int interpolation,
+                  void *stream)
+{
+    int rc = check_resize_args(what, src_h, src_w, dst_h, dst_w, interpolation);
     if (rc) return rc;
     if (n_frames > 0 && (!src || !dst)) BEVK_FAIL(BEVK_E_ARG, "%s: null src / dst", what);
     rc = bevk_require_device();
     if (rc) return rc;
     if (n_frames == 0) return BEVK_OK;
-    return bevk_launch_resize(src, dst, n_frames, src_h, src_w, channels, nv12, pitch, frame_stride, dst_h, dst_w,
+    return bevk_launch_resize(src, dst, n_frames, src_h, src_w, channels, src_format, pitch, frame_stride, dst_h, dst_w,
                               interpolation, (cudaStream_t)stream);
 }
 // The YUV 4:2:0 destinations (I420 or NV12 frames of h x w): even sizes, rows at least w bytes
@@ -620,6 +651,49 @@ int warp_yuv420(const char *what, const void *src, void *dst, int n_frames, int 
     build_groups(n_frames, n_mats, mat_index, maps, groups);
     return run_warp_yuv420(src, dst, a, groups, src_format, pitch, frame_stride, layout, dst_pitch, dst_frame_stride,
                            (cudaStream_t)stream);
+}
+
+// Bytes of one contiguous frame of h x w pixels in a video frame format.
+size_t video_frame_bytes(int format, int h, int w)
+{
+    return (size_t)w * h * (format == BEVK_BGR ? 2 : 1) * 3 / 2;
+}
+
+// The argument checks of the host video entry points: formats, even YUV sizes, frames below 4 GB
+// and the warp's own, before any device is looked for.
+int check_video_host(const char *what, const void *src, int src_format, void *dst, int dst_format, int n_frames,
+                     int src_h, int src_w, int dst_h, int dst_w, const double *M, int n_mats,
+                     const int32_t *mat_index, int flags, int border_mode, const double *border_value, WarpArgs &a)
+{
+    auto known = [](int f) { return f == BEVK_BGR || f == BEVK_YUV_I420 || f == BEVK_YUV_NV12; };
+    if (!known(src_format) || !known(dst_format))
+        BEVK_FAIL(BEVK_E_ARG, "%s: formats must be BEVK_YUV_I420 (0), BEVK_YUV_NV12 (1) or BEVK_BGR (2), got src %d, "
+                  "dst %d", what, src_format, dst_format);
+    int rc;
+    if (src_format != BEVK_BGR) {
+        rc = check_nv12_layout32(what, n_frames, src_h, src_w, src_w, (int64_t)src_w * src_h / 2 * 3);
+        if (rc) return rc;
+    }
+    if (dst_format != BEVK_BGR) {
+        rc = check_yuv420_dst(what, n_frames, dst_h, dst_w, dst_format, dst_w, (int64_t)dst_w * dst_h / 2 * 3);
+        if (rc) return rc;
+    }
+    return check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index, flags,
+                           border_mode, border_value, a);
+}
+
+// The warp of one chunk of contiguous video frames on the device, for a format pair.
+int run_video_warp(const void *src, void *dst, const WarpArgs &a, const std::vector<BevkWarpGroup> &groups,
+                   int src_format, int dst_format, cudaStream_t stream)
+{
+    const long long src_frame_bytes = (long long)video_frame_bytes(src_format, a.src_h, a.src_w);
+    if (dst_format != BEVK_BGR)
+        return run_warp_yuv420(src, dst, a, groups, src_format, src_format == BEVK_BGR ? 3LL * a.src_w : a.src_w,
+                               src_frame_bytes, dst_format, a.dst_w,
+                               (int64_t)video_frame_bytes(dst_format, a.dst_h, a.dst_w), stream);
+    if (src_format != BEVK_BGR)
+        return run_warp_yuv_bgr(src, dst, a, groups, src_format, a.src_w, src_frame_bytes, stream);
+    return run_warp_device(src, dst, a, groups, g_warp_path, stream);
 }
 }  // namespace
 
@@ -701,7 +775,7 @@ int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, 
     if (n_frames < 0) BEVK_FAIL(BEVK_E_ARG, "resize: n_frames must be >= 0");
     if (channels < 1 || channels > 4) BEVK_FAIL(BEVK_E_ARG, "resize: channels must be 1..4, got %d", channels);
     if (dtype != BEVK_U8) BEVK_FAIL(BEVK_E_ARG, "resize: only uint8 frames are implemented (dtype code %d)", dtype);
-    return resize_frames("resize", src, dst, n_frames, src_h, src_w, channels, 0, (long long)src_w * channels,
+    return resize_frames("resize", src, dst, n_frames, src_h, src_w, channels, BEVK_BGR, (long long)src_w * channels,
                          (long long)src_h * src_w * channels, dst_h, dst_w, interpolation, stream);
 }
 
@@ -717,8 +791,8 @@ int bevk_resize_nv12_interp(const void *src, void *dst, int n_frames, int src_h,
 {
     const int rc = check_nv12_layout32("resize_nv12", n_frames, src_h, src_w, pitch, frame_stride);
     if (rc) return rc;
-    return resize_frames("resize_nv12", src, dst, n_frames, src_h, src_w, 3, 1, pitch, frame_stride, dst_h, dst_w,
-                         interpolation, stream);
+    return resize_frames("resize_nv12", src, dst, n_frames, src_h, src_w, 3, BEVK_YUV_NV12, pitch, frame_stride, dst_h,
+                         dst_w, interpolation, stream);
 }
 
 int bevk_warp_host_rows(int src_h, int src_w, int dst_h, int dst_w, const double *M, int n_mats,
@@ -758,10 +832,12 @@ int bevk_warp_perspective_host(const void *src, void *dst, int n_frames, int src
     referenced_rows_union(maps, n_mats, a, r0, r1);
     const size_t row_bytes = (size_t)a.src_w * a.channels * a.elem_size;
     const size_t dst_frame_bytes = (size_t)a.dst_w * a.dst_h * a.channels * a.elem_size;
-    return host_pipeline(src, dst, a, maps, n_mats, mat_index, row_bytes * a.src_h, dst_frame_bytes,
-                         {{r0 * row_bytes, row_bytes * (size_t)(r1 - r0 + 1)}},
-                         [](const void *s, void *d, const WarpArgs &ac, const std::vector<BevkWarpGroup> &groups,
-                            cudaStream_t st) { return run_warp_device(s, d, ac, groups, g_warp_path, st); });
+    return host_pipeline(src, a, maps, n_mats, mat_index, row_bytes * a.src_h,
+                         {{r0 * row_bytes, row_bytes * (size_t)(r1 - r0 + 1)}}, {{dst, dst_frame_bytes}},
+                         [](const void *s, void *const *d, const WarpArgs &ac, int,
+                            const std::vector<BevkWarpGroup> &groups, cudaStream_t st) {
+                             return run_warp_device(s, d[0], ac, groups, g_warp_path, st);
+                         });
 }
 
 int bevk_warp_perspective_video_host(const void *src, int src_format, void *dst, int dst_format, int n_frames,
@@ -769,24 +845,9 @@ int bevk_warp_perspective_video_host(const void *src, int src_format, void *dst,
                                      const int32_t *mat_index, int flags, int border_mode,
                                      const double *border_value)
 {
-    const char *what = "warp_video_host";
-    auto known = [](int f) { return f == BEVK_BGR || f == BEVK_YUV_I420 || f == BEVK_YUV_NV12; };
-    if (!known(src_format) || !known(dst_format))
-        BEVK_FAIL(BEVK_E_ARG, "%s: formats must be BEVK_YUV_I420 (0), BEVK_YUV_NV12 (1) or BEVK_BGR (2), got src %d, "
-                  "dst %d", what, src_format, dst_format);
-    const bool yuv_src = src_format != BEVK_BGR, yuv_dst = dst_format != BEVK_BGR;
-    int rc;
-    if (yuv_src) {
-        rc = check_nv12_layout32(what, n_frames, src_h, src_w, src_w, (int64_t)src_w * src_h / 2 * 3);
-        if (rc) return rc;
-    }
-    if (yuv_dst) {
-        rc = check_yuv420_dst(what, n_frames, dst_h, dst_w, dst_format, dst_w, (int64_t)dst_w * dst_h / 2 * 3);
-        if (rc) return rc;
-    }
     WarpArgs a;
-    rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index, flags,
-                         border_mode, border_value, a);
+    int rc = check_video_host("warp_video_host", src, src_format, dst, dst_format, n_frames, src_h, src_w, dst_h,
+                              dst_w, M, n_mats, mat_index, flags, border_mode, border_value, a);
     if (rc) return rc;
     rc = bevk_require_device();
     if (rc) return rc;
@@ -798,13 +859,11 @@ int bevk_warp_perspective_video_host(const void *src, int src_format, void *dst,
     int r0, r1;
     referenced_rows_union(maps, n_mats, a, r0, r1);
     const size_t h = (size_t)src_h, w = (size_t)src_w, rows = (size_t)(r1 - r0 + 1);
-    size_t src_frame_bytes;
+    const size_t src_frame_bytes = video_frame_bytes(src_format, src_h, src_w);
     std::vector<HostBand> bands;
-    if (!yuv_src) {
-        src_frame_bytes = 3 * w * h;
+    if (src_format == BEVK_BGR) {
         bands.push_back({3 * w * r0, 3 * w * rows});
     } else {
-        src_frame_bytes = w * h / 2 * 3;
         bands.push_back({w * r0, w * rows});
         const size_t c0 = (size_t)(r0 / 2), nc = (size_t)(r1 / 2) - c0 + 1;
         if (src_format == BEVK_YUV_NV12) {
@@ -815,18 +874,59 @@ int bevk_warp_perspective_video_host(const void *src, int src_format, void *dst,
             bands.push_back({w * h + cw * (h / 2 + c0), cw * nc});
         }
     }
-    const size_t dst_frame_bytes = (size_t)dst_w * dst_h * (yuv_dst ? 1 : 2) * 3 / 2;
-    const long long pitch = yuv_src ? src_w : 3LL * src_w;
-    return host_pipeline(src, dst, a, maps, n_mats, mat_index, src_frame_bytes, dst_frame_bytes, bands,
-                         [&](const void *s, void *d, const WarpArgs &ac, const std::vector<BevkWarpGroup> &groups,
-                             cudaStream_t st) -> int {
-                             if (yuv_dst)
-                                 return run_warp_yuv420(s, d, ac, groups, src_format, pitch, src_frame_bytes,
-                                                        dst_format, dst_w, dst_frame_bytes, st);
-                             if (yuv_src)
-                                 return run_warp_yuv_bgr(s, d, ac, groups, src_format, src_w, src_frame_bytes, st);
-                             return run_warp_device(s, d, ac, groups, g_warp_path, st);
+    const size_t dst_frame_bytes = video_frame_bytes(dst_format, dst_h, dst_w);
+    return host_pipeline(src, a, maps, n_mats, mat_index, src_frame_bytes, bands, {{dst, dst_frame_bytes}},
+                         [&](const void *s, void *const *d, const WarpArgs &ac, int,
+                             const std::vector<BevkWarpGroup> &groups, cudaStream_t st) {
+                             return run_video_warp(s, d[0], ac, groups, src_format, dst_format, st);
                          });
+}
+
+int bevk_warp_perspective_video_host_small(const void *src, int src_format, void *dst, int dst_format, void *small,
+                                           void *dst_small, int n_frames, int src_h, int src_w, int dst_h, int dst_w,
+                                           int small_h, int small_w, const double *M, const double *M_small,
+                                           int n_mats, const int32_t *mat_index, int flags, int interpolation,
+                                           int border_mode, const double *border_value)
+{
+    const char *what = "warp_video_host_small";
+    WarpArgs a;
+    int rc = check_video_host(what, src, src_format, dst, dst_format, n_frames, src_h, src_w, dst_h, dst_w, M, n_mats,
+                              mat_index, flags, border_mode, border_value, a);
+    if (rc) return rc;
+    rc = check_resize_args(what, src_h, src_w, small_h, small_w, interpolation);
+    if (rc) return rc;
+    if (!M_small) BEVK_FAIL(BEVK_E_ARG, "%s: M_small is required (one small-frame matrix per matrix of M)", what);
+    if (n_frames > 0 && (!small || !dst_small)) BEVK_FAIL(BEVK_E_ARG, "%s: null small / dst_small", what);
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    std::vector<double> maps, maps_small;
+    effective_maps(M, n_mats, flags, maps);
+    effective_maps(M_small, n_mats, flags, maps_small);
+
+    // the resize reads every row: whole frames go up
+    const size_t src_frame_bytes = video_frame_bytes(src_format, src_h, src_w);
+    const size_t dst_frame_bytes = video_frame_bytes(dst_format, dst_h, dst_w);
+    const size_t small_frame_bytes = video_frame_bytes(BEVK_BGR, small_h, small_w);
+    const long long pitch = src_format == BEVK_BGR ? 3LL * src_w : src_w;
+    return host_pipeline(
+        src, a, maps, n_mats, mat_index, src_frame_bytes, {{0, src_frame_bytes}},
+        {{dst, dst_frame_bytes}, {small, small_frame_bytes}, {dst_small, dst_frame_bytes}},
+        [&](const void *s, void *const *d, const WarpArgs &ac, int f0, const std::vector<BevkWarpGroup> &groups,
+            cudaStream_t st) -> int {
+            // the small BGR frames (d[1]) are downloaded and are the source of the small warp
+            int rc = bevk_launch_resize(s, d[1], ac.n_frames, src_h, src_w, 3, src_format, pitch,
+                                        (long long)src_frame_bytes, small_h, small_w, interpolation, st);
+            if (rc) return rc;
+            rc = run_video_warp(s, d[0], ac, groups, src_format, dst_format, st);
+            if (rc) return rc;
+            std::vector<BevkWarpGroup> groups_small;
+            chunk_groups(maps_small, n_mats, mat_index, f0, ac.n_frames, groups_small);
+            WarpArgs as = ac;
+            as.src_h = small_h;
+            as.src_w = small_w;
+            return run_video_warp(d[1], d[2], as, groups_small, BEVK_BGR, dst_format, st);
+        });
 }
 
 }  // extern "C"

@@ -1,6 +1,6 @@
 // resize.cu -- batched cv2.resize of uint8 frames for sm_100a, INTER_LINEAR and INTER_AREA, from 1 to
-// 4-channel frames or fused with the NV12 -> BGR conversion for frames from a GPU video decoder:
-// cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12), dsize, interpolation).  INTER_LINEAR is the
+// 4-channel frames or fused with the NV12 / I420 -> BGR conversion for frames from a GPU or CPU
+// video decoder: cv2.resize(cv2.cvtColor(f, COLOR_YUV2BGR_NV12 / _I420), dsize, interpolation).  INTER_LINEAR is the
 // small-frame path of the reference's frame loop, `img_small = cv2.resize(img, (new_u, new_v))`
 // (vis_homo.py:90), whose result feeds the second warp at vis_homo.py:91 through the homography of
 // Calib.scale(align_corners=False) (bev/calib.py:142-198).  INTER_AREA is what OpenCV recommends
@@ -30,15 +30,15 @@
 //   any axis upscales: the bilinear resize above with the area coefficients
 //           sx = floor(dx * scale), fx = float((dx + 1) - (sx + 1) / scale),
 //           fx = fx <= 0 ? 0 : fx - floor(fx) (linear_area_coef).
-// An NV12 tap is converted to BGR with cv2's arithmetic (yuv_bgr.cuh) on its own, then
+// An NV12 or I420 tap is converted to BGR with cv2's arithmetic (yuv_bgr.cuh) on its own, then
 // interpolated.  The coefficients are recomputed per thread from (dx, dy) with unfused IEEE float /
 // double operations (the library is built with -fmad=false) -- no tables to upload, nothing to
 // keep alive across the asynchronous launch -- and amortised over the frames of the thread's chunk.
 //
 // One thread per dst pixel in every kernel.  The bilinear kernels take the coefficient rule as a
 // template parameter: a word-gather one for BGR frames (3 aligned words per window row, dp2a for
-// the horizontal pass, 32 pixels packed into one 96-byte store per warp), one for NV12 frames, and
-// a byte-wise one for every other channel count / width.  They are HBM-bound: every source row a
+// the horizontal pass, 32 pixels packed into one 96-byte store per warp), one each for NV12 and I420
+// frames, and a byte-wise one for every other channel count / width.  They are HBM-bound: every source row a
 // dst row references is read once (sector-wise), the small frame written once.  The area kernel
 // runs the other two INTER_AREA branches with byte loads.
 #include <cfloat>
@@ -278,6 +278,122 @@ __global__ void __launch_bounds__(256) resize_nv12_kernel(const __grid_constant_
     }
 }
 
+// ---- I420 frames to BGR ------------------------------------------------------------------------
+// Layout of frame n: luma rows 0..src_h-1, then the U plane and the V plane of (src_h / 2) x
+// (src_w / 2) bytes packed as cv2 packs them (yuv_src.cuh): U of block row r at row src_h + r / 2,
+// column (r % 2) * src_w / 2; V of block row r as U of block row r + src_h / 2.  cv2 converts I420
+// with the NV12 arithmetic, so resize_nv12_kernel's window, conversion and passes apply unchanged;
+// only the chroma gather differs: per window row the U and V samples of chroma columns cs / 2 and
+// (cs + 1) / 2, 1 byte each (an even cs: both columns share it) or 2 (an odd cs).  WORDS: aligned
+// words + funnel shifts as I420Src, the next word only when a 2-byte segment straddles it.  Kept
+// apart from resize_nv12_kernel so that kernel's register allocation and SASS stay as they are.
+template <bool AREA, bool WORDS, bool PACKED, int kBatch>
+__global__ void __launch_bounds__(256) resize_i420_kernel(const __grid_constant__ BevkResizeParams p)
+{
+    const int lane = threadIdx.x, x0 = blockIdx.x * 32;
+    const int x = x0 + lane, y = blockIdx.y * 8 + threadIdx.y;
+    if (y >= p.dst_h) return;  // a warp is one dst row segment: uniform exit, shuffles stay legal
+    int sx, a0, a1, sy, b0, b1;
+    bilinear_coef<AREA>(p, min(x, p.dst_w - 1), y, sx, a0, a1, sy, b0, b1);
+    const int cs = min(sx, p.src_w - 2);
+    const int wa = cs == sx ? a0 : a1, wb = cs == sx ? a1 : a0;  // sx == src_w - 1 has a1 == 0
+    const uint32_t w16 = (uint32_t)wa | ((uint32_t)wb << 16);
+    const int r0 = min(max(sy, 0), p.src_h - 1), r1 = min(max(sy + 1, 0), p.src_h - 1);
+    const uint32_t pitch = (uint32_t)p.pitch;
+    const uint32_t lo = (uint32_t)r0 * pitch + (uint32_t)cs;
+    const uint32_t l1 = (uint32_t)(r1 - r0) * pitch;
+    // byte offset of the U sample of block row r at chroma column cs / 2
+    const uint32_t c = (uint32_t)cs >> 1, vr = (uint32_t)p.src_h >> 1;
+    auto u_at = [&](uint32_t r) {
+        return ((uint32_t)p.src_h + (r >> 1)) * pitch + (r & 1u) * ((uint32_t)p.src_w >> 1) + c;
+    };
+    const uint32_t ca = (uint32_t)r0 >> 1, cb = (uint32_t)r1 >> 1;
+    const uint32_t co[4] = {u_at(ca), u_at(ca + vr), u_at(cb), u_at(cb + vr)};  // U0 V0 U1 V1
+    const uint32_t odd = cs & 1;
+    const bool l_two = (lo & 3u) == 3u;
+
+    const int j = lane >> 2, r4 = lane & 3;
+    const uint32_t sel_pack = r4 == 0 ? 0x4210u : (r4 == 1 ? 0x5421u : 0x6542u);
+    const bool st_ok = PACKED ? (r4 < 3 && 4 * j < min(32, p.dst_w - x0)) : x < p.dst_w;
+    uint8_t *dst = p.dst + ((long long)y * p.dst_w + x0) * 3 + (PACKED ? (3 * j + r4) * 4 : 3 * lane);
+
+    constexpr int kWords = WORDS ? 12 : 4;
+    auto LD = [](const uint8_t *a) { return ldg_sparse(reinterpret_cast<const uint32_t *>(a)); };
+    auto B = [](const uint8_t *a) { return (uint32_t)__ldg(a); };
+    auto load = [&](int f, uint32_t(&w)[kWords]) {
+        const uint8_t *s = p.src + (long long)f * p.src_frame;
+        if (WORDS) {
+            const uint8_t *la = s + (lo & ~3u);
+            w[0] = LD(la);
+            w[1] = l_two ? LD(la + 4) : 0u;
+            w[2] = LD(la + l1);
+            w[3] = l_two ? LD(la + l1 + 4) : 0u;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                const uint8_t *a = s + (co[i] & ~3u);
+                w[4 + 2 * i] = LD(a);
+                w[5 + 2 * i] = (odd && (co[i] & 3u) == 3u) ? LD(a + 4) : 0u;
+            }
+        } else {
+            const uint8_t *la = s + lo;
+            w[0] = B(la) | (B(la + 1) << 8);
+            w[1] = B(la + l1) | (B(la + l1 + 1) << 8);
+            w[2] = B(s + co[0]) | (B(s + co[1]) << 8) | (B(s + co[0] + odd) << 16) | (B(s + co[1] + odd) << 24);
+            w[3] = B(s + co[2]) | (B(s + co[3]) << 8) | (B(s + co[2] + odd) << 16) | (B(s + co[3] + odd) << 24);
+        }
+    };
+    auto finish = [&](int f, const uint32_t(&w)[kWords]) {
+        uint32_t L0, L1, C0, C1;  // [Y Y' . .] of window rows 0 / 1, [U V U' V'] under them
+        if (WORDS) {
+            // [U U' . .] and [V V' . .] of one chroma row -> [U V U' V'] (U V U V when cs is even)
+            const uint32_t csel = odd ? 0x5140u : 0x4040u;
+            L0 = __funnelshift_r(w[0], w[1], 8 * (lo & 3u));
+            L1 = __funnelshift_r(w[2], w[3], 8 * (lo & 3u));
+            C0 = prmt(__funnelshift_r(w[4], w[5], 8 * (co[0] & 3u)), __funnelshift_r(w[6], w[7], 8 * (co[1] & 3u)),
+                      csel);
+            C1 = prmt(__funnelshift_r(w[8], w[9], 8 * (co[2] & 3u)), __funnelshift_r(w[10], w[11], 8 * (co[3] & 3u)),
+                      csel);
+        } else {
+            L0 = w[0];
+            L1 = w[1];
+            C0 = w[2];
+            C1 = w[3];
+        }
+        const uint32_t p00 = yuv_to_bgr(byte_of(L0, 0), byte_of(C0, 0), byte_of(C0, 1));
+        const uint32_t p01 = yuv_to_bgr(byte_of(L0, 1), byte_of(C0, 2), byte_of(C0, 3));
+        const uint32_t p10 = yuv_to_bgr(byte_of(L1, 0), byte_of(C1, 0), byte_of(C1, 1));
+        const uint32_t p11 = yuv_to_bgr(byte_of(L1, 1), byte_of(C1, 2), byte_of(C1, 3));
+        const uint32_t xa = prmt(p00, p01, 0x5140u), ya = prmt(p00, p01, 0x0062u);
+        const uint32_t xb = prmt(p10, p11, 0x5140u), yb = prmt(p10, p11, 0x0062u);
+        const int s00 = __dp2a_lo(w16, xa, 0u), s01 = __dp2a_hi(w16, xa, 0u), s02 = __dp2a_lo(w16, ya, 0u);
+        const int s10 = __dp2a_lo(w16, xb, 0u), s11 = __dp2a_hi(w16, xb, 0u), s12 = __dp2a_lo(w16, yb, 0u);
+        const uint32_t P0 = vpass(b0, b1, s00, s10) | (vpass(b0, b1, s01, s11) << 8) | (vpass(b0, b1, s02, s12) << 16);
+        uint8_t *d = dst + (long long)f * p.dst_frame;
+        if (PACKED) {
+            const uint32_t word = prmt(P0, __shfl_down_sync(0xffffffffu, P0, 1), sel_pack);
+            if (st_ok) st_stream_free(reinterpret_cast<uint32_t *>(d), word);
+        } else if (st_ok) {
+            d[0] = (uint8_t)P0;
+            d[1] = (uint8_t)(P0 >> 8);
+            d[2] = (uint8_t)(P0 >> 16);
+        }
+    };
+    const int f0 = blockIdx.z * p.frames_per_chunk, f1 = min(f0 + p.frames_per_chunk, p.n_frames);
+    int f = f0;
+    for (; f + kBatch <= f1; f += kBatch) {
+        uint32_t w[kBatch][kWords];
+#pragma unroll
+        for (int u = 0; u < kBatch; ++u) load(f + u, w[u]);
+#pragma unroll
+        for (int u = 0; u < kBatch; ++u) finish(f + u, w[u]);
+    }
+    for (; f < f1; ++f) {
+        uint32_t w[kWords];
+        load(f, w);
+        finish(f, w);
+    }
+}
+
 // ---- INTER_AREA downscales: integer cells (FAST) and general cells ------------------------------
 // The entries of computeResizeAreaTab for dst position d along one axis: source indices s0 ..
 // s0 + n - 1, alpha a_first for the first, a_last for the last and a_mid for the others.
@@ -334,14 +450,33 @@ template <int C, bool NV12> struct Row {
     }
 };
 
+// One source row of an I420 frame: luma row y, and the U and V rows of its block row y / 2 (cv2's
+// packing, see resize_i420_kernel).
+struct RowI420 {
+    const uint8_t *l, *u, *v;
+    __device__ __forceinline__ RowI420(const uint8_t *s, const BevkResizeParams &p, int y)
+    {
+        const long long r = y >> 1, rv = r + (p.src_h >> 1), half = p.src_w >> 1;
+        l = s + (long long)y * p.pitch;
+        u = s + (p.src_h + (r >> 1)) * p.pitch + (r & 1) * half;
+        v = s + (p.src_h + (rv >> 1)) * p.pitch + (rv & 1) * half;
+    }
+    __device__ __forceinline__ void px(int x, int (&c)[3]) const
+    {
+        const uint32_t bgr = yuv_to_bgr(__ldg(l + x), __ldg(u + (x >> 1)), __ldg(v + (x >> 1)));
+        c[0] = (int)(bgr & 0xffu);
+        c[1] = (int)((bgr >> 8) & 0xffu);
+        c[2] = (int)(bgr >> 16);
+    }
+};
+
 __device__ __forceinline__ uint8_t sat_round(float v) { return (uint8_t)min(max(__float2int_rn(v), 0), 255); }
 
 // Each thread computes its tap window once per frame chunk and reads its taps with byte loads,
-// which serve any alignment and pitch; an NV12 tap is converted to BGR where it is read.
-template <int C, bool NV12, bool FAST>
-__global__ void __launch_bounds__(256) resize_area_kernel(const __grid_constant__ BevkResizeParams p)
+// which serve any alignment and pitch; a YUV tap is converted to BGR where it is read.  R is the
+// row type of the frame layout: Row<C, NV12> or RowI420.
+template <int C, class R, bool FAST> __device__ __forceinline__ void area_cells(const BevkResizeParams &p)
 {
-    static_assert(!NV12 || C == 3, "NV12 frames convert to BGR");
     const int x = blockIdx.x * 32 + threadIdx.x, y = blockIdx.y * 8 + threadIdx.y;
     if (x >= p.dst_w || y >= p.dst_h) return;
     const long long od = ((long long)y * p.dst_w + x) * C;
@@ -354,7 +489,7 @@ __global__ void __launch_bounds__(256) resize_area_kernel(const __grid_constant_
             const uint8_t *s = p.src + f * p.src_frame;
             int acc[C] = {};
             for (int j = 0; j < p.ky; ++j) {
-                const Row<C, NV12> r(s, p, sy0 + j);
+                const R r(s, p, sy0 + j);
                 for (int i = 0; i < p.kx; ++i) {
                     int v[C];
                     r.px(sx0 + i, v);
@@ -373,7 +508,7 @@ __global__ void __launch_bounds__(256) resize_area_kernel(const __grid_constant_
             const uint8_t *s = p.src + f * p.src_frame;
             float sum[C] = {};
             for (int j = 0; j < ay.n; ++j) {
-                const Row<C, NV12> r(s, p, ay.s0 + j);
+                const R r(s, p, ay.s0 + j);
                 float buf[C] = {};
                 for (int i = 0; i < ax.n; ++i) {
                     const float alpha = area_alpha(ax, i);
@@ -394,17 +529,39 @@ __global__ void __launch_bounds__(256) resize_area_kernel(const __grid_constant_
     }
 }
 
+template <int C, bool NV12, bool FAST>
+__global__ void __launch_bounds__(256) resize_area_kernel(const __grid_constant__ BevkResizeParams p)
+{
+    static_assert(!NV12 || C == 3, "NV12 frames convert to BGR");
+    area_cells<C, Row<C, NV12>, FAST>(p);
+}
+
+template <bool FAST>
+__global__ void __launch_bounds__(256) resize_area_i420_kernel(const __grid_constant__ BevkResizeParams p)
+{
+    area_cells<3, RowI420, FAST>(p);
+}
+
 // ---- launch ------------------------------------------------------------------------------------
 const dim3 kBlock(32, 8, 1);
 
 template <bool AREA>
-void launch_bilinear(const BevkResizeParams &p, int channels, bool nv12, dim3 grid, cudaStream_t st)
+void launch_bilinear(const BevkResizeParams &p, int channels, int src_format, dim3 grid, cudaStream_t st)
 {
-    if (nv12) {
+    if (src_format != BEVK_BGR) {
         constexpr int kBatch = 2;
         const bool words = ((uintptr_t)p.src % 4) == 0 && (p.pitch % 4) == 0 && (p.src_frame % 4) == 0;
         const bool packed = (p.dst_w % 4) == 0 && ((uintptr_t)p.dst % 4) == 0;
-        if (words && packed)
+        if (src_format == BEVK_YUV_I420) {
+            if (words && packed)
+                resize_i420_kernel<AREA, true, true, kBatch><<<grid, kBlock, 0, st>>>(p);
+            else if (words)
+                resize_i420_kernel<AREA, true, false, kBatch><<<grid, kBlock, 0, st>>>(p);
+            else if (packed)
+                resize_i420_kernel<AREA, false, true, kBatch><<<grid, kBlock, 0, st>>>(p);
+            else
+                resize_i420_kernel<AREA, false, false, kBatch><<<grid, kBlock, 0, st>>>(p);
+        } else if (words && packed)
             resize_nv12_kernel<AREA, true, true, kBatch><<<grid, kBlock, 0, st>>>(p);
         else if (words)
             resize_nv12_kernel<AREA, true, false, kBatch><<<grid, kBlock, 0, st>>>(p);
@@ -428,9 +585,14 @@ void launch_bilinear(const BevkResizeParams &p, int channels, bool nv12, dim3 gr
     }
 }
 
-template <bool FAST> void launch_area(const BevkResizeParams &p, int channels, bool nv12, dim3 grid, cudaStream_t st)
+template <bool FAST>
+void launch_area(const BevkResizeParams &p, int channels, int src_format, dim3 grid, cudaStream_t st)
 {
-    if (nv12) {
+    if (src_format == BEVK_YUV_I420) {
+        resize_area_i420_kernel<FAST><<<grid, kBlock, 0, st>>>(p);
+        return;
+    }
+    if (src_format == BEVK_YUV_NV12) {
         resize_area_kernel<3, true, FAST><<<grid, kBlock, 0, st>>>(p);
         return;
     }
@@ -451,7 +613,7 @@ bool integer_scale(double scale, int &k)
 
 }  // namespace
 
-int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels, int nv12,
+int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int channels, int src_format,
                        long long pitch, long long frame_stride, int dst_h, int dst_w, int interpolation,
                        cudaStream_t stream)
 {
@@ -463,16 +625,16 @@ int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int 
     // cv2's branch first, then the kernel for the frame layout
     int kx, ky;
     if (interpolation != BEVK_INTER_AREA) {
-        launch_bilinear<false>(p, channels, nv12, grid, stream);
+        launch_bilinear<false>(p, channels, src_format, grid, stream);
     } else if (p.scale_x < 1 || p.scale_y < 1) {
-        launch_bilinear<true>(p, channels, nv12, grid, stream);
+        launch_bilinear<true>(p, channels, src_format, grid, stream);
     } else if (integer_scale(p.scale_x, kx) && integer_scale(p.scale_y, ky)) {
         p.kx = kx;
         p.ky = ky;
         p.inv_area = 1.f / (float)(kx * ky);
-        launch_area<true>(p, channels, nv12, grid, stream);
+        launch_area<true>(p, channels, src_format, grid, stream);
     } else {
-        launch_area<false>(p, channels, nv12, grid, stream);
+        launch_area<false>(p, channels, src_format, grid, stream);
     }
     BEVK_CUDA(cudaGetLastError());
     return BEVK_OK;

@@ -335,6 +335,42 @@ def warp_img_to_bev_video_host(frames, calib, bspec, src_format="i420", dst_form
                                        flags=flags)
 
 
+def warp_perspective_video_host_small(src, M, M_small, dsize, small_size, src_format="bgr", dst_format="i420",
+                                      flags=INTER_LINEAR, interpolation=INTER_LINEAR, borderValue=0, mat_index=None,
+                                      dst=None, small=None, dst_small=None):
+    """:func:`warp_perspective_video_host` together with the small-frame leg of vis_homo.py:90-91,
+    from one upload of each frame.  Returns ``(bev, small, bev_small)`` as host arrays:
+
+    - ``bev``: what :func:`warp_perspective_video_host` returns for the same arguments;
+    - ``small``: (h, w, 3) or (N, h, w, 3) BGR, small_size = (w, h), byte-identical to
+      ``cv2.resize(bgr(f), small_size, interpolation=interpolation)`` (INTER_LINEAR or INTER_AREA),
+      where bgr() is ``cv2.cvtColor(f, COLOR_YUV2BGR_I420 / _NV12)`` for a YUV source;
+    - ``bev_small``: the BEV of each small frame through M_small (one matrix per matrix of M, picked
+      by mat_index like M), with ``flags`` and ``borderValue``, in dst_format -- cv2's
+      ``warpPerspective`` followed by ``cvtColor(BGR2YUV_I420)`` (or its NV12 relayout) for YUV.
+
+    dst, small and dst_small may be given as C-contiguous uint8 host arrays or CPU tensors (pinned
+    for full speed).  Whole frames are uploaded, since the resize reads every row.  Synchronous."""
+    return _native.warp_perspective_video_host_small(src, M, M_small, dsize, small_size, src_format, dst_format,
+                                                     flags, interpolation, BORDER_CONSTANT, borderValue, mat_index,
+                                                     dst, small, dst_small)
+
+
+def warp_img_and_small_to_bev_video_host(frames, calib, bspec, new_u, new_v, src_format="i420", dst_format="i420",
+                                         flags=INTER_LINEAR, interpolation=INTER_LINEAR):
+    """The three images of vis_homo.py:85-111 from host video frames of a CPU codec: the BEV
+    (:89, the homography of :func:`warp_img_to_bev_video_host`), the (new_u, new_v) small frame
+    (:90) and its BEV (:91, through the homography of ``Calib.scale(align_corners=False)``, as
+    :func:`warp_small_img_to_bev`).  Returns ``(bev, small, bev_small)``; see
+    :func:`warp_perspective_video_host_small`."""
+    H = compose_H_bev_img(calib, bspec)
+    calib_small = calib.scale(align_corners=False, new_u=new_u, new_v=new_v)
+    H_small = np.linalg.inv(bspec.gen_H_world_bev()).dot(calib_small.gen_H_world_img())
+    return warp_perspective_video_host_small(frames, H, H_small, (int(bspec.u_size), int(bspec.v_size)),
+                                             (int(new_u), int(new_v)), src_format, dst_format, flags=flags,
+                                             interpolation=interpolation)
+
+
 def warp_bev_to_img(bev_frames, calib, bspec, flags=INTER_LINEAR):
     """Inverse BEV -> image warp (north_star extension; same kernel, H inverted on the host)."""
     H = np.linalg.inv(compose_H_bev_img(calib, bspec))

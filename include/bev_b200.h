@@ -211,6 +211,31 @@ int bevk_warp_perspective_video_host(const void *src, int src_format, void *dst,
                                      const double *border_value);
 
 /*
+ * bevk_warp_perspective_video_host plus the small-frame leg of the frame loop (vis_homo.py:90-91)
+ * in one call, from one upload of each frame.  Three HOST outputs, with bgr(f) = f for BGR frames
+ * and cv2.cvtColor(f, COLOR_YUV2BGR_I420 / _NV12) for YUV ones:
+ *   dst        the BEVs, exactly what bevk_warp_perspective_video_host writes for these arguments
+ *   small      [n_frames][small_h][small_w][3] uint8 BGR:
+ *                  cv2.resize(bgr(src[i]), (small_w, small_h), interpolation=interpolation)
+ *   dst_small  the BEVs of the small frames, the size and format of dst:
+ *                  cv2.warpPerspective(small[i], M_small[k], (dst_w, dst_h), flags, BORDER_CONSTANT,
+ *                                      border_value)
+ *              followed by cv2.cvtColor(..., COLOR_BGR2YUV_I420) or its NV12 relayout for a YUV dst_format
+ *   M_small    HOST float64 [n_mats][9]: the small frames' matrices (the homography of
+ *              Calib.scale(align_corners=False), vis_homo.py:73-78), indexed like M (n_mats, mat_index)
+ *   interpolation  BEVK_INTER_LINEAR or BEVK_INTER_AREA; small_h, small_w 1..32767
+ * Everything else as for bevk_warp_perspective_video_host; flags, border_mode and border_value
+ * serve both warps.  The resize reads every row, so whole frames (luma and chroma) are uploaded:
+ * the row-band trimming of bevk_warp_host_rows does not apply.  Arguments are checked before a
+ * device is looked for.
+ */
+int bevk_warp_perspective_video_host_small(const void *src, int src_format, void *dst, int dst_format, void *small,
+                                           void *dst_small, int n_frames, int src_h, int src_w, int dst_h, int dst_w,
+                                           int small_h, int small_w, const double *M, const double *M_small,
+                                           int n_mats, const int32_t *mat_index, int flags, int interpolation,
+                                           int border_mode, const double *border_value);
+
+/*
  * Roofline accounting helper (SURVEY.md 8d): number of distinct in-bounds source pixels that the
  * coordinate map of one matrix references (4 taps bilinear / 1 tap nearest), computed on the
  * device with the same coordinate code as the warp.  row_range (HOST int[2], may be NULL)

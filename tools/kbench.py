@@ -593,6 +593,45 @@ def resize_nv12_area_bench(rounds=5):
         torch.cuda.empty_cache()
 
 
+def _duplex_ceiling(h_up, h_dn, dev):
+    """ms(nu, nd): the best of three plain pinned copies of nu bytes up from h_up and nd bytes down
+    to h_dn at the same time, on two streams -- the host link's ceiling for a route's bytes."""
+    import time
+    d_up = torch.empty(h_up.numel(), dtype=torch.uint8, device=dev)
+    d_dn = torch.empty(h_dn.numel(), dtype=torch.uint8, device=dev)
+    s_up, s_dn = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
+
+    def ceiling(nu, nd):
+        best = None
+        for _ in range(3):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            with torch.cuda.stream(s_up):
+                d_up[:nu].copy_(h_up[:nu], non_blocking=True)
+            with torch.cuda.stream(s_dn):
+                h_dn[:nd].copy_(d_dn[:nd], non_blocking=True)
+            s_up.synchronize()
+            s_dn.synchronize()
+            dt = (time.perf_counter() - t0) * 1e3
+            best = dt if best is None else min(best, dt)
+        return best
+    return ceiling
+
+
+def _kernel_ms(fn, names):
+    """Sum of the device durations of the kernels one fn() runs whose names contain one of names
+    (torch.profiler, in a run of its own)."""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    us = 0.0
+    for e in prof.key_averages():
+        if any(k in e.key for k in names):
+            us += getattr(e, "self_device_time_total", None) or getattr(e, "self_cuda_time_total", 0.0)
+    return us / 1e3
+
+
 def video_host_bench(rounds=5, n=256):
     """Host video frames to host BEVs through bevk_warp_perspective_video_host (vis_homo.py:85-111
     with a CPU codec): cfg 2, n pinned 1080p frames -> 1024^2 bilinear with the canonical map, for
@@ -604,7 +643,6 @@ def video_host_bench(rounds=5, n=256):
     the kernels one call runs (torch.profiler: the I420-source kernels have no device entry point
     to bracket with events).  Every route's output equals the device route on the same frames."""
     import time
-    from torch.profiler import ProfilerActivity, profile
     print("card: %s" % card(), flush=True)
     dev = torch.device("cuda", 0)
     H, ssize, dsize = bench.h_canon(1), (1920, 1080), (1024, 1024)
@@ -650,35 +688,10 @@ def video_host_bench(rounds=5, n=256):
     torch.cuda.empty_cache()
 
     # the link ceiling for each route's byte counts: plain pinned copies, both directions at once
-    flat = bgr.view(-1)
-    d_up = torch.empty(max(up.values()) * n, dtype=torch.uint8, device=dev)
-    d_dn = torch.empty(max(down.values()) * n, dtype=torch.uint8, device=dev)
-    h_dn = out[("bgr", "bgr")].view(-1)
-    s_up, s_dn = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
-
-    def ceiling(nu, nd):
-        best = None
-        for _ in range(3):
-            torch.cuda.synchronize()
-            t0 = time.perf_counter()
-            with torch.cuda.stream(s_up):
-                d_up[:nu].copy_(flat[:nu], non_blocking=True)
-            with torch.cuda.stream(s_dn):
-                h_dn[:nd].copy_(d_dn[:nd], non_blocking=True)
-            s_up.synchronize()
-            s_dn.synchronize()
-            dt = (time.perf_counter() - t0) * 1e3
-            best = dt if best is None else min(best, dt)
-        return best
+    ceiling = _duplex_ceiling(bgr.view(-1), out[("bgr", "bgr")].view(-1), dev)
 
     def kernel_ms(r):
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            call(r)
-        us = 0.0
-        for e in prof.key_averages():
-            if "warp" in e.key:
-                us += getattr(e, "self_device_time_total", None) or getattr(e, "self_cuda_time_total", 0.0)
-        return us / 1e3
+        return _kernel_ms(lambda: call(r), ("warp",))
 
     for r in routes:
         nu, nd = up[r[0]] * n, down[r[1]] * n
@@ -691,6 +704,88 @@ def video_host_bench(rounds=5, n=256):
                  nu / 1e6, nd / 1e6, ceil, (nu + nd) / ceil / 1e6, 100.0 * ceil / med, kernel_ms(r)), flush=True)
 
 
+def video_host_small_bench(rounds=5, n=256):
+    """The three images of vis_homo.py:85-111 -- the BEV, the 852x480 small frame and its BEV -- from
+    n pinned host 1080p frames of a CPU codec, cfg 2 (1024^2 BEVs through the canonical map, the small
+    frames' map scaled from it as Calib.scale(align_corners=False) scales a calibration), INTER_LINEAR
+    resize, bilinear warps.  Routes, alternated in rounds (host clock around each synchronous call):
+      bgr one pass    warp_perspective_video_host_small, BGR -> BGR
+      bgr today       warp_perspective_host for the BEV, then the whole frames uploaded (pinned), resize,
+                      warp_perspective of the small frames and the two downloads
+      i420 one pass   warp_perspective_video_host_small, I420 -> I420
+    Per route: the bytes it moves up and down, the link ceiling for them (plain pinned copies both
+    ways at once, measured in the same run), its share of that ceiling, and its kernel time
+    (torch.profiler).  The two BGR routes must give the same bytes."""
+    import time
+    print("card: %s" % card(), flush=True)
+    dev = torch.device("cuda", 0)
+    H, ssize, dsize, small_size = bench.h_canon(1), (1920, 1080), (1024, 1024), (852, 480)
+    w, h, dw, dh, sw, sh = ssize[0], ssize[1], dsize[0], dsize[1], small_size[0], small_size[1]
+    fx, fy = w / sw, h / sh  # small pixel centre x -> (x + 0.5) * fx - 0.5 in the frame
+    Hs = H @ np.array([[fx, 0.0, 0.5 * fx - 0.5], [0.0, fy, 0.5 * fy - 0.5], [0.0, 0.0, 1.0]])
+    r0, r1 = _native.warp_host_rows(ssize, dsize, H, 1)
+    band = 3 * w * (r1 - r0 + 1)
+    up = {"bgr one pass": 3 * w * h, "bgr today": band + 3 * w * h, "i420 one pass": w * h * 3 // 2}
+    dn_bgr = 3 * dw * dh * 2 + 3 * sw * sh
+    down = {"bgr one pass": dn_bgr, "bgr today": dn_bgr, "i420 one pass": dw * dh * 3 + 3 * sw * sh}
+    print("cfg2 x%d 1080p -> 1024^2 and 852x480 -> 1024^2, bilinear, INTER_LINEAR resize; BEV band rows [%d, %d]"
+          % (n, r0, r1), flush=True)
+
+    g = torch.Generator().manual_seed(1234)
+    bgr = torch.randint(0, 256, (n, h, w, 3), dtype=torch.uint8, generator=g).pin_memory()
+    i420 = torch.randint(0, 256, (n, h * 3 // 2, w), dtype=torch.uint8, generator=g).pin_memory()
+
+    def outs(fmt):
+        frame = (dh, dw, 3) if fmt == "bgr" else (dh * 3 // 2, dw)
+        return [torch.empty((n,) + s, dtype=torch.uint8).pin_memory() for s in (frame, (sh, sw, 3), frame)]
+    out = {r: outs(r.split()[0]) for r in up}
+    d_frames = torch.empty((n, h, w, 3), dtype=torch.uint8, device=dev)
+    d_small = torch.empty((n, sh, sw, 3), dtype=torch.uint8, device=dev)
+    d_bev_small = torch.empty((n, dh, dw, 3), dtype=torch.uint8, device=dev)
+
+    def today():
+        o = out["bgr today"]
+        _native.warp_perspective_host(bgr, H, dsize, dst=o[0])
+        d_frames.copy_(bgr, non_blocking=True)
+        homo.resize(d_frames, small_size, dst=d_small)
+        homo.warp_perspective(d_small, Hs, dsize, dst=d_bev_small)
+        o[1].copy_(d_small, non_blocking=True)
+        o[2].copy_(d_bev_small, non_blocking=True)
+        torch.cuda.synchronize()
+
+    def one_pass(src, fmt, o):
+        return lambda: homo.warp_perspective_video_host_small(src, H, Hs, dsize, small_size, fmt, fmt, dst=o[0],
+                                                              small=o[1], dst_small=o[2])
+    routes = {"bgr one pass": one_pass(bgr, "bgr", out["bgr one pass"]), "bgr today": today,
+              "i420 one pass": one_pass(i420, "i420", out["i420 one pass"])}
+    for fn in routes.values():  # warm-up: workspace allocations, module loads
+        fn()
+    times = {r: [] for r in routes}
+    for _ in range(rounds):
+        for r, fn in routes.items():
+            t0 = time.perf_counter()
+            fn()
+            times[r].append((time.perf_counter() - t0) * 1e3)
+    for a, b in zip(out["bgr one pass"], out["bgr today"]):
+        assert torch.equal(a, b), "the one-pass BGR route differs from today's route"
+    kernels = {r: _kernel_ms(fn, ("warp", "resize")) for r, fn in routes.items()}
+    del routes, out, d_frames, d_small, d_bev_small
+    torch.cuda.empty_cache()
+
+    # plain pinned copies of each route's bytes, both directions at once
+    ceiling = _duplex_ceiling(torch.empty(max(up.values()) * n, dtype=torch.uint8).pin_memory(),
+                              torch.empty(max(down.values()) * n, dtype=torch.uint8).pin_memory(), dev)
+    for r in up:
+        nu, nd = up[r] * n, down[r] * n
+        ceil = ceiling(nu, nd)
+        t = np.array(times[r])
+        med = float(np.median(t))
+        print("%s: median %.2f ms (min %.2f, max %.2f, spread %.1f %%) | H2D %.1f MB, D2H %.1f MB per step, "
+              "ceiling %.2f ms (%.1f GB/s both ways) -> %.1f %% of it | kernels %.2f ms"
+              % (r, med, t.min(), t.max(), 100.0 * (t.max() - t.min()) / med, nu / 1e6, nd / 1e6, ceil,
+                 (nu + nd) / ceil / 1e6, 100.0 * ceil / med, kernels[r]), flush=True)
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "nv12":
         nv12_bench()
@@ -698,6 +793,8 @@ if __name__ == "__main__":
         yuv420_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "video_host":
         video_host_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "video_host_small":
+        video_host_small_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_nv12":
         resize_nv12_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_area":
