@@ -704,6 +704,102 @@ def video_host_bench(rounds=5, n=256):
                  nu / 1e6, nd / 1e6, ceil, (nu + nd) / ceil / 1e6, 100.0 * ceil / med, kernel_ms(r)), flush=True)
 
 
+def frame_loop_bench(rounds=5, n=200):
+    """The live-camera loop of vis_homo.py:85-111 for one frame at a time (cfg 1: launch-bound): the
+    1024^2 BEV, the 852x480 small frame, its 1024^2 BEV and the YUV 4:2:0 (I420) frames of both BEVs
+    for an encoder, from one 1080p BGR frame and from one NV12 frame of a GPU decoder.  Four routes
+    per chain, alternated in rounds:
+      ctypes    the bev_b200.homo functions (ctypes, one Python call per entry point)
+      ops       the torch.ops.bev_cuda operators, eager
+      compile   the operator chain under torch.compile(fullgraph=True)
+      graph     one torch.cuda.graph replay of the operator chain
+    Per route: the host time per frame (host clock around n frames that ends in a synchronise, median
+    over the rounds) and the device time of the same work (the kernels' durations per frame,
+    torch.profiler over n frames in a run of its own).  All routes must give the same bytes."""
+    import time
+    from torch.profiler import ProfilerActivity, profile
+    from bev_b200 import torch_ops
+    torch_ops.load()
+    ops = torch.ops.bev_cuda
+    print("card: %s" % card(), flush=True)
+    dev = torch.device("cuda", 0)
+    H, (w, h), (dw, dh), (sw, sh) = bench.h_canon(1), (1920, 1080), (1024, 1024), (852, 480)
+    fx, fy = w / sw, h / sh  # Calib.scale(align_corners=False) of the calibration
+    Hs = H @ np.array([[fx, 0.0, 0.5 * fx - 0.5], [0.0, fy, 0.5 * fy - 0.5], [0.0, 0.0, 1.0]])
+    Ht, Hst = torch.from_numpy(H), torch.from_numpy(Hs)
+    g = torch.Generator(device=dev).manual_seed(1234)
+    bgr = torch.randint(0, 256, (h, w, 3), dtype=torch.uint8, device=dev, generator=g)
+    nv12 = torch.randint(0, 256, (h * 3 // 2, w), dtype=torch.uint8, device=dev, generator=g)
+
+    def bgr_ops(f):
+        bev = ops.warp_perspective(f, Ht, dw, dh)
+        small = ops.resize(f, sw, sh)
+        bev_small = ops.warp_perspective(small, Hst, dw, dh)
+        return bev, small, bev_small, ops.bgr_to_yuv420(bev), ops.bgr_to_yuv420(bev_small)
+
+    def bgr_ctypes(f):
+        bev = homo.warp_perspective(f, H, (dw, dh))
+        small = homo.resize(f, (sw, sh))
+        bev_small = homo.warp_perspective(small, Hs, (dw, dh))
+        return bev, small, bev_small, homo.bgr_to_yuv420(bev), homo.bgr_to_yuv420(bev_small)
+
+    def nv12_ops(f):
+        bev = ops.warp_perspective_nv12(f, Ht, dw, dh)
+        small = ops.resize_nv12(f, sw, sh)
+        bev_small = ops.warp_perspective(small, Hst, dw, dh)
+        return bev, small, bev_small, ops.warp_perspective_nv12_yuv420(f, Ht, dw, dh), ops.bgr_to_yuv420(bev_small)
+
+    def nv12_ctypes(f):
+        bev = homo.warp_perspective_nv12(f, H, (dw, dh))
+        small = homo.resize_nv12(f, (sw, sh))
+        bev_small = homo.warp_perspective(small, Hs, (dw, dh))
+        return (bev, small, bev_small, homo.warp_perspective_nv12_yuv420(f, H, (dw, dh)),
+                homo.bgr_to_yuv420(bev_small))
+
+    for label, frame, eager, ctypes_chain in (("bgr 1080p", bgr, bgr_ops, bgr_ctypes),
+                                              ("nv12 1080p", nv12, nv12_ops, nv12_ctypes)):
+        compiled = torch.compile(eager, fullgraph=True)
+        ref = eager(frame)
+        for _ in range(3):  # warm-up on a side stream before capture, as torch.cuda.graph asks
+            compiled(frame)
+        s = torch.cuda.Stream()
+        s.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(s):
+            for _ in range(3):
+                eager(frame)
+        torch.cuda.current_stream().wait_stream(s)
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph):
+            graph_out = eager(frame)
+        routes = {"ctypes": lambda: ctypes_chain(frame), "ops": lambda: eager(frame),
+                  "compile": lambda: compiled(frame), "graph": graph.replay}
+        graph.replay()
+        torch.cuda.synchronize()
+        for name, out in (("ctypes", ctypes_chain(frame)), ("compile", compiled(frame)), ("graph", graph_out)):
+            assert all(torch.equal(a, b) for a, b in zip(out, ref)), "%s route differs from the eager operators" % name
+        host = {r: [] for r in routes}
+        for _ in range(rounds):
+            for r, fn in routes.items():
+                fn()
+                torch.cuda.synchronize()
+                t0 = time.perf_counter()
+                for _ in range(n):
+                    fn()
+                torch.cuda.synchronize()
+                host[r].append((time.perf_counter() - t0) * 1e6 / n)
+        for r, fn in routes.items():
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                for _ in range(n):
+                    fn()
+                torch.cuda.synchronize()
+            kern = sum(e.self_device_time_total for e in prof.key_averages()
+                       if e.device_type == torch.autograd.DeviceType.CUDA) / n
+            t = np.array(host[r])
+            print("frame_loop %s -> 1024^2 + 852x480 + YUV | %-7s: host %.1f us/frame (min %.1f, max %.1f), "
+                  "device %.1f us/frame" % (label, r, float(np.median(t)), t.min(), t.max(), kern), flush=True)
+        del graph, graph_out, compiled
+
+
 def video_host_small_bench(rounds=5, n=256):
     """The three images of vis_homo.py:85-111 -- the BEV, the 852x480 small frame and its BEV -- from
     n pinned host 1080p frames of a CPU codec, cfg 2 (1024^2 BEVs through the canonical map, the small
@@ -795,6 +891,8 @@ if __name__ == "__main__":
         video_host_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "video_host_small":
         video_host_small_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "frame_loop":
+        frame_loop_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_nv12":
         resize_nv12_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_area":
