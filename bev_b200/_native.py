@@ -54,6 +54,15 @@ SIGNATURES = {
     "bevk_warp_perspective_nv12_yuv420": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int,
                                                    _c_int, _c_int, _c_i64, _dp, _c_int, _i32p, _c_int, _c_int, _dp,
                                                    _vp]),
+    "bevk_warp_perspective_dmat": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_int, _c_int,
+                                            _c_int, _dp, _c_int, _i32p, _c_int, _c_int, _dp, _vp]),
+    "bevk_warp_perspective_nv12_dmat": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int,
+                                                 _dp, _c_int, _i32p, _c_int, _c_int, _dp, _vp]),
+    "bevk_warp_perspective_yuv420_dmat": (_c_int, [_vp, _vp] + [_c_int] * 6 + [_c_int, _c_i64, _dp, _c_int, _i32p,
+                                                                               _c_int, _c_int, _dp, _vp]),
+    "bevk_warp_perspective_nv12_yuv420_dmat": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int,
+                                                        _c_int, _c_int, _c_int, _c_i64, _dp, _c_int, _i32p, _c_int,
+                                                        _c_int, _dp, _vp]),
     "bevk_resize": (_c_int, [_vp, _vp] + [_c_int] * 8 + [_vp]),
     "bevk_resize_nv12": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int, _vp]),
     "bevk_resize_nv12_interp": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_i64, _c_int, _c_int, _c_int,
@@ -204,6 +213,35 @@ def _prep_mats(M, n_frames, mat_index):
     return Ms, idx
 
 
+class _Mats:
+    """The matrices of one warp call as the C ABI takes them: ptr (host, or with dmat device, float64
+    3x3 matrices), n (their count) and idx (host int32 mat_index or None).  keep holds what ptr points
+    into for the length of the call."""
+
+    def __init__(self, M, n_frames, mat_index, dmat, device):
+        if not dmat:
+            Ms, self.idx = _prep_mats(M, n_frames, mat_index)
+            self.keep, self.ptr, self.n = Ms, _dptr(Ms), Ms.shape[0]
+            return
+        import torch
+        if not isinstance(M, torch.Tensor) or not M.is_cuda:
+            raise TypeError("M must be a CUDA tensor for the device-matrix warps, got %s"
+                            % (getattr(M, "device", type(M).__name__),))
+        if M.device != device:
+            raise ValueError("M is on %s, the frames on %s" % (M.device, device))
+        if M.dtype != torch.float64:
+            raise TypeError("M must be float64, got %s" % (M.dtype,))
+        Mt = (M[None] if M.dim() == 2 else M).contiguous()  # stream-ordered; no host read
+        if Mt.dim() != 3 or tuple(Mt.shape[1:]) != (3, 3) or Mt.shape[0] == 0:
+            raise ValueError("M must be 3x3 or (K,3,3), got %s" % (tuple(M.shape),))
+        # the indices are planned on the host: the same checks as for host matrices
+        _, self.idx = _prep_mats(np.zeros((Mt.shape[0], 3, 3)), n_frames, mat_index)
+        self.keep, self.ptr, self.n = Mt, ctypes.cast(Mt.data_ptr(), _dp), Mt.shape[0]
+
+    def idx_ptr(self):
+        return self.idx.ctypes.data_as(_i32p) if self.idx is not None else None
+
+
 def _border(borderValue):
     b = np.zeros(4, np.float64)
     v = np.atleast_1d(np.asarray(borderValue, dtype=np.float64)).reshape(-1)[:4]
@@ -229,6 +267,17 @@ def warp_perspective(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue
                      mat_index=None, path=None):
     """path: None (the calling thread's default, see set_warp_path), "auto", "generic" (direct-gather
     kernels) or "fast" (staged kernel; raises if the shape does not qualify)."""
+    return _warp_perspective(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, path, False)
+
+
+def warp_perspective_dmat(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue=0, mat_index=None):
+    """warp_perspective with M a CUDA float64 tensor (3,3) or (K,3,3) on src's device, read by the
+    kernels when they run on the current stream: no host sync, and a captured CUDA graph replays the
+    matrices last written into M.  Always the direct-gather kernels; mat_index stays on the host."""
+    return _warp_perspective(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, None, True)
+
+
+def _warp_perspective(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, path, dmat):
     import torch
     _require_cuda(src, "src")
     code = _warp_dtype(src)
@@ -236,19 +285,21 @@ def warp_perspective(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue
     s4 = s4.contiguous()
     n, h, w, c = s4.shape
     dw, dh = int(dsize[0]), int(dsize[1])
-    Ms, idx = _prep_mats(M, n, mat_index)
+    m = _Mats(M, n, mat_index, dmat, src.device)
     d4 = None
     if dst is not None:  # any rank whose (N, H, W, C) view has the output's shape
         _require_cuda(dst, "dst")
         d4, _ = _frames_view(dst)
     out4 = _out(d4, (n, dh, dw, c), src.dtype, src.device)
     b = _border(borderValue)
+    args = (_vp(s4.data_ptr()), _vp(out4.data_ptr()), n, h, w, dh, dw, c, code, m.ptr, m.n, m.idx_ptr(),
+            int(flags), int(borderMode), _dptr(b))
     with torch.cuda.device(src.device):
-        rc = lib().bevk_warp_perspective_path(
-            _vp(s4.data_ptr()), _vp(out4.data_ptr()), n, h, w, dh, dw, c, code, _dptr(Ms),
-            Ms.shape[0], idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags),
-            int(borderMode), _dptr(b), _PATHS.get(path, path), _stream_ptr(src))
-    _check(rc, "bevk_warp_perspective")
+        if dmat:
+            rc = lib().bevk_warp_perspective_dmat(*args, _stream_ptr(src))
+        else:
+            rc = lib().bevk_warp_perspective_path(*args, _PATHS.get(path, path), _stream_ptr(src))
+    _check(rc, "bevk_warp_perspective_dmat" if dmat else "bevk_warp_perspective")
     return dst if dst is not None else undo(out4)
 
 
@@ -324,18 +375,27 @@ def nv12_to_bgr(src, dst=None):
 def warp_perspective_nv12(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue=0, mat_index=None):
     """warp_perspective of nv12_to_bgr(src) in one pass: (H*3/2, W) -> (h, w, 3), (N, H*3/2, W) ->
     (N, h, w, 3) BGR uint8.  M / mat_index as for warp_perspective."""
+    return _warp_perspective_nv12(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, False)
+
+
+def warp_perspective_nv12_dmat(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue=0, mat_index=None):
+    """warp_perspective_nv12 with M a CUDA float64 tensor, as for warp_perspective_dmat."""
+    return _warp_perspective_nv12(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, True)
+
+
+def _warp_perspective_nv12(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, dmat):
     import torch
     s3, n, h, w, pitch, fstride = _nv12_frames(src)
     dw, dh = int(dsize[0]), int(dsize[1])
-    Ms, idx = _prep_mats(M, n, mat_index)
+    m = _Mats(M, n, mat_index, dmat, src.device)
     dst = _out(dst, (n, dh, dw, 3) if src.dim() == 3 else (dh, dw, 3), torch.uint8, src.device)
     b = _border(borderValue)
+    name = "bevk_warp_perspective_nv12_dmat" if dmat else "bevk_warp_perspective_nv12"
     with torch.cuda.device(src.device):
-        rc = lib().bevk_warp_perspective_nv12(
-            _vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride, dh, dw, _dptr(Ms), Ms.shape[0],
-            idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags), int(borderMode), _dptr(b),
-            _stream_ptr(src))
-    _check(rc, "bevk_warp_perspective_nv12")
+        rc = getattr(lib(), name)(
+            _vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride, dh, dw, m.ptr, m.n, m.idx_ptr(),
+            int(flags), int(borderMode), _dptr(b), _stream_ptr(src))
+    _check(rc, name)
     return dst
 
 
@@ -393,6 +453,16 @@ def warp_perspective_yuv420(src, M, dsize, layout="i420", dst=None, flags=1, bor
                             mat_index=None):
     """bgr_to_yuv420(warp_perspective(src, M, dsize, ...), layout) in one pass: CUDA uint8 BGR
     frames (H, W, 3) or (N, H, W, 3) -> (h*3/2, w) or (N, h*3/2, w)."""
+    return _warp_perspective_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index, False)
+
+
+def warp_perspective_yuv420_dmat(src, M, dsize, layout="i420", dst=None, flags=1, borderMode=0, borderValue=0,
+                                 mat_index=None):
+    """warp_perspective_yuv420 with M a CUDA float64 tensor, as for warp_perspective_dmat."""
+    return _warp_perspective_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index, True)
+
+
+def _warp_perspective_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index, dmat):
     import torch
     _require_cuda(src, "src")
     if src.dtype != torch.uint8 or src.dim() not in (3, 4) or src.shape[-1] != 3:
@@ -401,15 +471,15 @@ def warp_perspective_yuv420(src, M, dsize, layout="i420", dst=None, flags=1, bor
     s4 = (src[None] if src.dim() == 3 else src).contiguous()
     n, h, w, _ = s4.shape
     dw, dh = int(dsize[0]), int(dsize[1])
-    Ms, idx = _prep_mats(M, n, mat_index)
+    m = _Mats(M, n, mat_index, dmat, src.device)
     dst, d3, pitch, fstride = _yuv_dst(dst, n, dh, dw, src.dim() == 4, src.device)
     b = _border(borderValue)
+    name = "bevk_warp_perspective_yuv420_dmat" if dmat else "bevk_warp_perspective_yuv420"
     with torch.cuda.device(src.device):
-        rc = lib().bevk_warp_perspective_yuv420(
-            _vp(s4.data_ptr()), _vp(d3.data_ptr()), n, h, w, dh, dw, code, pitch, fstride, _dptr(Ms), Ms.shape[0],
-            idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags), int(borderMode), _dptr(b),
-            _stream_ptr(src))
-    _check(rc, "bevk_warp_perspective_yuv420")
+        rc = getattr(lib(), name)(
+            _vp(s4.data_ptr()), _vp(d3.data_ptr()), n, h, w, dh, dw, code, pitch, fstride, m.ptr, m.n, m.idx_ptr(),
+            int(flags), int(borderMode), _dptr(b), _stream_ptr(src))
+    _check(rc, name)
     return dst
 
 
@@ -417,19 +487,31 @@ def warp_perspective_nv12_yuv420(src, M, dsize, layout="i420", dst=None, flags=1
                                  mat_index=None):
     """bgr_to_yuv420(warp_perspective_nv12(src, M, dsize, ...), layout) in one pass: CUDA uint8 NV12
     frames (H*3/2, W) or (N, H*3/2, W), any pitch and frame stride -> (h*3/2, w) or (N, h*3/2, w)."""
+    return _warp_perspective_nv12_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index,
+                                         False)
+
+
+def warp_perspective_nv12_yuv420_dmat(src, M, dsize, layout="i420", dst=None, flags=1, borderMode=0,
+                                      borderValue=0, mat_index=None):
+    """warp_perspective_nv12_yuv420 with M a CUDA float64 tensor, as for warp_perspective_dmat."""
+    return _warp_perspective_nv12_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index,
+                                         True)
+
+
+def _warp_perspective_nv12_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index, dmat):
     import torch
     s3, n, h, w, pitch, fstride = _nv12_frames(src)
     code = _yuv_layout(layout)
     dw, dh = int(dsize[0]), int(dsize[1])
-    Ms, idx = _prep_mats(M, n, mat_index)
+    m = _Mats(M, n, mat_index, dmat, src.device)
     dst, d3, dpitch, dfstride = _yuv_dst(dst, n, dh, dw, src.dim() == 3, src.device)
     b = _border(borderValue)
+    name = "bevk_warp_perspective_nv12_yuv420_dmat" if dmat else "bevk_warp_perspective_nv12_yuv420"
     with torch.cuda.device(src.device):
-        rc = lib().bevk_warp_perspective_nv12_yuv420(
+        rc = getattr(lib(), name)(
             _vp(s3.data_ptr()), _vp(d3.data_ptr()), n, h, w, pitch, fstride, dh, dw, code, dpitch, dfstride,
-            _dptr(Ms), Ms.shape[0], idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags),
-            int(borderMode), _dptr(b), _stream_ptr(src))
-    _check(rc, "bevk_warp_perspective_nv12_yuv420")
+            m.ptr, m.n, m.idx_ptr(), int(flags), int(borderMode), _dptr(b), _stream_ptr(src))
+    _check(rc, name)
     return dst
 
 

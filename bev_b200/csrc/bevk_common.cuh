@@ -65,6 +65,14 @@ BEVK_HD double bevk_div(double a, double b)
     return a / b;
 #endif
 }
+BEVK_HD double bevk_sub(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __dsub_rn(a, b);
+#else
+    return a - b;
+#endif
+}
 BEVK_HD int bevk_round_sat(double v)
 {
     // clamp to int32 then round half to even
@@ -77,6 +85,36 @@ BEVK_HD int bevk_round_sat(double v)
 #endif
 }
 BEVK_HD int bevk_sat16(int v) { return v < -32768 ? -32768 : (v > 32767 ? 32767 : v); }
+
+// Adjugate inverse of a 3x3 matrix in the order cv2.invert evaluates it for doubles (cv2 inverts
+// the forward matrix of warpPerspective this way).  Returns 0 and the zero map when det == 0.  The
+// host (bevk_invert3x3) and the device-matrix kernels share it, so both give the same bits.
+BEVK_HD int bevk_invert_adj(const double *H, double *M)
+{
+    const double a00 = H[0], a01 = H[1], a02 = H[2];
+    const double a10 = H[3], a11 = H[4], a12 = H[5];
+    const double a20 = H[6], a21 = H[7], a22 = H[8];
+    auto cof = [](double a, double b, double c, double e) { return bevk_sub(bevk_mul(a, b), bevk_mul(c, e)); };
+    double d = bevk_add(bevk_sub(bevk_mul(a00, cof(a11, a22, a12, a21)), bevk_mul(a01, cof(a10, a22, a12, a20))),
+                        bevk_mul(a02, cof(a10, a21, a11, a20)));
+    if (d == 0.0) {
+        for (int i = 0; i < 9; ++i) M[i] = 0.0;
+        return 0;
+    }
+    d = bevk_div(1.0, d);
+    double t[9];
+    t[0] = bevk_mul(cof(a11, a22, a12, a21), d);
+    t[1] = bevk_mul(cof(a02, a21, a01, a22), d);
+    t[2] = bevk_mul(cof(a01, a12, a02, a11), d);
+    t[3] = bevk_mul(cof(a12, a20, a10, a22), d);
+    t[4] = bevk_mul(cof(a00, a22, a02, a20), d);
+    t[5] = bevk_mul(cof(a02, a10, a00, a12), d);
+    t[6] = bevk_mul(cof(a10, a21, a11, a20), d);
+    t[7] = bevk_mul(cof(a01, a20, a00, a21), d);
+    t[8] = bevk_mul(cof(a00, a11, a01, a10), d);
+    for (int i = 0; i < 9; ++i) M[i] = t[i];
+    return 1;
+}
 
 // cv2's block width for a dsize: min(16,h) rows -> 1024/rows columns, clipped to the width.
 BEVK_HD int bevk_block_width(int dst_w, int dst_h)
@@ -111,7 +149,13 @@ BEVK_HD void bevk_map_pixel(const double *M, int x, int y, int bw0, double scale
 #define BEVK_MAX_GROUPS 16
 
 struct BevkWarpGroup {
-    double M[9];     // dst->src map (already inverted on the host)
+    union {
+        double M[9];  // dst->src map (already inverted on the host)
+        struct {      // device-matrix launches (the _dmat entry points) instead:
+            const double *mat;  // the group's forward (or, !invert, dst->src) matrix in device memory
+            int invert;         // 1: the kernel inverts it (bevk_invert_adj), 0: WARP_INVERSE_MAP
+        } d;
+    };
     int first;       // first frame of the run
     int count;       // frames in the run
     int stride;      // frame index step
@@ -157,7 +201,8 @@ struct BevkYuvParams {
 };
 
 // kernels-side entry points implemented in the .cu files
-int bevk_launch_warp_generic(const BevkWarpParams &p, int channels, int dtype, int linear,
+// dmat: the groups point into a device matrix table (BevkWarpGroup::d) -- also for the two launchers below
+int bevk_launch_warp_generic(const BevkWarpParams &p, int channels, int dtype, int linear, bool dmat,
                              cudaStream_t stream);
 // fills frames_per_chunk, total_chunks and the groups' chunk0 for the direct-gather kernels
 int bevk_plan_generic_chunks(BevkWarpParams &p, int channels);
@@ -167,7 +212,7 @@ int bevk_launch_warp_fast(const BevkWarpParams &p, int channels, int dtype, int 
                           cudaStream_t stream);
 // NV12 or I420 (src_format BEVK_YUV_NV12 / BEVK_YUV_I420) -> BGR warp over the chunks
 // bevk_plan_generic_chunks planned for P.w
-int bevk_launch_warp_nv12(const BevkNv12Params &P, int src_format, int linear, cudaStream_t stream);
+int bevk_launch_warp_nv12(const BevkNv12Params &P, int src_format, int linear, bool dmat, cudaStream_t stream);
 int bevk_launch_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int w, int pitch,
                             long long frame_stride, cudaStream_t stream);
 // cv2.resize of n_frames > 0 frames with `interpolation` (BEVK_INTER_LINEAR or BEVK_INTER_AREA):
@@ -179,7 +224,8 @@ int bevk_launch_resize(const void *src, void *dst, int n_frames, int src_h, int 
                        cudaStream_t stream);
 // BGR, NV12 or I420 frames (src_format BEVK_BGR / BEVK_YUV_NV12 / BEVK_YUV_I420) warped to YUV
 // 4:2:0 (nv12_out: NV12, else I420) over the chunks planned for P.w on the grid of 2x2 dst blocks
-int bevk_launch_warp_yuv420(const BevkYuvParams &P, int src_format, int nv12_out, int linear, cudaStream_t stream);
+int bevk_launch_warp_yuv420(const BevkYuvParams &P, int src_format, int nv12_out, int linear, bool dmat,
+                            cudaStream_t stream);
 // n_frames > 0 contiguous BGR frames of h x w (both even) to YUV 4:2:0 (nv12_out: NV12, else I420)
 int bevk_launch_bgr_to_yuv420(const void *src, void *dst, int n_frames, int h, int w, int nv12_out, int dst_pitch,
                               long long dst_frame_stride, cudaStream_t stream);

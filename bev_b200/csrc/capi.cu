@@ -103,33 +103,8 @@ int bevk_device_info(int *sm_count, int *cc_major, int *cc_minor)
     return rc;
 }
 
-// Adjugate inverse evaluated in the order cv2.invert uses for 3x3 double matrices (host code in
-// this file is compiled with -ffp-contract=off, so no product-difference is fused).
-int bevk_invert3x3(const double H[9], double M[9])
-{
-    const double a00 = H[0], a01 = H[1], a02 = H[2];
-    const double a10 = H[3], a11 = H[4], a12 = H[5];
-    const double a20 = H[6], a21 = H[7], a22 = H[8];
-    double d = a00 * (a11 * a22 - a12 * a21) - a01 * (a10 * a22 - a12 * a20) +
-               a02 * (a10 * a21 - a11 * a20);
-    if (d == 0.0) {
-        for (int i = 0; i < 9; ++i) M[i] = 0.0;
-        return 0;
-    }
-    d = 1.0 / d;
-    double t[9];
-    t[0] = (a11 * a22 - a12 * a21) * d;
-    t[1] = (a02 * a21 - a01 * a22) * d;
-    t[2] = (a01 * a12 - a02 * a11) * d;
-    t[3] = (a12 * a20 - a10 * a22) * d;
-    t[4] = (a00 * a22 - a02 * a20) * d;
-    t[5] = (a02 * a10 - a00 * a12) * d;
-    t[6] = (a10 * a21 - a11 * a20) * d;
-    t[7] = (a01 * a20 - a00 * a21) * d;
-    t[8] = (a00 * a11 - a01 * a10) * d;
-    for (int i = 0; i < 9; ++i) M[i] = t[i];
-    return 1;
-}
+// Host code in this file is compiled with -ffp-contract=off, so no product-difference is fused.
+int bevk_invert3x3(const double H[9], double M[9]) { return bevk_invert_adj(H, M); }
 
 int bevk_warp_set_path(int path)
 {
@@ -147,6 +122,7 @@ struct WarpArgs {
     int n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, linear;
     size_t elem_size;
     float border[4];
+    bool dmat;  // the groups point into a device matrix table (the _dmat entry points)
 };
 
 // The frame sizes every warp and resize takes: 1..32767.
@@ -195,6 +171,7 @@ int check_warp_args(const void *src, void *dst, int n_frames, int src_h, int src
     a.linear = interp == BEVK_INTER_LINEAR;
     a.elem_size = dtype == BEVK_U8 ? 1 : (dtype == BEVK_F16 ? 2 : 4);
     for (int c = 0; c < 4; ++c) a.border[c] = border_value ? (float)border_value[c] : 0.0f;
+    a.dmat = false;
     return BEVK_OK;
 }
 
@@ -210,13 +187,15 @@ void effective_maps(const double *M, int n_mats, int flags, std::vector<double> 
     }
 }
 
-// Split the frames of every matrix into arithmetic runs (first, count, stride).
-void build_groups(int n_frames, int n_mats, const int32_t *mat_index, const std::vector<double> &maps,
-                  std::vector<BevkWarpGroup> &groups)
+// Split the frames of every matrix into arithmetic runs (first, count, stride): set_map(g, k) gives
+// the group of a run of matrix k its map.
+template <typename SetMap>
+void build_groups(int n_frames, int n_mats, const int32_t *mat_index, std::vector<BevkWarpGroup> &groups,
+                  SetMap set_map)
 {
     auto push = [&](int k, int first, int count, int stride) {
         BevkWarpGroup g;
-        memcpy(g.M, &maps[(size_t)k * 9], 9 * sizeof(double));
+        set_map(g, k);
         g.first = first;
         g.count = count;
         g.stride = stride;
@@ -249,6 +228,33 @@ void build_groups(int n_frames, int n_mats, const int32_t *mat_index, const std:
     }
 }
 
+// The groups of host dst->src maps.
+void build_groups(int n_frames, int n_mats, const int32_t *mat_index, const std::vector<double> &maps,
+                  std::vector<BevkWarpGroup> &groups)
+{
+    build_groups(n_frames, n_mats, mat_index, groups,
+                 [&](BevkWarpGroup &g, int k) { memcpy(g.M, &maps[(size_t)k * 9], 9 * sizeof(double)); });
+}
+
+// The groups of a device call on the n_mats matrices M: maps inverted here from host matrices, or
+// (a.dmat) pointers into the device table M that the kernels read and invert when they run.
+void device_groups(const WarpArgs &a, const double *M, int n_mats, const int32_t *mat_index, int flags,
+                   std::vector<BevkWarpGroup> &groups)
+{
+    if (a.dmat) {
+        const int invert = (flags & BEVK_WARP_INVERSE_MAP) ? 0 : 1;
+        build_groups(a.n_frames, n_mats, mat_index, groups, [&](BevkWarpGroup &g, int k) {
+            memset(g.M, 0, sizeof(g.M));
+            g.d.mat = M + (size_t)k * 9;
+            g.d.invert = invert;
+        });
+        return;
+    }
+    std::vector<double> maps;
+    effective_maps(M, n_mats, flags, maps);
+    build_groups(a.n_frames, n_mats, mat_index, maps, groups);
+}
+
 // Fill p from a and walk the groups in launches of up to BEVK_MAX_GROUPS: launch() plans and
 // launches the groups p holds.
 template <typename Launch>
@@ -278,12 +284,14 @@ int launch_warp_groups(BevkWarpParams &p, const void *src, void *dst, const Warp
 }
 
 // The BGR warp: the staged kernel where it qualifies (path 0 or 2), else the direct-gather kernels.
+// Device matrices (a.dmat) always take the direct-gather kernels: the staged kernel plans its tiles
+// on the host from the maps.
 int run_warp_device(const void *src, void *dst, const WarpArgs &a,
                     const std::vector<BevkWarpGroup> &groups, int path, cudaStream_t stream)
 {
     BevkWarpParams p;
     return launch_warp_groups(p, src, dst, a, groups, [&]() -> int {
-        if (path != 1) {
+        if (path != 1 && !a.dmat) {
             const int launched = bevk_launch_warp_fast(p, a.channels, a.dtype, a.linear, path == 2, stream);
             if (launched < 0) return launched;
             if (launched) return BEVK_OK;
@@ -291,7 +299,7 @@ int run_warp_device(const void *src, void *dst, const WarpArgs &a,
         }
         const int rc = bevk_plan_generic_chunks(p, a.channels);
         if (rc) return rc;
-        return bevk_launch_warp_generic(p, a.channels, a.dtype, a.linear, stream);
+        return bevk_launch_warp_generic(p, a.channels, a.dtype, a.linear, a.dmat, stream);
     });
 }
 
@@ -523,11 +531,27 @@ int bevk_warp_perspective_path(const void *src, void *dst, int n_frames, int src
     rc = bevk_require_device();
     if (rc) return rc;
     if (n_frames == 0) return BEVK_OK;
-    std::vector<double> maps;
-    effective_maps(M, n_mats, flags, maps);
     std::vector<BevkWarpGroup> groups;
-    build_groups(n_frames, n_mats, mat_index, maps, groups);
+    device_groups(a, M, n_mats, mat_index, flags, groups);
     return run_warp_device(src, dst, a, groups, path, (cudaStream_t)stream);
+}
+
+int bevk_warp_perspective_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
+                               int dst_w, int channels, int dtype, const double *M, int n_mats,
+                               const int32_t *mat_index, int flags, int border_mode, const double *border_value,
+                               void *stream)
+{
+    WarpArgs a;
+    int rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
+                             n_mats, mat_index, flags, border_mode, border_value, a);
+    if (rc) return rc;
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    a.dmat = true;
+    std::vector<BevkWarpGroup> groups;
+    device_groups(a, M, n_mats, mat_index, flags, groups);
+    return run_warp_device(src, dst, a, groups, 1, (cudaStream_t)stream);
 }
 
 }  // extern "C"
@@ -610,7 +634,7 @@ int run_warp_yuv420(const void *src, void *dst, const WarpArgs &a, const std::ve
         P.w.dst_w *= 2;
         P.w.dst_h *= 2;
         if (rc) return rc;
-        return bevk_launch_warp_yuv420(P, src_format, layout == BEVK_YUV_NV12, a.linear, stream);
+        return bevk_launch_warp_yuv420(P, src_format, layout == BEVK_YUV_NV12, a.linear, a.dmat, stream);
     });
 }
 
@@ -625,16 +649,17 @@ int run_warp_yuv_bgr(const void *src, void *dst, const WarpArgs &a, const std::v
     return launch_warp_groups(P.w, src, dst, a, groups, [&]() {
         const int rc = bevk_plan_generic_chunks(P.w, 3);
         if (rc) return rc;
-        return bevk_launch_warp_nv12(P, src_format, a.linear, stream);
+        return bevk_launch_warp_nv12(P, src_format, a.linear, a.dmat, stream);
     });
 }
 
 // The fused warps to YUV 4:2:0 after their source-layout checks: BGR (src_format BEVK_BGR,
 // contiguous frames) or NV12 frames, rows `pitch` and frames `frame_stride` bytes apart.
+// dmat: M is a device matrix table.
 int warp_yuv420(const char *what, const void *src, void *dst, int n_frames, int src_h, int src_w, int src_format,
                 long long pitch, long long frame_stride, int dst_h, int dst_w, int layout, int dst_pitch,
                 int64_t dst_frame_stride, const double *M, int n_mats, const int32_t *mat_index, int flags,
-                int border_mode, const double *border_value, void *stream)
+                int border_mode, const double *border_value, bool dmat, void *stream)
 {
     int rc = check_yuv420_dst(what, n_frames, dst_h, dst_w, layout, dst_pitch, dst_frame_stride);
     if (rc) return rc;
@@ -645,10 +670,9 @@ int warp_yuv420(const char *what, const void *src, void *dst, int n_frames, int 
     rc = bevk_require_device();
     if (rc) return rc;
     if (n_frames == 0) return BEVK_OK;
-    std::vector<double> maps;
-    effective_maps(M, n_mats, flags, maps);
+    a.dmat = dmat;
     std::vector<BevkWarpGroup> groups;
-    build_groups(n_frames, n_mats, mat_index, maps, groups);
+    device_groups(a, M, n_mats, mat_index, flags, groups);
     return run_warp_yuv420(src, dst, a, groups, src_format, pitch, frame_stride, layout, dst_pitch, dst_frame_stride,
                            (cudaStream_t)stream);
 }
@@ -695,6 +719,26 @@ int run_video_warp(const void *src, void *dst, const WarpArgs &a, const std::vec
         return run_warp_yuv_bgr(src, dst, a, groups, src_format, a.src_w, src_frame_bytes, stream);
     return run_warp_device(src, dst, a, groups, g_warp_path, stream);
 }
+
+// dmat: M is a device matrix table.
+int warp_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch, int64_t frame_stride,
+              int dst_h, int dst_w, const double *M, int n_mats, const int32_t *mat_index, int flags, int border_mode,
+              const double *border_value, bool dmat, void *stream)
+{
+    int rc = check_nv12_layout32("warp_nv12", n_frames, src_h, src_w, pitch, frame_stride);
+    if (rc) return rc;
+    WarpArgs a;
+    rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index,
+                         flags, border_mode, border_value, a);
+    if (rc) return rc;
+    rc = bevk_require_device();
+    if (rc) return rc;
+    if (n_frames == 0) return BEVK_OK;
+    a.dmat = dmat;
+    std::vector<BevkWarpGroup> groups;
+    device_groups(a, M, n_mats, mat_index, flags, groups);
+    return run_warp_yuv_bgr(src, dst, a, groups, BEVK_YUV_NV12, pitch, frame_stride, (cudaStream_t)stream);
+}
 }  // namespace
 
 extern "C" {
@@ -716,20 +760,17 @@ int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src
                                const double *M, int n_mats, const int32_t *mat_index, int flags,
                                int border_mode, const double *border_value, void *stream)
 {
-    int rc = check_nv12_layout32("warp_nv12", n_frames, src_h, src_w, pitch, frame_stride);
-    if (rc) return rc;
-    WarpArgs a;
-    rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index,
-                         flags, border_mode, border_value, a);
-    if (rc) return rc;
-    rc = bevk_require_device();
-    if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
-    std::vector<double> maps;
-    effective_maps(M, n_mats, flags, maps);
-    std::vector<BevkWarpGroup> groups;
-    build_groups(n_frames, n_mats, mat_index, maps, groups);
-    return run_warp_yuv_bgr(src, dst, a, groups, BEVK_YUV_NV12, pitch, frame_stride, (cudaStream_t)stream);
+    return warp_nv12(src, dst, n_frames, src_h, src_w, pitch, frame_stride, dst_h, dst_w, M, n_mats, mat_index,
+                     flags, border_mode, border_value, false, stream);
+}
+
+int bevk_warp_perspective_nv12_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                                    int64_t frame_stride, int dst_h, int dst_w, const double *M, int n_mats,
+                                    const int32_t *mat_index, int flags, int border_mode,
+                                    const double *border_value, void *stream)
+{
+    return warp_nv12(src, dst, n_frames, src_h, src_w, pitch, frame_stride, dst_h, dst_w, M, n_mats, mat_index,
+                     flags, border_mode, border_value, true, stream);
 }
 
 int bevk_bgr_to_yuv420(const void *src, void *dst, int n_frames, int h, int w, int layout, int dst_pitch,
@@ -753,7 +794,17 @@ int bevk_warp_perspective_yuv420(const void *src, void *dst, int n_frames, int s
 {
     return warp_yuv420("warp_yuv420", src, dst, n_frames, src_h, src_w, BEVK_BGR, 3LL * src_w,
                        3LL * src_w * src_h, dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index,
-                       flags, border_mode, border_value, stream);
+                       flags, border_mode, border_value, false, stream);
+}
+
+int bevk_warp_perspective_yuv420_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
+                                      int dst_w, int layout, int dst_pitch, int64_t dst_frame_stride,
+                                      const double *M, int n_mats, const int32_t *mat_index, int flags,
+                                      int border_mode, const double *border_value, void *stream)
+{
+    return warp_yuv420("warp_yuv420", src, dst, n_frames, src_h, src_w, BEVK_BGR, 3LL * src_w,
+                       3LL * src_w * src_h, dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index,
+                       flags, border_mode, border_value, true, stream);
 }
 
 int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
@@ -766,7 +817,20 @@ int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, 
     if (rc) return rc;
     return warp_yuv420("warp_nv12_yuv420", src, dst, n_frames, src_h, src_w, BEVK_YUV_NV12, pitch, frame_stride,
                        dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index, flags, border_mode,
-                       border_value, stream);
+                       border_value, false, stream);
+}
+
+int bevk_warp_perspective_nv12_yuv420_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                                           int64_t frame_stride, int dst_h, int dst_w, int layout, int dst_pitch,
+                                           int64_t dst_frame_stride, const double *M, int n_mats,
+                                           const int32_t *mat_index, int flags, int border_mode,
+                                           const double *border_value, void *stream)
+{
+    const int rc = check_nv12_layout32("warp_nv12_yuv420", n_frames, src_h, src_w, pitch, frame_stride);
+    if (rc) return rc;
+    return warp_yuv420("warp_nv12_yuv420", src, dst, n_frames, src_h, src_w, BEVK_YUV_NV12, pitch, frame_stride,
+                       dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index, flags, border_mode,
+                       border_value, true, stream);
 }
 
 int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h, int dst_w, int channels,

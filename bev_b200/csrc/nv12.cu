@@ -25,11 +25,17 @@ namespace {
 // of the window's one or two chroma columns).  WORDS (pitch, frame stride and src 4-byte aligned):
 // aligned 32-bit words + funnel shifts, the second word of a row only when the window straddles
 // it; otherwise byte loads.  PACKED (dst_w % 4 == 0): the warp packs 32 pixels into one coalesced
-// 96-byte store, otherwise every lane stores its 3 bytes.
-template <bool LINEAR, bool WORDS, bool PACKED, int kBatch>
+// 96-byte store, otherwise every lane stores its 3 bytes.  DMAT: the matrices are in a device table
+// (dmat_map).
+template <bool LINEAR, bool WORDS, bool PACKED, int kBatch, bool DMAT>
 __global__ void __launch_bounds__(256) warp_nv12_kernel(const __grid_constant__ BevkNv12Params P)
 {
     const BevkWarpParams &p = P.w;
+    const double *dm = nullptr;  // DMAT: the group's map, read from the device table
+    if constexpr (DMAT) {
+        __shared__ double sm[9];
+        dm = dmat_map(p, sm);
+    }
     const int lane = threadIdx.x, x0 = blockIdx.x * 32;
     const int x = x0 + lane, y = blockIdx.y * 8 + threadIdx.y;
     if (y >= p.dst_h) return;  // a warp is one dst row segment: uniform exit, shuffles stay legal
@@ -40,7 +46,7 @@ __global__ void __launch_bounds__(256) warp_nv12_kernel(const __grid_constant__ 
     const int f1 = min(f0 + p.frames_per_chunk, g.count);
 
     int X, Y;
-    bevk_map_pixel(g.M, min(x, p.dst_w - 1), y, p.bw0, LINEAR ? 32.0 : 1.0, X, Y);
+    bevk_map_pixel(DMAT ? dm : g.M, min(x, p.dst_w - 1), y, p.bw0, LINEAR ? 32.0 : 1.0, X, Y);
     int cs, rs, wc0, wc1, wr0, wr1;
     if (LINEAR) {
         window(bevk_sat16(X >> 5), X & 31, p.src_w, cs, wc0, wc1);
@@ -174,16 +180,16 @@ __global__ void __launch_bounds__(256) warp_nv12_kernel(const __grid_constant__ 
     }
 }
 
-template <bool LINEAR, bool WORDS>
+template <bool LINEAR, bool WORDS, bool DMAT>
 void launch_warp(const BevkNv12Params &P, bool packed, cudaStream_t stream)
 {
     constexpr int kBatch = LINEAR ? 2 : 4;
     dim3 block(32, 8, 1);
     dim3 grid((P.w.dst_w + 31) / 32, (P.w.dst_h + 7) / 8, P.w.total_chunks);
     if (packed)
-        warp_nv12_kernel<LINEAR, WORDS, true, kBatch><<<grid, block, 0, stream>>>(P);
+        warp_nv12_kernel<LINEAR, WORDS, true, kBatch, DMAT><<<grid, block, 0, stream>>>(P);
     else
-        warp_nv12_kernel<LINEAR, WORDS, false, kBatch><<<grid, block, 0, stream>>>(P);
+        warp_nv12_kernel<LINEAR, WORDS, false, kBatch, DMAT><<<grid, block, 0, stream>>>(P);
 }
 
 // warp_nv12_kernel over a source format S of yuv_src.cuh (S::make, S::load, S::math): the warp of
@@ -359,18 +365,30 @@ nv12_to_bgr_kernel(const uint8_t *__restrict__ src, uint8_t *__restrict__ dst, i
     }
 }
 
+// the four warp_nv12_kernel instances of one matrix source: bilinear / nearest, word / byte gathers
+template <bool DMAT>
+void launch_nv12(const BevkNv12Params &P, bool words, bool packed, int linear, cudaStream_t stream)
+{
+    if (linear)
+        words ? launch_warp<true, true, DMAT>(P, packed, stream) : launch_warp<true, false, DMAT>(P, packed, stream);
+    else
+        words ? launch_warp<false, true, DMAT>(P, packed, stream) : launch_warp<false, false, DMAT>(P, packed, stream);
+}
+
 }  // namespace
 
-int bevk_launch_warp_nv12(const BevkNv12Params &P, int src_format, int linear, cudaStream_t stream)
+int bevk_launch_warp_nv12(const BevkNv12Params &P, int src_format, int linear, bool dmat, cudaStream_t stream)
 {
     const bool words = ((uintptr_t)P.w.src % 4) == 0 && (P.pitch % 4) == 0 && (P.frame_stride % 4) == 0;
     const bool packed = (P.w.dst_w % 4) == 0 && ((uintptr_t)P.w.dst % 4) == 0;
-    if (src_format == BEVK_YUV_I420)
+    if (src_format == BEVK_YUV_I420) {
+        if (dmat) BEVK_FAIL(BEVK_E_ARG, "warp_nv12: I420 frames take host matrices");
         launch_yuv_src<I420Src>(P, words, packed, linear, stream);
-    else if (linear)
-        words ? launch_warp<true, true>(P, packed, stream) : launch_warp<true, false>(P, packed, stream);
-    else
-        words ? launch_warp<false, true>(P, packed, stream) : launch_warp<false, false>(P, packed, stream);
+    } else if (dmat) {
+        launch_nv12<true>(P, words, packed, linear, stream);
+    } else {
+        launch_nv12<false>(P, words, packed, linear, stream);
+    }
     BEVK_CUDA(cudaGetLastError());
     return BEVK_OK;
 }

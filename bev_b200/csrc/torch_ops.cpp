@@ -6,8 +6,11 @@
 // Every CUDA implementation only checks tensors, allocates the result with torch's caching
 // allocator, takes the current CUDA stream and calls the extern "C" entry point with raw pointers --
 // no arithmetic lives here.  Homographies, K and Rt are CPU float64 tensors (they stay on the host,
-// SURVEY.md 8b "Matrix ownership"), and so is a mat_index during CUDA-graph capture.  No CPU
-// implementation is registered: CPU tensors fail in the dispatcher, there is no CPU fallback.
+// SURVEY.md 8b "Matrix ownership"), and so is a mat_index during CUDA-graph capture -- except the M of
+// the four warps, which may also be a CUDA tensor on the frames' device: the kernels then read it
+// when they run (the *_dmat entry points), so nothing synchronises and a captured graph replays
+// whatever matrices were last written into it.  No CPU implementation is registered: CPU tensors
+// fail in the dispatcher, there is no CPU fallback.
 //
 // Each operator is ONE function, registered for both the CUDA and the Meta dispatch key: it checks
 // shapes and dtypes and allocates the output with SymInt sizes, and returns there for meta tensors
@@ -88,12 +91,16 @@ void check_mats(const at::Tensor &M, const char *what)
 
 // ---- shape and validation helpers, one per operator family ----------------------------------------
 
-// Warp matrices of n frames: (K, 3, 3) float64 on the host and the optional per-frame index.  During
-// CUDA-graph capture a CUDA mat_index cannot be read (the copy to the host synchronises): the captured
-// graph would bake in the index of capture time anyway, so a CPU one is asked for.
+// Warp matrices of n frames: (K, 3, 3) float64, on the host or (device) on the frames' device, and
+// the optional per-frame index.  During CUDA-graph capture a CUDA mat_index cannot be read (the copy to
+// the host synchronises): the captured graph would bake in the index of capture time anyway, so a CPU
+// one is asked for.
 struct WarpMats {
     at::Tensor M, idx;
+    bool device;  // M is a CUDA tensor: call the *_dmat twin of the entry point
     const int32_t *idx_ptr() const { return idx.defined() ? idx.data_ptr<int32_t>() : nullptr; }
+    // the entry point for M: host (host_fn) or device (dmat_fn) matrices; the twins share a signature
+    template <typename FN> FN *pick(FN *host_fn, FN *dmat_fn) const { return device ? dmat_fn : host_fn; }
 };
 
 void check_warp_mats(const at::Tensor &M, const c10::optional<at::Tensor> &mat_index, const SymInt &n)
@@ -104,10 +111,16 @@ void check_warp_mats(const at::Tensor &M, const c10::optional<at::Tensor> &mat_i
                         n, " frames");
 }
 
-WarpMats warp_mats(const at::Tensor &M, const c10::optional<at::Tensor> &mat_index)
+WarpMats warp_mats(const at::Tensor &M, const c10::optional<at::Tensor> &mat_index, const at::Tensor &src)
 {
     WarpMats m;
-    m.M = host_f64(M, "M").reshape({-1, 3, 3});
+    m.device = M.is_cuda();
+    if (m.device) {
+        check_cuda(M, src, "M");
+        m.M = M.to(at::kDouble).contiguous().reshape({-1, 3, 3});  // on the current stream, no host read
+    } else {
+        m.M = host_f64(M, "M").reshape({-1, 3, 3});
+    }
     if (mat_index.has_value()) {
         TORCH_CHECK(!mat_index->is_cuda() ||
                         c10::cuda::currentStreamCaptureStatusMayInitCtx() == c10::cuda::CaptureStatus::None,
@@ -239,9 +252,9 @@ at::Tensor warp_perspective(const at::Tensor &src, const at::Tensor &M, int64_t 
     TORCH_CHECK(src.is_cuda(), "src must be a CUDA tensor");
     c10::cuda::CUDAGuard guard(src.device());
     const at::Tensor s = src.contiguous();
-    const WarpMats m = warp_mats(M, mat_index);
+    const WarpMats m = warp_mats(M, mat_index, src);
     const double border[4] = {border_val, border_val, border_val, border_val};
-    check_rc(bevk_warp_perspective(s.data_ptr(), out.data_ptr(), (int)I(f.n), (int)I(f.h), (int)I(f.w), (int)h,
+    check_rc(m.pick(bevk_warp_perspective, bevk_warp_perspective_dmat)(s.data_ptr(), out.data_ptr(), (int)I(f.n), (int)I(f.h), (int)I(f.w), (int)h,
                                    (int)w, (int)I(f.c), dtype, m.M.data_ptr<double>(), (int)m.M.size(0),
                                    m.idx_ptr(), (int)flags, (int)border_mode, border, current_stream(src)),
              "bevk_warp_perspective");
@@ -289,9 +302,9 @@ at::Tensor warp_perspective_nv12(const at::Tensor &src, const at::Tensor &M, int
     TORCH_CHECK(src.is_cuda(), "src must be a CUDA tensor");
     c10::cuda::CUDAGuard guard(src.device());
     const Nv12View v = nv12_view(src, f);
-    const WarpMats m = warp_mats(M, mat_index);
+    const WarpMats m = warp_mats(M, mat_index, src);
     const double border[4] = {border_val, border_val, border_val, border_val};
-    check_rc(bevk_warp_perspective_nv12(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w,
+    check_rc(m.pick(bevk_warp_perspective_nv12, bevk_warp_perspective_nv12_dmat)(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w,
                                         (int)v.pitch, v.frame_stride, (int)h, (int)w, m.M.data_ptr<double>(),
                                         (int)m.M.size(0), m.idx_ptr(), (int)flags, (int)border_mode, border,
                                         current_stream(src)),
@@ -339,9 +352,9 @@ at::Tensor warp_perspective_yuv420(const at::Tensor &src, const at::Tensor &M, i
     TORCH_CHECK(src.is_cuda(), "src must be a CUDA tensor");
     c10::cuda::CUDAGuard guard(src.device());
     const at::Tensor s = src.contiguous();
-    const WarpMats m = warp_mats(M, mat_index);
+    const WarpMats m = warp_mats(M, mat_index, src);
     const double border[4] = {border_val, border_val, border_val, border_val};
-    check_rc(bevk_warp_perspective_yuv420(s.data_ptr(), out.data_ptr(), (int)I(f.n), (int)I(f.h), (int)I(f.w),
+    check_rc(m.pick(bevk_warp_perspective_yuv420, bevk_warp_perspective_yuv420_dmat)(s.data_ptr(), out.data_ptr(), (int)I(f.n), (int)I(f.h), (int)I(f.w),
                                           (int)h, (int)w, (int)layout, (int)w, w * (h / 2 * 3),
                                           m.M.data_ptr<double>(), (int)m.M.size(0), m.idx_ptr(), (int)flags,
                                           (int)border_mode, border, current_stream(src)),
@@ -360,9 +373,9 @@ at::Tensor warp_perspective_nv12_yuv420(const at::Tensor &src, const at::Tensor 
     TORCH_CHECK(src.is_cuda(), "src must be a CUDA tensor");
     c10::cuda::CUDAGuard guard(src.device());
     const Nv12View v = nv12_view(src, f);
-    const WarpMats m = warp_mats(M, mat_index);
+    const WarpMats m = warp_mats(M, mat_index, src);
     const double border[4] = {border_val, border_val, border_val, border_val};
-    check_rc(bevk_warp_perspective_nv12_yuv420(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w,
+    check_rc(m.pick(bevk_warp_perspective_nv12_yuv420, bevk_warp_perspective_nv12_yuv420_dmat)(v.s3.data_ptr(), out.data_ptr(), (int)v.n, (int)v.h, (int)v.w,
                                                (int)v.pitch, v.frame_stride, (int)h, (int)w, (int)layout, (int)w,
                                                w * (h / 2 * 3), m.M.data_ptr<double>(), (int)m.M.size(0),
                                                m.idx_ptr(), (int)flags, (int)border_mode, border,

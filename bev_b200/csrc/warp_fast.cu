@@ -1412,7 +1412,7 @@ int bevk_launch_warp_fast(const BevkWarpParams &p_in, int channels, int dtype, i
         if (e == cudaSuccess && split) {
             // the tiles the staged kernel marked, through the direct-gather kernel (same stream)
             rc2 = bevk_plan_generic_chunks(p, channels);
-            if (!rc2) rc2 = bevk_launch_warp_generic(p, channels, dtype, linear, stream);
+            if (!rc2) rc2 = bevk_launch_warp_generic(p, channels, dtype, linear, false, stream);
         }
     }
     const cudaError_t ef = cudaFreeAsync(scratch, stream);  // stream-ordered: after the kernels above

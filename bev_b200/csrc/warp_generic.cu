@@ -38,9 +38,14 @@ __device__ __forceinline__ uint8_t border_u8(float b)
 }
 
 // ---- bilinear ---------------------------------------------------------------------------------
-template <typename T, int C>
+template <typename T, int C, bool DMAT>
 __global__ void __launch_bounds__(256) warp_linear_kernel(const __grid_constant__ BevkWarpParams p)
 {
+    const double *dm = nullptr;  // DMAT: the group's map, read from the device table
+    if constexpr (DMAT) {
+        __shared__ double sm[9];
+        dm = dmat_map(p, sm);
+    }
     const int x = blockIdx.x * 32 + threadIdx.x;
     const int y = blockIdx.y * 8 + threadIdx.y;
     if (x >= p.dst_w || y >= p.dst_h) return;
@@ -52,7 +57,7 @@ __global__ void __launch_bounds__(256) warp_linear_kernel(const __grid_constant_
     const int f1 = min(f0 + p.frames_per_chunk, g.count);
 
     int X, Y;
-    bevk_map_pixel(g.M, x, y, p.bw0, 32.0, X, Y);
+    bevk_map_pixel(DMAT ? dm : g.M, x, y, p.bw0, 32.0, X, Y);
     const int sx = bevk_sat16(X >> 5), sy = bevk_sat16(Y >> 5);
     const int ax = X & 31, ay = Y & 31;
     const bool cx0 = (sx >= 0 && sx < p.src_w), cx1 = (sx + 1 >= 0 && sx + 1 < p.src_w);
@@ -138,9 +143,14 @@ __global__ void __launch_bounds__(256) warp_linear_kernel(const __grid_constant_
 }
 
 // ---- nearest ----------------------------------------------------------------------------------
-template <typename T, int C>
+template <typename T, int C, bool DMAT>
 __global__ void __launch_bounds__(256) warp_nearest_kernel(const __grid_constant__ BevkWarpParams p)
 {
+    const double *dm = nullptr;  // DMAT: the group's map, read from the device table
+    if constexpr (DMAT) {
+        __shared__ double sm[9];
+        dm = dmat_map(p, sm);
+    }
     const int x = blockIdx.x * 32 + threadIdx.x;
     const int y = blockIdx.y * 8 + threadIdx.y;
     if (x >= p.dst_w || y >= p.dst_h) return;
@@ -152,7 +162,7 @@ __global__ void __launch_bounds__(256) warp_nearest_kernel(const __grid_constant
     const int f1 = min(f0 + p.frames_per_chunk, g.count);
 
     int X, Y;
-    bevk_map_pixel(g.M, x, y, p.bw0, 1.0, X, Y);
+    bevk_map_pixel(DMAT ? dm : g.M, x, y, p.bw0, 1.0, X, Y);
     const int sx = bevk_sat16(X), sy = bevk_sat16(Y);
     const bool inside = (sx >= 0 && sx < p.src_w && sy >= 0 && sy < p.src_h);
     const long long os = ((long long)sy * p.src_w + sx) * C;
@@ -186,9 +196,14 @@ __global__ void __launch_bounds__(256) warp_nearest_kernel(const __grid_constant
 // its 32 pixels into 24 words -- one coalesced 96-byte store per warp and frame.  This is the
 // kernel for strongly minifying maps (BrnoCompSpeed-sized BEVs of 1080p frames), where a tile's
 // source box is mostly untouched pixels and staging it would move more data than the gather.
-template <bool LINEAR, int kBatch>
+template <bool LINEAR, int kBatch, bool DMAT>
 __global__ void __launch_bounds__(256) warp_u8c3_direct_kernel(const __grid_constant__ BevkWarpParams p)
 {
+    const double *dm = nullptr;  // DMAT: the group's map, read from the device table
+    if constexpr (DMAT) {
+        __shared__ double sm[9];
+        dm = dmat_map(p, sm);
+    }
     const int lane = threadIdx.x, x0 = blockIdx.x * 32;
     const int x = x0 + lane, y = blockIdx.y * 8 + threadIdx.y;
     if (y >= p.dst_h) return;  // a warp is one dst row segment: uniform exit, shuffles stay legal
@@ -200,7 +215,7 @@ __global__ void __launch_bounds__(256) warp_u8c3_direct_kernel(const __grid_cons
     const int f1 = min(f0 + p.frames_per_chunk, g.count);
 
     int X, Y;
-    bevk_map_pixel(g.M, min(x, p.dst_w - 1), y, p.bw0, LINEAR ? 32.0 : 1.0, X, Y);
+    bevk_map_pixel(DMAT ? dm : g.M, min(x, p.dst_w - 1), y, p.bw0, LINEAR ? 32.0 : 1.0, X, Y);
     int cs, rs, wc0, wc1, wr0, wr1;
     if (LINEAR) {
         window(bevk_sat16(X >> 5), X & 31, p.src_w, cs, wc0, wc1);
@@ -274,6 +289,7 @@ __global__ void __launch_bounds__(256) warp_u8c3_direct_kernel(const __grid_cons
 }
 
 // returns true if it launched
+template <bool DMAT>
 bool launch_u8c3_direct(const BevkWarpParams &p, int linear, cudaStream_t stream)
 {
     if (p.border[0] != 0.f || p.border[1] != 0.f || p.border[2] != 0.f) return false;
@@ -285,35 +301,50 @@ bool launch_u8c3_direct(const BevkWarpParams &p, int linear, cudaStream_t stream
     dim3 block(32, 8, 1);
     dim3 grid((p.dst_w + 31) / 32, (p.dst_h + 7) / 8, p.total_chunks);
     if (linear)
-        warp_u8c3_direct_kernel<true, 2><<<grid, block, 0, stream>>>(p);
+        warp_u8c3_direct_kernel<true, 2, DMAT><<<grid, block, 0, stream>>>(p);
     else
-        warp_u8c3_direct_kernel<false, 4><<<grid, block, 0, stream>>>(p);
+        warp_u8c3_direct_kernel<false, 4, DMAT><<<grid, block, 0, stream>>>(p);
     return true;
 }
 
-template <typename T, int C>
+template <typename T, int C, bool DMAT>
 int launch_tc(const BevkWarpParams &p, int linear, cudaStream_t stream)
 {
     dim3 block(32, 8, 1);
     dim3 grid((p.dst_w + 31) / 32, (p.dst_h + 7) / 8, p.total_chunks);
     if (linear)
-        warp_linear_kernel<T, C><<<grid, block, 0, stream>>>(p);
+        warp_linear_kernel<T, C, DMAT><<<grid, block, 0, stream>>>(p);
     else
-        warp_nearest_kernel<T, C><<<grid, block, 0, stream>>>(p);
+        warp_nearest_kernel<T, C, DMAT><<<grid, block, 0, stream>>>(p);
     BEVK_CUDA(cudaGetLastError());
     return BEVK_OK;
 }
 
-template <typename T>
+template <typename T, bool DMAT>
 int launch_t(const BevkWarpParams &p, int channels, int linear, cudaStream_t stream)
 {
     switch (channels) {
-    case 1: return launch_tc<T, 1>(p, linear, stream);
-    case 2: return launch_tc<T, 2>(p, linear, stream);
-    case 3: return launch_tc<T, 3>(p, linear, stream);
-    case 4: return launch_tc<T, 4>(p, linear, stream);
+    case 1: return launch_tc<T, 1, DMAT>(p, linear, stream);
+    case 2: return launch_tc<T, 2, DMAT>(p, linear, stream);
+    case 3: return launch_tc<T, 3, DMAT>(p, linear, stream);
+    case 4: return launch_tc<T, 4, DMAT>(p, linear, stream);
     }
     BEVK_FAIL(BEVK_E_ARG, "channels must be 1..4, got %d", channels);
+}
+
+template <bool DMAT>
+int launch_generic(const BevkWarpParams &p, int channels, int dtype, int linear, cudaStream_t stream)
+{
+    if (dtype == BEVK_U8 && channels == 3 && launch_u8c3_direct<DMAT>(p, linear, stream)) {
+        BEVK_CUDA(cudaGetLastError());
+        return BEVK_OK;
+    }
+    switch (dtype) {
+    case BEVK_U8: return launch_t<uint8_t, DMAT>(p, channels, linear, stream);
+    case BEVK_F16: return launch_t<__half, DMAT>(p, channels, linear, stream);
+    case BEVK_F32: return launch_t<float, DMAT>(p, channels, linear, stream);
+    }
+    BEVK_FAIL(BEVK_E_ARG, "warp dtype must be BEVK_U8/F16/F32, got %d", dtype);
 }
 
 }  // namespace
@@ -351,19 +382,11 @@ int bevk_plan_generic_chunks(BevkWarpParams &p, int channels)
     return BEVK_OK;
 }
 
-int bevk_launch_warp_generic(const BevkWarpParams &p, int channels, int dtype, int linear,
+int bevk_launch_warp_generic(const BevkWarpParams &p, int channels, int dtype, int linear, bool dmat,
                              cudaStream_t stream)
 {
-    if (dtype == BEVK_U8 && channels == 3 && launch_u8c3_direct(p, linear, stream)) {
-        BEVK_CUDA(cudaGetLastError());
-        return BEVK_OK;
-    }
-    switch (dtype) {
-    case BEVK_U8: return launch_t<uint8_t>(p, channels, linear, stream);
-    case BEVK_F16: return launch_t<__half>(p, channels, linear, stream);
-    case BEVK_F32: return launch_t<float>(p, channels, linear, stream);
-    }
-    BEVK_FAIL(BEVK_E_ARG, "warp dtype must be BEVK_U8/F16/F32, got %d", dtype);
+    return dmat ? launch_generic<true>(p, channels, dtype, linear, stream)
+                : launch_generic<false>(p, channels, dtype, linear, stream);
 }
 
 // ---- touched-pixel accounting -----------------------------------------------------------------

@@ -37,6 +37,29 @@ __device__ __forceinline__ const BevkWarpGroup &find_group(const BevkWarpParams 
     return p.g[gi];
 }
 
+// The dst->src map of this block's group in a device-matrix launch: thread 0 reads the group's
+// matrix from the caller's device table when the kernel runs, inverts it with bevk_invert_adj (the
+// bits bevk_invert3x3 gives on the host) or takes it as is for WARP_INVERSE_MAP, and shares it
+// through sm.  Holds a barrier: every thread of the block calls it, before any thread leaves.
+__device__ __forceinline__ const double *dmat_map(const BevkWarpParams &p, double *sm)
+{
+    if (threadIdx.x == 0 && threadIdx.y == 0) {
+        int gi;
+        const BevkWarpGroup &g = find_group(p, blockIdx.z, gi);
+        double H[9];
+#pragma unroll
+        for (int i = 0; i < 9; ++i) H[i] = g.d.mat[i];
+        if (g.d.invert) {
+            bevk_invert_adj(H, sm);
+        } else {
+#pragma unroll
+            for (int i = 0; i < 9; ++i) sm[i] = H[i];
+        }
+    }
+    __syncthreads();
+    return sm;
+}
+
 // 2-tap window along one axis: first index (clamped into the image) and the weight each of the
 // two window positions receives.  Taps outside [0, n) contribute nothing (border value 0).
 __device__ __forceinline__ void window(int s, int frac, int n, int &first, int &w0, int &w1)

@@ -254,10 +254,16 @@ template <bool LINEAR> struct BgrBytes {
     }
 };
 
-template <class S, bool NV12_OUT, int kBatch>
+// DMAT: the matrices are in a device table (dmat_map).
+template <class S, bool NV12_OUT, int kBatch, bool DMAT>
 __global__ void __launch_bounds__(256) warp_yuv420_kernel(const __grid_constant__ BevkYuvParams P)
 {
     const BevkWarpParams &p = P.w;
+    const double *dm = nullptr;  // DMAT: the group's map, read from the device table
+    if constexpr (DMAT) {
+        __shared__ double sm[9];
+        dm = dmat_map(p, sm);
+    }
     const int bx = blockIdx.x * 32 + threadIdx.x, by = blockIdx.y * 8 + threadIdx.y;  // the lane's 2x2 block
     if (2 * bx >= p.dst_w || 2 * by >= p.dst_h) return;  // no shuffles: lanes may leave on their own
     int gi;
@@ -268,7 +274,7 @@ __global__ void __launch_bounds__(256) warp_yuv420_kernel(const __grid_constant_
     const uint32_t bpx = border_bgr(p.border);
     typename S::Tap t[4];  // pixels (0,0), (1,0), (0,1), (1,1) of the block
 #pragma unroll
-    for (int q = 0; q < 4; ++q) t[q] = S::make(P, g.M, 2 * bx + (q & 1), 2 * by + (q >> 1), bpx);
+    for (int q = 0; q < 4; ++q) t[q] = S::make(P, DMAT ? dm : g.M, 2 * bx + (q & 1), 2 * by + (q >> 1), bpx);
     const uint8_t *src = (const uint8_t *)p.src;
     uint8_t *dst = (uint8_t *)p.dst;
 
@@ -301,45 +307,62 @@ __global__ void __launch_bounds__(256) warp_yuv420_kernel(const __grid_constant_
     }
 }
 
-template <class S, int kBatch>
+template <class S, int kBatch, bool DMAT>
 void launch_warp(const BevkYuvParams &P, bool nv12_out, cudaStream_t stream)
 {
     dim3 block(32, 8, 1);
     dim3 grid((P.w.dst_w / 2 + 31) / 32, (P.w.dst_h / 2 + 7) / 8, P.w.total_chunks);
     if (nv12_out)
-        warp_yuv420_kernel<S, true, kBatch><<<grid, block, 0, stream>>>(P);
+        warp_yuv420_kernel<S, true, kBatch, DMAT><<<grid, block, 0, stream>>>(P);
     else
-        warp_yuv420_kernel<S, false, kBatch><<<grid, block, 0, stream>>>(P);
+        warp_yuv420_kernel<S, false, kBatch, DMAT><<<grid, block, 0, stream>>>(P);
 }
 
 // the four kernels of a YUV source format: bilinear / nearest, word / byte gathers
-template <template <bool, bool> class S>
+template <template <bool, bool> class S, bool DMAT>
 void launch_yuv_src(const BevkYuvParams &P, bool aligned, bool out, int linear, cudaStream_t stream)
 {
     if (linear)
-        aligned ? launch_warp<S<true, true>, 1>(P, out, stream) : launch_warp<S<true, false>, 1>(P, out, stream);
+        aligned ? launch_warp<S<true, true>, 1, DMAT>(P, out, stream)
+                : launch_warp<S<true, false>, 1, DMAT>(P, out, stream);
     else
-        aligned ? launch_warp<S<false, true>, 2>(P, out, stream) : launch_warp<S<false, false>, 2>(P, out, stream);
+        aligned ? launch_warp<S<false, true>, 2, DMAT>(P, out, stream)
+                : launch_warp<S<false, false>, 2, DMAT>(P, out, stream);
 }
 
-}  // namespace
-
-int bevk_launch_warp_yuv420(const BevkYuvParams &P, int src_format, int nv12_out, int linear, cudaStream_t stream)
+// the kernels of BGR or NV12 sources for one matrix source (host maps or a device table)
+template <bool DMAT>
+void launch_bgr_nv12(const BevkYuvParams &P, int src_format, bool aligned, bool out, int linear, cudaStream_t stream)
 {
-    const bool out = nv12_out != 0;
-    const bool aligned = ((uintptr_t)P.w.src % 4) == 0 && (P.pitch % 4) == 0 && (P.frame_stride % 4) == 0;
     if (src_format == BEVK_YUV_NV12) {
-        launch_yuv_src<Nv12Src>(P, aligned, out, linear, stream);
-    } else if (src_format == BEVK_YUV_I420) {
-        launch_yuv_src<I420Src>(P, aligned, out, linear, stream);
+        launch_yuv_src<Nv12Src, DMAT>(P, aligned, out, linear, stream);
     } else {
         // word gathers: rows of a multiple of 4 bytes (both window rows share one word alignment)
         // and a 2x2 window inside the frame
         const bool words = aligned && P.w.src_w >= 2 && P.w.src_h >= 2;
         if (linear)
-            words ? launch_warp<BgrWords<true>, 1>(P, out, stream) : launch_warp<BgrBytes<true>, 1>(P, out, stream);
+            words ? launch_warp<BgrWords<true>, 1, DMAT>(P, out, stream)
+                  : launch_warp<BgrBytes<true>, 1, DMAT>(P, out, stream);
         else
-            words ? launch_warp<BgrWords<false>, 2>(P, out, stream) : launch_warp<BgrBytes<false>, 2>(P, out, stream);
+            words ? launch_warp<BgrWords<false>, 2, DMAT>(P, out, stream)
+                  : launch_warp<BgrBytes<false>, 2, DMAT>(P, out, stream);
+    }
+}
+
+}  // namespace
+
+int bevk_launch_warp_yuv420(const BevkYuvParams &P, int src_format, int nv12_out, int linear, bool dmat,
+                            cudaStream_t stream)
+{
+    const bool out = nv12_out != 0;
+    const bool aligned = ((uintptr_t)P.w.src % 4) == 0 && (P.pitch % 4) == 0 && (P.frame_stride % 4) == 0;
+    if (src_format == BEVK_YUV_I420) {
+        if (dmat) BEVK_FAIL(BEVK_E_ARG, "warp_yuv420: I420 frames take host matrices");
+        launch_yuv_src<I420Src, false>(P, aligned, out, linear, stream);
+    } else if (dmat) {
+        launch_bgr_nv12<true>(P, src_format, aligned, out, linear, stream);
+    } else {
+        launch_bgr_nv12<false>(P, src_format, aligned, out, linear, stream);
     }
     BEVK_CUDA(cudaGetLastError());
     return BEVK_OK;

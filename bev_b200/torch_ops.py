@@ -4,7 +4,8 @@
 ``__graft_entry__.build()``): a thin C++ extension whose operators check tensors, allocate the
 output with torch's caching allocator, take the current CUDA stream and call the extern "C" entry
 points of libbev_b200.so.  After ``load()`` (frames are CUDA tensors; M, H, K, Rt are CPU float64
-tensors; shapes with a leading N also take one unbatched frame and then return one):
+tensors, and the M of the four warps may also be a CUDA tensor on the frames' device; shapes with a
+leading N also take one unbatched frame and then return one):
 
   frames (uint8 BGR (N,H,W,3); NV12 / YUV 4:2:0 (N,H*3/2,W), NV12 with any row pitch / frame stride)
     warp_perspective(src, M, w, h, flags=1, border_mode=0, border_val=0., mat_index=None)
@@ -46,10 +47,17 @@ tests/test_torch_ops_compile_gpu.py).
 
 The operators work under FakeTensor, ``torch.compile(fullgraph=True)`` (also with dynamic batch
 sizes), ``torch.export`` and ``torch.library.opcheck``, and they can be captured in a
-``torch.cuda.graph``.  A captured graph replays the homographies and the mat_index of capture time
-(they live on the host and are read when the call is made): capture one graph per camera set-up and
-refill only the frame tensors between replays.  A CUDA mat_index cannot be captured (reading it
-synchronises); pass a CPU one.
+``torch.cuda.graph``.  Where the homographies live decides what a captured graph replays:
+
+  * CPU M / H: read on the host when the call is made, so fixed at capture time.
+  * CUDA M (warp_perspective, warp_perspective_nv12, warp_perspective_yuv420,
+    warp_perspective_nv12_yuv420): read by the kernels when they run, in stream order (a non-float64
+    one is converted on the stream).  A graph captured once replays whatever matrices were last
+    written into M (``M.copy_(new)`` between replays), and homographies made on the GPU cost no sync.
+    These calls always take the direct-gather warp kernels, not the staged one.
+
+mat_index is planned on the host and stays fixed at capture time; a CUDA mat_index cannot be
+captured (reading it synchronises): pass a CPU one.  The box and point operators take CPU H only.
 """
 import os
 

@@ -190,6 +190,39 @@ int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, 
                                       const double *border_value, void *stream);
 
 /*
+ * The four warps above with the matrices in DEVICE memory, so that homographies made on the GPU
+ * need no copy to the host, and a CUDA graph captured once replays whatever matrices were last
+ * written into the table.  Each takes the arguments of its twin (bevk_warp_perspective,
+ * bevk_warp_perspective_nv12, bevk_warp_perspective_yuv420, bevk_warp_perspective_nv12_yuv420) and
+ * writes the same bytes, except:
+ *   M          DEVICE pointer to n_mats row-major 3x3 float64 matrices (cv2 meaning, as for the
+ *              twin).  The kernels read them on `stream` when they run, and invert them there with
+ *              bevk_invert3x3's arithmetic; the caller keeps M alive and unchanged until then.
+ *   mat_index  stays a HOST array (or NULL with n_mats 1 or n_frames): frame runs, launches and
+ *              frame chunks are planned on the host from it, as for the twin.
+ * The BGR warp always runs the direct-gather kernels (bevk_warp_perspective_path 1 and
+ * bevk_warp_set_path do not apply): the staged kernel plans its tiles on the host from the matrices.
+ * Argument errors are the twin's, BEVK_E_ARG before any device is looked for; a NULL M is one.
+ */
+int bevk_warp_perspective_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
+                               int dst_w, int channels, int dtype, const double *M, int n_mats,
+                               const int32_t *mat_index, int flags, int border_mode, const double *border_value,
+                               void *stream);
+int bevk_warp_perspective_nv12_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                                    int64_t frame_stride, int dst_h, int dst_w, const double *M, int n_mats,
+                                    const int32_t *mat_index, int flags, int border_mode,
+                                    const double *border_value, void *stream);
+int bevk_warp_perspective_yuv420_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
+                                      int dst_w, int layout, int dst_pitch, int64_t dst_frame_stride,
+                                      const double *M, int n_mats, const int32_t *mat_index, int flags,
+                                      int border_mode, const double *border_value, void *stream);
+int bevk_warp_perspective_nv12_yuv420_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
+                                           int64_t frame_stride, int dst_h, int dst_w, int layout, int dst_pitch,
+                                           int64_t dst_frame_stride, const double *M, int n_mats,
+                                           const int32_t *mat_index, int flags, int border_mode,
+                                           const double *border_value, void *stream);
+
+/*
  * The host-buffer warp of video frames for CPU codecs: the frame loop of vis_homo.py:85-111 with a
  * CPU decoder and / or encoder (PyAV, an ffmpeg rawvideo pipe), whose native frames are planar
  * yuv420p.  dst[i] is byte-identical to cv2's chain for the format pair:

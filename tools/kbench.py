@@ -882,6 +882,104 @@ def video_host_small_bench(rounds=5, n=256):
                  (nu + nd) / ceil / 1e6, 100.0 * ceil / med, kernels[r]), flush=True)
 
 
+def device_mats_bench(rounds=5):
+    """Homographies in CUDA tensors (the *_dmat entry points, the operators given a CUDA M) against the
+    same calls with host matrices, alternated in rounds in one process; every pair of routes must give
+    the same bytes.  A device matrix is read and inverted by the kernels when they run, and always takes
+    the direct-gather kernels.
+      cfg 1  one torch.cuda.graph replay of the one-frame loop (1080p BGR frame -> 1024^2 BEV, 852x480
+             small frame, its 1024^2 BEV), captured with CPU H / Hs and with CUDA H / Hs
+      cfg 2  256 1080p frames -> 1024^2, bilinear and nearest: device matrices against the automatic
+             host-matrix route (the staged kernel) and the host-matrix direct-gather kernels
+      cfg 4  the 8 cameras of tests/golden/cfg4_cams.json x 1000 1080p frames, host against device"""
+    import json
+    from bev_b200 import torch_ops
+    torch_ops.load()
+    ops = torch.ops.bev_cuda
+    print("card: %s" % card(), flush=True)
+    peak, _ = bench.measured_peak()
+    dev = torch.device("cuda", 0)
+    g = torch.Generator(device=dev).manual_seed(1234)
+
+    # cfg 1: graph replays
+    H, (w, h), (sw, sh) = bench.h_canon(1), (1920, 1080), (852, 480)
+    fx, fy = w / sw, h / sh
+    Hs = H @ np.array([[fx, 0.0, 0.5 * fx - 0.5], [0.0, fy, 0.5 * fy - 0.5], [0.0, 0.0, 1.0]])
+    frame = torch.randint(0, 256, (1, h, w, 3), dtype=torch.uint8, device=dev, generator=g)
+    graphs, outs = {}, {}
+    for route, (Ht, Hst) in (("host H", (torch.from_numpy(H), torch.from_numpy(Hs))),
+                             ("device H", (torch.from_numpy(H).to(dev), torch.from_numpy(Hs).to(dev)))):
+        def loop(Ht=Ht, Hst=Hst):
+            small = ops.resize(frame, sw, sh)
+            return ops.warp_perspective(frame, Ht, 1024, 1024), small, ops.warp_perspective(small, Hst, 1024, 1024)
+        s = torch.cuda.Stream()
+        s.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(s):
+            for _ in range(3):
+                loop()
+        torch.cuda.current_stream().wait_stream(s)
+        graphs[route] = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graphs[route]):
+            outs[route] = loop()
+        graphs[route].replay()
+    torch.cuda.synchronize()
+    assert all(torch.equal(a, b) for a, b in zip(outs["host H"], outs["device H"])), "cfg 1: routes differ"
+    times = _alternate({r: gr.replay for r, gr in graphs.items()}, rounds, 200)
+    for r, t in times.items():
+        t = np.array(t) * 1e3
+        print("device_mats cfg1 graph replay | %-8s: median %.1f us (min %.1f, max %.1f)"
+              % (r, float(np.median(t)), t.min(), t.max()), flush=True)
+    del graphs, outs
+
+    # cfg 2
+    n, dsize = 256, (1024, 1024)
+    frames = torch.randint(0, 256, (n, h, w, 3), dtype=torch.uint8, device=dev, generator=g)
+    Hd = torch.from_numpy(H).to(dev)
+    for flags, label in ((1, "bilinear"), (0, "nearest")):
+        outs = {r: torch.empty((n, 1024, 1024, 3), dtype=torch.uint8, device=dev) for r in ("auto", "generic", "dmat")}
+        routes = {"host M auto (staged)": lambda: homo.warp_perspective(frames, H, dsize, dst=outs["auto"], flags=flags,
+                                                                         path="auto"),
+                  "host M direct gather": lambda: homo.warp_perspective(frames, H, dsize, dst=outs["generic"],
+                                                                        flags=flags, path="generic"),
+                  "device M": lambda: _native.warp_perspective_dmat(frames, Hd, dsize, dst=outs["dmat"], flags=flags)}
+        for fn in routes.values():
+            fn()
+        torch.cuda.synchronize()
+        assert torch.equal(outs["auto"], outs["dmat"]) and torch.equal(outs["generic"], outs["dmat"]), \
+            "cfg 2 %s: routes differ" % label
+        T, _, _ = _native.warp_touched_pixels((w, h), dsize, H, flags)
+        _report("device_mats cfg2 %s 256 x 1080p -> 1024^2" % label, _alternate(routes, rounds, 10),
+                (T + dsize[0] * dsize[1]) * 3 * n, peak)
+        del outs
+    del frames
+    torch.cuda.empty_cache()
+
+    # cfg 4
+    cams = json.load(open(os.path.join(ROOT, "tests", "golden", "cfg4_cams.json")))
+    n = 1000
+    frames = torch.randint(0, 256, (n, h, w, 3), dtype=torch.uint8, device=dev, generator=g)
+    tables = [(np.array(c["H_bev_img"]), (int(c["bspec"]["u_size"]), int(c["bspec"]["v_size"]))) for c in cams]
+    outs = [(torch.empty((n, d[1], d[0], 3), dtype=torch.uint8, device=dev),
+             torch.empty((n, d[1], d[0], 3), dtype=torch.uint8, device=dev)) for _, d in tables]
+    dev_tables = [torch.from_numpy(Hc).to(dev) for Hc, _ in tables]
+
+    def host_all():
+        for (Hc, d), (o, _) in zip(tables, outs):
+            homo.warp_perspective(frames, Hc, d, dst=o)
+
+    def dev_all():
+        for Hc, (_, d), (_, o) in zip(dev_tables, tables, outs):
+            _native.warp_perspective_dmat(frames, Hc, d, dst=o)
+
+    host_all()
+    dev_all()
+    torch.cuda.synchronize()
+    assert all(torch.equal(a, b) for a, b in outs), "cfg 4: routes differ"
+    algo = sum((_native.warp_touched_pixels((w, h), d, Hc, 1)[0] + d[0] * d[1]) * 3 * n for Hc, d in tables)
+    _report("device_mats cfg4 8 cameras x 1000 x 1080p", _alternate({"host M": host_all, "device M": dev_all},
+                                                                    rounds, 2), algo, peak)
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "nv12":
         nv12_bench()
@@ -893,6 +991,8 @@ if __name__ == "__main__":
         video_host_small_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "frame_loop":
         frame_loop_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "device_mats":
+        device_mats_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_nv12":
         resize_nv12_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_area":
