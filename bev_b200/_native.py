@@ -69,6 +69,7 @@ SIGNATURES = {
                                          _vp]),
     "bevk_composite_u8c3": (_c_int, [_vp, _vp, _vp, _vp, _c_i64, _c_int, _vp]),
     "bevk_composite_bev_u8c3": (_c_int, [_vp, _vp, _vp, _vp] + [_c_int] * 8 + [_dp, _dp, _c_int, _vp]),
+    "bevk_composite_bev_u8c3_dmat": (_c_int, [_vp, _vp, _vp, _vp] + [_c_int] * 8 + [_dp, _dp, _c_int, _vp]),
     "bevk_pts_project": (_c_int, [_vp, _vp, _c_i64, _c_int, _c_int, _dp, _vp]),
     "bevk_xywhr2xyxy": (_c_int, [_vp, _vp, _c_i64, _c_int, _c_int, _dp, _vp]),
     "bevk_xy82xywhr": (_c_int, [_vp, _vp, _c_i64, _c_int, _c_int, _dp, _vp]),
@@ -754,6 +755,30 @@ def composite_bev_u8c3(bg, fg, fg_mask, H_bg, H_fg, dsize, out=None):
     """Fused warp + warp + warp + blend (bev/tool/compo.py:26-50).  bg: (Hb,Wb,3) or (N,Hb,Wb,3);
     fg, fg_mask: (N,Hf,Wf,3) uint8 CUDA; H_bg, H_fg: forward 3x3 (or (N,3,3)) float64 on the host;
     dsize = (width, height) of the BEV.  Returns (N, height, width, 3)."""
+    return _composite_bev(bg, fg, fg_mask, H_bg, H_fg, dsize, out, False)
+
+
+def composite_bev_u8c3_dmat(bg, fg, fg_mask, H_bg, H_fg, dsize, out=None):
+    """composite_bev_u8c3 with H_bg, H_fg CUDA tensors (3,3) or (N,3,3) on fg's device, converted to
+    contiguous float64 on the current stream and read by the kernels when they run: no host sync, and
+    a captured CUDA graph replays the matrices last written into them.  Same bytes as the host call."""
+    return _composite_bev(bg, fg, fg_mask, H_bg, H_fg, dsize, out, True)
+
+
+def _composite_mats(H, what, device):
+    """(K, 9) float64 device matrices for bevk_composite_bev_u8c3_dmat, converted in stream order"""
+    import torch
+    if not isinstance(H, torch.Tensor) or not H.is_cuda:
+        raise TypeError("%s must be a CUDA tensor for the device-matrix compositor, got %s"
+                        % (what, getattr(H, "device", type(H).__name__)))
+    if H.device != device:
+        raise ValueError("%s is on %s, the frames on %s" % (what, H.device, device))
+    if H.numel() == 0 or H.numel() % 9:
+        raise ValueError("%s must be 3x3 or (N,3,3), got %s" % (what, tuple(H.shape)))
+    return H.to(torch.float64).contiguous().reshape(-1, 9)
+
+
+def _composite_bev(bg, fg, fg_mask, H_bg, H_fg, dsize, out, dmat):
     import torch
     for name, t in (("bg", bg), ("fg", fg), ("fg_mask", fg_mask)):
         _require_cuda(t, name)
@@ -767,8 +792,13 @@ def composite_bev_u8c3(bg, fg, fg_mask, H_bg, H_fg, dsize, out=None):
         bg = bg[None]
     if bg.dim() != 4 or bg.shape[0] not in (1, n):
         raise ValueError("bg must be (H, W, 3) or (N, H, W, 3) with N = %d; got %s" % (n, tuple(bg.shape)))
-    Hb = np.ascontiguousarray(np.asarray(_to_numpy(H_bg), np.float64).reshape(-1, 9))
-    Hf = np.ascontiguousarray(np.asarray(_to_numpy(H_fg), np.float64).reshape(-1, 9))
+    if dmat:
+        Hb, Hf = _composite_mats(H_bg, "H_bg", fg.device), _composite_mats(H_fg, "H_fg", fg.device)
+        pb, pf = ctypes.cast(Hb.data_ptr(), _dp), ctypes.cast(Hf.data_ptr(), _dp)
+    else:
+        Hb = np.ascontiguousarray(np.asarray(_to_numpy(H_bg), np.float64).reshape(-1, 9))
+        Hf = np.ascontiguousarray(np.asarray(_to_numpy(H_fg), np.float64).reshape(-1, 9))
+        pb, pf = _dptr(Hb), _dptr(Hf)
     if Hb.shape[0] != Hf.shape[0] or Hb.shape[0] not in (1, n):
         raise ValueError("need 1 or %d homography pairs, got %d / %d" % (n, Hb.shape[0], Hf.shape[0]))
     if not (bg.device == fg.device == fg_mask.device):
@@ -779,12 +809,13 @@ def composite_bev_u8c3(bg, fg, fg_mask, H_bg, H_fg, dsize, out=None):
     out = _out(out, (n, h, w, 3), torch.uint8, fg.device, "out")
     if out.data_ptr() % 4:
         raise ValueError("out must be 4-byte aligned")
+    name = "bevk_composite_bev_u8c3_dmat" if dmat else "bevk_composite_bev_u8c3"
     with torch.cuda.device(fg.device):
-        rc = lib().bevk_composite_bev_u8c3(
+        rc = getattr(lib(), name)(
             _vp(bg.data_ptr()), _vp(fg.data_ptr()), _vp(fg_mask.data_ptr()), _vp(out.data_ptr()),
             n, bg.shape[0], bg.shape[1], bg.shape[2], fg.shape[1], fg.shape[2], h, w,
-            _dptr(Hb), _dptr(Hf), Hb.shape[0], _stream_ptr(fg))
-    _check(rc, "bevk_composite_bev_u8c3")
+            pb, pf, Hb.shape[0], _stream_ptr(fg))
+    _check(rc, name)
     return out
 
 

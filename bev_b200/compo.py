@@ -64,25 +64,35 @@ def composite_bev_batch(bg, fg, fg_mask, H_img2bev_bg, H_img2bev_fg, dsize, fuse
 
     The batched form of compo.py:36-49.  ``fused=None`` picks the one-pass kernel
     (bevk_composite_bev_u8c3) whenever the shapes allow it, else three warps and a blend;
-    True / False force one route (both give identical bytes)."""
+    True / False force one route (both give identical bytes).
+
+    The homographies may also both be CUDA tensors on fg's device (e.g. a rendering camera's pose
+    made in torch): the kernels of either route then read them when they run, with no host sync, and
+    a captured CUDA graph replays whatever matrices were last written into them."""
     import torch
     n = fg.shape[0]
-    Hb = np.asarray(H_img2bev_bg, np.float64).reshape(-1, 3, 3)
-    Hf = np.asarray(H_img2bev_fg, np.float64).reshape(-1, 3, 3)
+    dmat = any(isinstance(H, torch.Tensor) and H.is_cuda for H in (H_img2bev_bg, H_img2bev_fg))
+    if dmat:
+        Hb = _native._composite_mats(H_img2bev_bg, "H_img2bev_bg", fg.device).reshape(-1, 3, 3)
+        Hf = _native._composite_mats(H_img2bev_fg, "H_img2bev_fg", fg.device).reshape(-1, 3, 3)
+        composite_bev, warp = _native.composite_bev_u8c3_dmat, _native.warp_perspective_dmat
+    else:
+        Hb = np.asarray(H_img2bev_bg, np.float64).reshape(-1, 3, 3)
+        Hf = np.asarray(H_img2bev_fg, np.float64).reshape(-1, 3, 3)
+        composite_bev, warp = _native.composite_bev_u8c3, _native.warp_perspective
     can_fuse = _native.composite_bev_fusable(bg, fg, dsize)
     if fused is None:
         fused = can_fuse
     if fused:
-        return _native.composite_bev_u8c3(bg, fg, fg_mask, Hb, Hf, dsize)
+        return composite_bev(bg, fg, fg_mask, Hb, Hf, dsize)
     if bg.shape[0] == 1 and len(Hb) > 1:  # one background seen through a camera per frame
         bg = bg.expand(n, -1, -1, -1).contiguous()
-    bg_bev = _native.warp_perspective(bg, Hb if len(Hb) > 1 else Hb[0], dsize, flags=INTER_LINEAR)
+    bg_bev = warp(bg, Hb if len(Hb) > 1 else Hb[0], dsize, flags=INTER_LINEAR)
     if bg_bev.shape[0] != n:
         bg_bev = bg_bev.expand(n, -1, -1, -1)
     if len(Hf) == 1:
-        fm = _native.warp_perspective(torch.cat([fg, fg_mask], 0), Hf[0], dsize, flags=INTER_LINEAR)
-    else:
+        fm = warp(torch.cat([fg, fg_mask], 0), Hf[0], dsize, flags=INTER_LINEAR)
+    else:  # mat_index stays on the host
         idx = np.concatenate([np.arange(n, dtype=np.int32)] * 2)
-        fm = _native.warp_perspective(torch.cat([fg, fg_mask], 0), Hf, dsize, flags=INTER_LINEAR,
-                                      mat_index=idx)
+        fm = warp(torch.cat([fg, fg_mask], 0), Hf, dsize, flags=INTER_LINEAR, mat_index=idx)
     return _native.composite_u8c3(bg_bev.contiguous(), fm[:n], fm[n:])

@@ -112,7 +112,16 @@ __global__ void __launch_bounds__(256) composite_kernel(const uint32_t *__restri
 constexpr int kCompoGroups = 32;
 
 struct CompoGroup {
-    double Mb[9], Mf[9];  // dst -> src maps of the background / foreground (inverted on the host)
+    // dst -> src maps of the background / foreground (inverted on the host), or in device-matrix
+    // launches (bevk_composite_bev_u8c3_dmat) the group's forward matrices in device memory
+    union {
+        double Mb[9];
+        const double *Hb;
+    };
+    union {
+        double Mf[9];
+        const double *Hf;
+    };
     int first, count;     // frames first .. first + count - 1
     int chunk0;           // first z-block of the group
     int pad;
@@ -174,23 +183,61 @@ __device__ __forceinline__ uint32_t gather_pixel(const Gather &t, const uint8_t 
     return gather_math(t, w);
 }
 
-template <int kBatch>
+// The group of this block's z-chunk.  DMAT blocks search with all loads in flight at once: the
+// search lies on their critical path, in front of the matrix loads and the barrier (DESIGN 3.13).
+// The host-matrix instances keep the serial loop they were tuned and measured with.
+template <bool DMAT>
+__device__ __forceinline__ const CompoGroup &compo_group(const CompoParams &p)
+{
+    int gi = 0;
+    if constexpr (DMAT) {
+        if (p.n_groups > 1) {
+#pragma unroll
+            for (int i = 1; i < kCompoGroups; ++i)
+                if (i < p.n_groups && (int)blockIdx.z >= p.g[i].chunk0) gi = i;
+        }
+    } else {
+#pragma unroll 1
+        for (int i = 1; i < p.n_groups; ++i)
+            if ((int)blockIdx.z >= p.g[i].chunk0) gi = i;
+    }
+    return p.g[gi];
+}
+
+// DMAT: the group holds device addresses of its forward matrices (CompoGroup::Hb / Hf).  Every
+// thread finds the group; threads 0 and 1 of the block each read one of the matrices when the kernel
+// runs, invert it with bevk_invert_adj (the bits bevk_invert3x3 gives on the host; a singular matrix
+// gives the zero map) and share the map through shared memory behind one barrier, which every
+// thread reaches before any thread leaves.
+template <int kBatch, bool DMAT>
 __global__ void __launch_bounds__(256) composite_bev_kernel(const __grid_constant__ CompoParams p)
 {
+    const double *dm = nullptr;        // DMAT: the background map, then the foreground map
+    const CompoGroup *dg = nullptr;    // DMAT: the block's group
+    if constexpr (DMAT) {
+        __shared__ double sm[18];
+        dg = &compo_group<true>(p);
+        const int t = threadIdx.y * 32 + threadIdx.x;
+        if (t < 2) {
+            const double *H = t ? dg->Hf : dg->Hb;
+            double h[9];
+#pragma unroll
+            for (int i = 0; i < 9; ++i) h[i] = H[i];
+            bevk_invert_adj(h, sm + 9 * t);
+        }
+        __syncthreads();
+        dm = sm;
+    }
     const int lane = threadIdx.x, x0 = blockIdx.x * 32;
     const int x = x0 + lane, y = blockIdx.y * 8 + threadIdx.y;
     if (y >= p.dst_h) return;  // a warp is one dst row segment: uniform exit
-    int gi = 0;
-#pragma unroll 1
-    for (int i = 1; i < p.n_groups; ++i)
-        if ((int)blockIdx.z >= p.g[i].chunk0) gi = i;
-    const CompoGroup &g = p.g[gi];
+    const CompoGroup &g = DMAT ? *dg : compo_group<false>(p);
     const int f0 = ((int)blockIdx.z - g.chunk0) * p.frames_per_chunk;
     const int f1 = min(f0 + p.frames_per_chunk, g.count);
 
     const int xc = min(x, p.dst_w - 1);
-    const Gather tb = make_gather(g.Mb, xc, y, p.bw0, p.bg_w, p.bg_h, p.bg_frame);
-    const Gather tf = make_gather(g.Mf, xc, y, p.bw0, p.fg_w, p.fg_h, p.fg_frame);
+    const Gather tb = make_gather(DMAT ? dm : g.Mb, xc, y, p.bw0, p.bg_w, p.bg_h, p.bg_frame);
+    const Gather tf = make_gather(DMAT ? dm + 9 : g.Mf, xc, y, p.bw0, p.fg_w, p.fg_h, p.fg_frame);
 
     const int j = lane >> 2, r4 = lane & 3;
     const uint32_t sel_pack = r4 == 0 ? 0x4210u : (r4 == 1 ? 0x5421u : 0x6542u);
@@ -258,10 +305,13 @@ extern "C" int bevk_composite_u8c3(const void *bg, const void *fg, const void *f
 }
 
 
-extern "C" int bevk_composite_bev_u8c3(const void *bg, const void *fg, const void *fg_mask, void *out,
-                                       int n_frames, int n_bg, int bg_h, int bg_w, int fg_h, int fg_w,
-                                       int dst_h, int dst_w, const double *H_bg, const double *H_fg,
-                                       int n_mats, void *stream)
+namespace {
+
+// The fused compositor with host matrices (inverted here) or, dmat, device matrices (read and
+// inverted by the kernels when they run).  Both plan runs, groups and frame chunks alike.
+int composite_bev(const void *bg, const void *fg, const void *fg_mask, void *out, int n_frames, int n_bg, int bg_h,
+                  int bg_w, int fg_h, int fg_w, int dst_h, int dst_w, const double *H_bg, const double *H_fg,
+                  int n_mats, bool dmat, void *stream)
 {
     if (n_frames < 0) BEVK_FAIL(BEVK_E_ARG, "composite_bev: n_frames must be >= 0");
     if (bg_h < 2 || bg_w < 2 || fg_h < 2 || fg_w < 2 || dst_h <= 0 || dst_w <= 0)
@@ -314,8 +364,14 @@ extern "C" int bevk_composite_bev_u8c3(const void *bg, const void *fg, const voi
         int z = 0;
         for (int i = 0; i < ng; ++i) {
             CompoGroup &g = p.g[i];
-            bevk_invert3x3(H_bg + (size_t)(r0 + i) * 9, g.Mb);  // cv2 inverts a forward matrix
-            bevk_invert3x3(H_fg + (size_t)(r0 + i) * 9, g.Mf);
+            const size_t k = (size_t)(r0 + i) * 9;
+            if (dmat) {
+                g.Hb = H_bg + k;
+                g.Hf = H_fg + k;
+            } else {
+                bevk_invert3x3(H_bg + k, g.Mb);  // cv2 inverts a forward matrix
+                bevk_invert3x3(H_fg + k, g.Mf);
+            }
             g.first = n_mats == 1 ? 0 : r0 + i;
             g.count = count;
             g.chunk0 = z;
@@ -327,11 +383,34 @@ extern "C" int bevk_composite_bev_u8c3(const void *bg, const void *fg, const voi
         dim3 block(32, 8, 1), grid((dst_w + 31) / 32, (dst_h + 7) / 8, z);
         // two frames of windows in flight per thread when runs are long enough to use them; the
         // one-frame build keeps more warps resident for the coordinate-bound camera-per-frame case
-        if (fpc >= 2)
-            composite_bev_kernel<2><<<grid, block, 0, st>>>(p);
+        if (dmat)
+            fpc >= 2 ? composite_bev_kernel<2, true><<<grid, block, 0, st>>>(p)
+                     : composite_bev_kernel<1, true><<<grid, block, 0, st>>>(p);
+        else if (fpc >= 2)
+            composite_bev_kernel<2, false><<<grid, block, 0, st>>>(p);
         else
-            composite_bev_kernel<1><<<grid, block, 0, st>>>(p);
+            composite_bev_kernel<1, false><<<grid, block, 0, st>>>(p);
         BEVK_CUDA(cudaGetLastError());
     }
     return BEVK_OK;
+}
+
+}  // namespace
+
+extern "C" int bevk_composite_bev_u8c3(const void *bg, const void *fg, const void *fg_mask, void *out,
+                                       int n_frames, int n_bg, int bg_h, int bg_w, int fg_h, int fg_w,
+                                       int dst_h, int dst_w, const double *H_bg, const double *H_fg,
+                                       int n_mats, void *stream)
+{
+    return composite_bev(bg, fg, fg_mask, out, n_frames, n_bg, bg_h, bg_w, fg_h, fg_w, dst_h, dst_w, H_bg, H_fg,
+                         n_mats, false, stream);
+}
+
+extern "C" int bevk_composite_bev_u8c3_dmat(const void *bg, const void *fg, const void *fg_mask, void *out,
+                                            int n_frames, int n_bg, int bg_h, int bg_w, int fg_h, int fg_w,
+                                            int dst_h, int dst_w, const double *H_bg, const double *H_fg,
+                                            int n_mats, void *stream)
+{
+    return composite_bev(bg, fg, fg_mask, out, n_frames, n_bg, bg_h, bg_w, fg_h, fg_w, dst_h, dst_w, H_bg, H_fg,
+                         n_mats, true, stream);
 }

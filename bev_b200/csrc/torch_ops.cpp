@@ -7,10 +7,10 @@
 // allocator, takes the current CUDA stream and calls the extern "C" entry point with raw pointers --
 // no arithmetic lives here.  Homographies, K and Rt are CPU float64 tensors (they stay on the host,
 // SURVEY.md 8b "Matrix ownership"), and so is a mat_index during CUDA-graph capture -- except the M of
-// the four warps, which may also be a CUDA tensor on the frames' device: the kernels then read it
-// when they run (the *_dmat entry points), so nothing synchronises and a captured graph replays
-// whatever matrices were last written into it.  No CPU implementation is registered: CPU tensors
-// fail in the dispatcher, there is no CPU fallback.
+// the four warps and the H_bg / H_fg of composite_bev, which may also be CUDA tensors on the frames'
+// device: the kernels then read them when they run (the *_dmat entry points), so nothing synchronises
+// and a captured graph replays whatever matrices were last written into them.  No CPU implementation
+// is registered: CPU tensors fail in the dispatcher, there is no CPU fallback.
 //
 // Each operator is ONE function, registered for both the CUDA and the Meta dispatch key: it checks
 // shapes and dtypes and allocates the output with SymInt sizes, and returns there for meta tensors
@@ -422,8 +422,17 @@ at::Tensor composite(const at::Tensor &bg, const at::Tensor &fg, const at::Tenso
     return out;
 }
 
+// The compositor's forward matrices as contiguous float64: on the host, or (device) on fg's device,
+// converted on the current stream with no host read
+at::Tensor composite_mats(const at::Tensor &H, bool device, const at::Tensor &fg, const char *what)
+{
+    if (!device) return host_f64(H, what);
+    check_cuda(H, fg, what);
+    return H.to(at::kDouble).contiguous();
+}
+
 // fg, mask (H, W, 3) or (N, H, W, 3); bg (H, W, 3), (1, H, W, 3) or (N, H, W, 3); H_bg, H_fg 1 or N
-// forward 3x3 matrices each -> (h, w, 3) or (N, h, w, 3)
+// forward 3x3 matrices each, both on the host or both on fg's device -> (h, w, 3) or (N, h, w, 3)
 at::Tensor composite_bev(const at::Tensor &bg, const at::Tensor &fg, const at::Tensor &mask, const at::Tensor &H_bg,
                          const at::Tensor &H_fg, int64_t w, int64_t h)
 {
@@ -450,12 +459,15 @@ at::Tensor composite_bev(const at::Tensor &bg, const at::Tensor &fg, const at::T
     check_cuda(mask, fg, "mask");
     const at::Tensor b = aligned(bg.dim() == 3 ? bg.unsqueeze(0) : bg, 16), f = aligned(fg, 16),
                      k = aligned(mask, 16);
-    const at::Tensor Hb = host_f64(H_bg, "H_bg"), Hf = host_f64(H_fg, "H_fg");
-    check_rc(bevk_composite_bev_u8c3(b.data_ptr(), f.data_ptr(), k.data_ptr(), out.data_ptr(), (int)I(fr.n),
-                                     (int)b.size(0), (int)b.size(1), (int)b.size(2), (int)I(fr.h), (int)I(fr.w),
-                                     (int)h, (int)w, Hb.data_ptr<double>(), Hf.data_ptr<double>(),
-                                     (int)(Hb.numel() / 9), current_stream(fg)),
-             "bevk_composite_bev_u8c3");
+    const bool device = H_bg.is_cuda() || H_fg.is_cuda();
+    TORCH_CHECK(H_bg.is_cuda() == H_fg.is_cuda(), "H_bg is on ", H_bg.device(), " and H_fg on ", H_fg.device(),
+                ": pass both homographies on the host or both on the frames' CUDA device");
+    const at::Tensor Hb = composite_mats(H_bg, device, fg, "H_bg"), Hf = composite_mats(H_fg, device, fg, "H_fg");
+    check_rc((device ? bevk_composite_bev_u8c3_dmat : bevk_composite_bev_u8c3)(
+                 b.data_ptr(), f.data_ptr(), k.data_ptr(), out.data_ptr(), (int)I(fr.n), (int)b.size(0),
+                 (int)b.size(1), (int)b.size(2), (int)I(fr.h), (int)I(fr.w), (int)h, (int)w, Hb.data_ptr<double>(),
+                 Hf.data_ptr<double>(), (int)(Hb.numel() / 9), current_stream(fg)),
+             device ? "bevk_composite_bev_u8c3_dmat" : "bevk_composite_bev_u8c3");
     return out;
 }
 

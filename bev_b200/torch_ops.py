@@ -4,8 +4,8 @@
 ``__graft_entry__.build()``): a thin C++ extension whose operators check tensors, allocate the
 output with torch's caching allocator, take the current CUDA stream and call the extern "C" entry
 points of libbev_b200.so.  After ``load()`` (frames are CUDA tensors; M, H, K, Rt are CPU float64
-tensors, and the M of the four warps may also be a CUDA tensor on the frames' device; shapes with a
-leading N also take one unbatched frame and then return one):
+tensors, and the M of the four warps and the H_bg / H_fg of composite_bev may also be CUDA tensors on
+the frames' device; shapes with a leading N also take one unbatched frame and then return one):
 
   frames (uint8 BGR (N,H,W,3); NV12 / YUV 4:2:0 (N,H*3/2,W), NV12 with any row pitch / frame stride)
     warp_perspective(src, M, w, h, flags=1, border_mode=0, border_val=0., mat_index=None)
@@ -55,6 +55,8 @@ sizes), ``torch.export`` and ``torch.library.opcheck``, and they can be captured
     one is converted on the stream).  A graph captured once replays whatever matrices were last
     written into M (``M.copy_(new)`` between replays), and homographies made on the GPU cost no sync.
     These calls always take the direct-gather warp kernels, not the staged one.
+  * CUDA H_bg and H_fg (composite_bev; both, not one of them): the same, through the fused
+    compositor's device-matrix kernels.
 
 mat_index is planned on the host and stays fixed at capture time; a CUDA mat_index cannot be
 captured (reading it synchronises): pass a CPU one.  The box and point operators take CPU H only.

@@ -338,6 +338,23 @@ int bevk_composite_bev_u8c3(const void *bg, const void *fg, const void *fg_mask,
                             int n_mats, void *stream);
 
 /*
+ * bevk_composite_bev_u8c3 with the homographies in DEVICE memory, like the warp _dmat entry points
+ * above: a rendering camera's pose made on the GPU needs no copy to the host, and a CUDA graph
+ * captured once replays whatever matrices were last written into H_bg / H_fg.  Takes the twin's
+ * arguments and writes the same bytes, except:
+ *   H_bg, H_fg  DEVICE pointers to n_mats row-major 3x3 float64 FORWARD matrices each.  The kernels
+ *               read them on `stream` when they run, and invert them there with bevk_invert3x3's
+ *               arithmetic; the caller keeps them alive and unchanged until then.
+ * Runs, launches and frame chunks are planned on the host from n_mats and n_frames, as for the
+ * twin.  Argument errors are the twin's, BEVK_E_ARG before any device is looked for; a NULL H_bg or
+ * H_fg is one.
+ */
+int bevk_composite_bev_u8c3_dmat(const void *bg, const void *fg, const void *fg_mask, void *out,
+                                 int n_frames, int n_bg, int bg_h, int bg_w, int fg_h, int fg_w,
+                                 int dst_h, int dst_w, const double *H_bg, const double *H_fg,
+                                 int n_mats, void *stream);
+
+/*
  * Homogeneous point projection with divide.  Replaces rbox.pts_world_bev (bev/rbox.py:136-151)
  * and the cv2.perspectiveTransform call sites (bev/visualizer/rbox_vis.py:54,61,74).
  *   pts/out [n][dim], dim 2 (w = 1 implied, 2 columns out) or 3 (homogeneous in, 3 columns out,

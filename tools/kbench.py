@@ -980,6 +980,67 @@ def device_mats_bench(rounds=5):
                                                                     rounds, 2), algo, peak)
 
 
+def compo_dmat_bench(rounds=5, n=64):
+    """The fused BEV compositor with CUDA H_bg / H_fg (bevk_composite_bev_u8c3_dmat) against the same
+    calls with host matrices, alternated in rounds in one process; each pair must give the same bytes.
+      x64    n 1080p renders + masks over ONE 1080p background -> 1024^2 BEVs (compo_bench's row),
+             with one shared homography pair and with one pair per frame
+      graph  one torch.cuda.graph replay of a single 1080p composite, captured with CPU and with
+             CUDA matrices"""
+    from bev_b200 import torch_ops
+    torch_ops.load()
+    ops = torch.ops.bev_cuda
+    print("card: %s" % card(), flush=True)
+    peak, _ = bench.measured_peak()
+    dev = torch.device("cuda", 0)
+    g = torch.Generator(device=dev).manual_seed(1234)
+    ssize, dsize = (1920, 1080), (1024, 1024)
+    B = torch.randint(0, 256, (1, 1080, 1920, 3), dtype=torch.uint8, device=dev, generator=g)
+    F = torch.randint(0, 256, (n, 1080, 1920, 3), dtype=torch.uint8, device=dev, generator=g)
+    M = torch.randint(0, 256, (n, 1080, 1920, 3), dtype=torch.uint8, device=dev, generator=g)
+    H = bench.h_canon(1)
+    T, _, _ = _native.warp_touched_pixels(ssize, dsize, H, 1)
+    D = dsize[0] * dsize[1]
+    algo = 3 * (T + n * (2 * T + D))  # as compo_bench: background once, render and mask per frame, output
+    for label, Hh in (("shared pair", H), ("pair per frame", np.repeat(H[None], n, 0))):
+        Hd = torch.from_numpy(np.ascontiguousarray(Hh)).to(dev)
+        outs = [torch.empty((n, 1024, 1024, 3), dtype=torch.uint8, device=dev) for _ in range(2)]
+        routes = {"host H": lambda: _native.composite_bev_u8c3(B, F, M, Hh, Hh, dsize, out=outs[0]),
+                  "device H": lambda: _native.composite_bev_u8c3_dmat(B, F, M, Hd, Hd, dsize, out=outs[1])}
+        for fn in routes.values():
+            fn()
+        torch.cuda.synchronize()
+        assert torch.equal(outs[0], outs[1]), "x%d %s: routes differ" % (n, label)
+        _report("compo_dmat x%d 1080p -> 1024^2 %s" % (n, label), _alternate(routes, rounds, 10), algo, peak)
+        del outs
+    del F, M
+    torch.cuda.empty_cache()
+
+    fg = torch.randint(0, 256, (1080, 1920, 3), dtype=torch.uint8, device=dev, generator=g)
+    mask = torch.randint(0, 256, (1080, 1920, 3), dtype=torch.uint8, device=dev, generator=g)
+    graphs, outs = {}, {}
+    for route, Ht in (("host H", torch.from_numpy(H)), ("device H", torch.from_numpy(H).to(dev))):
+        def one(Ht=Ht):
+            return ops.composite_bev(B[0], fg, mask, Ht, Ht, 1024, 1024)
+        s = torch.cuda.Stream()
+        s.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(s):
+            for _ in range(3):
+                one()
+        torch.cuda.current_stream().wait_stream(s)
+        graphs[route] = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graphs[route]):
+            outs[route] = one()
+        graphs[route].replay()
+    torch.cuda.synchronize()
+    assert torch.equal(outs["host H"], outs["device H"]), "graph: routes differ"
+    times = _alternate({r: gr.replay for r, gr in graphs.items()}, rounds, 200)
+    for r, t in times.items():
+        t = np.array(t) * 1e3
+        print("compo_dmat 1080p -> 1024^2 graph replay | %-8s: median %.1f us (min %.1f, max %.1f)"
+              % (r, float(np.median(t)), t.min(), t.max()), flush=True)
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "nv12":
         nv12_bench()
@@ -993,6 +1054,8 @@ if __name__ == "__main__":
         frame_loop_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "device_mats":
         device_mats_bench()
+    elif len(sys.argv) > 1 and sys.argv[1] == "compo_dmat":
+        compo_dmat_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_nv12":
         resize_nv12_bench()
     elif len(sys.argv) > 1 and sys.argv[1] == "resize_area":
