@@ -198,46 +198,38 @@ def _warp_dtype(t):
     return code
 
 
-def _prep_mats(M, n_frames, mat_index):
-    Ms = np.ascontiguousarray(_to_numpy(M), dtype=np.float64)
-    if Ms.ndim == 2:
-        Ms = Ms[None]
-    if Ms.ndim != 3 or Ms.shape[1:] != (3, 3):
-        raise ValueError("M must be 3x3 or (K,3,3), got %s" % (Ms.shape,))
-    idx = None
-    if mat_index is not None:
-        idx = np.ascontiguousarray(_to_numpy(mat_index), dtype=np.int32).reshape(-1)
-        if idx.shape[0] != n_frames:
-            raise ValueError("mat_index has %d entries for %d frames" % (idx.shape[0], n_frames))
-    elif Ms.shape[0] not in (1, n_frames):
-        raise ValueError("%d matrices for %d frames needs mat_index" % (Ms.shape[0], n_frames))
-    return Ms, idx
-
-
 class _Mats:
     """The matrices of one warp call as the C ABI takes them: ptr (host, or with dmat device, float64
     3x3 matrices), n (their count) and idx (host int32 mat_index or None).  keep holds what ptr points
     into for the length of the call."""
 
     def __init__(self, M, n_frames, mat_index, dmat, device):
-        if not dmat:
-            Ms, self.idx = _prep_mats(M, n_frames, mat_index)
-            self.keep, self.ptr, self.n = Ms, _dptr(Ms), Ms.shape[0]
-            return
-        import torch
-        if not isinstance(M, torch.Tensor) or not M.is_cuda:
-            raise TypeError("M must be a CUDA tensor for the device-matrix warps, got %s"
-                            % (getattr(M, "device", type(M).__name__),))
-        if M.device != device:
-            raise ValueError("M is on %s, the frames on %s" % (M.device, device))
-        if M.dtype != torch.float64:
-            raise TypeError("M must be float64, got %s" % (M.dtype,))
-        Mt = (M[None] if M.dim() == 2 else M).contiguous()  # stream-ordered; no host read
-        if Mt.dim() != 3 or tuple(Mt.shape[1:]) != (3, 3) or Mt.shape[0] == 0:
-            raise ValueError("M must be 3x3 or (K,3,3), got %s" % (tuple(M.shape),))
-        # the indices are planned on the host: the same checks as for host matrices
-        _, self.idx = _prep_mats(np.zeros((Mt.shape[0], 3, 3)), n_frames, mat_index)
-        self.keep, self.ptr, self.n = Mt, ctypes.cast(Mt.data_ptr(), _dp), Mt.shape[0]
+        if dmat:
+            import torch
+            if not isinstance(M, torch.Tensor) or not M.is_cuda:
+                raise TypeError("M must be a CUDA tensor for the device-matrix warps, got %s"
+                                % (getattr(M, "device", type(M).__name__),))
+            if M.device != device:
+                raise ValueError("M is on %s, the frames on %s" % (M.device, device))
+            if M.dtype != torch.float64:
+                raise TypeError("M must be float64, got %s" % (M.dtype,))
+            Ms = (M[None] if M.dim() == 2 else M).contiguous()  # stream-ordered; no host read
+            if Ms.dim() != 3 or tuple(Ms.shape[1:]) != (3, 3) or Ms.shape[0] == 0:
+                raise ValueError("M must be 3x3 or (K,3,3), got %s" % (tuple(M.shape),))
+        else:
+            Ms = np.ascontiguousarray(_to_numpy(M), dtype=np.float64)
+            Ms = Ms[None] if Ms.ndim == 2 else Ms
+            if Ms.ndim != 3 or Ms.shape[1:] != (3, 3):
+                raise ValueError("M must be 3x3 or (K,3,3), got %s" % (Ms.shape,))
+        self.ptr = ctypes.cast(Ms.data_ptr(), _dp) if dmat else _dptr(Ms)
+        self.keep, self.n, self.idx = Ms, Ms.shape[0], None
+        # the indices are planned on the host, for device matrices too
+        if mat_index is not None:
+            self.idx = np.ascontiguousarray(_to_numpy(mat_index), dtype=np.int32).reshape(-1)
+            if self.idx.shape[0] != n_frames:
+                raise ValueError("mat_index has %d entries for %d frames" % (self.idx.shape[0], n_frames))
+        elif self.n not in (1, n_frames):
+            raise ValueError("%d matrices for %d frames needs mat_index" % (self.n, n_frames))
 
     def idx_ptr(self):
         return self.idx.ctypes.data_as(_i32p) if self.idx is not None else None
@@ -268,40 +260,15 @@ def warp_perspective(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue
                      mat_index=None, path=None):
     """path: None (the calling thread's default, see set_warp_path), "auto", "generic" (direct-gather
     kernels) or "fast" (staged kernel; raises if the shape does not qualify)."""
-    return _warp_perspective(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, path, False)
+    return _warp(src, "frames", M, dsize, dst, "frames", flags, borderMode, borderValue, mat_index, False,
+                 path=_PATHS.get(path, path))
 
 
 def warp_perspective_dmat(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue=0, mat_index=None):
     """warp_perspective with M a CUDA float64 tensor (3,3) or (K,3,3) on src's device, read by the
     kernels when they run on the current stream: no host sync, and a captured CUDA graph replays the
     matrices last written into M.  Always the direct-gather kernels; mat_index stays on the host."""
-    return _warp_perspective(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, None, True)
-
-
-def _warp_perspective(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, path, dmat):
-    import torch
-    _require_cuda(src, "src")
-    code = _warp_dtype(src)
-    s4, undo = _frames_view(src)
-    s4 = s4.contiguous()
-    n, h, w, c = s4.shape
-    dw, dh = int(dsize[0]), int(dsize[1])
-    m = _Mats(M, n, mat_index, dmat, src.device)
-    d4 = None
-    if dst is not None:  # any rank whose (N, H, W, C) view has the output's shape
-        _require_cuda(dst, "dst")
-        d4, _ = _frames_view(dst)
-    out4 = _out(d4, (n, dh, dw, c), src.dtype, src.device)
-    b = _border(borderValue)
-    args = (_vp(s4.data_ptr()), _vp(out4.data_ptr()), n, h, w, dh, dw, c, code, m.ptr, m.n, m.idx_ptr(),
-            int(flags), int(borderMode), _dptr(b))
-    with torch.cuda.device(src.device):
-        if dmat:
-            rc = lib().bevk_warp_perspective_dmat(*args, _stream_ptr(src))
-        else:
-            rc = lib().bevk_warp_perspective_path(*args, _PATHS.get(path, path), _stream_ptr(src))
-    _check(rc, "bevk_warp_perspective_dmat" if dmat else "bevk_warp_perspective")
-    return dst if dst is not None else undo(out4)
+    return _warp(src, "frames", M, dsize, dst, "frames", flags, borderMode, borderValue, mat_index, True)
 
 
 def warp_perspective_host(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue=0,
@@ -315,25 +282,23 @@ def warp_perspective_host(src, M, dsize, dst=None, flags=1, borderMode=0, border
     s4 = np.ascontiguousarray(s4)
     n, h, w, c = s4.shape
     dw, dh = int(dsize[0]), int(dsize[1])
-    Ms, idx = _prep_mats(M, n, mat_index)
+    m = _Mats(M, n, mat_index, False, None)
     if dst is None:
         out4 = np.empty((n, dh, dw, c), s4.dtype)
     else:
-        out4 = _to_numpy(dst) if not isinstance(dst, np.ndarray) else dst
-        out4 = out4.reshape(n, dh, dw, c)
+        out4 = _to_numpy(dst).reshape(n, dh, dw, c)
         if out4.dtype != s4.dtype or not out4.flags["C_CONTIGUOUS"]:
             raise ValueError("dst must be C-contiguous with src's dtype")
     b = _border(borderValue)
     rc = lib().bevk_warp_perspective_host(
-        _vp(s4.ctypes.data), _vp(out4.ctypes.data), n, h, w, dh, dw, c, code, _dptr(Ms),
-        Ms.shape[0], idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags),
-        int(borderMode), _dptr(b))
+        _vp(s4.ctypes.data), _vp(out4.ctypes.data), n, h, w, dh, dw, c, code, m.ptr, m.n, m.idx_ptr(),
+        int(flags), int(borderMode), _dptr(b))
     _check(rc, "bevk_warp_perspective_host")
     return dst if dst is not None else undo(out4)
 
 
 def _nv12_frames(src):
-    """(frames view (N, H*3/2, W), N, H, W, pitch, frame stride) of an NV12 tensor (H*3/2, W) or
+    """(frames view (N, H*3/2, W), N, H, W, (pitch, frame stride)) of an NV12 tensor (H*3/2, W) or
     (N, H*3/2, W).  Pitch and frame stride come from the tensor's strides, so a decoder surface
     with padded rows is used as it is."""
     import torch
@@ -357,14 +322,14 @@ def _nv12_frames(src):
     if pitch < w:
         raise ValueError("NV12 row pitch %d is smaller than the width %d" % (pitch, w))
     fstride = s3.stride(0) if n > 1 else pitch * rows
-    return s3, n, rows // 3 * 2, w, pitch, fstride
+    return s3, n, rows // 3 * 2, w, (pitch, fstride)
 
 
 def nv12_to_bgr(src, dst=None):
     """cv2.cvtColor(f, COLOR_YUV2BGR_NV12) on CUDA uint8 NV12 frames (H*3/2, W) or (N, H*3/2, W)
     -> (H, W, 3) or (N, H, W, 3) BGR."""
     import torch
-    s3, n, h, w, pitch, fstride = _nv12_frames(src)
+    s3, n, h, w, (pitch, fstride) = _nv12_frames(src)
     dst = _out(dst, (n, h, w, 3) if src.dim() == 3 else (h, w, 3), torch.uint8, src.device)
     with torch.cuda.device(src.device):
         rc = lib().bevk_nv12_to_bgr(_vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride,
@@ -376,28 +341,12 @@ def nv12_to_bgr(src, dst=None):
 def warp_perspective_nv12(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue=0, mat_index=None):
     """warp_perspective of nv12_to_bgr(src) in one pass: (H*3/2, W) -> (h, w, 3), (N, H*3/2, W) ->
     (N, h, w, 3) BGR uint8.  M / mat_index as for warp_perspective."""
-    return _warp_perspective_nv12(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, False)
+    return _warp(src, "nv12", M, dsize, dst, "bgr", flags, borderMode, borderValue, mat_index, False)
 
 
 def warp_perspective_nv12_dmat(src, M, dsize, dst=None, flags=1, borderMode=0, borderValue=0, mat_index=None):
     """warp_perspective_nv12 with M a CUDA float64 tensor, as for warp_perspective_dmat."""
-    return _warp_perspective_nv12(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, True)
-
-
-def _warp_perspective_nv12(src, M, dsize, dst, flags, borderMode, borderValue, mat_index, dmat):
-    import torch
-    s3, n, h, w, pitch, fstride = _nv12_frames(src)
-    dw, dh = int(dsize[0]), int(dsize[1])
-    m = _Mats(M, n, mat_index, dmat, src.device)
-    dst = _out(dst, (n, dh, dw, 3) if src.dim() == 3 else (dh, dw, 3), torch.uint8, src.device)
-    b = _border(borderValue)
-    name = "bevk_warp_perspective_nv12_dmat" if dmat else "bevk_warp_perspective_nv12"
-    with torch.cuda.device(src.device):
-        rc = getattr(lib(), name)(
-            _vp(s3.data_ptr()), _vp(dst.data_ptr()), n, h, w, pitch, fstride, dh, dw, m.ptr, m.n, m.idx_ptr(),
-            int(flags), int(borderMode), _dptr(b), _stream_ptr(src))
-    _check(rc, name)
-    return dst
+    return _warp(src, "nv12", M, dsize, dst, "bgr", flags, borderMode, borderValue, mat_index, True)
 
 
 YUV_LAYOUTS = {"i420": 0, "nv12": 1}
@@ -410,42 +359,15 @@ def _yuv_layout(layout):
     return code
 
 
-def _yuv_dst(dst, n, h, w, batched, device):
-    """(frames view (N, H*3/2, W), pitch, frame stride) of a new or given YUV 4:2:0 dst of n frames of
-    h x w: (H*3/2, W) or (N, H*3/2, W) uint8.  Pitch and frame stride come from the tensor's strides,
-    so an encoder surface with padded rows is written as it is."""
-    import torch
-    if h % 2 or w % 2:
-        raise ValueError("YUV 4:2:0 frames need an even width and height, got %dx%d" % (w, h))
-    shape = (n, h * 3 // 2, w) if batched else (h * 3 // 2, w)
-    if dst is None:
-        dst = torch.empty(shape, dtype=torch.uint8, device=device)
-    _require_cuda(dst, "dst")
-    if tuple(dst.shape) != shape or dst.dtype != torch.uint8 or dst.device != device:
-        raise ValueError("dst must be a uint8 tensor of shape %s on %s, got %s %s on %s"
-                         % (shape, device, dst.dtype, tuple(dst.shape), dst.device))
-    d3 = dst if batched else dst[None]
-    if d3.stride(2) != 1 or d3.stride(1) < w:
-        raise ValueError("dst rows must be contiguous and at least %d bytes apart, got strides %s"
-                         % (w, tuple(d3.stride())))
-    pitch = d3.stride(1)
-    return dst, d3, pitch, d3.stride(0) if n > 1 else pitch * (h * 3 // 2)
-
-
 def bgr_to_yuv420(src, layout="i420", dst=None):
     """cv2.cvtColor(f, COLOR_BGR2YUV_I420) (layout "i420") or its NV12 relayout ("nv12") on CUDA
     uint8 BGR frames (H, W, 3) or (N, H, W, 3) -> (H*3/2, W) or (N, H*3/2, W)."""
     import torch
-    _require_cuda(src, "src")
-    if src.dtype != torch.uint8 or src.dim() not in (3, 4) or src.shape[-1] != 3:
-        raise ValueError("src must be uint8 (H, W, 3) or (N, H, W, 3), got %s %s" % (src.dtype, tuple(src.shape)))
+    s4, n, h, w, batched, _ = _warp_src(src, "bgr")
     code = _yuv_layout(layout)
-    s4 = (src[None] if src.dim() == 3 else src).contiguous()
-    n, h, w, _ = s4.shape
-    dst, d3, pitch, fstride = _yuv_dst(dst, n, h, w, src.dim() == 4, src.device)
+    dst, d3, dst_args = _warp_dst(dst, "yuv", src, s4, n, h, w, batched, code)
     with torch.cuda.device(src.device):
-        rc = lib().bevk_bgr_to_yuv420(_vp(s4.data_ptr()), _vp(d3.data_ptr()), n, h, w, code, pitch, fstride,
-                                      _stream_ptr(src))
+        rc = lib().bevk_bgr_to_yuv420(_vp(s4.data_ptr()), _vp(d3.data_ptr()), n, h, w, *dst_args, _stream_ptr(src))
     _check(rc, "bevk_bgr_to_yuv420")
     return dst
 
@@ -454,97 +376,147 @@ def warp_perspective_yuv420(src, M, dsize, layout="i420", dst=None, flags=1, bor
                             mat_index=None):
     """bgr_to_yuv420(warp_perspective(src, M, dsize, ...), layout) in one pass: CUDA uint8 BGR
     frames (H, W, 3) or (N, H, W, 3) -> (h*3/2, w) or (N, h*3/2, w)."""
-    return _warp_perspective_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index, False)
+    return _warp(src, "bgr", M, dsize, dst, "yuv", flags, borderMode, borderValue, mat_index, False, layout)
 
 
 def warp_perspective_yuv420_dmat(src, M, dsize, layout="i420", dst=None, flags=1, borderMode=0, borderValue=0,
                                  mat_index=None):
     """warp_perspective_yuv420 with M a CUDA float64 tensor, as for warp_perspective_dmat."""
-    return _warp_perspective_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index, True)
-
-
-def _warp_perspective_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index, dmat):
-    import torch
-    _require_cuda(src, "src")
-    if src.dtype != torch.uint8 or src.dim() not in (3, 4) or src.shape[-1] != 3:
-        raise ValueError("src must be uint8 (H, W, 3) or (N, H, W, 3), got %s %s" % (src.dtype, tuple(src.shape)))
-    code = _yuv_layout(layout)
-    s4 = (src[None] if src.dim() == 3 else src).contiguous()
-    n, h, w, _ = s4.shape
-    dw, dh = int(dsize[0]), int(dsize[1])
-    m = _Mats(M, n, mat_index, dmat, src.device)
-    dst, d3, pitch, fstride = _yuv_dst(dst, n, dh, dw, src.dim() == 4, src.device)
-    b = _border(borderValue)
-    name = "bevk_warp_perspective_yuv420_dmat" if dmat else "bevk_warp_perspective_yuv420"
-    with torch.cuda.device(src.device):
-        rc = getattr(lib(), name)(
-            _vp(s4.data_ptr()), _vp(d3.data_ptr()), n, h, w, dh, dw, code, pitch, fstride, m.ptr, m.n, m.idx_ptr(),
-            int(flags), int(borderMode), _dptr(b), _stream_ptr(src))
-    _check(rc, name)
-    return dst
+    return _warp(src, "bgr", M, dsize, dst, "yuv", flags, borderMode, borderValue, mat_index, True, layout)
 
 
 def warp_perspective_nv12_yuv420(src, M, dsize, layout="i420", dst=None, flags=1, borderMode=0, borderValue=0,
                                  mat_index=None):
     """bgr_to_yuv420(warp_perspective_nv12(src, M, dsize, ...), layout) in one pass: CUDA uint8 NV12
     frames (H*3/2, W) or (N, H*3/2, W), any pitch and frame stride -> (h*3/2, w) or (N, h*3/2, w)."""
-    return _warp_perspective_nv12_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index,
-                                         False)
+    return _warp(src, "nv12", M, dsize, dst, "yuv", flags, borderMode, borderValue, mat_index, False, layout)
 
 
 def warp_perspective_nv12_yuv420_dmat(src, M, dsize, layout="i420", dst=None, flags=1, borderMode=0,
                                       borderValue=0, mat_index=None):
     """warp_perspective_nv12_yuv420 with M a CUDA float64 tensor, as for warp_perspective_dmat."""
-    return _warp_perspective_nv12_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index,
-                                         True)
+    return _warp(src, "nv12", M, dsize, dst, "yuv", flags, borderMode, borderValue, mat_index, True, layout)
 
 
-def _warp_perspective_nv12_yuv420(src, M, dsize, layout, dst, flags, borderMode, borderValue, mat_index, dmat):
+def _warp_src(src, kind):
+    """(frames view, n, h, w, whether src has a frame axis, C arguments) of CUDA frames of a warp dtype
+    (H,W), (H,W,C) or (N,H,W,C) ("frames"), uint8 BGR (H, W, 3) or (N, H, W, 3) ("bgr") or NV12 ("nv12")."""
     import torch
-    s3, n, h, w, pitch, fstride = _nv12_frames(src)
-    code = _yuv_layout(layout)
+    if kind == "nv12":
+        s3, n, h, w, args = _nv12_frames(src)
+        return s3, n, h, w, src.dim() == 3, args
+    _require_cuda(src, "src")
+    if kind == "bgr" and (src.dtype != torch.uint8 or src.dim() not in (3, 4) or src.shape[-1] != 3):
+        raise ValueError("src must be uint8 (H, W, 3) or (N, H, W, 3), got %s %s" % (src.dtype, tuple(src.shape)))
+    _warp_dtype(src)
+    s4 = _frames_view(src)[0].contiguous()
+    return s4, s4.shape[0], s4.shape[1], s4.shape[2], src.dim() == 4, ()
+
+
+def _warp_dst(dst, kind, src, s, n, h, w, batched, layout):
+    """(what the call returns, frames view written, C arguments) of a new or given dst of n h x w frames,
+    batched as src: frames shaped as src ("frames"), uint8 BGR ("bgr") or YUV 4:2:0 of this layout code
+    ("yuv"; pitch and frame stride from the strides, so padded encoder surfaces are written in place)."""
+    import torch
+    if kind == "frames":  # a given dst may have any rank whose (N, H, W, C) view has the output's shape
+        if dst is not None:
+            _require_cuda(dst, "dst")
+        out4 = _out(None if dst is None else _frames_view(dst)[0], (n, h, w, s.shape[3]), src.dtype, src.device)
+        return dst if dst is not None else _frames_view(src)[1](out4), out4, (s.shape[3], _warp_dtype(src))
+    if kind == "bgr":
+        dst = _out(dst, (n, h, w, 3) if batched else (h, w, 3), torch.uint8, src.device)
+        return dst, dst, ()
+    if h % 2 or w % 2:
+        raise ValueError("YUV 4:2:0 frames need an even width and height, got %dx%d" % (w, h))
+    shape = (n, h * 3 // 2, w) if batched else (h * 3 // 2, w)
+    if dst is None:
+        dst = torch.empty(shape, dtype=torch.uint8, device=src.device)
+    _require_cuda(dst, "dst")
+    if tuple(dst.shape) != shape or dst.dtype != torch.uint8 or dst.device != src.device:
+        raise ValueError("dst must be a uint8 tensor of shape %s on %s, got %s %s on %s"
+                         % (shape, src.device, dst.dtype, tuple(dst.shape), dst.device))
+    d3 = dst if batched else dst[None]
+    if d3.stride(2) != 1 or d3.stride(1) < w:
+        raise ValueError("dst rows must be contiguous and at least %d bytes apart, got strides %s"
+                         % (w, tuple(d3.stride())))
+    pitch = d3.stride(1)
+    return dst, d3, (layout, pitch, d3.stride(0) if n > 1 else pitch * (h * 3 // 2))
+
+
+# (source kind, destination kind, device matrices) -> entry point
+_WARPS = {
+    ("frames", "frames", False): "bevk_warp_perspective",
+    ("frames", "frames", True): "bevk_warp_perspective_dmat",
+    ("nv12", "bgr", False): "bevk_warp_perspective_nv12",
+    ("nv12", "bgr", True): "bevk_warp_perspective_nv12_dmat",
+    ("bgr", "yuv", False): "bevk_warp_perspective_yuv420",
+    ("bgr", "yuv", True): "bevk_warp_perspective_yuv420_dmat",
+    ("nv12", "yuv", False): "bevk_warp_perspective_nv12_yuv420",
+    ("nv12", "yuv", True): "bevk_warp_perspective_nv12_yuv420_dmat",
+}
+
+
+def _warp(src, src_kind, M, dsize, dst, dst_kind, flags, borderMode, borderValue, mat_index, dmat, layout=None,
+          path=None):
+    """The device warps.  layout: a YUV destination's layout name; path: the BGR warp's kernel family
+    code, passed to the entry point's _path form.  The C arguments compose as (src, dst, n, h, w)
+    + the source's + (dh, dw) + the destination's + (M, n_mats, mat_index, flags, border) [+ path]."""
+    import torch
+    s, n, h, w, batched, src_args = _warp_src(src, src_kind)
+    code = _yuv_layout(layout) if dst_kind == "yuv" else None
     dw, dh = int(dsize[0]), int(dsize[1])
     m = _Mats(M, n, mat_index, dmat, src.device)
-    dst, d3, dpitch, dfstride = _yuv_dst(dst, n, dh, dw, src.dim() == 3, src.device)
+    out, d, dst_args = _warp_dst(dst, dst_kind, src, s, n, dh, dw, batched, code)
     b = _border(borderValue)
-    name = "bevk_warp_perspective_nv12_yuv420_dmat" if dmat else "bevk_warp_perspective_nv12_yuv420"
+    name = _WARPS[src_kind, dst_kind, dmat]
+    args = ((_vp(s.data_ptr()), _vp(d.data_ptr()), n, h, w) + src_args + (dh, dw) + dst_args
+            + (m.ptr, m.n, m.idx_ptr(), int(flags), int(borderMode), _dptr(b)) + (() if path is None else (path,)))
     with torch.cuda.device(src.device):
-        rc = getattr(lib(), name)(
-            _vp(s3.data_ptr()), _vp(d3.data_ptr()), n, h, w, pitch, fstride, dh, dw, code, dpitch, dfstride,
-            m.ptr, m.n, m.idx_ptr(), int(flags), int(borderMode), _dptr(b), _stream_ptr(src))
+        rc = getattr(lib(), name if path is None else name + "_path")(*args, _stream_ptr(src))
     _check(rc, name)
-    return dst
+    return out
 
 
 VIDEO_FORMATS = {"i420": 0, "nv12": 1, "bgr": 2}
 
 
-def _video_frames(a, fmt, what, caller="warp_perspective_video_host"):
-    """(frames view, n, h, w, batched) of a host BGR (H, W, 3) / (N, H, W, 3) or YUV 4:2:0
-    (H*3/2, W) / (N, H*3/2, W) uint8 buffer (numpy array or CPU tensor)."""
-    if hasattr(a, "detach"):
-        if a.is_cuda:
-            raise ValueError("%s is on %s: %s takes host buffers" % (what, a.device, caller))
-        a = a.detach().numpy()
-    a = np.asarray(a)
+def _video_call(src, src_format, dst_format, sizes, caller="warp_perspective_video_host"):
+    """The first checks of the host video calls, in order: format names, the host source frames (BGR or
+    YUV 4:2:0 uint8), the (width, height) sizes, dsize first and even for YUV BEVs.  Returns (frames
+    view, n, h, w, leading dims of the outputs, BEV frame shape, the sizes as ints)."""
+    for name, fmt in (("src_format", src_format), ("dst_format", dst_format)):
+        if fmt not in VIDEO_FORMATS:
+            raise ValueError("%s must be 'bgr', 'i420' or 'nv12', got %r" % (name, fmt))
+    if hasattr(src, "detach"):
+        if src.is_cuda:
+            raise ValueError("src is on %s: %s takes host buffers" % (src.device, caller))
+        src = src.detach().numpy()
+    a = np.asarray(src)
     if a.dtype != np.uint8:
-        raise ValueError("%s frames are uint8, got %s" % (what, a.dtype))
+        raise ValueError("src frames are uint8, got %s" % (a.dtype,))
     if not a.flags["C_CONTIGUOUS"]:
-        raise ValueError("%s must be C-contiguous" % what)
-    if fmt == "bgr":
+        raise ValueError("src must be C-contiguous")
+    batched = a.ndim == (4 if src_format == "bgr" else 3)
+    f = a if batched else a[None]
+    if src_format == "bgr":
         if a.ndim not in (3, 4) or a.shape[-1] != 3:
-            raise ValueError("%s BGR frames must be (H, W, 3) or (N, H, W, 3), got shape %s" % (what, a.shape))
-        f = a[None] if a.ndim == 3 else a
-        return f, f.shape[0], f.shape[1], f.shape[2], a.ndim == 4
-    if a.ndim not in (2, 3):
-        raise ValueError("%s %s frames must be (H*3/2, W) or (N, H*3/2, W), got shape %s"
-                         % (what, fmt.upper(), a.shape))
-    f = a[None] if a.ndim == 2 else a
-    rows, w = f.shape[1], f.shape[2]
-    if rows == 0 or rows % 3 or w % 2 or w == 0:
-        raise ValueError("%s %s frames need H*3/2 rows for an even H and an even width W, got %d rows x %d"
-                         % (what, fmt.upper(), rows, w))
-    return f, f.shape[0], rows // 3 * 2, w, a.ndim == 3
+            raise ValueError("src BGR frames must be (H, W, 3) or (N, H, W, 3), got shape %s" % (a.shape,))
+        h, w = f.shape[1], f.shape[2]
+    else:
+        if a.ndim not in (2, 3):
+            raise ValueError("src %s frames must be (H*3/2, W) or (N, H*3/2, W), got shape %s"
+                             % (src_format.upper(), a.shape))
+        rows, w = f.shape[1], f.shape[2]
+        if rows == 0 or rows % 3 or w % 2 or w == 0:
+            raise ValueError("src %s frames need H*3/2 rows for an even H and an even width W, got %d rows x %d"
+                             % (src_format.upper(), rows, w))
+        h = rows // 3 * 2
+    sizes = [(int(z[0]), int(z[1])) for z in sizes]
+    dw, dh = sizes[0]
+    if dst_format != "bgr" and (dw % 2 or dh % 2):
+        raise ValueError("YUV 4:2:0 frames need an even width and height, got dsize %dx%d" % (dw, dh))
+    frame = (dh, dw, 3) if dst_format == "bgr" else (dh * 3 // 2, dw)
+    return f, f.shape[0], h, w, f.shape[:1] if batched else (), frame, sizes
 
 
 def _host_out(dst, shape, what, caller="warp_perspective_video_host"):
@@ -565,21 +537,13 @@ def warp_perspective_video_host(src, M, dsize, src_format="bgr", dst_format="i42
     """Host-buffer warp between video frame formats ("bgr", "i420", "nv12"): src / dst are numpy
     arrays or CPU tensors (pinned for full speed), BGR (H, W, 3) / (N, H, W, 3) or YUV 4:2:0
     (H*3/2, W) / (N, H*3/2, W) uint8."""
-    for name, fmt in (("src_format", src_format), ("dst_format", dst_format)):
-        if fmt not in VIDEO_FORMATS:
-            raise ValueError("%s must be 'bgr', 'i420' or 'nv12', got %r" % (name, fmt))
-    s, n, h, w, batched = _video_frames(src, src_format, "src")
-    dw, dh = int(dsize[0]), int(dsize[1])
-    if dst_format != "bgr" and (dw % 2 or dh % 2):
-        raise ValueError("YUV 4:2:0 frames need an even width and height, got dsize %dx%d" % (dw, dh))
-    Ms, idx = _prep_mats(M, n, mat_index)
-    frame = (dh, dw, 3) if dst_format == "bgr" else (dh * 3 // 2, dw)
-    out = _host_out(dst, (n,) + frame if batched else frame, "dst")
+    s, n, h, w, lead, frame, [(dw, dh)] = _video_call(src, src_format, dst_format, [dsize])
+    m = _Mats(M, n, mat_index, False, None)
+    out = _host_out(dst, lead + frame, "dst")
     b = _border(borderValue)
     rc = lib().bevk_warp_perspective_video_host(
         _vp(s.ctypes.data), VIDEO_FORMATS[src_format], _vp(out.ctypes.data), VIDEO_FORMATS[dst_format], n, h, w,
-        dh, dw, _dptr(Ms), Ms.shape[0], idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags),
-        int(borderMode), _dptr(b))
+        dh, dw, m.ptr, m.n, m.idx_ptr(), int(flags), int(borderMode), _dptr(b))
     _check(rc, "bevk_warp_perspective_video_host")
     return dst if dst is not None else out
 
@@ -589,35 +553,25 @@ def warp_perspective_video_host_small(src, M, M_small, dsize, small_size, src_fo
                                       dst=None, small=None, dst_small=None):
     """warp_perspective_video_host plus the small frames (BGR, small_size = (w, h)) and their BEVs
     through M_small, from one upload of each frame.  Returns (dst, small, dst_small)."""
-    for name, fmt in (("src_format", src_format), ("dst_format", dst_format)):
-        if fmt not in VIDEO_FORMATS:
-            raise ValueError("%s must be 'bgr', 'i420' or 'nv12', got %r" % (name, fmt))
     caller = "warp_perspective_video_host_small"
-    s, n, h, w, batched = _video_frames(src, src_format, "src", caller)
-    dw, dh = int(dsize[0]), int(dsize[1])
-    sw, sh = int(small_size[0]), int(small_size[1])
-    if dst_format != "bgr" and (dw % 2 or dh % 2):
-        raise ValueError("YUV 4:2:0 frames need an even width and height, got dsize %dx%d" % (dw, dh))
+    s, n, h, w, lead, frame, [(dw, dh), (sw, sh)] = _video_call(src, src_format, dst_format, [dsize, small_size],
+                                                                 caller)
     if interpolation not in (1, 3):
         raise ValueError("interpolation must be INTER_LINEAR (1) or INTER_AREA (3), got %r" % (interpolation,))
-    Ms, idx = _prep_mats(M, n, mat_index)
+    m = _Mats(M, n, mat_index, False, None)
     Mss = np.ascontiguousarray(_to_numpy(M_small), dtype=np.float64)
-    if Mss.ndim == 2:
-        Mss = Mss[None]
-    if Mss.shape != Ms.shape:
+    Mss = Mss[None] if Mss.ndim == 2 else Mss
+    if Mss.shape != m.keep.shape:
         raise ValueError("M_small must hold one 3x3 matrix per matrix of M, shape %s, got %s"
-                         % (Ms.shape, Mss.shape))
-    lead = (n,) if batched else ()
-    frame = (dh, dw, 3) if dst_format == "bgr" else (dh * 3 // 2, dw)
+                         % (m.keep.shape, Mss.shape))
     out = _host_out(dst, lead + frame, "dst", caller)
     out_small = _host_out(small, lead + (sh, sw, 3), "small", caller)
     out_bev_small = _host_out(dst_small, lead + frame, "dst_small", caller)
     b = _border(borderValue)
     rc = lib().bevk_warp_perspective_video_host_small(
         _vp(s.ctypes.data), VIDEO_FORMATS[src_format], _vp(out.ctypes.data), VIDEO_FORMATS[dst_format],
-        _vp(out_small.ctypes.data), _vp(out_bev_small.ctypes.data), n, h, w, dh, dw, sh, sw, _dptr(Ms), _dptr(Mss),
-        Ms.shape[0], idx.ctypes.data_as(_i32p) if idx is not None else None, int(flags), int(interpolation),
-        int(borderMode), _dptr(b))
+        _vp(out_small.ctypes.data), _vp(out_bev_small.ctypes.data), n, h, w, dh, dw, sh, sw, m.ptr, _dptr(Mss),
+        m.n, m.idx_ptr(), int(flags), int(interpolation), int(borderMode), _dptr(b))
     _check(rc, "bevk_warp_perspective_video_host_small")
     return (dst if dst is not None else out, small if small is not None else out_small,
             dst_small if dst_small is not None else out_bev_small)
@@ -707,7 +661,7 @@ def resize_nv12(src, dsize, dst=None, interpolation=1):
     (H*3/2, W) or (N, H*3/2, W) -> (h, w, 3) or (N, h, w, 3) BGR; dsize = (width, height);
     interpolation INTER_LINEAR = 1 or INTER_AREA = 3."""
     import torch
-    s3, n, h, w, pitch, fstride = _nv12_frames(src)
+    s3, n, h, w, (pitch, fstride) = _nv12_frames(src)
     dw, dh = int(dsize[0]), int(dsize[1])
     dst = _out(dst, (n, dh, dw, 3) if src.dim() == 3 else (dh, dw, 3), torch.uint8, src.device)
     with torch.cuda.device(src.device):

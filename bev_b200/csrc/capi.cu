@@ -228,12 +228,16 @@ void build_groups(int n_frames, int n_mats, const int32_t *mat_index, std::vecto
     }
 }
 
-// The groups of host dst->src maps.
-void build_groups(int n_frames, int n_mats, const int32_t *mat_index, const std::vector<double> &maps,
+// The groups of frames [f0, f0 + nf) of a call on maps, the dst->src maps of all n_mats matrices:
+// the frames' slice of mat_index, or of the per-frame matrices.
+void chunk_groups(const std::vector<double> &maps, int n_mats, const int32_t *mat_index, int f0, int nf,
                   std::vector<BevkWarpGroup> &groups)
 {
-    build_groups(n_frames, n_mats, mat_index, groups,
-                 [&](BevkWarpGroup &g, int k) { memcpy(g.M, &maps[(size_t)k * 9], 9 * sizeof(double)); });
+    groups.clear();
+    const int k0 = (!mat_index && n_mats != 1) ? f0 : 0;  // one matrix per frame: frame f0 has matrix f0
+    build_groups(nf, n_mats, mat_index ? mat_index + f0 : nullptr, groups, [&](BevkWarpGroup &g, int k) {
+        memcpy(g.M, &maps[(size_t)(k0 + k) * 9], 9 * sizeof(double));
+    });
 }
 
 // The groups of a device call on the n_mats matrices M: maps inverted here from host matrices, or
@@ -241,18 +245,17 @@ void build_groups(int n_frames, int n_mats, const int32_t *mat_index, const std:
 void device_groups(const WarpArgs &a, const double *M, int n_mats, const int32_t *mat_index, int flags,
                    std::vector<BevkWarpGroup> &groups)
 {
-    if (a.dmat) {
-        const int invert = (flags & BEVK_WARP_INVERSE_MAP) ? 0 : 1;
-        build_groups(a.n_frames, n_mats, mat_index, groups, [&](BevkWarpGroup &g, int k) {
-            memset(g.M, 0, sizeof(g.M));
-            g.d.mat = M + (size_t)k * 9;
-            g.d.invert = invert;
-        });
-        return;
+    if (!a.dmat) {
+        std::vector<double> maps;
+        effective_maps(M, n_mats, flags, maps);
+        return chunk_groups(maps, n_mats, mat_index, 0, a.n_frames, groups);
     }
-    std::vector<double> maps;
-    effective_maps(M, n_mats, flags, maps);
-    build_groups(a.n_frames, n_mats, mat_index, maps, groups);
+    const int invert = (flags & BEVK_WARP_INVERSE_MAP) ? 0 : 1;
+    build_groups(a.n_frames, n_mats, mat_index, groups, [&](BevkWarpGroup &g, int k) {
+        memset(g.M, 0, sizeof(g.M));
+        g.d.mat = M + (size_t)k * 9;
+        g.d.invert = invert;
+    });
 }
 
 // Fill p from a and walk the groups in launches of up to BEVK_MAX_GROUPS: launch() plans and
@@ -387,23 +390,6 @@ struct HostOut {
     size_t frame_bytes;
 };
 
-// The (matrix, frame-run) groups of frames [f0, f0 + nf) of a host call: the chunk's slice of
-// mat_index, or of the per-frame matrices.
-void chunk_groups(const std::vector<double> &maps, int n_mats, const int32_t *mat_index, int f0, int nf,
-                  std::vector<BevkWarpGroup> &groups)
-{
-    groups.clear();
-    if (mat_index) {
-        const std::vector<int32_t> idx(mat_index + f0, mat_index + f0 + nf);
-        build_groups(nf, n_mats, idx.data(), maps, groups);
-    } else if (n_mats != 1) {  // one matrix per frame: this chunk's slice
-        const std::vector<double> chunk_maps(maps.begin() + (size_t)f0 * 9, maps.begin() + (size_t)(f0 + nf) * 9);
-        build_groups(nf, nf, nullptr, chunk_maps, groups);
-    } else {
-        build_groups(nf, 1, nullptr, maps, groups);
-    }
-}
-
 // The pipelined host-buffer warp of the n_frames > 0 frames of a: frames of src_frame_bytes, of which
 // only `bands` are uploaded, to one or more outputs.  Chunks of frames go through the device
 // workspace, kHostSlots at a time, so that the copies and kernels of neighbouring chunks overlap.
@@ -504,59 +490,6 @@ int host_pipeline(const void *src, const WarpArgs &a, const std::vector<double> 
 #undef BEVK_CUDA_DRAIN
 }
 
-}  // namespace
-
-extern "C" {
-
-int bevk_warp_perspective(const void *src, void *dst, int n_frames, int src_h, int src_w,
-                          int dst_h, int dst_w, int channels, int dtype, const double *M,
-                          int n_mats, const int32_t *mat_index, int flags, int border_mode,
-                          const double *border_value, void *stream)
-{
-    return bevk_warp_perspective_path(src, dst, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
-                                      n_mats, mat_index, flags, border_mode, border_value, -1, stream);
-}
-
-int bevk_warp_perspective_path(const void *src, void *dst, int n_frames, int src_h, int src_w,
-                               int dst_h, int dst_w, int channels, int dtype, const double *M,
-                               int n_mats, const int32_t *mat_index, int flags, int border_mode,
-                               const double *border_value, int path, void *stream)
-{
-    if (path < -1 || path > 2) BEVK_FAIL(BEVK_E_ARG, "warp: path must be -1 (thread default), 0, 1 or 2");
-    if (path < 0) path = g_warp_path;
-    WarpArgs a;
-    int rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
-                             n_mats, mat_index, flags, border_mode, border_value, a);
-    if (rc) return rc;
-    rc = bevk_require_device();
-    if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
-    std::vector<BevkWarpGroup> groups;
-    device_groups(a, M, n_mats, mat_index, flags, groups);
-    return run_warp_device(src, dst, a, groups, path, (cudaStream_t)stream);
-}
-
-int bevk_warp_perspective_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
-                               int dst_w, int channels, int dtype, const double *M, int n_mats,
-                               const int32_t *mat_index, int flags, int border_mode, const double *border_value,
-                               void *stream)
-{
-    WarpArgs a;
-    int rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
-                             n_mats, mat_index, flags, border_mode, border_value, a);
-    if (rc) return rc;
-    rc = bevk_require_device();
-    if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
-    a.dmat = true;
-    std::vector<BevkWarpGroup> groups;
-    device_groups(a, M, n_mats, mat_index, flags, groups);
-    return run_warp_device(src, dst, a, groups, 1, (cudaStream_t)stream);
-}
-
-}  // extern "C"
-
-namespace {
 // The NV12 frame rules of the NV12 entry points: even sizes, rows at least a luma row apart.
 int check_nv12_layout(const char *what, int n_frames, int h, int w, int pitch, int64_t frame_stride)
 {
@@ -614,18 +547,38 @@ int check_yuv420_dst(const char *what, int n_frames, int h, int w, int layout, i
     return check_nv12_layout32(what, n_frames, h, w, pitch, frame_stride);
 }
 
-// The fused warps to YUV 4:2:0 of these groups on device buffers: BGR (src_format BEVK_BGR,
-// contiguous frames), NV12 or I420 frames, rows `pitch` and frames `frame_stride` bytes apart.
-int run_warp_yuv420(const void *src, void *dst, const WarpArgs &a, const std::vector<BevkWarpGroup> &groups,
-                    int src_format, long long pitch, long long frame_stride, int layout, int dst_pitch,
-                    int64_t dst_frame_stride, cudaStream_t stream)
+// The layout of the YUV 4:2:0 frames on one side of a warp: format BEVK_YUV_NV12 or BEVK_YUV_I420
+// (a destination's layout code, checked with it), rows `pitch` and frames `frame_stride` bytes
+// apart.  A BGR side has no layout (nullptr): its frames are contiguous, of the WarpArgs' channels
+// and dtype.
+struct FrameLayout {
+    int format;
+    long long pitch, frame_stride;
+};
+
+// Bytes of one contiguous frame of h x w pixels in a video frame format.
+size_t video_frame_bytes(int format, int h, int w)
 {
-    BevkYuvParams P;
-    memset(&P, 0, sizeof(P));
-    P.pitch = (int)pitch;
-    P.frame_stride = frame_stride;
-    P.dst_pitch = dst_pitch;
-    P.dst_frame_stride = dst_frame_stride;
+    return (size_t)w * h * (format == BEVK_BGR ? 2 : 1) * 3 / 2;
+}
+
+// The layout L of contiguous video frames of a format; nullptr for BGR frames, which run_warp lays out.
+const FrameLayout *video_layout(int format, int h, int w, FrameLayout &L)
+{
+    L = {format, format == BEVK_BGR ? 3LL * w : w, (long long)video_frame_bytes(format, h, w)};
+    return format == BEVK_BGR ? nullptr : &L;
+}
+
+// The fused warps to YUV 4:2:0 frames (dstL) of these groups on device buffers, from BGR, NV12 or
+// I420 frames (srcL).
+int run_warp_yuv420(const void *src, const FrameLayout &srcL, void *dst, const FrameLayout &dstL, const WarpArgs &a,
+                    const std::vector<BevkWarpGroup> &groups, cudaStream_t stream)
+{
+    BevkYuvParams P = {};  // launch_warp_groups fills P.w
+    P.pitch = (int)srcL.pitch;
+    P.frame_stride = srcL.frame_stride;
+    P.dst_pitch = (int)dstL.pitch;
+    P.dst_frame_stride = dstL.frame_stride;
     return launch_warp_groups(P.w, src, dst, a, groups, [&]() {
         // a thread owns a 2x2 dst block: plan the frame chunks over the grid of blocks
         P.w.dst_w /= 2;
@@ -634,57 +587,73 @@ int run_warp_yuv420(const void *src, void *dst, const WarpArgs &a, const std::ve
         P.w.dst_w *= 2;
         P.w.dst_h *= 2;
         if (rc) return rc;
-        return bevk_launch_warp_yuv420(P, src_format, layout == BEVK_YUV_NV12, a.linear, a.dmat, stream);
+        return bevk_launch_warp_yuv420(P, srcL.format, dstL.format == BEVK_YUV_NV12, a.linear, a.dmat, stream);
     });
 }
 
-// The NV12 or I420 (src_format) to BGR warp of these groups on device buffers.
-int run_warp_yuv_bgr(const void *src, void *dst, const WarpArgs &a, const std::vector<BevkWarpGroup> &groups,
-                     int src_format, int pitch, int64_t frame_stride, cudaStream_t stream)
+// The NV12 or I420 (srcL) to BGR warp of these groups on device buffers.
+int run_warp_yuv_bgr(const void *src, const FrameLayout &srcL, void *dst, const WarpArgs &a,
+                     const std::vector<BevkWarpGroup> &groups, cudaStream_t stream)
 {
-    BevkNv12Params P;
-    memset(&P, 0, sizeof(P));
-    P.pitch = pitch;
-    P.frame_stride = frame_stride;
+    BevkNv12Params P = {};  // launch_warp_groups fills P.w
+    P.pitch = (int)srcL.pitch;
+    P.frame_stride = srcL.frame_stride;
     return launch_warp_groups(P.w, src, dst, a, groups, [&]() {
         const int rc = bevk_plan_generic_chunks(P.w, 3);
         if (rc) return rc;
-        return bevk_launch_warp_nv12(P, src_format, a.linear, a.dmat, stream);
+        return bevk_launch_warp_nv12(P, srcL.format, a.linear, a.dmat, stream);
     });
 }
 
-// The fused warps to YUV 4:2:0 after their source-layout checks: BGR (src_format BEVK_BGR,
-// contiguous frames) or NV12 frames, rows `pitch` and frames `frame_stride` bytes apart.
-// dmat: M is a device matrix table.
-int warp_yuv420(const char *what, const void *src, void *dst, int n_frames, int src_h, int src_w, int src_format,
-                long long pitch, long long frame_stride, int dst_h, int dst_w, int layout, int dst_pitch,
-                int64_t dst_frame_stride, const double *M, int n_mats, const int32_t *mat_index, int flags,
-                int border_mode, const double *border_value, bool dmat, void *stream)
+// The kernel family of a warp between two sides (nullptr: BGR frames): the warps to YUV 4:2:0, else
+// the YUV to BGR warp, else the BGR warp on `path`.
+int run_warp(const void *src, const FrameLayout *yuv_src, void *dst, const FrameLayout *yuv_dst, const WarpArgs &a,
+             const std::vector<BevkWarpGroup> &groups, int path, cudaStream_t stream)
 {
-    int rc = check_yuv420_dst(what, n_frames, dst_h, dst_w, layout, dst_pitch, dst_frame_stride);
+    const FrameLayout bgr = {BEVK_BGR, 3LL * a.src_w, 3LL * a.src_w * a.src_h};  // the YUV warps' BGR source
+    if (yuv_dst) return run_warp_yuv420(src, yuv_src ? *yuv_src : bgr, dst, *yuv_dst, a, groups, stream);
+    if (yuv_src) return run_warp_yuv_bgr(src, *yuv_src, dst, a, groups, stream);
+    return run_warp_device(src, dst, a, groups, path, stream);
+}
+
+// The argument checks of a warp between two sides (nullptr: BGR frames), in this order: the NV12 /
+// I420 source's, the YUV 4:2:0 destination's, then the warp's own.
+int check_frames(const char *what, const void *src, const FrameLayout *yuv_src, void *dst, const FrameLayout *yuv_dst,
+                 int n_frames, int src_h, int src_w, int dst_h, int dst_w, int channels, int dtype, const double *M,
+                 int n_mats, const int32_t *mat_index, int flags, int border_mode, const double *border_value,
+                 WarpArgs &a)
+{
+    int rc = BEVK_OK;
+    if (yuv_src) rc = check_nv12_layout32(what, n_frames, src_h, src_w, (int)yuv_src->pitch, yuv_src->frame_stride);
+    if (!rc && yuv_dst)
+        rc = check_yuv420_dst(what, n_frames, dst_h, dst_w, yuv_dst->format, (int)yuv_dst->pitch,
+                              yuv_dst->frame_stride);
     if (rc) return rc;
+    return check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M, n_mats, mat_index,
+                           flags, border_mode, border_value, a);
+}
+
+// The device warp entry points: every argument check before the device probe, then the launches.
+// dmat: M is a device matrix table.  path: the BGR warp's kernel family, -1 the calling thread's.
+int warp_frames(const char *what, const void *src, const FrameLayout *yuv_src, void *dst, const FrameLayout *yuv_dst,
+                int n_frames, int src_h, int src_w, int dst_h, int dst_w, int channels, int dtype, const double *M,
+                int n_mats, const int32_t *mat_index, int flags, int border_mode, const double *border_value,
+                bool dmat, int path, void *stream)
+{
     WarpArgs a;
-    rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index, flags,
-                         border_mode, border_value, a);
+    int rc = check_frames(what, src, yuv_src, dst, yuv_dst, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
+                          n_mats, mat_index, flags, border_mode, border_value, a);
     if (rc) return rc;
     rc = bevk_require_device();
-    if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
+    if (rc || n_frames == 0) return rc;
     a.dmat = dmat;
     std::vector<BevkWarpGroup> groups;
     device_groups(a, M, n_mats, mat_index, flags, groups);
-    return run_warp_yuv420(src, dst, a, groups, src_format, pitch, frame_stride, layout, dst_pitch, dst_frame_stride,
-                           (cudaStream_t)stream);
+    return run_warp(src, yuv_src, dst, yuv_dst, a, groups, path < 0 ? g_warp_path : path, (cudaStream_t)stream);
 }
 
-// Bytes of one contiguous frame of h x w pixels in a video frame format.
-size_t video_frame_bytes(int format, int h, int w)
-{
-    return (size_t)w * h * (format == BEVK_BGR ? 2 : 1) * 3 / 2;
-}
-
-// The argument checks of the host video entry points: formats, even YUV sizes, frames below 4 GB
-// and the warp's own, before any device is looked for.
+// The argument checks of the host video entry points on contiguous frames: formats, then those of
+// the warp, before any device is looked for.
 int check_video_host(const char *what, const void *src, int src_format, void *dst, int dst_format, int n_frames,
                      int src_h, int src_w, int dst_h, int dst_w, const double *M, int n_mats,
                      const int32_t *mat_index, int flags, int border_mode, const double *border_value, WarpArgs &a)
@@ -693,55 +662,79 @@ int check_video_host(const char *what, const void *src, int src_format, void *ds
     if (!known(src_format) || !known(dst_format))
         BEVK_FAIL(BEVK_E_ARG, "%s: formats must be BEVK_YUV_I420 (0), BEVK_YUV_NV12 (1) or BEVK_BGR (2), got src %d, "
                   "dst %d", what, src_format, dst_format);
-    int rc;
-    if (src_format != BEVK_BGR) {
-        rc = check_nv12_layout32(what, n_frames, src_h, src_w, src_w, (int64_t)src_w * src_h / 2 * 3);
-        if (rc) return rc;
-    }
-    if (dst_format != BEVK_BGR) {
-        rc = check_yuv420_dst(what, n_frames, dst_h, dst_w, dst_format, dst_w, (int64_t)dst_w * dst_h / 2 * 3);
-        if (rc) return rc;
-    }
-    return check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index, flags,
-                           border_mode, border_value, a);
+    FrameLayout sL, dL;
+    return check_frames(what, src, video_layout(src_format, src_h, src_w, sL), dst,
+                        video_layout(dst_format, dst_h, dst_w, dL), n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8,
+                        M, n_mats, mat_index, flags, border_mode, border_value, a);
 }
 
-// The warp of one chunk of contiguous video frames on the device, for a format pair.
-int run_video_warp(const void *src, void *dst, const WarpArgs &a, const std::vector<BevkWarpGroup> &groups,
-                   int src_format, int dst_format, cudaStream_t stream)
+// The host-buffer warps of checked, contiguous frames (nullptr: BGR frames of a.channels x a.dtype)
+// through the host pipeline: only the source rows the maps reference go up, and for YUV sources the
+// chroma rows under them.
+int warp_host_frames(const void *src, const FrameLayout *yuv_src, void *dst, const FrameLayout *yuv_dst,
+                     const WarpArgs &a, const double *M, int n_mats, const int32_t *mat_index, int flags)
 {
-    const long long src_frame_bytes = (long long)video_frame_bytes(src_format, a.src_h, a.src_w);
-    if (dst_format != BEVK_BGR)
-        return run_warp_yuv420(src, dst, a, groups, src_format, src_format == BEVK_BGR ? 3LL * a.src_w : a.src_w,
-                               src_frame_bytes, dst_format, a.dst_w,
-                               (int64_t)video_frame_bytes(dst_format, a.dst_h, a.dst_w), stream);
-    if (src_format != BEVK_BGR)
-        return run_warp_yuv_bgr(src, dst, a, groups, src_format, a.src_w, src_frame_bytes, stream);
-    return run_warp_device(src, dst, a, groups, g_warp_path, stream);
-}
+    const int rc = bevk_require_device();
+    if (rc || a.n_frames == 0) return rc;
+    std::vector<double> maps;
+    effective_maps(M, n_mats, flags, maps);
 
-// dmat: M is a device matrix table.
-int warp_nv12(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch, int64_t frame_stride,
-              int dst_h, int dst_w, const double *M, int n_mats, const int32_t *mat_index, int flags, int border_mode,
-              const double *border_value, bool dmat, void *stream)
-{
-    int rc = check_nv12_layout32("warp_nv12", n_frames, src_h, src_w, pitch, frame_stride);
-    if (rc) return rc;
-    WarpArgs a;
-    rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M, n_mats, mat_index,
-                         flags, border_mode, border_value, a);
-    if (rc) return rc;
-    rc = bevk_require_device();
-    if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
-    a.dmat = dmat;
-    std::vector<BevkWarpGroup> groups;
-    device_groups(a, M, n_mats, mat_index, flags, groups);
-    return run_warp_yuv_bgr(src, dst, a, groups, BEVK_YUV_NV12, pitch, frame_stride, (cudaStream_t)stream);
+    // the referenced luma (BGR) row band [r0, r1] and, for YUV, the chroma rows under it
+    int r0, r1;
+    referenced_rows_union(maps, n_mats, a, r0, r1);
+    const size_t h = (size_t)a.src_h, w = (size_t)a.src_w, rows = (size_t)(r1 - r0 + 1);
+    const size_t row_bytes = yuv_src ? w : w * a.channels * a.elem_size;
+    std::vector<HostBand> bands = {{row_bytes * r0, row_bytes * rows}};
+    if (yuv_src) {
+        const size_t c0 = (size_t)(r0 / 2), nc = (size_t)(r1 / 2) - c0 + 1;
+        if (yuv_src->format == BEVK_YUV_NV12) {
+            bands.push_back({w * (h + c0), w * nc});
+        } else {  // the U plane, then the V plane: (h / 2) x (w / 2) each, contiguous
+            const size_t cw = w / 2;
+            bands.push_back({w * h + cw * c0, cw * nc});
+            bands.push_back({w * h + cw * (h / 2 + c0), cw * nc});
+        }
+    }
+    const size_t src_frame_bytes = yuv_src ? (size_t)yuv_src->frame_stride : row_bytes * h;
+    const size_t dst_frame_bytes =
+        yuv_dst ? (size_t)yuv_dst->frame_stride : (size_t)a.dst_w * a.dst_h * a.channels * a.elem_size;
+    return host_pipeline(src, a, maps, n_mats, mat_index, src_frame_bytes, bands, {{dst, dst_frame_bytes}},
+                         [&](const void *s, void *const *d, const WarpArgs &ac, int,
+                             const std::vector<BevkWarpGroup> &groups, cudaStream_t st) {
+                             return run_warp(s, yuv_src, d[0], yuv_dst, ac, groups, g_warp_path, st);
+                         });
 }
 }  // namespace
 
 extern "C" {
+
+int bevk_warp_perspective(const void *src, void *dst, int n_frames, int src_h, int src_w,
+                          int dst_h, int dst_w, int channels, int dtype, const double *M,
+                          int n_mats, const int32_t *mat_index, int flags, int border_mode,
+                          const double *border_value, void *stream)
+{
+    return warp_frames("warp", src, nullptr, dst, nullptr, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
+                       n_mats, mat_index, flags, border_mode, border_value, false, -1, stream);
+}
+
+int bevk_warp_perspective_path(const void *src, void *dst, int n_frames, int src_h, int src_w,
+                               int dst_h, int dst_w, int channels, int dtype, const double *M,
+                               int n_mats, const int32_t *mat_index, int flags, int border_mode,
+                               const double *border_value, int path, void *stream)
+{
+    if (path < -1 || path > 2) BEVK_FAIL(BEVK_E_ARG, "warp: path must be -1 (thread default), 0, 1 or 2");
+    return warp_frames("warp", src, nullptr, dst, nullptr, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
+                       n_mats, mat_index, flags, border_mode, border_value, false, path, stream);
+}
+
+int bevk_warp_perspective_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
+                               int dst_w, int channels, int dtype, const double *M, int n_mats,
+                               const int32_t *mat_index, int flags, int border_mode, const double *border_value,
+                               void *stream)
+{
+    return warp_frames("warp", src, nullptr, dst, nullptr, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
+                       n_mats, mat_index, flags, border_mode, border_value, true, -1, stream);
+}
 
 int bevk_nv12_to_bgr(const void *src, void *dst, int n_frames, int h, int w, int pitch,
                      int64_t frame_stride, void *stream)
@@ -760,8 +753,9 @@ int bevk_warp_perspective_nv12(const void *src, void *dst, int n_frames, int src
                                const double *M, int n_mats, const int32_t *mat_index, int flags,
                                int border_mode, const double *border_value, void *stream)
 {
-    return warp_nv12(src, dst, n_frames, src_h, src_w, pitch, frame_stride, dst_h, dst_w, M, n_mats, mat_index,
-                     flags, border_mode, border_value, false, stream);
+    const FrameLayout srcL = {BEVK_YUV_NV12, pitch, frame_stride};
+    return warp_frames("warp_nv12", src, &srcL, dst, nullptr, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M,
+                       n_mats, mat_index, flags, border_mode, border_value, false, -1, stream);
 }
 
 int bevk_warp_perspective_nv12_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
@@ -769,8 +763,9 @@ int bevk_warp_perspective_nv12_dmat(const void *src, void *dst, int n_frames, in
                                     const int32_t *mat_index, int flags, int border_mode,
                                     const double *border_value, void *stream)
 {
-    return warp_nv12(src, dst, n_frames, src_h, src_w, pitch, frame_stride, dst_h, dst_w, M, n_mats, mat_index,
-                     flags, border_mode, border_value, true, stream);
+    const FrameLayout srcL = {BEVK_YUV_NV12, pitch, frame_stride};
+    return warp_frames("warp_nv12", src, &srcL, dst, nullptr, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M,
+                       n_mats, mat_index, flags, border_mode, border_value, true, -1, stream);
 }
 
 int bevk_bgr_to_yuv420(const void *src, void *dst, int n_frames, int h, int w, int layout, int dst_pitch,
@@ -792,9 +787,9 @@ int bevk_warp_perspective_yuv420(const void *src, void *dst, int n_frames, int s
                                  int n_mats, const int32_t *mat_index, int flags, int border_mode,
                                  const double *border_value, void *stream)
 {
-    return warp_yuv420("warp_yuv420", src, dst, n_frames, src_h, src_w, BEVK_BGR, 3LL * src_w,
-                       3LL * src_w * src_h, dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index,
-                       flags, border_mode, border_value, false, stream);
+    const FrameLayout dstL = {layout, dst_pitch, dst_frame_stride};
+    return warp_frames("warp_yuv420", src, nullptr, dst, &dstL, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M,
+                       n_mats, mat_index, flags, border_mode, border_value, false, -1, stream);
 }
 
 int bevk_warp_perspective_yuv420_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h,
@@ -802,9 +797,9 @@ int bevk_warp_perspective_yuv420_dmat(const void *src, void *dst, int n_frames, 
                                       const double *M, int n_mats, const int32_t *mat_index, int flags,
                                       int border_mode, const double *border_value, void *stream)
 {
-    return warp_yuv420("warp_yuv420", src, dst, n_frames, src_h, src_w, BEVK_BGR, 3LL * src_w,
-                       3LL * src_w * src_h, dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index,
-                       flags, border_mode, border_value, true, stream);
+    const FrameLayout dstL = {layout, dst_pitch, dst_frame_stride};
+    return warp_frames("warp_yuv420", src, nullptr, dst, &dstL, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8, M,
+                       n_mats, mat_index, flags, border_mode, border_value, true, -1, stream);
 }
 
 int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
@@ -813,11 +808,9 @@ int bevk_warp_perspective_nv12_yuv420(const void *src, void *dst, int n_frames, 
                                       const int32_t *mat_index, int flags, int border_mode,
                                       const double *border_value, void *stream)
 {
-    const int rc = check_nv12_layout32("warp_nv12_yuv420", n_frames, src_h, src_w, pitch, frame_stride);
-    if (rc) return rc;
-    return warp_yuv420("warp_nv12_yuv420", src, dst, n_frames, src_h, src_w, BEVK_YUV_NV12, pitch, frame_stride,
-                       dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index, flags, border_mode,
-                       border_value, false, stream);
+    const FrameLayout srcL = {BEVK_YUV_NV12, pitch, frame_stride}, dstL = {layout, dst_pitch, dst_frame_stride};
+    return warp_frames("warp_nv12_yuv420", src, &srcL, dst, &dstL, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8,
+                       M, n_mats, mat_index, flags, border_mode, border_value, false, -1, stream);
 }
 
 int bevk_warp_perspective_nv12_yuv420_dmat(const void *src, void *dst, int n_frames, int src_h, int src_w, int pitch,
@@ -826,11 +819,9 @@ int bevk_warp_perspective_nv12_yuv420_dmat(const void *src, void *dst, int n_fra
                                            const int32_t *mat_index, int flags, int border_mode,
                                            const double *border_value, void *stream)
 {
-    const int rc = check_nv12_layout32("warp_nv12_yuv420", n_frames, src_h, src_w, pitch, frame_stride);
-    if (rc) return rc;
-    return warp_yuv420("warp_nv12_yuv420", src, dst, n_frames, src_h, src_w, BEVK_YUV_NV12, pitch, frame_stride,
-                       dst_h, dst_w, layout, dst_pitch, dst_frame_stride, M, n_mats, mat_index, flags, border_mode,
-                       border_value, true, stream);
+    const FrameLayout srcL = {BEVK_YUV_NV12, pitch, frame_stride}, dstL = {layout, dst_pitch, dst_frame_stride};
+    return warp_frames("warp_nv12_yuv420", src, &srcL, dst, &dstL, n_frames, src_h, src_w, dst_h, dst_w, 3, BEVK_U8,
+                       M, n_mats, mat_index, flags, border_mode, border_value, true, -1, stream);
 }
 
 int bevk_resize(const void *src, void *dst, int n_frames, int src_h, int src_w, int dst_h, int dst_w, int channels,
@@ -882,26 +873,10 @@ int bevk_warp_perspective_host(const void *src, void *dst, int n_frames, int src
                                const double *border_value)
 {
     WarpArgs a;
-    int rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
-                             n_mats, mat_index, flags, border_mode, border_value, a);
+    const int rc = check_warp_args(src, dst, n_frames, src_h, src_w, dst_h, dst_w, channels, dtype, M,
+                                   n_mats, mat_index, flags, border_mode, border_value, a);
     if (rc) return rc;
-    rc = bevk_require_device();
-    if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
-    std::vector<double> maps;
-    effective_maps(M, n_mats, flags, maps);
-
-    // union of the source rows any matrix references: only those are uploaded
-    int r0, r1;
-    referenced_rows_union(maps, n_mats, a, r0, r1);
-    const size_t row_bytes = (size_t)a.src_w * a.channels * a.elem_size;
-    const size_t dst_frame_bytes = (size_t)a.dst_w * a.dst_h * a.channels * a.elem_size;
-    return host_pipeline(src, a, maps, n_mats, mat_index, row_bytes * a.src_h,
-                         {{r0 * row_bytes, row_bytes * (size_t)(r1 - r0 + 1)}}, {{dst, dst_frame_bytes}},
-                         [](const void *s, void *const *d, const WarpArgs &ac, int,
-                            const std::vector<BevkWarpGroup> &groups, cudaStream_t st) {
-                             return run_warp_device(s, d[0], ac, groups, g_warp_path, st);
-                         });
+    return warp_host_frames(src, nullptr, dst, nullptr, a, M, n_mats, mat_index, flags);
 }
 
 int bevk_warp_perspective_video_host(const void *src, int src_format, void *dst, int dst_format, int n_frames,
@@ -910,40 +885,12 @@ int bevk_warp_perspective_video_host(const void *src, int src_format, void *dst,
                                      const double *border_value)
 {
     WarpArgs a;
-    int rc = check_video_host("warp_video_host", src, src_format, dst, dst_format, n_frames, src_h, src_w, dst_h,
-                              dst_w, M, n_mats, mat_index, flags, border_mode, border_value, a);
+    const int rc = check_video_host("warp_video_host", src, src_format, dst, dst_format, n_frames, src_h, src_w,
+                                    dst_h, dst_w, M, n_mats, mat_index, flags, border_mode, border_value, a);
     if (rc) return rc;
-    rc = bevk_require_device();
-    if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
-    std::vector<double> maps;
-    effective_maps(M, n_mats, flags, maps);
-
-    // the referenced luma (BGR) row band [r0, r1] and, for YUV, the chroma rows under it
-    int r0, r1;
-    referenced_rows_union(maps, n_mats, a, r0, r1);
-    const size_t h = (size_t)src_h, w = (size_t)src_w, rows = (size_t)(r1 - r0 + 1);
-    const size_t src_frame_bytes = video_frame_bytes(src_format, src_h, src_w);
-    std::vector<HostBand> bands;
-    if (src_format == BEVK_BGR) {
-        bands.push_back({3 * w * r0, 3 * w * rows});
-    } else {
-        bands.push_back({w * r0, w * rows});
-        const size_t c0 = (size_t)(r0 / 2), nc = (size_t)(r1 / 2) - c0 + 1;
-        if (src_format == BEVK_YUV_NV12) {
-            bands.push_back({w * (h + c0), w * nc});
-        } else {  // the U plane, then the V plane: (h / 2) x (w / 2) each, contiguous
-            const size_t cw = w / 2;
-            bands.push_back({w * h + cw * c0, cw * nc});
-            bands.push_back({w * h + cw * (h / 2 + c0), cw * nc});
-        }
-    }
-    const size_t dst_frame_bytes = video_frame_bytes(dst_format, dst_h, dst_w);
-    return host_pipeline(src, a, maps, n_mats, mat_index, src_frame_bytes, bands, {{dst, dst_frame_bytes}},
-                         [&](const void *s, void *const *d, const WarpArgs &ac, int,
-                             const std::vector<BevkWarpGroup> &groups, cudaStream_t st) {
-                             return run_video_warp(s, d[0], ac, groups, src_format, dst_format, st);
-                         });
+    FrameLayout sL, dL;
+    return warp_host_frames(src, video_layout(src_format, src_h, src_w, sL), dst,
+                            video_layout(dst_format, dst_h, dst_w, dL), a, M, n_mats, mat_index, flags);
 }
 
 int bevk_warp_perspective_video_host_small(const void *src, int src_format, void *dst, int dst_format, void *small,
@@ -962,34 +909,33 @@ int bevk_warp_perspective_video_host_small(const void *src, int src_format, void
     if (!M_small) BEVK_FAIL(BEVK_E_ARG, "%s: M_small is required (one small-frame matrix per matrix of M)", what);
     if (n_frames > 0 && (!small || !dst_small)) BEVK_FAIL(BEVK_E_ARG, "%s: null small / dst_small", what);
     rc = bevk_require_device();
-    if (rc) return rc;
-    if (n_frames == 0) return BEVK_OK;
+    if (rc || n_frames == 0) return rc;
     std::vector<double> maps, maps_small;
     effective_maps(M, n_mats, flags, maps);
     effective_maps(M_small, n_mats, flags, maps_small);
 
     // the resize reads every row: whole frames go up
-    const size_t src_frame_bytes = video_frame_bytes(src_format, src_h, src_w);
-    const size_t dst_frame_bytes = video_frame_bytes(dst_format, dst_h, dst_w);
-    const size_t small_frame_bytes = video_frame_bytes(BEVK_BGR, small_h, small_w);
-    const long long pitch = src_format == BEVK_BGR ? 3LL * src_w : src_w;
+    FrameLayout sL, dL;
+    const FrameLayout *yuv_src = video_layout(src_format, src_h, src_w, sL);
+    const FrameLayout *yuv_dst = video_layout(dst_format, dst_h, dst_w, dL);
+    const size_t src_frame_bytes = sL.frame_stride, dst_frame_bytes = dL.frame_stride;
     return host_pipeline(
         src, a, maps, n_mats, mat_index, src_frame_bytes, {{0, src_frame_bytes}},
-        {{dst, dst_frame_bytes}, {small, small_frame_bytes}, {dst_small, dst_frame_bytes}},
+        {{dst, dst_frame_bytes}, {small, video_frame_bytes(BEVK_BGR, small_h, small_w)}, {dst_small, dst_frame_bytes}},
         [&](const void *s, void *const *d, const WarpArgs &ac, int f0, const std::vector<BevkWarpGroup> &groups,
             cudaStream_t st) -> int {
             // the small BGR frames (d[1]) are downloaded and are the source of the small warp
-            int rc = bevk_launch_resize(s, d[1], ac.n_frames, src_h, src_w, 3, src_format, pitch,
-                                        (long long)src_frame_bytes, small_h, small_w, interpolation, st);
+            int rc = bevk_launch_resize(s, d[1], ac.n_frames, src_h, src_w, 3, src_format, sL.pitch, sL.frame_stride,
+                                        small_h, small_w, interpolation, st);
             if (rc) return rc;
-            rc = run_video_warp(s, d[0], ac, groups, src_format, dst_format, st);
+            rc = run_warp(s, yuv_src, d[0], yuv_dst, ac, groups, g_warp_path, st);
             if (rc) return rc;
             std::vector<BevkWarpGroup> groups_small;
             chunk_groups(maps_small, n_mats, mat_index, f0, ac.n_frames, groups_small);
             WarpArgs as = ac;
             as.src_h = small_h;
             as.src_w = small_w;
-            return run_video_warp(d[1], d[2], as, groups_small, BEVK_BGR, dst_format, st);
+            return run_warp(d[1], nullptr, d[2], yuv_dst, as, groups_small, g_warp_path, st);
         });
 }
 
